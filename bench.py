@@ -16,6 +16,11 @@ A ray = one BVH traversal launched (camera, bounce, light-shadow, sky-shadow eac
 
 At N = 1 the default run also carries `extra.c5`: BASELINE.json configs[4] (closest-hit microbenchmark, 10 M-triangle
 heightfield, 2 x 2^24 incoherent Philox rays) with its own roofline block — the one config where the HBM roofline binds.
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) as DIR/<name>.npy, so that two builds run with the
+same arguments can be compared output for output: a render workload's mean image (`image`, H x W x 3 float32; above 2^21
+pixels a fixed seeded sample of them, `image` N x 3 at `pixel_index`); for closest_hit the hits of the step's rays, above
+2^21 rays a fixed seeded sample (`ray_index`, `t`, `prim`, `uv`; a miss is prim 2^32 - 1). 56 MiB at most.
 """
 from __future__ import annotations
 
@@ -54,7 +59,12 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-c5-leg", action="store_true", help="skip extra.c5 (N = 1 default workload only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------- workloads
@@ -122,6 +132,41 @@ def ncu_evidence(key):
             return json.load(f).get(key)
     except Exception:
         return None
+
+
+DUMP_ROWS = 1 << 21   # pixels / rays --dump-outputs writes at most: <= 56 MiB in all; a 1920 x 1080 image fits whole
+
+
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy; float32 stays float32, anything else is written as float64."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
+def dump_index(n):
+    """The rows of an n-row output that --dump-outputs writes: all of them, or a fixed seeded sample of DUMP_ROWS."""
+    import numpy as np
+    return np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+
+
+def dump_image(out_dir, img):
+    """The mean image (H, W, 3) whole, or the pixels of dump_index (`pixel_index` into the row-major H * W pixels)."""
+    index = dump_index(img.shape[0] * img.shape[1])
+    if len(index) == img.shape[0] * img.shape[1]:
+        dump_outputs(out_dir, image=img)
+    else:
+        dump_outputs(out_dir, pixel_index=index, image=img.reshape(-1, 3)[index])
+
+
+def dump_hits(out_dir, n, hits_of):
+    """The hits of the rays of dump_index(n) in an n-ray step; `hits_of(index)` returns their hit_dtype records."""
+    import numpy as np
+    index = dump_index(n)
+    h = hits_of(index)
+    dump_outputs(out_dir, ray_index=index, t=h["t"], prim=h["prim"], uv=np.stack([h["u"], h["v"]], 1))
 
 
 class ClockSampler:
@@ -214,10 +259,12 @@ def run_reference(args):
     # one step = a bounded sample of the workload: 1 spp of the full-resolution image
     total_rays, total_s = 0, 0.0
     for i in range(args.warmup + args.steps):
-        _, counts, secs = o.render(w, h, 1, method, seed=0, sample_offset=i)
+        acc, counts, secs = o.render(w, h, 1, method, seed=0, sample_offset=i)
         if i >= args.warmup:
             total_rays += counts["camera"] + counts["bounce"] + counts["shadow_light"] + counts["shadow_sky"]
             total_s += secs
+    if args.dump_outputs:
+        dump_image(args.dump_outputs, acc)   # the sum of one sample per pixel is its mean
     v = total_rays / total_s / 1e6
     sample = (f"{w}x{h} x 1 spp per step on all host threads; reference SAH BVH (built once in {o.build_seconds():.2f} s, not "
               "timed), BFS un-culled candidates, test-all closest hit")
@@ -249,10 +296,12 @@ def run_reference_closest_hit(args, O):
     for i in range(args.warmup + args.steps):
         rays = ptb200.meshgen.philox_rays(n, first=i * n)
         t0 = time.perf_counter()
-        o.closest_hit(rays)
+        hits = o.closest_hit(rays)
         dt = time.perf_counter() - t0
         if i >= args.warmup:
             total += n; secs += dt
+    if args.dump_outputs:
+        dump_hits(args.dump_outputs, n, lambda index: hits[index])
     v = total / secs / 1e6
     sample = f"{n} rays per step on all host threads, reference SAH BVH + BFS candidates"
     print(json.dumps({"impl": "reference", "metric": "Mrays/s", "value": v, "unit": "Mrays/s", "n_gpus": args.gpus,
@@ -325,7 +374,7 @@ def run_ours(args):
     args.gpus = world
 
     if args.workload == "closest_hit":
-        out = run_closest_hit(args, rank, world, local, args.tris, args.rays, cpu=not args.no_cpu)
+        out = run_closest_hit(args, rank, world, local, args.tris, args.rays, cpu=not args.no_cpu, dump_dir=args.dump_outputs)
         if rank == 0:
             print(json.dumps(out))
         if world > 1:
@@ -390,6 +439,9 @@ def run_ours(args):
     dev_ms = e0.elapsed_time(e1)
     st = ctx.stats()
     ctx.set_option(ptb200._lib.OPT_TIME_KERNELS, 0)
+    if args.dump_outputs and rank == 0:   # rank 0's accumulator holds the reduced sums of all step_span samples
+        ctx.accum_set_samples(step_span)
+        dump_image(args.dump_outputs, ctx.accum_read(w, h, normalise=True))
     t = torch.tensor([dev_ms, float(st.rays_total), float(st.kernel_launches)], dtype=torch.float64, device="cuda")
     tmax = t.clone()
     if world > 1:
@@ -620,9 +672,9 @@ def binary_tree_label(ctx):
     return f"device SAH builder ({levels} levels of binned splits + per-warp sweeps)" if builder == 4 else "Karras LBVH"
 
 
-def run_closest_hit(args, rank, world, local, n_tris, n_rays, cpu=True, steps=None, warmup=None):
+def run_closest_hit(args, rank, world, local, n_tris, n_rays, cpu=True, steps=None, warmup=None, dump_dir=""):
     """C5: incoherent Philox rays vs a synthetic heightfield BVH, intersection only (rays sharded across ranks).
-    Returns the JSON object (rank 0) — also used as the `extra.c5` leg of the default run."""
+    Returns the JSON object (rank 0) — also used as the `extra.c5` leg of the default run. `dump_dir`: --dump-outputs."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -679,6 +731,9 @@ def run_closest_hit(args, rank, world, local, n_tris, n_rays, cpu=True, steps=No
     total_ms = float(tm[0])
     value = batch * K * world / (total_ms * 1e-3) / 1e6
     hit_frac = float((d_hits[:, 1].view(torch.int32) != -1).float().mean())
+    if dump_dir and rank == 0:   # d_hits still holds the last timed step's hits
+        dump_hits(dump_dir, batch, lambda index: d_hits[torch.from_numpy(index).cuda()].cpu().numpy()
+                  .view(ptb200.hit_dtype).reshape(-1))
     # V, T on one batch (untimed)
     ctx.set_option(ptb200._lib.OPT_COUNT_TRAVERSAL, 1)
     ctx.stats_reset()

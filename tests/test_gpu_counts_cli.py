@@ -51,8 +51,9 @@ def test_cli_matches_binding(ptb, gpu_ctx, root, tmp_path):
     assert os.path.exists(cli), "build the frontend with `make cli`"
     out = tmp_path / "img.pfm"
     scene_path = os.path.join(root, "scenes", "overshadowed.ssml")
-    r = subprocess.run([cli, "-f", scene_path, "-s", "8", "-x", "96", "-y", "54", "-r", "naive", "-o", str(out), "--seed", "5"],
-                       capture_output=True, text=True, timeout=300)
+    # -o takes exactly one '.' in the whole path (output/src/lib.rs:81-85): a relative name, run inside tmp_path
+    r = subprocess.run([cli, "-f", scene_path, "-s", "8", "-x", "96", "-y", "54", "-r", "naive", "-o", out.name, "--seed", "5"],
+                       capture_output=True, text=True, timeout=300, cwd=tmp_path)
     assert r.returncode == 0, r.stderr
     assert "Render started:" in r.stderr and "Rays shot:" in r.stderr and "Mray/s" in r.stderr
     raw = out.read_bytes()
@@ -78,10 +79,10 @@ def test_cli_gpus_flag_and_exr_output(ptb, gpu_ctx, root, tmp_path):
     cli = os.path.join(root, "raytracing-rust_b200", "ptb200-cli")
     out = tmp_path / "img.exr"
     scene_path = os.path.join(root, "scenes", "rtweekend1.ssml")
-    r = subprocess.run([cli, "-f", scene_path, "-s", "6", "-x", "96", "-y", "54", "-r", "mis", "-o", str(out), "--seed", "9",
-                        "--gpus", str(gpus)], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([cli, "-f", scene_path, "-s", "6", "-x", "96", "-y", "54", "-r", "mis", "-o", out.name, "--seed", "9",
+                        "--gpus", str(gpus)], capture_output=True, text=True, timeout=600, cwd=tmp_path)
     assert r.returncode == 0, r.stderr
-    assert f"{gpus} GPU(s)" in r.stderr and f"Image {out} saved" in r.stderr
+    assert f"{gpus} GPU(s)" in r.stderr and f"Image {out.name} saved" in r.stderr
     raw = out.read_bytes()
     assert struct.unpack_from("<I", raw, 0)[0] == 20000630
     w, h = 96, 54
@@ -104,8 +105,8 @@ def test_cli_bvh_type(ptb, root, tmp_path):
     imgs = {}
     for bvh in ("sah", "middle", "equal-counts"):
         out = tmp_path / f"img_{bvh}.pfm"
-        r = subprocess.run([cli, "-f", scene_path, "-s", "4", "-x", "64", "-y", "36", "-r", "mis", "-o", str(out), "--seed", "3", "-b", bvh],
-                           capture_output=True, text=True, timeout=300)
+        r = subprocess.run([cli, "-f", scene_path, "-s", "4", "-x", "64", "-y", "36", "-r", "mis", "-o", out.name, "--seed", "3", "-b", bvh],
+                           capture_output=True, text=True, timeout=300, cwd=tmp_path)
         assert r.returncode == 0, r.stderr
         assert ("no equal-counts builder" in r.stderr) == (bvh == "equal-counts")
         raw = out.read_bytes()

@@ -156,20 +156,21 @@ def test_obj_without_normals_is_rejected(ptb, tmp_path):
     assert s.triangles["material"].tolist() == [0, 0, 0]        # no usemtl, no "default" material -> __DEFAULT_MAT
 
 
-def test_image_save(ptb, tmp_path):
+def test_image_save(ptb, tmp_path, monkeypatch):
+    monkeypatch.chdir(tmp_path)      # relative names: the one-'.' rule covers the whole path, so a '.' in tmp_path would trip it
     img = np.linspace(0, 1.2, 8 * 4 * 3, dtype=np.float32).reshape(4, 8, 3)
     for ext in ("ppm", "bmp", "png", "pfm"):
         p = tmp_path / f"out.{ext}"
-        ptb.save_image(str(p), 8, 4, img, 2.2)
+        ptb.save_image(p.name, 8, 4, img, 2.2)
         assert p.stat().st_size > 0
     raw = (tmp_path / "out.ppm").read_bytes()
     px = np.frombuffer(raw[raw.index(b"255\n") + 4:], np.uint8)
     vals = np.power(img.ravel(), np.float32(1 / 2.2)) * np.float32(255.999)
     assert np.array_equal(px, np.clip(vals, 0, 255).astype(np.uint8))     # output/src/lib.rs:92-95
     with pytest.raises(ptb.PtbError):
-        ptb.save_image(str(tmp_path / "a.b.png"), 8, 4, img)                # filename must split into exactly two parts
+        ptb.save_image("a.b.png", 8, 4, img)                                # filename must split into exactly two parts
     with pytest.raises(ptb.PtbError):
-        ptb.save_image(str(tmp_path / "out.webp"), 8, 4, img)
+        ptb.save_image("out.webp", 8, 4, img)
 
 
 def _read_exr(path):
@@ -206,10 +207,11 @@ def _read_exr(path):
     return img
 
 
-def test_image_save_every_reference_extension(ptb, tmp_path):
+def test_image_save_every_reference_extension(ptb, tmp_path, monkeypatch):
     """SURVEY.md §8(f) N2 — output/src/lib.rs:89-107: png | jpg | jpeg | tiff | ppm | bmp through the 8-bit gamma mapping,
     exr as linear f32. The files are read back with independent decoders (Pillow; the EXR layout parser above)."""
     from PIL import Image
+    monkeypatch.chdir(tmp_path)      # relative names, as in test_image_save
     w, h = 67, 45                                                    # not multiples of the 8 x 8 JPEG block
     yy, xx = np.mgrid[0:h, 0:w]
     img = np.stack([xx / w, yy / h, 0.5 + 0.5 * np.sin(xx / 5.0) * np.cos(yy / 7.0)], -1).astype(np.float32)
@@ -218,11 +220,11 @@ def test_image_save_every_reference_extension(ptb, tmp_path):
     want8 = np.clip(np.nan_to_num(np.power(img, np.float32(1 / 2.2)) * np.float32(255.999), nan=0.0), 0, 255).astype(np.uint8)
     for ext in ("png", "tiff", "bmp", "ppm"):
         f = tmp_path / f"o.{ext}"
-        ptb.save_image(str(f), w, h, img, 2.2)
+        ptb.save_image(f.name, w, h, img, 2.2)
         assert np.array_equal(np.asarray(Image.open(f).convert("RGB")), want8), ext
     for ext in ("jpg", "jpeg"):
         f = tmp_path / f"o.{ext}"
-        ptb.save_image(str(f), w, h, img, 2.2)
+        ptb.save_image(f.name, w, h, img, 2.2)
         im = Image.open(f)
         assert im.format == "JPEG" and im.size == (w, h)
         got = np.asarray(im.convert("RGB")).astype(np.float64)
@@ -232,6 +234,6 @@ def test_image_save_every_reference_extension(ptb, tmp_path):
         theirs = np.sqrt(np.mean((np.asarray(Image.open(g)).astype(np.float64) - want8) ** 2))
         assert ours < 1.25 * theirs + 0.5, (ours, theirs)
     f = tmp_path / "o.exr"
-    ptb.save_image(str(f), w, h, img, 2.2)                           # gamma is ignored for exr (lib.rs:98-99)
+    ptb.save_image(f.name, w, h, img, 2.2)                           # gamma is ignored for exr (lib.rs:98-99)
     back = _read_exr(f)
     assert np.array_equal(back.view(np.uint32), img.view(np.uint32))    # linear f32, bit for bit (NaN included)

@@ -222,7 +222,8 @@ def _png_bytes(arr, bit_depth=8, colour_type=2, level=6):
             + chunk(b"IDAT", zlib.compress(bytes(raw), level)) + chunk(b"IEND", b""))
 
 
-def test_image_decoders(ptb, tmp_path):
+def test_image_decoders(ptb, tmp_path, monkeypatch):
+    monkeypatch.chdir(tmp_path)      # save_image takes exactly one '.' in the whole path: relative names for the writers below
     rng = np.random.default_rng(5)
     img8 = rng.integers(0, 256, (9, 11, 3)).astype(np.uint8)
     want = img8.astype(np.float32) / 255.0                                  # to_rgb32f
@@ -256,11 +257,11 @@ def test_image_decoders(ptb, tmp_path):
     assert np.array_equal(ptb.load_image(str(f)), want)
     lin = rng.uniform(0, 4, (9, 11, 3)).astype(np.float32)
     f = tmp_path / "e.pfm"
-    ptb.save_image(str(f), 11, 9, lin, 2.2)
+    ptb.save_image(f.name, 11, 9, lin, 2.2)
     assert np.array_equal(ptb.load_image(str(f)), lin)
     for ext in ("bmp", "png", "ppm"):
         f = tmp_path / f"w.{ext}"
-        ptb.save_image(str(f), 11, 9, want, 1.0)                            # gamma 1: v * 255.999 as u8
+        ptb.save_image(f.name, 11, 9, want, 1.0)                            # gamma 1: v * 255.999 as u8
         assert np.array_equal(ptb.load_image(str(f)), np.floor(want * 255.999).astype(np.float32) / 255.0), ext
     with pytest.raises(ptb.PtbError):
         ptb.load_image(str(tmp_path / "missing.png"))
