@@ -73,6 +73,28 @@ impl CudaScene {
 }
 
 impl CudaScene {
+    /// AccelerationStructure::check_hit_index (acceleration/mod.rs:226-263) for a batch: is primitive `index[i]` (loader
+    /// order) the first thing ray i hits? Some((t, b1, b2)) when it is, None when it is blocked, missed or out of range.
+    pub fn check_hit_index(&self, rays: &[Ray], index: &[u32]) -> Result<Vec<Option<(Float, Float, Float)>>, String> {
+        assert_eq!(rays.len(), index.len());
+        let r: Vec<ptb_ray> = rays.iter().map(|r| ptb_ray { o: [r.origin.x, r.origin.y, r.origin.z], _pad0: 0.0,
+                                                           d: [r.direction.x, r.direction.y, r.direction.z], _pad1: 0.0 }).collect();
+        let mut hits = vec![ptb_hit { t: 0.0, prim: PTB_MISS, u: 0.0, v: 0.0 }; rays.len()];
+        check(self.ctx, unsafe { ptb_check_hit_index(self.ctx, r.as_ptr(), index.as_ptr(), r.len(), hits.as_mut_ptr()) })?;
+        Ok(hits.iter().map(|h| if h.prim == PTB_MISS { None } else { Some((h.t, h.u, h.v)) }).collect())
+    }
+
+    /// Shadow rays: true when a primitive other than `exclude` (loader order; PTB_MISS: none) lies at 0 < t < tmax along
+    /// the normalised direction. tmax = Float::INFINITY asks whether the ray hits anything (the sky test, mis.rs:104-115).
+    pub fn occluded(&self, rays: &[(Ray, Float, u32)]) -> Result<Vec<bool>, String> {
+        let r: Vec<ptb_occlusion_ray> = rays.iter().map(|(r, tmax, exclude)| ptb_occlusion_ray {
+            o: [r.origin.x, r.origin.y, r.origin.z], tmax: *tmax, d: [r.direction.x, r.direction.y, r.direction.z], exclude: *exclude,
+        }).collect();
+        let mut out = vec![0u8; r.len()];
+        check(self.ctx, unsafe { ptb_occluded(self.ctx, r.as_ptr(), r.len(), out.as_mut_ptr()) })?;
+        Ok(out.iter().map(|&o| o != 0).collect())
+    }
+
     /// The reference's own contract: `presentation_update` sees the single-sample image of every pass
     /// (Sampler::sample_image, samplers/mod.rs:7-20). `f` returns true to stop, like the Rust closure.
     pub fn render_with_update<T, F: Fn(&mut T, &SamplerProgress, u64) -> bool>(&self, opts: RenderOptions, seed: u64, data: &mut T, f: F) -> Result<(), String> {

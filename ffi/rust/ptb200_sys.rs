@@ -17,6 +17,8 @@ pub const PTB_METHOD_MIS: u32 = 1;
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_sky { pub texture: u32, pub sampler_res_x: u32, pub sampler_res_y: u32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_ray { pub o: [f32; 3], pub _pad0: f32, pub d: [f32; 3], pub _pad1: f32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_hit { pub t: f32, pub prim: u32, pub u: f32, pub v: f32 }
+/// occlusion query (32 B): origin | tmax, un-normalised direction | excluded primitive (original id, PTB_MISS: none)
+#[repr(C)] #[derive(Clone, Copy)] pub struct ptb_occlusion_ray { pub o: [f32; 3], pub tmax: f32, pub d: [f32; 3], pub exclude: u32 }
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct ptb_render_opts {
     pub width: u32, pub height: u32, pub samples_per_pixel: u32, pub sample_offset: u32,
@@ -63,6 +65,11 @@ extern "C" {
     pub fn ptb_bvh_builder(ctx: *mut ptb_ctx, builder: *mut u32, sah_levels: *mut u32) -> i32;
     pub fn ptb_bvh_wide_export(ctx: *mut ptb_ctx, nodes96: *mut c_void, slot_prim: *mut u32) -> i32;
     pub fn ptb_closest_hit(ctx: *mut ptb_ctx, rays: *const ptb_ray, n: usize, hits: *mut ptb_hit) -> i32;
+    pub fn ptb_closest_hit_device(ctx: *mut ptb_ctx, d_rays: *const c_void, n: usize, d_hits: *mut c_void) -> i32;
+    pub fn ptb_check_hit_index(ctx: *mut ptb_ctx, rays: *const ptb_ray, index: *const u32, n: usize, hits: *mut ptb_hit) -> i32;
+    pub fn ptb_check_hit_index_device(ctx: *mut ptb_ctx, d_rays: *const c_void, d_index: *const c_void, n: usize, d_hits: *mut c_void) -> i32;
+    pub fn ptb_occluded(ctx: *mut ptb_ctx, rays: *const ptb_occlusion_ray, n: usize, occluded: *mut u8) -> i32;
+    pub fn ptb_occluded_device(ctx: *mut ptb_ctx, d_rays: *const c_void, n: usize, d_occluded: *mut c_void) -> i32;
     pub fn ptb_render(ctx: *mut ptb_ctx, opts: *const ptb_render_opts, progress: ptb_progress_fn, user: *mut c_void) -> i32;
     pub fn ptb_render_passes(ctx: *mut ptb_ctx, opts: *const ptb_render_opts, update: ptb_pass_fn, user: *mut c_void) -> i32;
     pub fn ptb_render_multi(ctxs: *const *mut ptb_ctx, n: i32, opts: *const ptb_render_opts) -> i32;

@@ -173,7 +173,7 @@ typedef struct ptb_stats {
   uint64_t nodes_fetched;      /* PTB_OPT_COUNT_TRAVERSAL: 64-byte BVH nodes fetched by closest-hit traversals */
   uint64_t prims_tested;       /* PTB_OPT_COUNT_TRAVERSAL: primitives tested by closest-hit traversals          */
   uint64_t rays_counted;       /* PTB_OPT_COUNT_TRAVERSAL: closest-hit traversals the two counters cover        */
-  uint64_t trace_launches;     /* closest-hit kernel launches (k_trace / k_closest_hit_api)                     */
+  uint64_t trace_launches;     /* traversal kernel launches (k_trace / k_closest_hit_api / k_visibility_api)    */
   double   build_ms;           /* last ptb_scene_commit: device LBVH build time               */
   double   render_ms;          /* last ptb_render: device time (CUDA events)                  */
   double   ms_generate;        /* PTB_OPT_TIME_KERNELS: summed CUDA-event time per kernel class */
@@ -257,6 +257,40 @@ int32_t ptb_bvh_wide_export(ptb_ctx* ctx, void* nodes96, uint32_t* slot_prim);
 int32_t ptb_closest_hit(ptb_ctx* ctx, const ptb_ray* rays, size_t n, ptb_hit* hits);
 /* Same, buffers already resident in device memory (kernel only; used for roofline timing). */
 int32_t ptb_closest_hit_device(ptb_ctx* ctx, const void* d_rays, size_t n, void* d_hits);
+
+/* ----------------------------------------------------------- visibility -- */
+/* 32 B, two float4 like ptb_ray: origin | tmax, un-normalised direction | excluded primitive (original id, PTB_MISS: none) */
+typedef struct ptb_occlusion_ray {
+  float ox, oy, oz, tmax;
+  float dx, dy, dz;
+  uint32_t exclude;
+} ptb_occlusion_ray;
+
+/* Batch visibility queries. Rays are handled as in ptb_closest_hit. The direction is normalised as Ray::new does it
+ * (make_ray_from_raw), and t is measured along the normalised direction. The primitive's own intersector decides each
+ * hit, with the same arithmetic as closest hit.
+ *
+ * check_hit_index, per acceleration/mod.rs:226-263. The target index[i] is an original primitive id. It is visible when
+ * the target's own intersector gives t_target > 0 and no other primitive has 0 < t < t_target. The test is strict: a
+ * blocker at exactly t_target does not block. If visible, hits[i] = {t_target, index[i], b1, b2}, the same record
+ * ptb_closest_hit reports when that primitive is the closest. Otherwise hits[i] = {0, PTB_MISS, 0, 0}. A target
+ * >= n_prims is not visible. It is not an error, because the device variant cannot check without a synchronise. Both
+ * variants answer the same way.
+ *
+ * occluded: occluded[i] = 1 iff some primitive p != exclude has 0 < t_p < tmax, else 0. tmax = +inf asks "does the ray
+ * hit anything". tmax <= 0 or NaN gives 0. An exclude of PTB_MISS or out of range excludes nothing.
+ *
+ * Errors. A call before commit returns PTB_ERR_INVALID. So does a null buffer with n > 0, and more than 0xFFFFFFF0 rays
+ * in one device call (the same as ptb_closest_hit_device). n == 0 returns PTB_OK. In an empty scene nothing is occluded
+ * and nothing is visible.
+ *
+ * The host variants stream their buffers like ptb_closest_hit (PTB_HIT_BATCH, PTB_HIT_SORT). The _device variants
+ * enqueue on the context's stream and return without synchronising, like ptb_closest_hit_device. Both count in
+ * ptb_stats.kernel_launches / trace_launches only, not in the closest-hit traversal counters. */
+int32_t ptb_check_hit_index(ptb_ctx* ctx, const ptb_ray* rays, const uint32_t* index, size_t n, ptb_hit* hits);
+int32_t ptb_check_hit_index_device(ptb_ctx* ctx, const void* d_rays, const void* d_index, size_t n, void* d_hits);
+int32_t ptb_occluded(ptb_ctx* ctx, const ptb_occlusion_ray* rays, size_t n, uint8_t* occluded);
+int32_t ptb_occluded_device(ptb_ctx* ctx, const void* d_rays, size_t n, void* d_occluded);
 
 /* --------------------------------------------------------------- render -- */
 /* Replaces Sampler::sample_image (samplers/mod.rs:7-20, random_sampler.rs:10-99) + the running mean of

@@ -39,6 +39,7 @@ camera_dtype = np.dtype([("origin", "<f4", 3), ("lower_left", "<f4", 3), ("horiz
 sky_dtype = np.dtype([("texture", "<u4"), ("sampler_res_x", "<u4"), ("sampler_res_y", "<u4")])
 ray_dtype = np.dtype([("o", "<f4", 3), ("_pad0", "<f4"), ("d", "<f4", 3), ("_pad1", "<f4")])
 hit_dtype = np.dtype([("t", "<f4"), ("prim", "<u4"), ("u", "<f4"), ("v", "<f4")])
+occlusion_ray_dtype = np.dtype([("o", "<f4", 3), ("tmax", "<f4"), ("d", "<f4", 3), ("exclude", "<u4")])
 bvh_node_dtype = np.dtype([("lmin", "<f4", 3), ("lmax", "<f4", 3), ("rmin", "<f4", 3), ("rmax", "<f4", 3),
                            ("left", "<u4"), ("right", "<u4"), ("parent", "<u4"), ("_pad", "<u4")])
 
@@ -109,6 +110,10 @@ SYMBOLS = [
     ("ptb_bvh_wide_export", C.c_int32, [_P, _P, _P]),
     ("ptb_closest_hit", C.c_int32, [_P, _P, C.c_size_t, _P]),
     ("ptb_closest_hit_device", C.c_int32, [_P, _P, C.c_size_t, _P]),
+    ("ptb_check_hit_index", C.c_int32, [_P, _P, _P, C.c_size_t, _P]),
+    ("ptb_check_hit_index_device", C.c_int32, [_P, _P, _P, C.c_size_t, _P]),
+    ("ptb_occluded", C.c_int32, [_P, _P, C.c_size_t, _P]),
+    ("ptb_occluded_device", C.c_int32, [_P, _P, C.c_size_t, _P]),
     ("ptb_render", C.c_int32, [_P, C.POINTER(RenderOpts), _P, _P]),
     ("ptb_render_passes", C.c_int32, [_P, C.POINTER(RenderOpts), _P, _P]),
     ("ptb_accum_clear", C.c_int32, [_P]),

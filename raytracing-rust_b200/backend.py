@@ -1,7 +1,8 @@
 """The `--backend cuda` path as seen from Python: a thin, typed wrapper over the C ABI.
 
 Names follow the reference's interface for this path:
-  Bvh            <- implementations::acceleration::Bvh            (acceleration/mod.rs:43-93, check_hit :265-298)
+  Bvh            <- implementations::acceleration::Bvh            (acceleration/mod.rs:43-93, check_hit :265-298,
+                                                                   check_hit_index :226-263)
   RenderOptions  <- implementations::samplers::RenderOptions       (samplers/mod.rs:22-41)
   RandomSampler  <- implementations::samplers::random_sampler::RandomSampler.sample_image (random_sampler.rs:10-99)
   Scene.render   <- frontend Scene::render                         (src/scene.rs:35-42)
@@ -156,6 +157,36 @@ class Context:
     def closest_hit_device(self, d_rays_ptr: int, n: int, d_hits_ptr: int):
         _check(self._h, L.lib.ptb_closest_hit_device(self._h, C.c_void_p(d_rays_ptr), n, C.c_void_p(d_hits_ptr)))
 
+    # ---- visibility
+    def check_hit_index(self, rays: np.ndarray, index: np.ndarray, out: np.ndarray | None = None) -> np.ndarray:
+        """AccelerationStructure::check_hit_index per ray: is original primitive index[i] the first thing rays[i] hits?
+        Visible: the hit record closest_hit reports for that primitive; otherwise {0, PTB_MISS, 0, 0} (an out-of-range
+        target included). `out`: optional caller-owned hit buffer."""
+        rays = np.ascontiguousarray(rays, dtype=L.ray_dtype)
+        index = np.ascontiguousarray(index, dtype=np.uint32)
+        assert index.shape == (len(rays),)
+        hits = np.zeros(len(rays), L.hit_dtype) if out is None else out
+        assert hits.dtype == L.hit_dtype and len(hits) == len(rays) and hits.flags.c_contiguous
+        _check(self._h, L.lib.ptb_check_hit_index(self._h, L.ptr(rays), L.ptr(index), len(rays), L.ptr(hits)))
+        return hits
+
+    def check_hit_index_device(self, d_rays_ptr: int, d_index_ptr: int, n: int, d_hits_ptr: int):
+        _check(self._h, L.lib.ptb_check_hit_index_device(self._h, C.c_void_p(d_rays_ptr), C.c_void_p(d_index_ptr), n,
+                                                          C.c_void_p(d_hits_ptr)))
+
+    def occluded(self, rays: np.ndarray, out: np.ndarray | None = None) -> np.ndarray:
+        """Occlusion per ray (occlusion_ray_dtype, see make_occlusion_rays): True iff a primitive other than `exclude` is
+        hit at 0 < t < tmax. `out`: optional caller-owned bool buffer."""
+        rays = np.ascontiguousarray(rays, dtype=L.occlusion_ray_dtype)
+        occ = np.zeros(len(rays), bool) if out is None else out
+        assert occ.dtype == bool and len(occ) == len(rays) and occ.flags.c_contiguous
+        _check(self._h, L.lib.ptb_occluded(self._h, L.ptr(rays), len(rays), L.ptr(occ)))
+        return occ
+
+    def occluded_device(self, d_rays_ptr: int, n: int, d_occluded_ptr: int):
+        """d_occluded: n bytes, 1 = occluded."""
+        _check(self._h, L.lib.ptb_occluded_device(self._h, C.c_void_p(d_rays_ptr), n, C.c_void_p(d_occluded_ptr)))
+
     # ---- render
     def render(self, opts: RenderOptions, progress=None):
         cb = None
@@ -242,6 +273,12 @@ class Bvh:
     def check_hit(self, rays: np.ndarray) -> np.ndarray:
         return self.ctx.closest_hit(rays)
 
+    def check_hit_index(self, rays: np.ndarray, index: np.ndarray) -> np.ndarray:
+        return self.ctx.check_hit_index(rays, index)
+
+    def occluded(self, rays: np.ndarray) -> np.ndarray:
+        return self.ctx.occluded(rays)
+
 
 class RandomSampler:
     """RandomSampler::sample_image on the device: `spp` samples of every pixel into the accumulator."""
@@ -284,4 +321,15 @@ def make_rays(origins: np.ndarray, directions: np.ndarray) -> np.ndarray:
     r = np.zeros(len(origins), L.ray_dtype)
     r["o"] = origins
     r["d"] = directions
+    return r
+
+
+def make_occlusion_rays(origins: np.ndarray, directions: np.ndarray, tmax=np.inf, exclude=L.PTB_MISS) -> np.ndarray:
+    """Occlusion rays: `tmax` (distance along the normalised direction) and `exclude` (original primitive id that does not
+    block, PTB_MISS: none) are scalars or one value per ray."""
+    r = np.zeros(len(origins), L.occlusion_ray_dtype)
+    r["o"] = origins
+    r["d"] = directions
+    r["tmax"] = tmax
+    r["exclude"] = exclude
     return r

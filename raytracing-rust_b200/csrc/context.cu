@@ -339,7 +339,83 @@ int32_t ptb_bvh_wide_export(ptb_ctx* ctx, void* nodes96, uint32_t* slot_prim) {
   return PTB_OK;
 }
 
-// ---------------------------------------------------------------- closest hit
+// ---------------------------------------------------------------- batch queries (closest hit, visibility)
+// A query over host buffers: in_bytes per record of `in` (plus in2_bytes of `in2`, when given) up, out_bytes per record of
+// `out` back. Batches of 4 Mi records through two staging pairs: upload k+1 | traverse k | read back k-1. With pinned
+// host buffers the three overlap and the call runs at PCIe speed; pageable buffers still work (the copies then serialise
+// inside the driver).
+typedef int32_t (*BatchLaunch)(Ctx* c, const void* d_in, const void* d_in2, size_t n, void* d_out);
+static int32_t staged_batches(Ctx* c, size_t n, const void* in, size_t in_bytes, const void* in2, size_t in2_bytes, void* out,
+                              size_t out_bytes, BatchLaunch launch) {
+  size_t chunk = (size_t)1 << 22;
+  if (const char* e = getenv("PTB_HIT_BATCH")) { size_t v = strtoull(e, nullptr, 10); if (v >= 1024) chunk = v; }
+  const size_t cap = n < chunk ? n : chunk;
+  DevBuf* dr[2] = {&c->d_rays, &c->d_rays2};
+  DevBuf* dx[2] = {&c->d_index, &c->d_index2};
+  DevBuf* dh[2] = {&c->d_hits, &c->d_hits2};
+  const int nbuf = n > chunk ? 2 : 1;
+  for (int b = 0; b < nbuf; ++b) {
+    PTB_CUDA_TRY(c, dr[b]->reserve(cap * in_bytes));
+    if (in2) PTB_CUDA_TRY(c, dx[b]->reserve(cap * in2_bytes));
+    PTB_CUDA_TRY(c, dh[b]->reserve(cap * out_bytes));
+  }
+  if (!c->s_in) {
+    PTB_CUDA_TRY(c, cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
+    PTB_CUDA_TRY(c, cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
+    for (int b = 0; b < 2; ++b) {
+      PTB_CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_in[b], cudaEventDisableTiming));
+      PTB_CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_kernel[b], cudaEventDisableTiming));
+      PTB_CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_out[b], cudaEventDisableTiming));
+    }
+  }
+  // On any failure the copies of earlier batches may still be in flight against the caller's buffers: drain all three
+  // streams before returning, the caller is free to release its buffers as soon as the call is back.
+  auto drain = [&](int32_t rc) {
+    cudaStreamSynchronize(c->s_out);
+    cudaStreamSynchronize(c->s_in);
+    cudaStreamSynchronize(c->stream);
+    return rc;
+  };
+#define PTB_TRY_DRAIN(expr)                                                  \
+  do {                                                                       \
+    cudaError_t _e = (expr);                                                 \
+    if (_e != cudaSuccess) return drain(ptb::check_cuda(c, _e, #expr));      \
+  } while (0)
+  const char* src = static_cast<const char*>(in);
+  const char* src2 = static_cast<const char*>(in2);
+  char* dst = static_cast<char*>(out);
+  // the staging buffers may still be in use by earlier work on the main stream
+  PTB_TRY_DRAIN(cudaEventRecord(c->ev_kernel[0], c->stream));
+  PTB_TRY_DRAIN(cudaStreamWaitEvent(c->s_in, c->ev_kernel[0], 0));
+  size_t k = 0;
+  for (size_t off = 0; off < n; off += chunk, ++k) {
+    const size_t m = n - off < chunk ? n - off : chunk;
+    const int b = (int)(k & 1u);
+    if (k >= 2) PTB_TRY_DRAIN(cudaStreamWaitEvent(c->s_in, c->ev_kernel[b], 0));  // batch k-2 no longer reads d_rays[b]
+    PTB_TRY_DRAIN(cudaMemcpyAsync(dr[b]->p, src + off * in_bytes, m * in_bytes, cudaMemcpyHostToDevice, c->s_in));
+    if (in2) PTB_TRY_DRAIN(cudaMemcpyAsync(dx[b]->p, src2 + off * in2_bytes, m * in2_bytes, cudaMemcpyHostToDevice, c->s_in));
+    PTB_TRY_DRAIN(cudaEventRecord(c->ev_in[b], c->s_in));
+    PTB_TRY_DRAIN(cudaStreamWaitEvent(c->stream, c->ev_in[b], 0));
+    if (k >= 2) PTB_TRY_DRAIN(cudaStreamWaitEvent(c->stream, c->ev_out[b], 0));     // batch k-2's results left d_hits[b]
+    int32_t rc = launch(c, dr[b]->p, in2 ? dx[b]->p : nullptr, m, dh[b]->p);
+    if (rc != PTB_OK) return drain(rc);
+    PTB_TRY_DRAIN(cudaEventRecord(c->ev_kernel[b], c->stream));
+    PTB_TRY_DRAIN(cudaStreamWaitEvent(c->s_out, c->ev_kernel[b], 0));
+    PTB_TRY_DRAIN(cudaMemcpyAsync(dst + off * out_bytes, dh[b]->p, m * out_bytes, cudaMemcpyDeviceToHost, c->s_out));
+    PTB_TRY_DRAIN(cudaEventRecord(c->ev_out[b], c->s_out));
+  }
+  PTB_TRY_DRAIN(cudaStreamSynchronize(c->s_out));
+  PTB_TRY_DRAIN(cudaStreamSynchronize(c->stream));
+#undef PTB_TRY_DRAIN
+  return PTB_OK;
+}
+static int32_t closest_hit_batch(Ctx* c, const void* d_rays, const void*, size_t n, void* d_hits) {
+  return launch_closest_hit(c, d_rays, n, d_hits);
+}
+static int32_t visibility_batch(Ctx* c, const void* d_rays, const void* d_index, size_t n, void* d_out) {
+  return launch_visibility(c, d_rays, d_index, n, d_out);
+}
+
 int32_t ptb_closest_hit_device(ptb_ctx* ctx, const void* d_rays, size_t n, void* d_hits) {
   CTX_OR_FAIL(ctx);
   if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
@@ -352,64 +428,37 @@ int32_t ptb_closest_hit(ptb_ctx* ctx, const ptb_ray* rays, size_t n, ptb_hit* hi
   if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
   if (n == 0) return PTB_OK;
   if (!rays || !hits) return set_error(c, PTB_ERR_INVALID, "null host buffer");
-  // Batches of 4 Mi rays (128 MiB in, 64 MiB out) through two staging pairs: upload k+1 | traverse k | read back k-1.
-  // With pinned host buffers the three overlap and the call runs at PCIe speed; pageable buffers still work (the copies
-  // then serialise inside the driver).
-  size_t chunk = (size_t)1 << 22;
-  if (const char* e = getenv("PTB_HIT_BATCH")) { size_t v = strtoull(e, nullptr, 10); if (v >= 1024) chunk = v; }
-  const size_t cap = n < chunk ? n : chunk;
-  DevBuf* dr[2] = {&c->d_rays, &c->d_rays2};
-  DevBuf* dh[2] = {&c->d_hits, &c->d_hits2};
-  const int nbuf = n > chunk ? 2 : 1;
-  for (int b = 0; b < nbuf; ++b) {
-    PTB_CUDA_TRY(c, dr[b]->reserve(cap * sizeof(ptb_ray)));
-    PTB_CUDA_TRY(c, dh[b]->reserve(cap * sizeof(ptb_hit)));
-  }
-  if (!c->s_in) {
-    PTB_CUDA_TRY(c, cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
-    PTB_CUDA_TRY(c, cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
-    for (int b = 0; b < 2; ++b) {
-      PTB_CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_in[b], cudaEventDisableTiming));
-      PTB_CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_kernel[b], cudaEventDisableTiming));
-      PTB_CUDA_TRY(c, cudaEventCreateWithFlags(&c->ev_out[b], cudaEventDisableTiming));
-    }
-  }
-  // On any failure the copies of earlier batches may still be in flight against the caller's `rays` / `hits`: drain all
-  // three streams before returning, the caller is free to release its buffers as soon as the call is back.
-  auto drain = [&](int32_t rc) {
-    cudaStreamSynchronize(c->s_out);
-    cudaStreamSynchronize(c->s_in);
-    cudaStreamSynchronize(c->stream);
-    return rc;
-  };
-#define PTB_TRY_DRAIN(expr)                                                  \
-  do {                                                                       \
-    cudaError_t _e = (expr);                                                 \
-    if (_e != cudaSuccess) return drain(ptb::check_cuda(c, _e, #expr));      \
-  } while (0)
-  // the staging buffers may still be in use by earlier work on the main stream
-  PTB_TRY_DRAIN(cudaEventRecord(c->ev_kernel[0], c->stream));
-  PTB_TRY_DRAIN(cudaStreamWaitEvent(c->s_in, c->ev_kernel[0], 0));
-  size_t k = 0;
-  for (size_t off = 0; off < n; off += chunk, ++k) {
-    const size_t m = n - off < chunk ? n - off : chunk;
-    const int b = (int)(k & 1u);
-    if (k >= 2) PTB_TRY_DRAIN(cudaStreamWaitEvent(c->s_in, c->ev_kernel[b], 0));  // batch k-2 no longer reads d_rays[b]
-    PTB_TRY_DRAIN(cudaMemcpyAsync(dr[b]->p, rays + off, m * sizeof(ptb_ray), cudaMemcpyHostToDevice, c->s_in));
-    PTB_TRY_DRAIN(cudaEventRecord(c->ev_in[b], c->s_in));
-    PTB_TRY_DRAIN(cudaStreamWaitEvent(c->stream, c->ev_in[b], 0));
-    if (k >= 2) PTB_TRY_DRAIN(cudaStreamWaitEvent(c->stream, c->ev_out[b], 0));     // batch k-2's hits left d_hits[b]
-    int32_t rc = launch_closest_hit(c, dr[b]->p, m, dh[b]->p);
-    if (rc != PTB_OK) return drain(rc);
-    PTB_TRY_DRAIN(cudaEventRecord(c->ev_kernel[b], c->stream));
-    PTB_TRY_DRAIN(cudaStreamWaitEvent(c->s_out, c->ev_kernel[b], 0));
-    PTB_TRY_DRAIN(cudaMemcpyAsync(hits + off, dh[b]->p, m * sizeof(ptb_hit), cudaMemcpyDeviceToHost, c->s_out));
-    PTB_TRY_DRAIN(cudaEventRecord(c->ev_out[b], c->s_out));
-  }
-  PTB_TRY_DRAIN(cudaStreamSynchronize(c->s_out));
-  PTB_TRY_DRAIN(cudaStreamSynchronize(c->stream));
-#undef PTB_TRY_DRAIN
-  return PTB_OK;
+  return staged_batches(c, n, rays, sizeof(ptb_ray), nullptr, 0, hits, sizeof(ptb_hit), closest_hit_batch);
+}
+
+int32_t ptb_check_hit_index_device(ptb_ctx* ctx, const void* d_rays, const void* d_index, size_t n, void* d_hits) {
+  CTX_OR_FAIL(ctx);
+  if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
+  if (n && (!d_rays || !d_index || !d_hits)) return set_error(c, PTB_ERR_INVALID, "null device buffer");
+  return launch_visibility(c, d_rays, d_index, n, d_hits);
+}
+
+int32_t ptb_check_hit_index(ptb_ctx* ctx, const ptb_ray* rays, const uint32_t* index, size_t n, ptb_hit* hits) {
+  CTX_OR_FAIL(ctx);
+  if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
+  if (n == 0) return PTB_OK;
+  if (!rays || !index || !hits) return set_error(c, PTB_ERR_INVALID, "null host buffer");
+  return staged_batches(c, n, rays, sizeof(ptb_ray), index, sizeof(uint32_t), hits, sizeof(ptb_hit), visibility_batch);
+}
+
+int32_t ptb_occluded_device(ptb_ctx* ctx, const void* d_rays, size_t n, void* d_occluded) {
+  CTX_OR_FAIL(ctx);
+  if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
+  if (n && (!d_rays || !d_occluded)) return set_error(c, PTB_ERR_INVALID, "null device buffer");
+  return launch_visibility(c, d_rays, nullptr, n, d_occluded);
+}
+
+int32_t ptb_occluded(ptb_ctx* ctx, const ptb_occlusion_ray* rays, size_t n, uint8_t* occluded) {
+  CTX_OR_FAIL(ctx);
+  if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
+  if (n == 0) return PTB_OK;
+  if (!rays || !occluded) return set_error(c, PTB_ERR_INVALID, "null host buffer");
+  return staged_batches(c, n, rays, sizeof(ptb_occlusion_ray), nullptr, 0, occluded, 1, visibility_batch);
 }
 
 // ---------------------------------------------------------------- render

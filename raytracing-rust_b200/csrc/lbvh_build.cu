@@ -642,8 +642,8 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   DevBuf &raw_spheres = c->d_raw_spheres, &raw_tris = c->d_raw_tris;
   DevBuf &bmin = c->scratch[0], &bmax = c->scratch[1], &bounds = c->scratch[2], &keys_a = c->scratch[3], &keys_b = c->scratch[4],
          &vals_a = c->scratch[5], &vals_b = c->scratch[6], &hist = c->scratch[7], &leaf_parent = c->scratch[8],
-         &nbmin = c->scratch[9], &nbmax = c->scratch[10], &flags = c->scratch[11], &prim_slot = c->scratch[12],
-         &d_light_prims = c->scratch[13], &d_light_tmp = c->scratch[14], &d_light_out = c->scratch[15], &d_qframe = c->scratch[16];
+         &nbmin = c->scratch[9], &nbmax = c->scratch[10], &flags = c->scratch[11], &prim_slot = c->d_prim_slot,
+         &d_light_prims = c->scratch[12], &d_light_tmp = c->scratch[13], &d_light_out = c->scratch[14], &d_qframe = c->scratch[15];
   const uint32_t n32 = (uint32_t)n, ns32 = (uint32_t)ns, nt32 = (uint32_t)nt;
   PTB_CUDA_TRY(c, bmin.reserve(n * 16));
   PTB_CUDA_TRY(c, bmax.reserve(n * 16));

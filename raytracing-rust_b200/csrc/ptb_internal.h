@@ -93,7 +93,7 @@ struct Ctx {
   // are kept on the host until commit
   DevBuf d_raw_spheres, d_raw_tris;
   size_t n_spheres = 0, n_tris = 0;
-  DevBuf scratch[17];  // LBVH build temporaries, grow-only (lbvh_build.cu)
+  DevBuf scratch[16];  // LBVH build temporaries, grow-only (lbvh_build.cu)
   std::vector<ptb_material> materials;
   std::vector<ptb_texture> textures;
   struct TexData { uint32_t width = 0, height = 0; std::vector<float> data; };
@@ -107,6 +107,7 @@ struct Ctx {
 
   // device scene
   DevScene dev{};
+  DevBuf d_prim_slot;  // original primitive id -> slot (k_gather; valid until the next commit: lights, visibility API)
   DevBuf d_geom, d_normals, d_slot_prim, d_slot_mat, d_nodes, d_qnodes, d_cw_nodes, d_prim_sorted, d_morton, d_materials, d_textures, d_tex_data, d_lights;
   DevBuf d_sky_ycdf, d_sky_ypdf, d_sky_xcdf, d_sky_xpdf;
   uint64_t n_prims = 0, n_nodes = 0, n_cw_nodes = 0;
@@ -145,6 +146,7 @@ struct Ctx {
   // closest-hit staging: two buffer pairs + copy streams so that the upload of batch k+1, the traversal of batch k and the
   // read-back of batch k-1 overlap (ptb_closest_hit with host buffers)
   DevBuf d_rays, d_hits, d_rays2, d_hits2;
+  DevBuf d_index, d_index2;  // the second input of ptb_check_hit_index (target ids), staged with the rays
   DevBuf d_hit_sort;  // ray ordering scratch of the closest-hit API: 4 x n words (keys / indices, ping-pong) + histogram
   cudaStream_t s_in = nullptr, s_out = nullptr;
   cudaEvent_t ev_in[2] = {}, ev_kernel[2] = {}, ev_out[2] = {};
@@ -187,6 +189,8 @@ size_t radix_sort_hist_words(uint32_t n);
 // wavefront.cu
 int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progress, void* user);
 int32_t launch_closest_hit(Ctx* c, const void* d_rays, size_t n, void* d_hits);
+// check_hit_index (d_index != nullptr: ptb_ray in, ptb_hit out) or occlusion (ptb_occlusion_ray in, one byte out)
+int32_t launch_visibility(Ctx* c, const void* d_rays, const void* d_index, size_t n, void* d_out);
 void free_render_state(Ctx* c);
 int32_t sampler_hook(Ctx* c, const ptb_sampler_query& q, size_t n, const float* dirs_in, float* dirs_out, float* pdf_out);
 

@@ -1572,6 +1572,69 @@ k_closest_hit_api(DevScene sc, const float4* __restrict__ rays, const uint32_t* 
   }
 }
 
+// ------------------------------------------------------------------------------------------ visibility API kernel
+// Batch any-hit through the walk k_shadow runs (persistent_trace<TR, ANYHIT = true>), fed from caller records.
+//   CHI  : check_hit_index (acceleration/mod.rs:226-263): ptb_ray + target id in, ptb_hit out. The target's own hit is
+//          computed first, as k_shade does for a light sample; the walk then looks for a blocker at 0 < t < t_target with
+//          the target excluded. A missed target keeps its lane with tmax = 0, which nothing can block, and answers a miss.
+//   !CHI : occlusion: ptb_occlusion_ray in (origin | tmax, direction | excluded original id), one byte out.
+// Ids arrive in the original order and are mapped to slots through prim_slot (k_gather's map, kept with the scene).
+template <bool CHI>
+struct VisFetch {
+  const DevScene& sc;
+  const float4* __restrict__ rays;
+  const uint32_t* __restrict__ index;      // CHI: target id per record
+  const uint32_t* __restrict__ order;      // nullptr: trace in the caller's order
+  const uint32_t* __restrict__ prim_slot;  // original id -> slot
+  uint32_t n_spheres;
+  uint32_t idx;
+  uint4 hit;  // CHI: the target's record, written when nothing blocks it
+  PTB_DEV void operator()(uint32_t i, Ray& r, float& tmax, uint32_t& exclude) {
+    idx = order ? order[i] : i;
+    const float4 o = __ldg(rays + 2u * (size_t)idx), d = __ldg(rays + 2u * (size_t)idx + 1u);
+    r = make_ray_from_raw(from4(o), from4(d));
+    if (CHI) {
+      const uint32_t p = __ldg(index + idx);
+      hit = make_uint4(__float_as_uint(0.0f), PTB_MISS, 0u, 0u);
+      tmax = 0.0f;
+      exclude = kNone;
+      if (p < sc.n_prims) {
+        const uint32_t slot = __ldg(prim_slot + p);
+        HitRec h;
+        if (prim_hit(sc, r, (p < n_spheres ? kSphereBit : 0u) | slot, h) && h.t > 0.0f) {  // acceleration/mod.rs:231-243
+          hit = make_uint4(__float_as_uint(h.t), p, __float_as_uint(h.b1), __float_as_uint(h.b2));
+          tmax = h.t;
+          exclude = slot;
+        }
+      }
+    } else {
+      const uint32_t x = __float_as_uint(d.w);
+      tmax = o.w;
+      exclude = x < sc.n_prims ? __ldg(prim_slot + x) : kNone;
+    }
+  }
+};
+template <bool CHI>
+struct VisRetire {
+  void* __restrict__ out;
+  const VisFetch<CHI>& f;
+  PTB_DEV void operator()(bool fin, const TraceResult& tr, const Ray&) {
+    if (!fin) return;
+    if (CHI) static_cast<uint4*>(out)[f.idx] = tr.ref == kNone ? f.hit : make_uint4(__float_as_uint(0.0f), PTB_MISS, 0u, 0u);
+    else static_cast<uint8_t*>(out)[f.idx] = tr.ref != kNone ? 1u : 0u;
+  }
+};
+template <class TR, bool CHI>
+__global__ void __launch_bounds__(256, TR::kApiMinBlocks)
+k_visibility_api(DevScene sc, const float4* __restrict__ rays, const uint32_t* __restrict__ index,
+                 const uint32_t* __restrict__ order, const uint32_t* __restrict__ prim_slot, uint32_t n_spheres, uint32_t n,
+                 void* __restrict__ out, uint32_t* head) {
+  uint32_t a = 0, b = 0, r = 0;
+  VisFetch<CHI> fetch{sc, rays, index, order, prim_slot, n_spheres, 0u, make_uint4(0u, 0u, 0u, 0u)};
+  VisRetire<CHI> retire{out, fetch};
+  persistent_trace<TR, true, false>(sc, n, head, fetch, retire, a, b, r);
+}
+
 // ------------------------------------------------------------------------------------------ sampler test hook
 // ptb_sample_only / ptb_sampler_pdf (include/ptb200.h): the reference's best-pinned tests are chi-squared tests of its
 // samplers against their pdfs (statistics/spherical_sampling.rs:64-226, bxdfs/lambertian.rs:30-48,
@@ -1680,6 +1743,10 @@ static const void* api_kernel(const Ctx* c, bool count) {
   if (c->wide) return count ? (const void*)k_closest_hit_api<CwTrav, true> : (const void*)k_closest_hit_api<CwTrav, false>;
   return count ? (const void*)k_closest_hit_api<BinTrav, true> : (const void*)k_closest_hit_api<BinTrav, false>;
 }
+static const void* visibility_kernel(const Ctx* c, bool chi) {
+  if (c->wide) return chi ? (const void*)k_visibility_api<CwTrav, true> : (const void*)k_visibility_api<CwTrav, false>;
+  return chi ? (const void*)k_visibility_api<BinTrav, true> : (const void*)k_visibility_api<BinTrav, false>;
+}
 template <class TR>
 static const void* tail_kernel_of(bool mis, bool full) {
   if (mis) return full ? (const void*)k_tail<TR, PTB_METHOD_MIS, true> : (const void*)k_tail<TR, PTB_METHOD_MIS, false>;
@@ -1703,19 +1770,19 @@ static int persistent_grid(Ctx* c, const void* kernel, int threads) {
   return c->sm_count * per_sm;
 }
 
-int32_t launch_closest_hit(Ctx* c, const void* d_rays, size_t n, void* d_hits) {
-  if (n == 0) return PTB_OK;
+// Work cursor and counters of one batch-API launch (in the scratch after the wavefront counters: [0] work cursor,
+// [8..24) node / primitive counters), zeroed on the stream, and the order the batch is traced in: batches of >= 65 536
+// rays are ordered by k_ray_sort_keys (which reads only the .xyz of the two float4 of a record, so ptb_ray and
+// ptb_occlusion_ray sort alike); PTB_HIT_SORT=0 traces in the caller's order (*order = nullptr).
+static int32_t prepare_batch(Ctx* c, const float4* r4, size_t n, uint32_t** head, unsigned long long** counts,
+                             const uint32_t** order) {
   if (n > 0xFFFFFFF0ull) return set_error(c, PTB_ERR_INVALID, "too many rays in one batch");
   PTB_CUDA_TRY(c, c->d_counters.reserve(sizeof(WaveCounters) + 64));
-  // scratch after the wavefront counters: [0] work cursor, [8..24) node / primitive counters
   char* scratch = c->d_counters.as<char>() + sizeof(WaveCounters);
-  uint32_t* head = reinterpret_cast<uint32_t*>(scratch);
-  unsigned long long* counts = reinterpret_cast<unsigned long long*>(scratch + 8);
+  *head = reinterpret_cast<uint32_t*>(scratch);
+  *counts = reinterpret_cast<unsigned long long*>(scratch + 8);
   PTB_CUDA_TRY(c, cudaMemsetAsync(scratch, 0, 24, c->stream));
-  const float4* r4 = reinterpret_cast<const float4*>(d_rays);
-  uint4* h4 = reinterpret_cast<uint4*>(d_hits);
-  // order the batch (see k_ray_sort_keys); PTB_HIT_SORT=0 traces in the caller's order
-  const uint32_t* order = nullptr;
+  *order = nullptr;
   bool sort = n >= (1u << 16) && c->n_prims > 0;
   if (const char* e = getenv("PTB_HIT_SORT")) sort = sort && atoi(e) != 0;
   if (sort) {
@@ -1726,8 +1793,20 @@ int32_t launch_closest_hit(Ctx* c, const void* d_rays, size_t n, void* d_hits) {
     k_ray_sort_keys<<<(n32 + 255u) / 256u, 256, 0, c->stream>>>(c->dev, r4, n32, ka, va);
     c->stats.kernel_launches += 1;
     radix_sort_pairs(c, ka, va, kb, vb, n32, 3, hist);
-    order = va;
+    *order = va;
   }
+  return PTB_OK;
+}
+
+int32_t launch_closest_hit(Ctx* c, const void* d_rays, size_t n, void* d_hits) {
+  if (n == 0) return PTB_OK;
+  const float4* r4 = reinterpret_cast<const float4*>(d_rays);
+  uint4* h4 = reinterpret_cast<uint4*>(d_hits);
+  uint32_t* head;
+  unsigned long long* counts;
+  const uint32_t* order;
+  const int32_t rc = prepare_batch(c, r4, n, &head, &counts, &order);
+  if (rc != PTB_OK) return rc;
   {
     const void* fn = api_kernel(c, c->opt_count_traversal);
     const int grid = persistent_grid(c, fn, 256);
@@ -1743,6 +1822,28 @@ int32_t launch_closest_hit(Ctx* c, const void* d_rays, size_t n, void* d_hits) {
     c->stats.prims_tested += hc[1];
     c->stats.rays_counted += n;
   }
+  c->stats.kernel_launches += 1;
+  c->stats.trace_launches += 1;
+  PTB_CUDA_TRY(c, cudaGetLastError());
+  return PTB_OK;
+}
+
+int32_t launch_visibility(Ctx* c, const void* d_rays, const void* d_index, size_t n, void* d_out) {
+  if (n == 0) return PTB_OK;
+  const float4* r4 = reinterpret_cast<const float4*>(d_rays);
+  const uint32_t* index = static_cast<const uint32_t*>(d_index);
+  uint32_t* head;
+  unsigned long long* counts;
+  const uint32_t* order;
+  const int32_t rc = prepare_batch(c, r4, n, &head, &counts, &order);
+  if (rc != PTB_OK) return rc;
+  const void* fn = visibility_kernel(c, index != nullptr);
+  const int grid = persistent_grid(c, fn, 256);
+  const uint32_t* prim_slot = c->d_prim_slot.as<uint32_t>();
+  uint32_t ns = (uint32_t)c->n_spheres, n32 = (uint32_t)n;
+  void* args[] = {(void*)&c->dev, (void*)&r4, (void*)&index, (void*)&order, (void*)&prim_slot, (void*)&ns, (void*)&n32,
+                  (void*)&d_out, (void*)&head};
+  PTB_CUDA_TRY(c, cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(256), args, 0, c->stream));
   c->stats.kernel_launches += 1;
   c->stats.trace_launches += 1;
   PTB_CUDA_TRY(c, cudaGetLastError());
