@@ -10,7 +10,7 @@ type Prim<'a> = AllPrimitives<'a, Mat<'a>>;
 
 fn v(p: Vec3) -> ptb_vec3 { ptb_vec3 { x: p.x, y: p.y, z: p.z } }
 
-pub struct CudaScene { ctx: *mut ptb_ctx }
+pub struct CudaScene { ctx: *mut ptb_ctx, mat_ids: HashMap<*const Mat, u32> }
 
 impl CudaScene {
     /// `primitives` in loader order (spheres first, then mesh triangles: loader/src/lib.rs:234-240).
@@ -53,7 +53,7 @@ impl CudaScene {
             check(ctx, ptb_scene_set_sky(ctx, &sky))?;
             check(ctx, ptb_scene_commit(ctx, 0))?; // Bvh::new
         }
-        Ok(Self { ctx })
+        Ok(Self { ctx, mat_ids })
     }
 
     /// Scene::render (src/scene.rs:35-42) for the cuda backend: the accumulator comes back as the running-mean image the
@@ -73,6 +73,41 @@ impl CudaScene {
 }
 
 impl CudaScene {
+    /// Animation: overwrite triangles [first, first + tris.len()) of the scene (triangle order, i.e. loader order after the
+    /// spheres) with new geometry. Their materials must be ones the scene was created with. Call `refit` afterwards.
+    pub fn update_triangles(&self, first: usize, tris: &[Prim]) -> Result<(), String> {
+        let mut out = Vec::with_capacity(tris.len());
+        for p in tris {
+            let (pts, nrm, m) = match p {
+                Prim::Triangle(t) => (t.points.map(v), t.normals.map(v), t.material),
+                Prim::MeshTriangle(t) => (t.point_indices.map(|i| v(t.mesh.vertices[i])), t.normal_indices.map(|i| v(t.mesh.normals[i])), t.material),
+                Prim::Sphere(_) => return Err("update_triangles: a sphere in the triangle range".into()),
+            };
+            let material = *self.mat_ids.get(&(m as *const _)).ok_or("update_triangles: a material the scene does not have")?;
+            out.push(ptb_triangle { p: pts, n: nrm, material });
+        }
+        check(self.ctx, unsafe { ptb_scene_update_triangles(self.ctx, first, out.as_ptr(), out.len()) })
+    }
+
+    /// Commit the updates keeping the tree (PTB_BUILD_REFIT); returns the refitted tree's SAH cost, which the caller
+    /// compares with the cost after the last full build to decide when to call `rebuild`.
+    pub fn refit(&self) -> Result<f64, String> {
+        check(self.ctx, unsafe { ptb_scene_commit(self.ctx, PTB_BUILD_REFIT) })?;
+        self.sah_cost()
+    }
+
+    /// A full commit (Bvh::new's tree for the primitives as they are now); returns its SAH cost.
+    pub fn rebuild(&self) -> Result<f64, String> {
+        check(self.ctx, unsafe { ptb_scene_commit(self.ctx, PTB_BUILD_DEFAULT) })?;
+        self.sah_cost()
+    }
+
+    fn sah_cost(&self) -> Result<f64, String> {
+        let mut c = 0.0f64;
+        check(self.ctx, unsafe { ptb_bvh_sah_cost(self.ctx, &mut c) })?;
+        Ok(c)
+    }
+
     /// AccelerationStructure::check_hit_index (acceleration/mod.rs:226-263) for a batch: is primitive `index[i]` (loader
     /// order) the first thing ray i hits? Some((t, b1, b2)) when it is, None when it is blocked, missed or out of range.
     pub fn check_hit_index(&self, rays: &[Ray], index: &[u32]) -> Result<Vec<Option<(Float, Float, Float)>>, String> {

@@ -46,6 +46,7 @@ pub const PTB_BUILD_DEFAULT: u32 = 0;
 pub const PTB_BUILD_BINARY: u32 = 1; // Karras LBVH
 pub const PTB_BUILD_WIDE: u32 = 2;   // LBVH collapsed into the compressed 8-wide tree
 pub const PTB_BUILD_SAH: u32 = 4;    // top-down SAH builder (Bvh::new with Split::Sah, acceleration/mod.rs:58-160)
+pub const PTB_BUILD_REFIT: u32 = 8;  // keep the last full commit's binary tree, refit its boxes (same primitive counts)
 
 extern "C" {
     pub fn ptb_abi_version() -> u32;
@@ -59,7 +60,12 @@ extern "C" {
     pub fn ptb_scene_set_texture_data(ctx: *mut ptb_ctx, texture: u32, width: u32, height: u32, data: *const f32, n_floats: usize) -> i32;
     pub fn ptb_scene_set_camera(ctx: *mut ptb_ctx, cam: *const ptb_camera) -> i32;
     pub fn ptb_scene_set_sky(ctx: *mut ptb_ctx, sky: *const ptb_sky) -> i32;
+    pub fn ptb_scene_update_spheres(ctx: *mut ptb_ctx, first: usize, p: *const ptb_sphere, n: usize) -> i32;
+    pub fn ptb_scene_update_triangles(ctx: *mut ptb_ctx, first: usize, p: *const ptb_triangle, n: usize) -> i32;
+    pub fn ptb_scene_update_spheres_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
+    pub fn ptb_scene_update_triangles_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
     pub fn ptb_scene_commit(ctx: *mut ptb_ctx, build_flags: u32) -> i32;
+    pub fn ptb_bvh_sah_cost(ctx: *mut ptb_ctx, cost: *mut f64) -> i32;
     pub fn ptb_bvh_export_quantised(ctx: *mut ptb_ctx, frame: *mut f32, nodes32: *mut c_void) -> i32;
     pub fn ptb_bvh_wide_info(ctx: *mut ptb_ctx, n_nodes: *mut u64, max_leaf: *mut u32) -> i32;
     pub fn ptb_bvh_builder(ctx: *mut ptb_ctx, builder: *mut u32, sah_levels: *mut u32) -> i32;

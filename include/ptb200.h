@@ -174,7 +174,7 @@ typedef struct ptb_stats {
   uint64_t prims_tested;       /* PTB_OPT_COUNT_TRAVERSAL: primitives tested by closest-hit traversals          */
   uint64_t rays_counted;       /* PTB_OPT_COUNT_TRAVERSAL: closest-hit traversals the two counters cover        */
   uint64_t trace_launches;     /* traversal kernel launches (k_trace / k_closest_hit_api / k_visibility_api)    */
-  double   build_ms;           /* last ptb_scene_commit: device LBVH build time               */
+  double   build_ms;           /* last ptb_scene_commit: device LBVH build time (refit time for PTB_BUILD_REFIT) */
   double   render_ms;          /* last ptb_render: device time (CUDA events)                  */
   double   ms_generate;        /* PTB_OPT_TIME_KERNELS: summed CUDA-event time per kernel class */
   double   ms_trace;
@@ -225,12 +225,44 @@ int32_t ptb_scene_set_sky(ptb_ctx* ctx, const ptb_sky* sky);
  * the replacement for the QUALITY of build_bvh + Split::Sah, acceleration/mod.rs:97-160, split.rs:78-187; CPU definition
  * oracle/sah_ref.hpp; 2..2^24 primitives, otherwise the LBVH is built). Same hits, fewer nodes per ray, a slower commit.
  * PTB_BUILD_DEFAULT follows the environment (PTB_BVH=binary|lbvh|sah|wide) and otherwise the library's default. */
-enum { PTB_BUILD_DEFAULT = 0, PTB_BUILD_BINARY = 1, PTB_BUILD_WIDE = 2, PTB_BUILD_SAH = 4 };
+enum { PTB_BUILD_DEFAULT = 0, PTB_BUILD_BINARY = 1, PTB_BUILD_WIDE = 2, PTB_BUILD_SAH = 4, PTB_BUILD_REFIT = 8 };
 int32_t ptb_scene_commit(ptb_ctx* ctx, uint32_t build_flags);
+
+/* Dynamic scenes. PTB_BUILD_REFIT commits whatever was set since the last commit but KEEPS the binary tree of the last full
+ * commit: its topology (child / parent links) and its primitive slot order stay, and its boxes are refitted bottom-up to
+ * the primitives as they are now. Materials, textures, camera, sky table, material-index validation and the light list are
+ * redone as in a full commit; Morton codes, sort, hierarchy and SAH build are skipped. Hits do not depend on the tree, so a
+ * refitted scene answers every query exactly as a fresh commit of the same primitives does; only the traversal cost
+ * changes as the primitives move away from the layout the tree was built for (see ptb_bvh_sah_cost).
+ *   - Requirements: the last full commit of this context succeeded (a full commit that fails drops the kept tree), the
+ *     numbers of spheres and triangles are those of that commit, and the flag is passed alone. Otherwise the commit fails
+ *     with PTB_ERR_INVALID and a message naming the reason; a full commit always works afterwards.
+ *   - A scene committed with the compressed 8-wide tree answers PTB_ERR_UNSUPPORTED.
+ *   - ptb_bvh_builder keeps reporting the builder that made the topology; ptb_stats.build_ms is the refit's device time;
+ *     ptb_bvh_export's morton_sorted keeps the codes of the last full build.
+ * Typical animation loop: ptb_scene_update_* -> ptb_scene_commit(PTB_BUILD_REFIT) -> ptb_accum_clear -> ptb_render, with a
+ * full commit whenever ptb_bvh_sah_cost has grown too far above the value of a fresh build. */
+/* Overwrite primitives [first, first + n) of the current arrays, in original (loader) order, in place; the counts do not
+ * change. Like ptb_scene_set_*, they leave the scene uncommitted. first + n beyond the current count (overflow-safe) and a
+ * null pointer with n > 0 give PTB_ERR_INVALID; n == 0 is a no-op. The host variants copy before returning. */
+int32_t ptb_scene_update_spheres(ptb_ctx* ctx, size_t first, const ptb_sphere* spheres, size_t n);
+int32_t ptb_scene_update_triangles(ptb_ctx* ctx, size_t first, const ptb_triangle* triangles, size_t n);
+/* Same from device memory: a device-to-device copy enqueued on the context's stream, returning without synchronising. The
+ * caller's buffer must be ready when the stream reaches the copy (produce it on the same stream, see ptb_set_stream, or
+ * synchronise first) and must stay valid until the next commit or ptb_synchronize. */
+int32_t ptb_scene_update_spheres_device(ptb_ctx* ctx, size_t first, const void* d_spheres, size_t n);
+int32_t ptb_scene_update_triangles_device(ptb_ctx* ctx, size_t first, const void* d_triangles, size_t n);
+/* SAH cost of the committed binary tree in the reference's cost model (traversal 0.125, intersection 1, split.rs:161-176):
+ * (0.125 * sum over inner nodes of SA(node) + sum over leaves of SA(leaf box)) / SA(root), SA = 2 (xy + yz + zx) of the f32
+ * box evaluated in f64, root box = union of node 0's two child boxes. 1 primitive: 1.125; 0 primitives or a root of zero
+ * area: 0. A device reduction in a fixed order: the same tree gives the same bits on every call. The wide tree answers
+ * PTB_ERR_UNSUPPORTED. The signal for refit-or-rebuild: compare with the cost right after the last full commit. */
+int32_t ptb_bvh_sah_cost(ptb_ctx* ctx, double* cost);
 
 /* Bit-exact test hooks: n_prims Morton codes and primitive ids in sorted order, n_prims-1 nodes
  * (1 node when n_prims == 1). Any pointer may be NULL. After an SAH build prim_sorted is the SAH tree's own primitive
- * order (what its leaf references index) while morton_sorted still holds the sorted codes of the order it started from. */
+ * order (what its leaf references index) while morton_sorted still holds the sorted codes of the order it started from.
+ * After a PTB_BUILD_REFIT commit morton_sorted and prim_sorted are those of the last full build. */
 int32_t ptb_bvh_info(ptb_ctx* ctx, uint64_t* n_prims, uint64_t* n_nodes);
 int32_t ptb_bvh_export(ptb_ctx* ctx, uint32_t* morton_sorted, uint32_t* prim_sorted, ptb_bvh_node* nodes);
 /* The same binary tree as the traversal kernels read it (bit-exact test hook): 32 bytes per node, both children's boxes

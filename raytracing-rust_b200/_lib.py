@@ -28,7 +28,7 @@ TEX_CHECKERED, TEX_SOLID, TEX_IMAGE, TEX_LERP, TEX_PERLIN = range(5)
 METHOD_NAIVE, METHOD_MIS = 0, 1
 PERLIN_TABLE_WORDS = 1024
 OPT_TIME_KERNELS, OPT_COUNT_TRAVERSAL = 1, 2
-BUILD_DEFAULT, BUILD_BINARY, BUILD_WIDE, BUILD_SAH = 0, 1, 2, 4
+BUILD_DEFAULT, BUILD_BINARY, BUILD_WIDE, BUILD_SAH, BUILD_REFIT = 0, 1, 2, 4, 8
 
 # numpy mirrors of the POD structs (sizes asserted against the header's layout in tests/test_abi.py)
 sphere_dtype = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4")])
@@ -101,7 +101,12 @@ SYMBOLS = [
     ("ptb_scene_set_texture_data", C.c_int32, [_P, C.c_uint32, C.c_uint32, C.c_uint32, _P, C.c_size_t]),
     ("ptb_scene_set_camera", C.c_int32, [_P, _P]),
     ("ptb_scene_set_sky", C.c_int32, [_P, _P]),
+    ("ptb_scene_update_spheres", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_triangles", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_spheres_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_triangles_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
     ("ptb_scene_commit", C.c_int32, [_P, C.c_uint32]),
+    ("ptb_bvh_sah_cost", C.c_int32, [_P, C.POINTER(C.c_double)]),
     ("ptb_bvh_info", C.c_int32, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     ("ptb_bvh_export", C.c_int32, [_P, _P, _P, _P]),
     ("ptb_bvh_export_quantised", C.c_int32, [_P, _P, _P]),

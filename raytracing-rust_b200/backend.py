@@ -99,8 +99,36 @@ class Context:
     def commit(self, flags: int = 0):
         """Bvh::new: device build of the acceleration structure. L.BUILD_BINARY: Karras LBVH; L.BUILD_SAH: top-down SAH
         builder (sah_build.cu); L.BUILD_WIDE: the LBVH collapsed into the compressed 8-wide tree; L.BUILD_DEFAULT follows
-        PTB_BVH=binary|lbvh|sah|wide, else the library default."""
+        PTB_BVH=binary|lbvh|sah|wide, else the library default. L.BUILD_REFIT (alone) keeps the binary tree of the last
+        full commit and refits its boxes to the primitives as they are now (see update_triangles)."""
         _check(self._h, L.lib.ptb_scene_commit(self._h, flags))
+
+    # ---- dynamic scenes: overwrite primitives in place, then commit(L.BUILD_REFIT)
+    def update_spheres(self, first: int, spheres: np.ndarray):
+        """Overwrite spheres [first, first + len(spheres)) (sphere_dtype, original order); the count does not change."""
+        a = np.ascontiguousarray(spheres, dtype=L.sphere_dtype)
+        _check(self._h, L.lib.ptb_scene_update_spheres(self._h, first, L.ptr(a), len(a)))
+
+    def update_triangles(self, first: int, triangles: np.ndarray):
+        """Overwrite triangles [first, first + len(triangles)) (triangle_dtype; triangle ids, not primitive ids)."""
+        a = np.ascontiguousarray(triangles, dtype=L.triangle_dtype)
+        _check(self._h, L.lib.ptb_scene_update_triangles(self._h, first, L.ptr(a), len(a)))
+
+    def update_spheres_device(self, first: int, d_ptr: int, n: int):
+        """Same from device memory (n records of sphere_dtype's layout), enqueued on the context's stream without a
+        synchronise: the buffer must be ready when the stream gets there (produce it on that stream, see set_stream)."""
+        _check(self._h, L.lib.ptb_scene_update_spheres_device(self._h, first, C.c_void_p(d_ptr), n))
+
+    def update_triangles_device(self, first: int, d_ptr: int, n: int):
+        """Same from device memory (n records of triangle_dtype's layout, 76 bytes each)."""
+        _check(self._h, L.lib.ptb_scene_update_triangles_device(self._h, first, C.c_void_p(d_ptr), n))
+
+    def bvh_sah_cost(self) -> float:
+        """SAH cost of the committed binary tree (traversal 0.125, intersection 1; normalised by the root's area). Compare
+        it with the value right after a full commit to decide when a refitted tree should be rebuilt."""
+        v = C.c_double()
+        _check(self._h, L.lib.ptb_bvh_sah_cost(self._h, C.byref(v)))
+        return v.value
 
     def bvh_info(self):
         a, b = C.c_uint64(), C.c_uint64()

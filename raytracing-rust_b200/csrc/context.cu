@@ -182,6 +182,34 @@ int32_t ptb_scene_set_triangles(ptb_ctx* ctx, const ptb_triangle* p, size_t n) {
   c->n_tris = n;
   return PTB_OK;
 }
+// ptb_scene_update_*: primitives [first, first + n) of `raw` (count `have`, records of `rec` bytes) in place
+static int32_t update_prims(Ctx* c, DevBuf& raw, size_t have, size_t rec, size_t first, const void* p, size_t n,
+                            cudaMemcpyKind kind, const char* what) {
+  if (first > have || n > have - first)
+    return set_error(c, PTB_ERR_INVALID, "%s update [%zu, %zu + %zu) outside the %zu the scene holds", what, first, first, n, have);
+  if (n == 0) return PTB_OK;
+  if (!p) return set_error(c, PTB_ERR_INVALID, "null %s", what);
+  c->committed = false;
+  PTB_CUDA_TRY(c, cudaMemcpyAsync(static_cast<char*>(raw.p) + first * rec, p, n * rec, kind, c->stream));
+  if (kind == cudaMemcpyHostToDevice) PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));  // the caller may reuse its buffer
+  return PTB_OK;
+}
+int32_t ptb_scene_update_spheres(ptb_ctx* ctx, size_t first, const ptb_sphere* p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_prims(c, c->d_raw_spheres, c->n_spheres, sizeof(ptb_sphere), first, p, n, cudaMemcpyHostToDevice, "spheres");
+}
+int32_t ptb_scene_update_triangles(ptb_ctx* ctx, size_t first, const ptb_triangle* p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_prims(c, c->d_raw_tris, c->n_tris, sizeof(ptb_triangle), first, p, n, cudaMemcpyHostToDevice, "triangles");
+}
+int32_t ptb_scene_update_spheres_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_prims(c, c->d_raw_spheres, c->n_spheres, sizeof(ptb_sphere), first, d_p, n, cudaMemcpyDeviceToDevice, "spheres");
+}
+int32_t ptb_scene_update_triangles_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_prims(c, c->d_raw_tris, c->n_tris, sizeof(ptb_triangle), first, d_p, n, cudaMemcpyDeviceToDevice, "triangles");
+}
 int32_t ptb_scene_set_materials(ptb_ctx* ctx, const ptb_material* p, size_t n) {
   CTX_OR_FAIL(ctx);
   if (n && !p) return set_error(c, PTB_ERR_INVALID, "null materials");
@@ -284,6 +312,14 @@ int32_t ptb_bvh_builder(ptb_ctx* ctx, uint32_t* builder, uint32_t* sah_levels) {
   if (builder) *builder = c->wide ? PTB_BUILD_WIDE : (c->sah ? PTB_BUILD_SAH : PTB_BUILD_BINARY);
   if (sah_levels) *sah_levels = c->sah ? c->sah_levels : 0u;
   return PTB_OK;
+}
+
+int32_t ptb_bvh_sah_cost(ptb_ctx* ctx, double* cost) {
+  CTX_OR_FAIL(ctx);
+  if (!cost) return set_error(c, PTB_ERR_INVALID, "null cost");
+  if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
+  if (c->wide) return set_error(c, PTB_ERR_UNSUPPORTED, "the SAH cost is defined for the binary tree; the committed scene uses the 8-wide tree");
+  return tree_sah_cost(c, cost);
 }
 
 int32_t ptb_bvh_export(ptb_ctx* ctx, uint32_t* morton_sorted, uint32_t* prim_sorted, ptb_bvh_node* nodes) {

@@ -459,6 +459,144 @@ __global__ void k_light_slots(const uint32_t* __restrict__ light_prims, uint32_t
   lights[i] = (p < n_spheres ? kSphereBit : 0u) | prim_slot[p];
 }
 
+// ------------------------------------------------------------------------------------------ refit of a kept tree
+// PTB_BUILD_REFIT: one thread per slot of the binary tree of the last full commit. It reads its primitive once, writes the
+// slot's records as k_gather does, computes the box with k_prim_bounds' arithmetic (bit-identical), stores it in slot order
+// and climbs leaf_parent with k_refit's arrival flags. A leaf child's box comes from the slot-ordered array, so an arrival
+// costs no dependent prim_sorted -> bmin[p] load, and nothing goes through original order or the global bounds atomics.
+__global__ void k_refit_slots(const ptb_sphere* __restrict__ spheres, uint32_t n_spheres, const ptb_triangle* __restrict__ tris,
+                              uint32_t n_prims, const uint32_t* __restrict__ slot_prim, const uint32_t* __restrict__ leaf_parent,
+                              const DevMaterial* __restrict__ mats, uint32_t n_mats, float4* __restrict__ geom,
+                              float4* __restrict__ normals, uint32_t* __restrict__ slot_mat, float4* sbmin, float4* sbmax,
+                              BvhNode* nodes, float4* nbmin, float4* nbmax, uint32_t* flags) {
+  const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
+  if (slot >= n_prims) return;
+  const uint32_t p = slot_prim[slot];
+  uint32_t mat;
+  float4 g0, g1, g2, m0, m1, m2;
+  v3 mn, mx;
+  if (p < n_spheres) {
+    const ptb_sphere s = spheres[p];
+    const v3 c = mk(s.center.x, s.center.y, s.center.z);
+    mn = c - s.radius * mk(1.0f, 1.0f, 1.0f);
+    mx = c + s.radius * mk(1.0f, 1.0f, 1.0f);
+    g0 = make_float4(s.center.x, s.center.y, s.center.z, s.radius);
+    g1 = g2 = m0 = m1 = m2 = make_float4(0.f, 0.f, 0.f, 0.f);
+    mat = s.material;
+  } else {
+    const ptb_triangle* t = tris + (p - n_spheres);
+    const v3 p0 = mk(t->p[0].x, t->p[0].y, t->p[0].z), p1 = mk(t->p[1].x, t->p[1].y, t->p[1].z),
+             p2 = mk(t->p[2].x, t->p[2].y, t->p[2].z);
+    mn = vmin(p0, vmin(p1, p2));
+    mx = vmax(p0, vmax(p1, p2));
+    g0 = make_float4(p0.x, p0.y, p0.z, 0.f);
+    g1 = make_float4(p1.x, p1.y, p1.z, 0.f);
+    g2 = make_float4(p2.x, p2.y, p2.z, 0.f);
+    m0 = make_float4(t->n[0].x, t->n[0].y, t->n[0].z, 0.f);
+    m1 = make_float4(t->n[1].x, t->n[1].y, t->n[1].z, 0.f);
+    m2 = make_float4(t->n[2].x, t->n[2].y, t->n[2].z, 0.f);
+    mat = t->material;
+  }
+  geom[3 * (size_t)slot + 0] = g0;
+  geom[3 * (size_t)slot + 1] = g1;
+  geom[3 * (size_t)slot + 2] = g2;
+  normals[3 * (size_t)slot + 0] = m0;
+  normals[3 * (size_t)slot + 1] = m1;
+  normals[3 * (size_t)slot + 2] = m2;
+  const uint32_t kind = mat < n_mats ? mats[mat].kind : 0u;  // out of range: reported by k_collect_lights, as in k_gather
+  slot_mat[slot] = (kind << 24) | (mat & 0x00FFFFFFu);
+  __stcg(sbmin + slot, make_float4(mn.x, mn.y, mn.z, 0.0f));
+  __stcg(sbmax + slot, make_float4(mx.x, mx.y, mx.z, 0.0f));
+  if (n_prims < 2) return;  // the single node is k_single_node's
+  uint32_t cur = leaf_parent[slot];
+  while (cur != kNone) {
+    __threadfence();
+    if (atomicAdd(flags + cur, 1u) == 0u) return;  // first arrival: the sibling subtree is not finished yet
+    __threadfence();
+    const uint4 links = nodes[cur].n3;
+    v3 lmn, lmx, rmn, rmx;
+    const float4 *lo = (links.x & PTB_LEAF_BIT) ? sbmin + (links.x & kSlotMask) : nbmin + links.x,
+                 *hi = (links.x & PTB_LEAF_BIT) ? sbmax + (links.x & kSlotMask) : nbmax + links.x;
+    lmn = from4(__ldcg(lo));  // written by another thread of this launch: read through L2
+    lmx = from4(__ldcg(hi));
+    lo = (links.y & PTB_LEAF_BIT) ? sbmin + (links.y & kSlotMask) : nbmin + links.y;
+    hi = (links.y & PTB_LEAF_BIT) ? sbmax + (links.y & kSlotMask) : nbmax + links.y;
+    rmn = from4(__ldcg(lo));
+    rmx = from4(__ldcg(hi));
+    nodes[cur].n0 = make_float4(lmn.x, lmn.y, lmn.z, lmx.x);
+    nodes[cur].n1 = make_float4(lmx.y, lmx.z, rmn.x, rmn.y);
+    nodes[cur].n2 = make_float4(rmn.z, rmx.x, rmx.y, rmx.z);
+    const v3 bmn = vmin(lmn, rmn), bmx = vmax(lmx, rmx);
+    __stcg(nbmin + cur, make_float4(bmn.x, bmn.y, bmn.z, 0.0f));
+    __stcg(nbmax + cur, make_float4(bmx.x, bmx.y, bmx.z, 0.0f));
+    cur = links.z;
+  }
+}
+
+// ------------------------------------------------------------------------------------------ SAH cost of the binary tree
+// (0.125 * sum over inner nodes of SA(node) + sum over leaves of SA(leaf box)) / SA(root), SA = 2 (xy + yz + zx) of the f32
+// box in f64 (the reference's cost model, split.rs:161-163,176). A node's own box is the union of its two child boxes, a
+// leaf's box is the child box its parent stores. Fixed summation order: block partials, then one block in index order.
+PTB_DEV double box_area(float lx, float ly, float lz, float hx, float hy, float hz) {
+  const double dx = (double)hx - (double)lx, dy = (double)hy - (double)ly, dz = (double)hz - (double)lz;
+  return 2.0 * (dx * dy + dy * dz + dz * dx);
+}
+constexpr int kCostThreads = 256;
+__device__ __forceinline__ double block_sum_fixed(double v, double* sh) {
+  sh[threadIdx.x] = v;
+  __syncthreads();
+  for (int s = kCostThreads / 2; s > 0; s >>= 1) {
+    if ((int)threadIdx.x < s) sh[threadIdx.x] += sh[threadIdx.x + s];
+    __syncthreads();
+  }
+  return sh[0];
+}
+__global__ void __launch_bounds__(kCostThreads)
+k_sah_cost_partial(const BvhNode* __restrict__ nodes, uint32_t n_nodes, uint32_t n_prims, double* __restrict__ partial) {
+  __shared__ double sh[kCostThreads];
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  double v = 0.0;
+  if (i < n_nodes) {
+    const BvhNode nd = nodes[i];
+    v = 0.125 * box_area(fminf(nd.n0.x, nd.n1.z), fminf(nd.n0.y, nd.n1.w), fminf(nd.n0.z, nd.n2.x), fmaxf(nd.n0.w, nd.n2.y),
+                         fmaxf(nd.n1.x, nd.n2.z), fmaxf(nd.n1.y, nd.n2.w));
+    if (nd.n3.x & PTB_LEAF_BIT) v += box_area(nd.n0.x, nd.n0.y, nd.n0.z, nd.n0.w, nd.n1.x, nd.n1.y);
+    if ((nd.n3.y & PTB_LEAF_BIT) && n_prims > 1)  // one primitive: both child slots name the same leaf
+      v += box_area(nd.n1.z, nd.n1.w, nd.n2.x, nd.n2.y, nd.n2.z, nd.n2.w);
+  }
+  const double s = block_sum_fixed(v, sh);
+  if (threadIdx.x == 0) partial[blockIdx.x] = s;
+}
+__global__ void __launch_bounds__(kCostThreads)
+k_sah_cost_final(const double* __restrict__ partial, uint32_t n_partial, const BvhNode* __restrict__ nodes, double* __restrict__ out) {
+  __shared__ double sh[kCostThreads];
+  const uint32_t per = (n_partial + kCostThreads - 1) / kCostThreads;
+  const uint32_t b = threadIdx.x * per, e = min(b + per, n_partial);
+  double v = 0.0;
+  for (uint32_t k = b; k < e; ++k) v += partial[k];
+  const double s = block_sum_fixed(v, sh);
+  if (threadIdx.x == 0) {
+    const BvhNode r = nodes[0];
+    const double root = box_area(fminf(r.n0.x, r.n1.z), fminf(r.n0.y, r.n1.w), fminf(r.n0.z, r.n2.x), fmaxf(r.n0.w, r.n2.y),
+                                 fmaxf(r.n1.x, r.n2.z), fmaxf(r.n1.y, r.n2.w));
+    *out = root > 0.0 ? s / root : 0.0;
+  }
+}
+int32_t tree_sah_cost(Ctx* c, double* cost) {
+  *cost = 0.0;
+  if (c->n_prims == 0) return PTB_OK;
+  const uint32_t n_nodes = (uint32_t)c->n_nodes, nb = (n_nodes + kCostThreads - 1) / kCostThreads;
+  DevBuf& tmp = c->scratch[2];  // build temporary (the bounds words), free between commits
+  PTB_CUDA_TRY(c, tmp.reserve(((size_t)nb + 1) * sizeof(double)));
+  double* d = tmp.as<double>();
+  k_sah_cost_partial<<<nb, kCostThreads, 0, c->stream>>>(c->d_nodes.as<BvhNode>(), n_nodes, (uint32_t)c->n_prims, d + 1);
+  k_sah_cost_final<<<1, kCostThreads, 0, c->stream>>>(d + 1, nb, c->d_nodes.as<BvhNode>(), d);
+  c->stats.kernel_launches += 2;
+  PTB_CUDA_TRY(c, cudaMemcpyAsync(cost, d, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  return PTB_OK;
+}
+
 // ------------------------------------------------------------------------------------------ host: sky table
 // Sky::new (implementations/src/sky.rs:20-37) = generate_values (textures/mod.rs:32-50) + Distribution2D::new
 // (statistics/distributions.rs:11-44, 82-99), in the reference's f32 operation order.
@@ -553,9 +691,10 @@ __global__ void k_collect_lights(const ptb_sphere* __restrict__ spheres, uint32_
 // triangles and 38.8 instead of 4.2 ms at 10 M (profiles/r2_sweeps.md section 12); the reference's own default is its SAH split
 #define PTB_DEFAULT_SAH 1
 #endif
-int32_t build_scene(Ctx* c, uint32_t build_flags) {
-  const size_t ns = c->n_spheres, nt = c->n_tris;
-  const size_t n = ns + nt;
+// What every commit redoes, full or refit: validation of the small tables, materials / textures / camera to the device, the
+// sky table.
+static int32_t commit_tables(Ctx* c) {
+  const size_t n = c->n_spheres + c->n_tris;
   if (n >= (size_t)kSlotMask) return set_error(c, PTB_ERR_INVALID, "too many primitives (%zu)", n);
   if (!c->have_camera) return set_error(c, PTB_ERR_INVALID, "scene has no camera");
   if (c->materials.empty() || c->textures.empty()) return set_error(c, PTB_ERR_INVALID, "scene has no materials/textures");
@@ -619,10 +758,117 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   c->dev.cam_lower_left = mk(c->camera.lower_left.x, c->camera.lower_left.y, c->camera.lower_left.z);
   c->dev.cam_horizontal = mk(c->camera.horizontal.x, c->camera.horizontal.y, c->camera.horizontal.z);
   c->dev.cam_vertical = mk(c->camera.vertical.x, c->camera.vertical.y, c->camera.vertical.z);
+  return build_sky(c);
+}
+
+// Light list, after k_collect_lights: count + validation flag back to the host (8 bytes, with whatever else the stream
+// has queued for the host), ids sorted into original order with the radix passes, then mapped to slots.
+static int32_t light_list(Ctx* c, uint32_t ns32, uint32_t* n_lights) {
+  cudaStream_t st = c->stream;
+  DevBuf &keys_b = c->scratch[4], &vals_b = c->scratch[6], &hist = c->scratch[7], &d_light_prims = c->scratch[12],
+         &d_light_tmp = c->scratch[13], &d_light_out = c->scratch[14];
+  uint32_t h_light_out[2] = {0u, 0u};
+  PTB_CUDA_TRY(c, cudaMemcpyAsync(h_light_out, d_light_out.p, 8, cudaMemcpyDeviceToHost, st));
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(st));
+  if (h_light_out[1]) return set_error(c, PTB_ERR_INVALID, "primitive material index out of range");
+  const uint32_t nl = h_light_out[0];
+  if (nl) {
+    PTB_CUDA_TRY(c, c->d_lights.reserve((size_t)nl * 4));
+    uint32_t *la = d_light_prims.as<uint32_t>(), *lb = d_light_tmp.as<uint32_t>();
+    if (nl > 1) {
+      // nl <= n: the histogram scratch is large enough
+      // values ride along unused: keys double as values (keys_b / vals_b are free again)
+      uint32_t *lva = keys_b.as<uint32_t>(), *lvb = vals_b.as<uint32_t>();
+      radix_sort_pairs(c, la, lva, lb, lvb, nl, 4, hist.as<uint32_t>());
+    }
+    k_light_slots<<<(nl + 255) / 256, 256, 0, st>>>(la, nl, ns32, c->d_prim_slot.as<uint32_t>(), c->d_lights.as<uint32_t>());
+    c->stats.kernel_launches += 1;
+  }
+  *n_lights = nl;
+  return PTB_OK;
+}
+
+// PTB_BUILD_REFIT: keeps the binary tree of the last full commit (links, leaf_parent, slot order, Morton codes) and refits
+// its boxes to the primitives as they are now; materials, textures, camera, sky and the light list are redone as in a
+// full commit.
+static int32_t refit_scene(Ctx* c, uint32_t build_flags) {
+  if (build_flags != PTB_BUILD_REFIT)
+    return set_error(c, PTB_ERR_INVALID, "PTB_BUILD_REFIT cannot be combined with another build flag (flags 0x%x)", build_flags);
+  if (!c->refittable)
+    return set_error(c, PTB_ERR_INVALID, "PTB_BUILD_REFIT needs a tree to keep: the last full commit of this context failed or there was none");
+  if (c->wide)
+    return set_error(c, PTB_ERR_UNSUPPORTED, "PTB_BUILD_REFIT: the compressed 8-wide tree cannot be refitted; commit with a binary builder");
+  if (c->n_spheres != c->topo_spheres || c->n_tris != c->topo_tris)
+    return set_error(c, PTB_ERR_INVALID, "PTB_BUILD_REFIT keeps the tree of %zu spheres and %zu triangles, the scene now has %zu and %zu",
+                     c->topo_spheres, c->topo_tris, c->n_spheres, c->n_tris);
+  int32_t rc = commit_tables(c);
+  if (rc != PTB_OK) return rc;
+  const size_t n = c->n_prims;
+  if (n == 0) {
+    c->committed = true;
+    c->stats.build_ms = 0.0;
+    return PTB_OK;
+  }
+  cudaStream_t st = c->stream;
+  // the full commit of the same counts reserved every one of these (grow-only): no allocation happens here
+  DevBuf &sbmin = c->scratch[0], &sbmax = c->scratch[1], &nbmin = c->scratch[9], &nbmax = c->scratch[10], &flags = c->scratch[11],
+         &d_light_prims = c->scratch[12], &d_light_out = c->scratch[14], &d_qframe = c->scratch[15];
+  PTB_CUDA_TRY(c, sbmin.reserve(n * 16));
+  PTB_CUDA_TRY(c, sbmax.reserve(n * 16));
+  const uint32_t n32 = (uint32_t)n, ns32 = (uint32_t)c->n_spheres;
+  const int T = 256;
+  const uint32_t gn = (n32 + T - 1) / T;
+  PTB_CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
+  PTB_CUDA_TRY(c, cudaMemsetAsync(d_light_out.p, 0, 8, st));
+  k_collect_lights<<<gn, T, 0, st>>>(c->d_raw_spheres.as<ptb_sphere>(), ns32, c->d_raw_tris.as<ptb_triangle>(), n32,
+                                     c->d_materials.as<DevMaterial>(), (uint32_t)c->materials.size(), d_light_out.as<uint32_t>(),
+                                     d_light_prims.as<uint32_t>());
+  if (n > 1) PTB_CUDA_TRY(c, cudaMemsetAsync(flags.p, 0, c->n_nodes * 4, st));
+  k_refit_slots<<<gn, T, 0, st>>>(c->d_raw_spheres.as<ptb_sphere>(), ns32, c->d_raw_tris.as<ptb_triangle>(), n32,
+                                  c->d_slot_prim.as<uint32_t>(), c->d_leaf_parent.as<uint32_t>(), c->d_materials.as<DevMaterial>(),
+                                  (uint32_t)c->materials.size(), c->d_geom.as<float4>(), c->d_normals.as<float4>(),
+                                  c->d_slot_mat.as<uint32_t>(), sbmin.as<float4>(), sbmax.as<float4>(), c->d_nodes.as<BvhNode>(),
+                                  nbmin.as<float4>(), nbmax.as<float4>(), flags.as<uint32_t>());
+  c->stats.kernel_launches += 2;
+  if (n == 1) {  // slot 0 holds primitive 0: the slot-ordered box is also the original-order one k_single_node reads
+    k_single_node<<<1, 1, 0, st>>>(c->d_slot_prim.as<uint32_t>(), ns32, sbmin.as<float4>(), sbmax.as<float4>(), c->d_nodes.as<BvhNode>());
+    c->stats.kernel_launches += 1;
+  }
+  float h_qframe[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  if (PTB_QNODES) {  // the grid follows the root box
+    k_qframe<<<1, 1, 0, st>>>(c->d_nodes.as<BvhNode>(), d_qframe.as<float>());
+    k_quantise_nodes<<<((uint32_t)c->n_nodes + T - 1) / T, T, 0, st>>>(c->d_nodes.as<BvhNode>(), (uint32_t)c->n_nodes, d_qframe.as<float>(),
+                                                                     c->d_qnodes.as<uint4>());
+    PTB_CUDA_TRY(c, cudaMemcpyAsync(h_qframe, d_qframe.p, sizeof h_qframe, cudaMemcpyDeviceToHost, st));
+    c->stats.kernel_launches += 2;
+  }
+  uint32_t nl = 0;
+  rc = light_list(c, ns32, &nl);
+  if (rc != PTB_OK) return rc;
+  PTB_CUDA_TRY(c, cudaEventRecord(c->ev_b, st));
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(st));
+  PTB_CUDA_TRY(c, cudaGetLastError());
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev_a, c->ev_b);
+  c->stats.build_ms = ms;
+  if (PTB_QNODES)
+    for (int k = 0; k < 3; ++k) { c->dev.q_min[k] = h_qframe[k]; c->dev.q_step[k] = h_qframe[3 + k]; }
+  c->dev.lights = c->d_lights.as<uint32_t>();
+  c->dev.n_lights = nl;
+  c->committed = true;
+  return PTB_OK;
+}
+
+int32_t build_scene(Ctx* c, uint32_t build_flags) {
+  if (build_flags & PTB_BUILD_REFIT) return refit_scene(c, build_flags);
+  c->refittable = false;  // from here on the kept topology is being replaced
   {
-    int32_t rc = build_sky(c);
+    int32_t rc = commit_tables(c);
     if (rc != PTB_OK) return rc;
   }
+  const size_t ns = c->n_spheres, nt = c->n_tris;
+  const size_t n = ns + nt;
+  cudaStream_t st = c->stream;
 
   c->n_prims = n;
   c->n_nodes = n == 0 ? 0 : (n == 1 ? 1 : n - 1);
@@ -633,6 +879,9 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   c->wide = false;
   if (n == 0) {
     c->committed = true;
+    c->refittable = true;
+    c->topo_spheres = ns;
+    c->topo_tris = nt;
     c->stats.build_ms = 0.0;
     return PTB_OK;
   }
@@ -641,7 +890,7 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   // and only ever grow: a re-commit of a same-sized scene performs no cudaMalloc / cudaFree at all.
   DevBuf &raw_spheres = c->d_raw_spheres, &raw_tris = c->d_raw_tris;
   DevBuf &bmin = c->scratch[0], &bmax = c->scratch[1], &bounds = c->scratch[2], &keys_a = c->scratch[3], &keys_b = c->scratch[4],
-         &vals_a = c->scratch[5], &vals_b = c->scratch[6], &hist = c->scratch[7], &leaf_parent = c->scratch[8],
+         &vals_a = c->scratch[5], &vals_b = c->scratch[6], &hist = c->scratch[7], &leaf_parent = c->d_leaf_parent,
          &nbmin = c->scratch[9], &nbmax = c->scratch[10], &flags = c->scratch[11], &prim_slot = c->d_prim_slot,
          &d_light_prims = c->scratch[12], &d_light_tmp = c->scratch[13], &d_light_out = c->scratch[14], &d_qframe = c->scratch[15];
   const uint32_t n32 = (uint32_t)n, ns32 = (uint32_t)ns, nt32 = (uint32_t)nt;
@@ -701,7 +950,6 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   const uint32_t gn = (n32 + T - 1) / T;
   PTB_CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
   // lights + material-index validation (device), then the light ids are put in ORIGINAL primitive order (deterministic)
-  uint32_t h_light_out[2] = {0u, 0u};
   PTB_CUDA_TRY(c, cudaMemsetAsync(d_light_out.p, 0, 8, st));
   k_collect_lights<<<gn, T, 0, st>>>(raw_spheres.as<ptb_sphere>(), ns32, raw_tris.as<ptb_triangle>(), n32,
                                      c->d_materials.as<DevMaterial>(), (uint32_t)c->materials.size(), d_light_out.as<uint32_t>(),
@@ -766,22 +1014,10 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   // keep the sorted keys / ids for ptb_bvh_export and the traversal's tie-break
   PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_morton.p, ka, n * 4, cudaMemcpyDeviceToDevice, st));
   PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_slot_prim.p, slot_order, n * 4, cudaMemcpyDeviceToDevice, st));
-  // light list: count + validation flag back to the host (8 bytes), ids sorted with the same radix passes
-  PTB_CUDA_TRY(c, cudaMemcpyAsync(h_light_out, d_light_out.p, 8, cudaMemcpyDeviceToHost, st));
-  PTB_CUDA_TRY(c, cudaStreamSynchronize(st));
-  if (h_light_out[1]) return set_error(c, PTB_ERR_INVALID, "primitive material index out of range");
-  const uint32_t nl = h_light_out[0];
-  if (nl) {
-    PTB_CUDA_TRY(c, c->d_lights.reserve((size_t)nl * 4));
-    uint32_t *la = d_light_prims.as<uint32_t>(), *lb = d_light_tmp.as<uint32_t>();
-    if (nl > 1) {
-      // nl <= n: the histogram scratch is large enough
-      // values ride along unused: keys double as values (keys_b / vals_b are free again)
-      uint32_t *lva = keys_b.as<uint32_t>(), *lvb = vals_b.as<uint32_t>();
-      radix_sort_pairs(c, la, lva, lb, lvb, nl, 4, hist.as<uint32_t>());
-    }
-    k_light_slots<<<(nl + T - 1) / T, T, 0, st>>>(la, nl, ns32, prim_slot.as<uint32_t>(), c->d_lights.as<uint32_t>());
-    c->stats.kernel_launches += 1;
+  uint32_t nl = 0;
+  {
+    const int32_t rcl = light_list(c, ns32, &nl);
+    if (rcl != PTB_OK) return rcl;
   }
   PTB_CUDA_TRY(c, cudaEventRecord(c->ev_b, st));
   PTB_CUDA_TRY(c, cudaStreamSynchronize(st));
@@ -804,6 +1040,9 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   c->dev.lights = c->d_lights.as<uint32_t>();
   c->dev.n_lights = nl;
   c->committed = true;
+  c->refittable = true;
+  c->topo_spheres = ns;
+  c->topo_tris = nt;
   return PTB_OK;
 }
 

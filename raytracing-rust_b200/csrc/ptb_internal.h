@@ -108,6 +108,11 @@ struct Ctx {
   // device scene
   DevScene dev{};
   DevBuf d_prim_slot;  // original primitive id -> slot (k_gather; valid until the next commit: lights, visibility API)
+  DevBuf d_leaf_parent;  // slot -> parent node of the binary tree (k_hierarchy / SAH build; the refit climbs from it)
+  // The binary tree of the last full commit can be refitted (PTB_BUILD_REFIT): set when a full commit succeeds, cleared
+  // when one starts. Its topology (d_nodes links, d_leaf_parent, d_slot_prim) belongs to these primitive counts.
+  bool refittable = false;
+  size_t topo_spheres = 0, topo_tris = 0;
   DevBuf d_geom, d_normals, d_slot_prim, d_slot_mat, d_nodes, d_qnodes, d_cw_nodes, d_prim_sorted, d_morton, d_materials, d_textures, d_tex_data, d_lights;
   DevBuf d_sky_ycdf, d_sky_ypdf, d_sky_xcdf, d_sky_xpdf;
   uint64_t n_prims = 0, n_nodes = 0, n_cw_nodes = 0;
@@ -159,6 +164,8 @@ int32_t check_cuda(Ctx* c, cudaError_t e, const char* what);
 
 // lbvh_build.cu — uploads the host scene and builds the device LBVH (K2..K6)
 int32_t build_scene(Ctx* c, uint32_t flags);
+// SAH cost of the committed binary tree (ptb_bvh_sah_cost)
+int32_t tree_sah_cost(Ctx* c, double* cost);
 // cwbvh_build.cu — collapses the LBVH into the compressed 8-wide tree; leaves the final primitive order in
 // `final_prim` (final slot -> original primitive id, n words, device)
 struct CwBuildInputs {

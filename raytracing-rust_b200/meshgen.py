@@ -2,6 +2,7 @@
 
   c3_scene()          1 000 000 triangles: 800 000-triangle Lambertian terrain + 200 000-triangle dielectric UV sphere,
                       Lerp sky as scenes/rtweekend1.ssml, 16:9 camera                         (SURVEY.md §8d "C3")
+  c3_deform()         one frame of an animated C3: terrain wave + glass sphere pushed into the terrain (same counts)
   heightfield_scene() R x C quads in [-1,1]^2 x [-0.2,0.2]; 2500 x 2000 -> 10 000 000 triangles      ("C5")
   philox_rays()       incoherent rays from Philox4x32-10 (seed 0x5EED, counter = ray index): origin uniform in the
                       ball of radius 2 about the mesh centre, direction uniform on the sphere
@@ -9,6 +10,8 @@
 All arithmetic is float32 numpy; the arrays ARE the input (oracle and device receive identical bytes).
 """
 from __future__ import annotations
+
+import copy
 
 import numpy as np
 
@@ -94,6 +97,24 @@ def c3_scene(scale: float = 1.0) -> HostScene:
     tri["p"][len(tp):], tri["n"][len(tp):], tri["material"][len(tp):] = sp_, sn, 1
     s.triangles = tri
     s.set_camera((0.0, -1.5, 1.6), (0.0, 4.0, 0.7), (0.0, 0.0, 1.0), 60.0, 16.0 / 9.0, 0.0, 1.0)
+    return s
+
+
+C3_GLASS_RADIUS = 0.8
+
+
+def c3_deform(scene: HostScene, wave: float, shift: float) -> HostScene:
+    """A frame of an animated C3 (same counts, same order, for PTB_BUILD_REFIT): every terrain vertex's height is scaled by
+    1 + wave * sin(0.7 x + 0.4 y), and the glass sphere is moved by `shift` radii along (0.6, 0, -0.8), into the terrain.
+    The function of a vertex is a function of its position, so shared vertices stay shared; normals are kept."""
+    s = copy.deepcopy(scene)
+    tri = s.triangles
+    glass = tri["material"] == 1
+    p = tri["p"][~glass]
+    x, y = p[..., 0], p[..., 1]
+    p[..., 2] = p[..., 2] * (F(1) + F(wave) * np.sin(F(0.7) * x + F(0.4) * y))
+    tri["p"][~glass] = p
+    tri["p"][glass] = tri["p"][glass] + (F(shift) * F(C3_GLASS_RADIUS) * np.array([0.6, 0.0, -0.8], F)).astype(F)
     return s
 
 
