@@ -10,11 +10,24 @@ type Prim<'a> = AllPrimitives<'a, Mat<'a>>;
 
 fn v(p: Vec3) -> ptb_vec3 { ptb_vec3 { x: p.x, y: p.y, z: p.z } }
 
-pub struct CudaScene { ctx: *mut ptb_ctx, mat_ids: HashMap<*const Mat, u32> }
+/// `mesh_base`: for a scene made by `new_indexed`, where each interned MeshData starts in the vertex / normal pools.
+pub struct CudaScene { ctx: *mut ptb_ctx, mat_ids: HashMap<*const Mat, u32>, mesh_base: HashMap<*const MeshData, (usize, usize)> }
 
 impl CudaScene {
     /// `primitives` in loader order (spheres first, then mesh triangles: loader/src/lib.rs:234-240).
     pub fn new(primitives: &[Prim], camera: &SimpleCamera, sky_tex: &Tex, sampler_res: (usize, usize), device: i32) -> Result<Self, String> {
+        Self::create(primitives, camera, sky_tex, sampler_res, device, false)
+    }
+
+    /// As `new`, but the triangles go up as an indexed mesh (ptb_scene_set_mesh) and are expanded on the device: every
+    /// MeshData is interned by address into one vertex pool and one normal pool (its indices offset by where it starts), a
+    /// Prim::Triangle's corners are appended as fresh entries. About half the upload of `new` for grid-like meshes, and
+    /// animation can move vertices with `update_mesh_vertices` instead of re-sending whole triangles.
+    pub fn new_indexed(primitives: &[Prim], camera: &SimpleCamera, sky_tex: &Tex, sampler_res: (usize, usize), device: i32) -> Result<Self, String> {
+        Self::create(primitives, camera, sky_tex, sampler_res, device, true)
+    }
+
+    fn create(primitives: &[Prim], camera: &SimpleCamera, sky_tex: &Tex, sampler_res: (usize, usize), device: i32, indexed: bool) -> Result<Self, String> {
         let mut ctx = ptr::null_mut();
         check(ptr::null_mut(), unsafe { ptb_create(device, &mut ctx) })?;
         // intern textures / materials by address: the arena (crates/region) keeps them alive and unique
@@ -29,16 +42,35 @@ impl CudaScene {
         });
         let sky_id = tex_id(sky_tex);
         let (mut spheres, mut tris) = (Vec::new(), Vec::new());
+        // indexed: the vertex / normal pools and the mesh triangles that index them
+        let (mut verts, mut nrms, mut mtris) = (Vec::<ptb_vec3>::new(), Vec::<ptb_vec3>::new(), Vec::<ptb_mesh_triangle>::new());
+        let mut mesh_base = HashMap::<*const MeshData, (usize, usize)>::new();
         for p in primitives {
             let m = match p { Prim::Sphere(s) => s.material, Prim::Triangle(t) => t.material, Prim::MeshTriangle(t) => t.material };
             let mid = *mat_ids.entry(m as *const _).or_insert_with(|| { mats.push(flatten_material(m, &mut tex_id)); mats.len() as u32 - 1 });
             match p {
                 Prim::Sphere(s) => spheres.push(ptb_sphere { center: v(s.center), radius: s.radius, material: mid }),
+                Prim::Triangle(t) if indexed => {
+                    let (bp, bn) = (verts.len() as u32, nrms.len() as u32);
+                    verts.extend(t.points.map(v));
+                    nrms.extend(t.normals.map(v));
+                    mtris.push(ptb_mesh_triangle { p: [bp, bp + 1, bp + 2], n: [bn, bn + 1, bn + 2], material: mid });
+                }
+                Prim::MeshTriangle(t) if indexed => {
+                    let (bp, bn) = *mesh_base.entry(t.mesh as *const _).or_insert_with(|| {
+                        let b = (verts.len(), nrms.len());
+                        verts.extend(t.mesh.vertices.iter().map(|&p| v(p)));
+                        nrms.extend(t.mesh.normals.iter().map(|&p| v(p)));
+                        b
+                    });
+                    mtris.push(ptb_mesh_triangle { p: t.point_indices.map(|i| (bp + i) as u32), n: t.normal_indices.map(|i| (bn + i) as u32), material: mid });
+                }
                 Prim::Triangle(t) => tris.push(ptb_triangle { p: t.points.map(v), n: t.normals.map(v), material: mid }),
                 Prim::MeshTriangle(t) => tris.push(ptb_triangle {
                     p: t.point_indices.map(|i| v(t.mesh.vertices[i])), n: t.normal_indices.map(|i| v(t.mesh.normals[i])), material: mid }),
             }
         }
+        if verts.len() > u32::MAX as usize || nrms.len() > u32::MAX as usize { return Err("new_indexed: more than 2^32 - 1 vertices or normals".into()); }
         let cam = ptb_camera { origin: v(camera.origin), lower_left: v(camera.lower_left), horizontal: v(camera.horizontal), vertical: v(camera.vertical) };
         let sky = ptb_sky { texture: sky_id, sampler_res_x: sampler_res.0 as u32, sampler_res_y: sampler_res.1 as u32 };
         unsafe {
@@ -48,12 +80,16 @@ impl CudaScene {
             }
             check(ctx, ptb_scene_set_materials(ctx, mats.as_ptr(), mats.len()))?;
             check(ctx, ptb_scene_set_spheres(ctx, spheres.as_ptr(), spheres.len()))?;
-            check(ctx, ptb_scene_set_triangles(ctx, tris.as_ptr(), tris.len()))?;
+            if indexed {
+                check(ctx, ptb_scene_set_mesh(ctx, verts.as_ptr(), verts.len(), nrms.as_ptr(), nrms.len(), mtris.as_ptr(), mtris.len()))?;
+            } else {
+                check(ctx, ptb_scene_set_triangles(ctx, tris.as_ptr(), tris.len()))?;
+            }
             check(ctx, ptb_scene_set_camera(ctx, &cam))?;
             check(ctx, ptb_scene_set_sky(ctx, &sky))?;
             check(ctx, ptb_scene_commit(ctx, 0))?; // Bvh::new
         }
-        Ok(Self { ctx, mat_ids })
+        Ok(Self { ctx, mat_ids, mesh_base })
     }
 
     /// Scene::render (src/scene.rs:35-42) for the cuda backend: the accumulator comes back as the running-mean image the
@@ -87,6 +123,15 @@ impl CudaScene {
             out.push(ptb_triangle { p: pts, n: nrm, material });
         }
         check(self.ctx, unsafe { ptb_scene_update_triangles(self.ctx, first, out.as_ptr(), out.len()) })
+    }
+
+    /// Animation of a scene made by `new_indexed`: overwrite the vertices of `mesh` (one of the scene's MeshData) with
+    /// `positions` (as many as the mesh has). Call `refit` afterwards; the device expands the moved mesh at the commit.
+    pub fn update_mesh_vertices(&self, mesh: &MeshData, positions: &[Vec3]) -> Result<(), String> {
+        let &(base, _) = self.mesh_base.get(&(mesh as *const _)).ok_or("update_mesh_vertices: not a mesh of this indexed scene")?;
+        if positions.len() != mesh.vertices.len() { return Err("update_mesh_vertices: one position per vertex of the mesh".into()); }
+        let out: Vec<ptb_vec3> = positions.iter().map(|&p| v(p)).collect();
+        check(self.ctx, unsafe { ptb_scene_update_mesh_vertices(self.ctx, base, out.as_ptr(), out.len()) })
     }
 
     /// Commit the updates keeping the tree (PTB_BUILD_REFIT); returns the refitted tree's SAH cost, which the caller

@@ -11,6 +11,8 @@ pub const PTB_METHOD_MIS: u32 = 1;
 #[repr(C)] #[derive(Clone, Copy, Default)] pub struct ptb_vec3 { pub x: f32, pub y: f32, pub z: f32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_sphere { pub center: ptb_vec3, pub radius: f32, pub material: u32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_triangle { pub p: [ptb_vec3; 3], pub n: [ptb_vec3; 3], pub material: u32 }
+/// MeshTriangle (implementations/primitives/triangle.rs:30-36): indices into the scene's vertex / normal arrays (28 B)
+#[repr(C)] #[derive(Clone, Copy)] pub struct ptb_mesh_triangle { pub p: [u32; 3], pub n: [u32; 3], pub material: u32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_material { pub kind: u32, pub texture: u32, pub param: f32, pub ior: ptb_vec3, pub metallic: f32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_texture { pub kind: u32, pub a: ptb_vec3, pub b: ptb_vec3 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_camera { pub origin: ptb_vec3, pub lower_left: ptb_vec3, pub horizontal: ptb_vec3, pub vertical: ptb_vec3 }
@@ -64,6 +66,14 @@ extern "C" {
     pub fn ptb_scene_update_triangles(ctx: *mut ptb_ctx, first: usize, p: *const ptb_triangle, n: usize) -> i32;
     pub fn ptb_scene_update_spheres_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
     pub fn ptb_scene_update_triangles_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
+    pub fn ptb_scene_set_mesh(ctx: *mut ptb_ctx, vertices: *const ptb_vec3, n_vertices: usize, normals: *const ptb_vec3, n_normals: usize,
+                              triangles: *const ptb_mesh_triangle, n_triangles: usize) -> i32;
+    pub fn ptb_scene_update_mesh_vertices(ctx: *mut ptb_ctx, first: usize, p: *const ptb_vec3, n: usize) -> i32;
+    pub fn ptb_scene_update_mesh_normals(ctx: *mut ptb_ctx, first: usize, p: *const ptb_vec3, n: usize) -> i32;
+    pub fn ptb_scene_update_mesh_triangles(ctx: *mut ptb_ctx, first: usize, p: *const ptb_mesh_triangle, n: usize) -> i32;
+    pub fn ptb_scene_update_mesh_vertices_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
+    pub fn ptb_scene_update_mesh_normals_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
+    pub fn ptb_scene_update_mesh_triangles_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
     pub fn ptb_scene_commit(ctx: *mut ptb_ctx, build_flags: u32) -> i32;
     pub fn ptb_bvh_sah_cost(ctx: *mut ptb_ctx, cost: *mut f64) -> i32;
     pub fn ptb_bvh_export_quantised(ctx: *mut ptb_ctx, frame: *mut f32, nodes32: *mut c_void) -> i32;

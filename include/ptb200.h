@@ -252,6 +252,40 @@ int32_t ptb_scene_update_triangles(ptb_ctx* ctx, size_t first, const ptb_triangl
  * synchronise first) and must stay valid until the next commit or ptb_synchronize. */
 int32_t ptb_scene_update_spheres_device(ptb_ctx* ctx, size_t first, const void* d_spheres, size_t n);
 int32_t ptb_scene_update_triangles_device(ptb_ctx* ctx, size_t first, const void* d_triangles, size_t n);
+
+/* Indexed triangle meshes. implementations/primitives/triangle.rs:30-36 MeshTriangle: indices into the scene's vertex and
+ * normal arrays (the reference's MeshData) plus a material. 28 bytes. */
+typedef struct ptb_mesh_triangle {
+  uint32_t p[3];     /* vertex indices */
+  uint32_t n[3];     /* normal indices */
+  uint32_t material;
+} ptb_mesh_triangle;
+/* The scene's triangles come from one source at a time: the flat array of ptb_scene_set_triangles or an indexed mesh.
+ * ptb_scene_set_mesh replaces the triangle array with the mesh (host pointers, copied before returning): triangle id i is
+ * mesh triangle i, and primitive ids are still spheres first, then triangles. At commit (full or PTB_BUILD_REFIT) the
+ * device expands the mesh into the same ptb_triangle records the flat path uploads, when the mesh changed since the last
+ * successful commit; the expansion counts in ptb_stats.build_ms and kernel_launches. A mesh scene therefore builds, traverses
+ * and renders bit for bit as the flat scene it expands to. ptb_scene_set_triangles puts the scene back in flat mode and
+ * drops the mesh.
+ *   - Indices are checked on the device at commit: a vertex index >= n_vertices or a normal index >= n_normals fails the
+ *     commit with PTB_ERR_INVALID and a message naming the first such triangle (the expansion never reads out of range).
+ *     Fix it with ptb_scene_update_mesh_triangles and commit again.
+ *   - More than 2^32 - 1 vertices or normals: PTB_ERR_INVALID.
+ *   - PTB_BUILD_REFIT keeps the tree while the sphere and triangle counts are those of the last full commit; the vertex and
+ *     normal counts may differ. */
+int32_t ptb_scene_set_mesh(ptb_ctx* ctx, const ptb_vec3* vertices, size_t n_vertices, const ptb_vec3* normals, size_t n_normals,
+                           const ptb_mesh_triangle* triangles, size_t n_triangles);
+/* Overwrite entries [first, first + n) of the mesh's vertex, normal or triangle array in place, with the range and pointer
+ * rules of ptb_scene_update_* (host variants copy before returning; _device variants copy device to device on the
+ * context's stream without synchronising). They need a mesh scene: on a flat scene they fail with PTB_ERR_INVALID, and so
+ * does ptb_scene_update_triangles(_device) on a mesh scene (the next expansion would overwrite it). The usual animation
+ * loop moves vertices only: ptb_scene_update_mesh_vertices -> ptb_scene_commit(PTB_BUILD_REFIT). */
+int32_t ptb_scene_update_mesh_vertices(ptb_ctx* ctx, size_t first, const ptb_vec3* vertices, size_t n);
+int32_t ptb_scene_update_mesh_normals(ptb_ctx* ctx, size_t first, const ptb_vec3* normals, size_t n);
+int32_t ptb_scene_update_mesh_triangles(ptb_ctx* ctx, size_t first, const ptb_mesh_triangle* triangles, size_t n);
+int32_t ptb_scene_update_mesh_vertices_device(ptb_ctx* ctx, size_t first, const void* d_vertices, size_t n);
+int32_t ptb_scene_update_mesh_normals_device(ptb_ctx* ctx, size_t first, const void* d_normals, size_t n);
+int32_t ptb_scene_update_mesh_triangles_device(ptb_ctx* ctx, size_t first, const void* d_triangles, size_t n);
 /* SAH cost of the committed binary tree in the reference's cost model (traversal 0.125, intersection 1, split.rs:161-176):
  * (0.125 * sum over inner nodes of SA(node) + sum over leaves of SA(leaf box)) / SA(root), SA = 2 (xy + yz + zx) of the f32
  * box evaluated in f64, root box = union of node 0's two child boxes. 1 primitive: 1.125; 0 primitives or a root of zero

@@ -33,6 +33,7 @@ BUILD_DEFAULT, BUILD_BINARY, BUILD_WIDE, BUILD_SAH, BUILD_REFIT = 0, 1, 2, 4, 8
 # numpy mirrors of the POD structs (sizes asserted against the header's layout in tests/test_abi.py)
 sphere_dtype = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4")])
 triangle_dtype = np.dtype([("p", "<f4", (3, 3)), ("n", "<f4", (3, 3)), ("material", "<u4")])
+mesh_triangle_dtype = np.dtype([("p", "<u4", 3), ("n", "<u4", 3), ("material", "<u4")])  # indices into vertices / normals
 material_dtype = np.dtype([("kind", "<u4"), ("texture", "<u4"), ("param", "<f4"), ("ior", "<f4", 3), ("metallic", "<f4")])
 texture_dtype = np.dtype([("kind", "<u4"), ("a", "<f4", 3), ("b", "<f4", 3)])
 camera_dtype = np.dtype([("origin", "<f4", 3), ("lower_left", "<f4", 3), ("horizontal", "<f4", 3), ("vertical", "<f4", 3)])
@@ -105,6 +106,13 @@ SYMBOLS = [
     ("ptb_scene_update_triangles", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
     ("ptb_scene_update_spheres_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
     ("ptb_scene_update_triangles_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_set_mesh", C.c_int32, [_P, _P, C.c_size_t, _P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_mesh_vertices", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_mesh_normals", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_mesh_triangles", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_mesh_vertices_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_mesh_normals_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_mesh_triangles_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
     ("ptb_scene_commit", C.c_int32, [_P, C.c_uint32]),
     ("ptb_bvh_sah_cost", C.c_int32, [_P, C.POINTER(C.c_double)]),
     ("ptb_bvh_info", C.c_int32, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),

@@ -16,7 +16,7 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import _lib as L
-from .scene import HostScene
+from .scene import HostScene, IndexedMesh
 
 
 def _check(ctx_handle, rc: int):
@@ -84,15 +84,19 @@ class Context:
     def synchronize(self):
         _check(self._h, L.lib.ptb_synchronize(self._h))
 
-    def upload(self, s: HostScene):
-        """ptb_scene_set_* for every array (host -> library copy)."""
+    def upload(self, s: HostScene, mesh: IndexedMesh | None = None):
+        """ptb_scene_set_* for every array (host -> library copy). With `mesh`, the scene's triangles are that indexed mesh
+        (set_mesh) and s.triangles is not uploaded."""
         h = self._h
         _check(h, L.lib.ptb_scene_set_textures(h, L.ptr(s.textures), len(s.textures)))
         for i, (w, hh, words) in s.texture_data.items():
             _check(h, L.lib.ptb_scene_set_texture_data(h, i, w, hh, L.ptr(words), words.size))
         _check(h, L.lib.ptb_scene_set_materials(h, L.ptr(s.materials), len(s.materials)))
         _check(h, L.lib.ptb_scene_set_spheres(h, L.ptr(s.spheres), len(s.spheres)))
-        _check(h, L.lib.ptb_scene_set_triangles(h, L.ptr(s.triangles), len(s.triangles)))
+        if mesh is None:
+            _check(h, L.lib.ptb_scene_set_triangles(h, L.ptr(s.triangles), len(s.triangles)))
+        else:
+            self.set_mesh(mesh)
         _check(h, L.lib.ptb_scene_set_camera(h, L.ptr(s.camera)))
         _check(h, L.lib.ptb_scene_set_sky(h, L.ptr(s.sky)))
 
@@ -122,6 +126,38 @@ class Context:
     def update_triangles_device(self, first: int, d_ptr: int, n: int):
         """Same from device memory (n records of triangle_dtype's layout, 76 bytes each)."""
         _check(self._h, L.lib.ptb_scene_update_triangles_device(self._h, first, C.c_void_p(d_ptr), n))
+
+    # ---- indexed meshes: the device expands them into the triangle records at commit
+    def set_mesh(self, mesh: IndexedMesh):
+        """The scene's triangles become `mesh` (triangle id i = mesh triangle i); set_triangles goes back to flat ones."""
+        v, n, t = mesh.vertices, mesh.normals, mesh.triangles
+        _check(self._h, L.lib.ptb_scene_set_mesh(self._h, L.ptr(v), len(v), L.ptr(n), len(n), L.ptr(t), len(t)))
+
+    def update_mesh_vertices(self, first: int, vertices: np.ndarray):
+        """Overwrite mesh vertices [first, first + len(vertices)) ((k, 3) float32); then commit, e.g. with L.BUILD_REFIT."""
+        a = np.ascontiguousarray(vertices, np.float32).reshape(-1, 3)
+        _check(self._h, L.lib.ptb_scene_update_mesh_vertices(self._h, first, L.ptr(a), len(a)))
+
+    def update_mesh_normals(self, first: int, normals: np.ndarray):
+        a = np.ascontiguousarray(normals, np.float32).reshape(-1, 3)
+        _check(self._h, L.lib.ptb_scene_update_mesh_normals(self._h, first, L.ptr(a), len(a)))
+
+    def update_mesh_triangles(self, first: int, triangles: np.ndarray):
+        """Overwrite mesh triangles [first, first + len(triangles)) (mesh_triangle_dtype)."""
+        a = np.ascontiguousarray(triangles, L.mesh_triangle_dtype)
+        _check(self._h, L.lib.ptb_scene_update_mesh_triangles(self._h, first, L.ptr(a), len(a)))
+
+    def update_mesh_vertices_device(self, first: int, d_ptr: int, n: int):
+        """Same from device memory (n x 12 bytes), enqueued on the context's stream without a synchronise (as
+        update_triangles_device)."""
+        _check(self._h, L.lib.ptb_scene_update_mesh_vertices_device(self._h, first, C.c_void_p(d_ptr), n))
+
+    def update_mesh_normals_device(self, first: int, d_ptr: int, n: int):
+        _check(self._h, L.lib.ptb_scene_update_mesh_normals_device(self._h, first, C.c_void_p(d_ptr), n))
+
+    def update_mesh_triangles_device(self, first: int, d_ptr: int, n: int):
+        """n records of mesh_triangle_dtype's layout (28 bytes each)."""
+        _check(self._h, L.lib.ptb_scene_update_mesh_triangles_device(self._h, first, C.c_void_p(d_ptr), n))
 
     def bvh_sah_cost(self) -> float:
         """SAH cost of the committed binary tree (traversal 0.125, intersection 1; normalised by the root's area). Compare

@@ -176,10 +176,42 @@ int32_t ptb_scene_set_triangles(ptb_ctx* ctx, const ptb_triangle* p, size_t n) {
   if (n && !p) return set_error(c, PTB_ERR_INVALID, "null triangles");
   c->committed = false;
   c->n_tris = 0;
+  if (c->mesh) {  // flat mode: the mesh is dropped
+    PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));  // a device update may still read into its buffers
+    c->mesh = c->mesh_dirty = false;
+    c->n_mesh_vertices = c->n_mesh_normals = 0;
+    c->d_mesh_vertices.release();
+    c->d_mesh_normals.release();
+    c->d_mesh_tris.release();
+  }
   PTB_CUDA_TRY(c, c->d_raw_tris.reserve(n * sizeof(ptb_triangle)));
   if (n) PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_raw_tris.p, p, n * sizeof(ptb_triangle), cudaMemcpyHostToDevice, c->stream));
   PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   c->n_tris = n;
+  return PTB_OK;
+}
+int32_t ptb_scene_set_mesh(ptb_ctx* ctx, const ptb_vec3* v, size_t nv, const ptb_vec3* nrm, size_t nn, const ptb_mesh_triangle* t,
+                           size_t nt) {
+  CTX_OR_FAIL(ctx);
+  if ((nv && !v) || (nn && !nrm) || (nt && !t)) return set_error(c, PTB_ERR_INVALID, "null mesh array");
+  if (nv > 0xFFFFFFFFull || nn > 0xFFFFFFFFull)
+    return set_error(c, PTB_ERR_INVALID, "a mesh holds at most 2^32 - 1 vertices and normals (%zu vertices, %zu normals)", nv, nn);
+  c->committed = false;
+  c->n_tris = 0;
+  c->mesh = false;
+  c->n_mesh_vertices = c->n_mesh_normals = 0;
+  PTB_CUDA_TRY(c, c->d_mesh_vertices.reserve(nv * sizeof(ptb_vec3)));
+  PTB_CUDA_TRY(c, c->d_mesh_normals.reserve(nn * sizeof(ptb_vec3)));
+  PTB_CUDA_TRY(c, c->d_mesh_tris.reserve(nt * sizeof(ptb_mesh_triangle)));
+  PTB_CUDA_TRY(c, c->d_raw_tris.reserve(nt * sizeof(ptb_triangle)));  // the expansion's output
+  if (nv) PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_mesh_vertices.p, v, nv * sizeof(ptb_vec3), cudaMemcpyHostToDevice, c->stream));
+  if (nn) PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_mesh_normals.p, nrm, nn * sizeof(ptb_vec3), cudaMemcpyHostToDevice, c->stream));
+  if (nt) PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_mesh_tris.p, t, nt * sizeof(ptb_mesh_triangle), cudaMemcpyHostToDevice, c->stream));
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  c->n_mesh_vertices = nv;
+  c->n_mesh_normals = nn;
+  c->n_tris = nt;
+  c->mesh = c->mesh_dirty = true;
   return PTB_OK;
 }
 // ptb_scene_update_*: primitives [first, first + n) of `raw` (count `have`, records of `rec` bytes) in place
@@ -198,8 +230,15 @@ int32_t ptb_scene_update_spheres(ptb_ctx* ctx, size_t first, const ptb_sphere* p
   CTX_OR_FAIL(ctx);
   return update_prims(c, c->d_raw_spheres, c->n_spheres, sizeof(ptb_sphere), first, p, n, cudaMemcpyHostToDevice, "spheres");
 }
+// the triangles of a mesh scene are the mesh's expansion: the next commit would overwrite a flat update
+#define FLAT_TRIANGLES_OR_FAIL(c)                                                                                        \
+  if ((c)->mesh)                                                                                                         \
+    return set_error(c, PTB_ERR_INVALID,                                                                                 \
+                     "the scene's triangles are an indexed mesh: update it with ptb_scene_update_mesh_* (or go back to " \
+                     "flat triangles with ptb_scene_set_triangles)")
 int32_t ptb_scene_update_triangles(ptb_ctx* ctx, size_t first, const ptb_triangle* p, size_t n) {
   CTX_OR_FAIL(ctx);
+  FLAT_TRIANGLES_OR_FAIL(c);
   return update_prims(c, c->d_raw_tris, c->n_tris, sizeof(ptb_triangle), first, p, n, cudaMemcpyHostToDevice, "triangles");
 }
 int32_t ptb_scene_update_spheres_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
@@ -208,7 +247,41 @@ int32_t ptb_scene_update_spheres_device(ptb_ctx* ctx, size_t first, const void* 
 }
 int32_t ptb_scene_update_triangles_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
   CTX_OR_FAIL(ctx);
+  FLAT_TRIANGLES_OR_FAIL(c);
   return update_prims(c, c->d_raw_tris, c->n_tris, sizeof(ptb_triangle), first, d_p, n, cudaMemcpyDeviceToDevice, "triangles");
+}
+// ptb_scene_update_mesh_*: update_prims on one of the mesh arrays, which the next commit expands again
+static int32_t update_mesh(Ctx* c, DevBuf& raw, size_t have, size_t rec, size_t first, const void* p, size_t n,
+                           cudaMemcpyKind kind, const char* what) {
+  if (!c->mesh)
+    return set_error(c, PTB_ERR_INVALID, "%s update: the scene's triangles are flat, not an indexed mesh (ptb_scene_set_mesh)", what);
+  const int32_t rc = update_prims(c, raw, have, rec, first, p, n, kind, what);
+  if (rc == PTB_OK && n) c->mesh_dirty = true;
+  return rc;
+}
+int32_t ptb_scene_update_mesh_vertices(ptb_ctx* ctx, size_t first, const ptb_vec3* p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_mesh(c, c->d_mesh_vertices, c->n_mesh_vertices, sizeof(ptb_vec3), first, p, n, cudaMemcpyHostToDevice, "mesh vertices");
+}
+int32_t ptb_scene_update_mesh_normals(ptb_ctx* ctx, size_t first, const ptb_vec3* p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_mesh(c, c->d_mesh_normals, c->n_mesh_normals, sizeof(ptb_vec3), first, p, n, cudaMemcpyHostToDevice, "mesh normals");
+}
+int32_t ptb_scene_update_mesh_triangles(ptb_ctx* ctx, size_t first, const ptb_mesh_triangle* p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_mesh(c, c->d_mesh_tris, c->n_tris, sizeof(ptb_mesh_triangle), first, p, n, cudaMemcpyHostToDevice, "mesh triangles");
+}
+int32_t ptb_scene_update_mesh_vertices_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_mesh(c, c->d_mesh_vertices, c->n_mesh_vertices, sizeof(ptb_vec3), first, d_p, n, cudaMemcpyDeviceToDevice, "mesh vertices");
+}
+int32_t ptb_scene_update_mesh_normals_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_mesh(c, c->d_mesh_normals, c->n_mesh_normals, sizeof(ptb_vec3), first, d_p, n, cudaMemcpyDeviceToDevice, "mesh normals");
+}
+int32_t ptb_scene_update_mesh_triangles_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_mesh(c, c->d_mesh_tris, c->n_tris, sizeof(ptb_mesh_triangle), first, d_p, n, cudaMemcpyDeviceToDevice, "mesh triangles");
 }
 int32_t ptb_scene_set_materials(ptb_ctx* ctx, const ptb_material* p, size_t n) {
   CTX_OR_FAIL(ctx);

@@ -669,6 +669,69 @@ static int32_t build_sky(Ctx* c) {
   return PTB_OK;
 }
 
+// ------------------------------------------------------------------------------------------ indexed mesh expansion
+// ptb_scene_set_mesh: mesh triangle i becomes ptb_triangle record i of d_raw_tris, before anything else of the commit reads
+// that array. The words are copied, never computed on, so the records are bit-identical to a host-side gather. An index out
+// of range is not dereferenced: its corner becomes (0, 0, 0) and the commit fails through the word the material check uses
+// (out[1] |= 2 for a vertex index, 4 for a normal index; out[2] / out[3] = max of ~triangle, i.e. the first such triangle).
+constexpr uint32_t kExpandThreads = 256;
+constexpr uint32_t kMeshWords = sizeof(ptb_mesh_triangle) / 4, kTriWords = sizeof(ptb_triangle) / 4;  // 7, 19
+static_assert(sizeof(ptb_mesh_triangle) == 28 && sizeof(ptb_triangle) == 76, "record layouts");
+
+__device__ __forceinline__ void expand_record(const uint32_t* idx, uint32_t* rec, uint32_t tri, const uint32_t* __restrict__ vtx,
+                                              uint32_t nv, const uint32_t* __restrict__ nrm, uint32_t nn, uint32_t* out) {
+  bool bad_v = false, bad_n = false;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const uint32_t a = idx[k], b = idx[3 + k];
+    uint32_t p[3] = {0u, 0u, 0u}, q[3] = {0u, 0u, 0u};
+    if (a < nv) { p[0] = vtx[3 * (size_t)a]; p[1] = vtx[3 * (size_t)a + 1]; p[2] = vtx[3 * (size_t)a + 2]; }
+    else bad_v = true;
+    if (b < nn) { q[0] = nrm[3 * (size_t)b]; q[1] = nrm[3 * (size_t)b + 1]; q[2] = nrm[3 * (size_t)b + 2]; }
+    else bad_n = true;
+#pragma unroll
+    for (int w = 0; w < 3; ++w) {
+      rec[3 * k + w] = p[w];
+      rec[9 + 3 * k + w] = q[w];
+    }
+  }
+  rec[18] = idx[6];
+  if (bad_v) { atomicOr(out + 1, 2u); atomicMax(out + 2, ~tri); }
+  if (bad_n) { atomicOr(out + 1, 4u); atomicMax(out + 3, ~tri); }
+}
+__global__ void __launch_bounds__(kExpandThreads)
+k_expand_mesh(const uint32_t* __restrict__ vtx, uint32_t nv, const uint32_t* __restrict__ nrm, uint32_t nn,
+              const uint32_t* __restrict__ mesh_tris, uint32_t n_tris, uint32_t* __restrict__ tris, uint32_t* out) {
+  // A block reads its index records and writes its output records with 16-byte accesses through shared memory: 3.3x
+  // faster on B200 than 4-byte per-thread accesses to the 28- and 76-byte records (profiles/mesh_b200.md). A block's
+  // records start at 16-byte boundaries (256 x 28 and 256 x 76 bytes per block from cudaMalloc'd bases).
+  __shared__ __align__(16) uint32_t s_idx[kExpandThreads * kMeshWords];
+  __shared__ __align__(16) uint32_t s_rec[kExpandThreads * kTriWords];
+  const uint32_t first = blockIdx.x * kExpandThreads, count = min(kExpandThreads, n_tris - first);
+  const uint32_t in_words = count * kMeshWords, out_words = count * kTriWords;
+  const uint32_t* src = mesh_tris + (size_t)first * kMeshWords;
+  for (uint32_t q = threadIdx.x; q < in_words / 4; q += kExpandThreads)
+    reinterpret_cast<uint4*>(s_idx)[q] = __ldg(reinterpret_cast<const uint4*>(src) + q);
+  for (uint32_t w = (in_words & ~3u) + threadIdx.x; w < in_words; w += kExpandThreads) s_idx[w] = src[w];
+  __syncthreads();
+  if (threadIdx.x < count)  // odd word strides (7, 19): no bank conflicts
+    expand_record(s_idx + threadIdx.x * kMeshWords, s_rec + threadIdx.x * kTriWords, first + threadIdx.x, vtx, nv, nrm, nn, out);
+  __syncthreads();
+  uint32_t* dst = tris + (size_t)first * kTriWords;
+  for (uint32_t q = threadIdx.x; q < out_words / 4; q += kExpandThreads)
+    reinterpret_cast<uint4*>(dst)[q] = reinterpret_cast<const uint4*>(s_rec)[q];
+  for (uint32_t w = (out_words & ~3u) + threadIdx.x; w < out_words; w += kExpandThreads) dst[w] = s_rec[w];
+}
+// Enqueued after the memset of the light-list words and before k_collect_lights, in both commit paths.
+static void expand_mesh(Ctx* c, uint32_t* out) {
+  if (!c->mesh || !c->mesh_dirty || c->n_tris == 0) return;
+  const uint32_t nt = (uint32_t)c->n_tris;
+  k_expand_mesh<<<(nt + kExpandThreads - 1) / kExpandThreads, kExpandThreads, 0, c->stream>>>(
+      c->d_mesh_vertices.as<uint32_t>(), (uint32_t)c->n_mesh_vertices, c->d_mesh_normals.as<uint32_t>(), (uint32_t)c->n_mesh_normals,
+      c->d_mesh_tris.as<uint32_t>(), nt, c->d_raw_tris.as<uint32_t>(), out);
+  c->stats.kernel_launches += 1;
+}
+
 // ------------------------------------------------------------------------------------------ host: build
 // Material-index validation + light list, on the device: the host never walks the primitive arrays.
 // out[0] = number of lights, out[1] = 1 if some material index is out of range; list = light primitive ids (unordered).
@@ -761,15 +824,21 @@ static int32_t commit_tables(Ctx* c) {
   return build_sky(c);
 }
 
-// Light list, after k_collect_lights: count + validation flag back to the host (8 bytes, with whatever else the stream
+// Light list, after k_collect_lights: count + validation flags back to the host (16 bytes, with whatever else the stream
 // has queued for the host), ids sorted into original order with the radix passes, then mapped to slots.
 static int32_t light_list(Ctx* c, uint32_t ns32, uint32_t* n_lights) {
   cudaStream_t st = c->stream;
   DevBuf &keys_b = c->scratch[4], &vals_b = c->scratch[6], &hist = c->scratch[7], &d_light_prims = c->scratch[12],
          &d_light_tmp = c->scratch[13], &d_light_out = c->scratch[14];
-  uint32_t h_light_out[2] = {0u, 0u};
-  PTB_CUDA_TRY(c, cudaMemcpyAsync(h_light_out, d_light_out.p, 8, cudaMemcpyDeviceToHost, st));
+  uint32_t h_light_out[4] = {0u, 0u, 0u, 0u};
+  PTB_CUDA_TRY(c, cudaMemcpyAsync(h_light_out, d_light_out.p, 16, cudaMemcpyDeviceToHost, st));
   PTB_CUDA_TRY(c, cudaStreamSynchronize(st));
+  if (h_light_out[1] & 2u)
+    return set_error(c, PTB_ERR_INVALID, "mesh triangle %u: vertex index out of range (the mesh has %zu vertices)", ~h_light_out[2],
+                     c->n_mesh_vertices);
+  if (h_light_out[1] & 4u)
+    return set_error(c, PTB_ERR_INVALID, "mesh triangle %u: normal index out of range (the mesh has %zu normals)", ~h_light_out[3],
+                     c->n_mesh_normals);
   if (h_light_out[1]) return set_error(c, PTB_ERR_INVALID, "primitive material index out of range");
   const uint32_t nl = h_light_out[0];
   if (nl) {
@@ -819,7 +888,8 @@ static int32_t refit_scene(Ctx* c, uint32_t build_flags) {
   const int T = 256;
   const uint32_t gn = (n32 + T - 1) / T;
   PTB_CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
-  PTB_CUDA_TRY(c, cudaMemsetAsync(d_light_out.p, 0, 8, st));
+  PTB_CUDA_TRY(c, cudaMemsetAsync(d_light_out.p, 0, 16, st));
+  expand_mesh(c, d_light_out.as<uint32_t>());
   k_collect_lights<<<gn, T, 0, st>>>(c->d_raw_spheres.as<ptb_sphere>(), ns32, c->d_raw_tris.as<ptb_triangle>(), n32,
                                      c->d_materials.as<DevMaterial>(), (uint32_t)c->materials.size(), d_light_out.as<uint32_t>(),
                                      d_light_prims.as<uint32_t>());
@@ -856,6 +926,7 @@ static int32_t refit_scene(Ctx* c, uint32_t build_flags) {
   c->dev.lights = c->d_lights.as<uint32_t>();
   c->dev.n_lights = nl;
   c->committed = true;
+  c->mesh_dirty = false;
   return PTB_OK;
 }
 
@@ -909,7 +980,7 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   PTB_CUDA_TRY(c, prim_slot.reserve(n * 4));
   PTB_CUDA_TRY(c, d_light_prims.reserve(n * 4));
   PTB_CUDA_TRY(c, d_light_tmp.reserve(n * 4));
-  PTB_CUDA_TRY(c, d_light_out.reserve(8));
+  PTB_CUDA_TRY(c, d_light_out.reserve(16));
   PTB_CUDA_TRY(c, c->d_nodes.reserve(c->n_nodes * sizeof(BvhNode)));
   if (PTB_QNODES) PTB_CUDA_TRY(c, c->d_qnodes.reserve(c->n_nodes * 32));
   PTB_CUDA_TRY(c, d_qframe.reserve(6 * 4));
@@ -950,7 +1021,8 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   const uint32_t gn = (n32 + T - 1) / T;
   PTB_CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
   // lights + material-index validation (device), then the light ids are put in ORIGINAL primitive order (deterministic)
-  PTB_CUDA_TRY(c, cudaMemsetAsync(d_light_out.p, 0, 8, st));
+  PTB_CUDA_TRY(c, cudaMemsetAsync(d_light_out.p, 0, 16, st));
+  expand_mesh(c, d_light_out.as<uint32_t>());
   k_collect_lights<<<gn, T, 0, st>>>(raw_spheres.as<ptb_sphere>(), ns32, raw_tris.as<ptb_triangle>(), n32,
                                      c->d_materials.as<DevMaterial>(), (uint32_t)c->materials.size(), d_light_out.as<uint32_t>(),
                                      d_light_prims.as<uint32_t>());
@@ -1040,6 +1112,7 @@ int32_t build_scene(Ctx* c, uint32_t build_flags) {
   c->dev.lights = c->d_lights.as<uint32_t>();
   c->dev.n_lights = nl;
   c->committed = true;
+  c->mesh_dirty = false;
   c->refittable = true;
   c->topo_spheres = ns;
   c->topo_tris = nt;

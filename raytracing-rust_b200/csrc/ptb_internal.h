@@ -93,6 +93,11 @@ struct Ctx {
   // are kept on the host until commit
   DevBuf d_raw_spheres, d_raw_tris;
   size_t n_spheres = 0, n_tris = 0;
+  // indexed mesh (ptb_scene_set_mesh): when `mesh` is set, d_raw_tris is the mesh's expansion (k_expand_mesh), redone at
+  // the next commit whenever `mesh_dirty`; n_tris is the number of mesh triangles
+  DevBuf d_mesh_vertices, d_mesh_normals, d_mesh_tris;
+  size_t n_mesh_vertices = 0, n_mesh_normals = 0;
+  bool mesh = false, mesh_dirty = false;
   DevBuf scratch[16];  // LBVH build temporaries, grow-only (lbvh_build.cu)
   std::vector<ptb_material> materials;
   std::vector<ptb_texture> textures;

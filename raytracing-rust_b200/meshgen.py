@@ -3,6 +3,8 @@
   c3_scene()          1 000 000 triangles: 800 000-triangle Lambertian terrain + 200 000-triangle dielectric UV sphere,
                       Lerp sky as scenes/rtweekend1.ssml, 16:9 camera                         (SURVEY.md §8d "C3")
   c3_deform()         one frame of an animated C3: terrain wave + glass sphere pushed into the terrain (same counts)
+  c3_indexed(), heightfield_indexed(), c3_deform_vertices()
+                      the same scenes as indexed meshes over their grid points (expand() == the flat triangles)
   heightfield_scene() R x C quads in [-1,1]^2 x [-0.2,0.2]; 2500 x 2000 -> 10 000 000 triangles      ("C5")
   philox_rays()       incoherent rays from Philox4x32-10 (seed 0x5EED, counter = ray index): origin uniform in the
                       ball of radius 2 about the mesh centre, direction uniform on the sphere
@@ -16,17 +18,23 @@ import copy
 import numpy as np
 
 from . import _lib as L
-from .scene import HostScene
+from .scene import HostScene, IndexedMesh
 
 F = np.float32
 
 
-def _grid_triangles(xs: np.ndarray, ys: np.ndarray, height_fn, normal_fn):
-    """(len(xs)-1) x (len(ys)-1) quads -> 2 triangles each; returns positions (T,3,3) and normals (T,3,3)."""
+def _grid_vertices(xs: np.ndarray, ys: np.ndarray, height_fn, normal_fn):
+    """Positions and normals at the grid points: (len(xs), len(ys), 3) each."""
     X, Y = np.meshgrid(xs.astype(F), ys.astype(F), indexing="ij")
     Z = height_fn(X, Y).astype(F)
     P = np.stack([X, Y, Z], axis=-1)              # (nx, ny, 3)
     N = normal_fn(X, Y).astype(F)
+    return P, N
+
+
+def _grid_triangles(xs: np.ndarray, ys: np.ndarray, height_fn, normal_fn):
+    """(len(xs)-1) x (len(ys)-1) quads -> 2 triangles each; returns positions (T,3,3) and normals (T,3,3)."""
+    P, N = _grid_vertices(xs, ys, height_fn, normal_fn)
     p00, p10, p01, p11 = P[:-1, :-1], P[1:, :-1], P[:-1, 1:], P[1:, 1:]
     n00, n10, n01, n11 = N[:-1, :-1], N[1:, :-1], N[:-1, 1:], N[1:, 1:]
     t0 = np.stack([p00, p10, p11], axis=2)         # (nx-1, ny-1, 3, 3)
@@ -49,8 +57,8 @@ def _terrain_normal(X, Y):
     return n / np.linalg.norm(n, axis=-1, keepdims=True)
 
 
-def uv_sphere(center, radius: float, slices: int, stacks: int):
-    """2 * slices * (stacks - 1) triangles (poles are fans); normals are radial."""
+def _uv_sphere_vertices(center, radius: float, slices: int, stacks: int):
+    """Positions and radial normals at the (stacks + 1) x (slices + 1) grid points of the UV sphere."""
     c = np.asarray(center, F)
     theta = (np.arange(stacks + 1, dtype=F) / F(stacks)) * F(np.pi)        # 0 .. pi
     phi = (np.arange(slices + 1, dtype=F) / F(slices)) * F(2 * np.pi)
@@ -60,6 +68,12 @@ def uv_sphere(center, radius: float, slices: int, stacks: int):
     st[0] = st[-1] = F(0)
     D = np.stack([st[:, None] * cp[None, :], st[:, None] * sp[None, :], np.repeat(ct[:, None], slices + 1, 1)], -1).astype(F)
     P = c + F(radius) * D
+    return P, D
+
+
+def uv_sphere(center, radius: float, slices: int, stacks: int):
+    """2 * slices * (stacks - 1) triangles (poles are fans); normals are radial."""
+    P, D = _uv_sphere_vertices(center, radius, slices, stacks)
     tris_p, tris_n = [], []
     for k in range(stacks):
         a, b = k, k + 1
@@ -83,21 +97,83 @@ def _base_scene(sky_like_rtweekend: bool = True) -> HostScene:
     return s
 
 
+def _grid_indices(nx: int, ny: int) -> np.ndarray:
+    """Corner indices (T, 3) into an (nx, ny) grid of points flattened row-major, in _grid_triangles' order."""
+    g = np.arange(nx * ny, dtype=np.uint32).reshape(nx, ny)
+    i00, i10, i01, i11 = g[:-1, :-1], g[1:, :-1], g[:-1, 1:], g[1:, 1:]
+    t0 = np.stack([i00, i10, i11], axis=-1)
+    t1 = np.stack([i00, i11, i01], axis=-1)
+    return np.stack([t0, t1], axis=2).reshape(-1, 3)
+
+
+def _uv_sphere_indices(slices: int, stacks: int) -> np.ndarray:
+    """Corner indices (T, 3) into the flattened (stacks + 1) x (slices + 1) sphere grid, in uv_sphere's order."""
+    g = np.arange((stacks + 1) * (slices + 1), dtype=np.uint32).reshape(stacks + 1, slices + 1)
+    out = []
+    for k in range(stacks):
+        a0, a1, b0, b1 = g[k, :-1], g[k, 1:], g[k + 1, :-1], g[k + 1, 1:]
+        if k != 0:
+            out.append(np.stack([a0, b1, a1], 1))
+        if k != stacks - 1:
+            out.append(np.stack([a0, b0, b1], 1))
+    return np.concatenate(out)
+
+
+def _mesh(parts) -> IndexedMesh:
+    """One IndexedMesh from (positions grid, normals grid, corner indices (T, 3), material) parts; a triangle's position
+    and normal indices are the same grid point."""
+    verts, nrms, tris, base = [], [], [], 0
+    for P, N, idx, material in parts:
+        t = np.zeros(len(idx), L.mesh_triangle_dtype)
+        t["p"] = idx + np.uint32(base)
+        t["n"] = idx + np.uint32(base)
+        t["material"] = material
+        verts.append(P.reshape(-1, 3))
+        nrms.append(N.reshape(-1, 3))
+        tris.append(t)
+        base += len(verts[-1])
+    return IndexedMesh(np.concatenate(verts), np.concatenate(nrms), np.concatenate(tris))
+
+
+def _c3_dims(scale: float):
+    return (max(2, int(round(1000 * scale))), max(2, int(round(400 * scale))), max(3, int(round(500 * scale))),
+            max(3, int(round(201 * scale))))
+
+
+def _c3_axes(nx: int, ny: int):
+    return (np.linspace(-12.5, 12.5, nx + 1, dtype=np.float64).astype(F), np.linspace(0.0, 10.0, ny + 1, dtype=np.float64).astype(F))
+
+
+C3_CAMERA = ((0.0, -1.5, 1.6), (0.0, 4.0, 0.7), (0.0, 0.0, 1.0), 60.0, 16.0 / 9.0, 0.0, 1.0)
+
+
 def c3_scene(scale: float = 1.0) -> HostScene:
     """scale=1 -> exactly 1 000 000 triangles; scale<1 shrinks every grid dimension (tests)."""
-    nx, ny = max(2, int(round(1000 * scale))), max(2, int(round(400 * scale)))
-    slices, stacks = max(3, int(round(500 * scale))), max(3, int(round(201 * scale)))
+    nx, ny, slices, stacks = _c3_dims(scale)
     s = _base_scene()
-    xs = np.linspace(-12.5, 12.5, nx + 1, dtype=np.float64).astype(F)
-    ys = np.linspace(0.0, 10.0, ny + 1, dtype=np.float64).astype(F)
+    xs, ys = _c3_axes(nx, ny)
     tp, tn = _grid_triangles(xs, ys, _terrain_height, _terrain_normal)
     sp_, sn = uv_sphere((0.0, 4.0, 1.0), 0.8, slices, stacks)
     tri = np.zeros(len(tp) + len(sp_), L.triangle_dtype)
     tri["p"][: len(tp)], tri["n"][: len(tp)], tri["material"][: len(tp)] = tp, tn, 0
     tri["p"][len(tp):], tri["n"][len(tp):], tri["material"][len(tp):] = sp_, sn, 1
     s.triangles = tri
-    s.set_camera((0.0, -1.5, 1.6), (0.0, 4.0, 0.7), (0.0, 0.0, 1.0), 60.0, 16.0 / 9.0, 0.0, 1.0)
+    s.set_camera(*C3_CAMERA)
     return s
+
+
+def c3_indexed(scale: float = 1.0):
+    """C3 as an indexed mesh: (scene without triangles, mesh). The vertices are the grid points of the terrain
+    ((nx + 1) x (ny + 1)) and of the sphere ((stacks + 1) x (slices + 1)), 502 603 at scale 1; mesh.expand() equals
+    c3_scene(scale).triangles byte for byte."""
+    nx, ny, slices, stacks = _c3_dims(scale)
+    s = _base_scene()
+    xs, ys = _c3_axes(nx, ny)
+    P, N = _grid_vertices(xs, ys, _terrain_height, _terrain_normal)
+    SP, SN = _uv_sphere_vertices((0.0, 4.0, 1.0), 0.8, slices, stacks)
+    mesh = _mesh([(P, N, _grid_indices(nx + 1, ny + 1), 0), (SP, SN, _uv_sphere_indices(slices, stacks), 1)])
+    s.set_camera(*C3_CAMERA)
+    return s, mesh
 
 
 C3_GLASS_RADIUS = 0.8
@@ -118,27 +194,59 @@ def c3_deform(scene: HostScene, wave: float, shift: float) -> HostScene:
     return s
 
 
+def c3_deform_vertices(mesh: IndexedMesh, wave: float, shift: float) -> IndexedMesh:
+    """c3_deform's motion applied to the vertex array of c3_indexed's mesh (normals and triangles are shared, not copied).
+    A vertex belongs to the sphere when a glass triangle uses it. numpy may evaluate sin differently for arrays of other
+    shapes, so compare with expand() of the result, not with c3_deform."""
+    glass = np.zeros(len(mesh.vertices), bool)
+    glass[mesh.triangles["p"][mesh.triangles["material"] == 1].reshape(-1)] = True
+    v = mesh.vertices.copy()
+    t = v[~glass]
+    x, y = t[:, 0], t[:, 1]
+    t[:, 2] = t[:, 2] * (F(1) + F(wave) * np.sin(F(0.7) * x + F(0.4) * y))
+    v[~glass] = t
+    v[glass] = v[glass] + (F(shift) * F(C3_GLASS_RADIUS) * np.array([0.6, 0.0, -0.8], F)).astype(F)
+    return IndexedMesh(v, mesh.normals, mesh.triangles)
+
+
+def _hf_height(X, Y):
+    return F(0.1) * np.sin(F(9.0) * X) * np.cos(F(7.0) * Y) + F(0.1) * np.sin(F(23.0) * X + F(17.0) * Y)
+
+
+def _hf_normal(X, Y):
+    dx = F(0.9) * np.cos(F(9.0) * X) * np.cos(F(7.0) * Y) + F(2.3) * np.cos(F(23.0) * X + F(17.0) * Y)
+    dy = -F(0.7) * np.sin(F(9.0) * X) * np.sin(F(7.0) * Y) + F(1.7) * np.cos(F(23.0) * X + F(17.0) * Y)
+    n = np.stack([-dx, -dy, np.ones_like(dx)], -1)
+    return n / np.linalg.norm(n, axis=-1, keepdims=True)
+
+
+def _hf_axes(rows: int, cols: int):
+    return (np.linspace(-1.0, 1.0, rows + 1, dtype=np.float64).astype(F), np.linspace(-1.0, 1.0, cols + 1, dtype=np.float64).astype(F))
+
+
+HF_CAMERA = ((0.0, -3.0, 1.5), (0.0, 0.0, 0.0), (0.0, 0.0, 1.0), 50.0, 16.0 / 9.0, 0.0, 1.0)
+
+
 def heightfield_scene(rows: int = 2500, cols: int = 2000) -> HostScene:
     """rows x cols quads -> 2*rows*cols triangles in [-1,1]^2 x [-0.2,0.2] (C5: 10 000 000)."""
     s = _base_scene()
-    xs = np.linspace(-1.0, 1.0, rows + 1, dtype=np.float64).astype(F)
-    ys = np.linspace(-1.0, 1.0, cols + 1, dtype=np.float64).astype(F)
-
-    def h(X, Y):
-        return F(0.1) * np.sin(F(9.0) * X) * np.cos(F(7.0) * Y) + F(0.1) * np.sin(F(23.0) * X + F(17.0) * Y)
-
-    def nrm(X, Y):
-        dx = F(0.9) * np.cos(F(9.0) * X) * np.cos(F(7.0) * Y) + F(2.3) * np.cos(F(23.0) * X + F(17.0) * Y)
-        dy = -F(0.7) * np.sin(F(9.0) * X) * np.sin(F(7.0) * Y) + F(1.7) * np.cos(F(23.0) * X + F(17.0) * Y)
-        n = np.stack([-dx, -dy, np.ones_like(dx)], -1)
-        return n / np.linalg.norm(n, axis=-1, keepdims=True)
-
-    tp, tn = _grid_triangles(xs, ys, h, nrm)
+    xs, ys = _hf_axes(rows, cols)
+    tp, tn = _grid_triangles(xs, ys, _hf_height, _hf_normal)
     tri = np.zeros(len(tp), L.triangle_dtype)
     tri["p"], tri["n"], tri["material"] = tp, tn, 0
     s.triangles = tri
-    s.set_camera((0.0, -3.0, 1.5), (0.0, 0.0, 0.0), (0.0, 0.0, 1.0), 50.0, 16.0 / 9.0, 0.0, 1.0)
+    s.set_camera(*HF_CAMERA)
     return s
+
+
+def heightfield_indexed(rows: int = 2500, cols: int = 2000):
+    """The heightfield as an indexed mesh over its (rows + 1) x (cols + 1) grid points: (scene without triangles, mesh),
+    mesh.expand() equal to heightfield_scene(rows, cols).triangles byte for byte."""
+    s = _base_scene()
+    P, N = _grid_vertices(*_hf_axes(rows, cols), _hf_height, _hf_normal)
+    mesh = _mesh([(P, N, _grid_indices(rows + 1, cols + 1), 0)])
+    s.set_camera(*HF_CAMERA)
+    return s, mesh
 
 
 # ---- Philox4x32-10 in numpy (vectorised over counters) ---------------------------------------------------------

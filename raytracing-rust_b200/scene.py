@@ -94,6 +94,55 @@ class HostScene:
         self.sky["texture"], self.sky["sampler_res_x"], self.sky["sampler_res_y"] = texture, sampler_res[0], sampler_res[1]
 
 
+@dataclass
+class IndexedMesh:
+    """The reference's MeshData + MeshTriangle (implementations/primitives/triangle.rs:30-36): vertex and normal arrays and
+    triangles that index them (mesh_triangle_dtype). Uploaded with Context.set_mesh; the device expands it into the
+    triangle_dtype records expand() returns."""
+    vertices: np.ndarray   # (V, 3) float32
+    normals: np.ndarray    # (N, 3) float32
+    triangles: np.ndarray  # (T,) mesh_triangle_dtype
+
+    def __post_init__(self):
+        self.vertices = np.ascontiguousarray(self.vertices, np.float32).reshape(-1, 3)
+        self.normals = np.ascontiguousarray(self.normals, np.float32).reshape(-1, 3)
+        self.triangles = np.ascontiguousarray(self.triangles, L.mesh_triangle_dtype)
+
+    def expand(self) -> np.ndarray:
+        """The flat triangles (triangle_dtype) this mesh stands for: a host-side gather, byte for byte what the device
+        expansion writes. An index out of range raises IndexError."""
+        tri = np.zeros(len(self.triangles), L.triangle_dtype)
+        tri["p"] = self.vertices[self.triangles["p"]]
+        tri["n"] = self.normals[self.triangles["n"]]
+        tri["material"] = self.triangles["material"]
+        return tri
+
+    def nbytes(self) -> int:
+        return int(self.vertices.nbytes + self.normals.nbytes + self.triangles.nbytes)
+
+
+def _dedup_rows(a: np.ndarray):
+    """Distinct float32 3-vectors of `a` (rows compared by their bytes, so -0.0 != 0.0 and NaNs keep their payload) and
+    the index of each row among them."""
+    rows = np.ascontiguousarray(a, np.float32).reshape(-1, 3)
+    keys = rows.view(np.dtype((np.void, 12))).reshape(-1)
+    _, first, inverse = np.unique(keys, return_index=True, return_inverse=True)
+    return rows[first], inverse.reshape(-1).astype(np.uint32)
+
+
+def index_triangles(tri: np.ndarray) -> IndexedMesh:
+    """Indexed form of a flat triangle array: positions and normals deduplicated by their bytes. expand() of the result
+    equals `tri` byte for byte."""
+    tri = np.ascontiguousarray(tri, L.triangle_dtype)
+    vertices, pi = _dedup_rows(tri["p"])
+    normals, ni = _dedup_rows(tri["n"])
+    m = np.zeros(len(tri), L.mesh_triangle_dtype)
+    m["p"] = pi.reshape(-1, 3)
+    m["n"] = ni.reshape(-1, 3)
+    m["material"] = tri["material"]
+    return IndexedMesh(vertices, normals, m)
+
+
 def _copy_array(handle, getter, dtype) -> np.ndarray:
     p = C.c_void_p()
     n = getter(handle, C.byref(p))
