@@ -365,9 +365,8 @@ int32_t ptb_occluded_device(ptb_ctx* ctx, const void* d_rays, size_t n, void* d_
  * 133 B with MIS), never more than half of the memory that was free at the context's first large render. A call that fits
  * (124 Mi paths, 64 Mi with MIS) runs as one chunk; a larger one runs chunk by chunk in two slots of half the budget each,
  * the wide iterations of chunk k+1 overlapping the latency-bound tail of chunk k. PTB_POOL_PATHS=<paths> sets the slot size directly,
- * PTB_TAIL_PATHS=<paths> the live-path count (default 65 536) below which a chunk is handed to the fused tail kernel (0: never),
- * PTB_WAVEFRONT=queue selects the small-pool regenerating mode. The
- * image is a pure function of (scene, opts): pool size, chunking and GPU count only change the f32 summation order
+ * PTB_TAIL_PATHS=<paths> the live-path count (default 65 536) below which a chunk is handed to the fused tail kernel (0: never).
+ * The image is a pure function of (scene, opts): pool size, chunking and GPU count only change the f32 summation order
  * (finished paths are added with float atomics, so two runs of the same call agree to ~1e-6 relative, not bit for bit).
  * A non-zero return of `progress` stops the call with PTB_ERR_ABORTED and CLEARS the accumulator (samples of earlier
  * calls included): a partially rendered call has no sample count to normalise by. */

@@ -94,7 +94,6 @@ int32_t ptb_create(int32_t device, ptb_ctx** out) {
   c->own_stream = true;
   if ((e = cudaEventCreate(&c->ev_a)) != cudaSuccess) return fail(e, "cudaEventCreate");
   if ((e = cudaEventCreate(&c->ev_b)) != cudaSuccess) return fail(e, "cudaEventCreate");
-  if ((e = cudaEventCreate(&c->ev_iter)) != cudaSuccess) return fail(e, "cudaEventCreate");
   *out = ctx;
   return PTB_OK;
 }
@@ -110,7 +109,6 @@ int32_t ptb_destroy(ptb_ctx* ctx) {
     if (h) cudaFreeHost(h);
   if (c->ev_a) cudaEventDestroy(c->ev_a);
   if (c->ev_b) cudaEventDestroy(c->ev_b);
-  if (c->ev_iter) cudaEventDestroy(c->ev_iter);
   for (int b = 0; b < 2; ++b) {
     if (c->ev_in[b]) cudaEventDestroy(c->ev_in[b]);
     if (c->ev_kernel[b]) cudaEventDestroy(c->ev_kernel[b]);

@@ -50,30 +50,20 @@ struct PathPool {
 };
 constexpr uint32_t kMaxSampleIndex = 1u << 23;  // sample index shares a word with depth (8 bits) and one flag
 
-constexpr int kNumKinds = 6;  // shade queues: 0 = miss (sky), 1 + PTB_MAT_* otherwise
+constexpr int kNumKinds = 6;  // material kinds of k_shade's block sort: 0 = miss (sky), 1 + PTB_MAT_* otherwise
 
-struct WaveCounters {  // lives in device memory; mirrored to pinned host memory once per iteration
-  uint32_t n_free;          // entries in q_free
-  uint32_t n_active[2];     // entries in q_active[k]
-  uint32_t n_new;           // camera paths generated this iteration
+struct WaveCounters {  // one per chunk slot, in device memory; mirrored to pinned host memory once per iteration
   uint32_t n_trace;         // rays to trace this iteration
-  uint32_t free_base;       // q_free[free_base .. free_base + n_new) feed the generator
-  uint32_t n_kind[kNumKinds];
-  uint32_t n_shadow;
-  uint32_t cur;             // which q_active is the trace queue
-  uint32_t trace_head, shade_head, shadow_head;  // persistent-kernel work cursors
-  // window mode, decided ON THE DEVICE by k_win_prepare so that the host never has to wait for an iteration before it
-  // enqueues the next: 0 wavefront iterations running, 1 this iteration hands the chunk's last n_tail paths to k_tail,
-  // 2 chunk finished, 3 handed over earlier — in every state but 0 the wavefront kernels find n_trace == 0 and return
+  uint32_t trace_head, shadow_head;  // persistent-kernel work cursors
+  // decided ON THE DEVICE by k_win_prepare so that the host never has to wait for an iteration before it enqueues the
+  // next: 0 wavefront iterations running, 1 this iteration hands the chunk's last n_tail paths to k_tail, 2 chunk
+  // finished, 3 handed over earlier — in every state but 0 the wavefront kernels find n_trace == 0 and return
   uint32_t mode;
   uint32_t n_tail, tail_iter;  // set ONCE per chunk: live paths handed over, and the iteration whose k_tail launch takes them
   uint32_t tail_head, _pad2;   // k_tail's work cursor (its lanes pull paths one by one)
-  // k_shade's queue cursors, packed so that one warp needs ONE returning atomic per pair (the kernel used to spend 40 % of
-  // its stall samples waiting for three serial same-address atomics): push_pair = finished-slot cursor << 32 | next-active
-  // cursor, shadow_pair = sky NEE rays << 32 | shadow-queue cursor. k_prepare unpacks them between iterations.
-  unsigned long long push_pair, shadow_pair;
-  unsigned long long next_sample;   // next global sample index (pixel-major within a pass)
-  unsigned long long total_samples;
+  // k_shade's shadow-queue cursor, packed so that one warp needs ONE returning atomic: sky NEE rays << 32 | entries.
+  // k_win_prepare unpacks it between iterations.
+  unsigned long long shadow_pair;
   // statistics (ptb_stats)
   unsigned long long rays_camera, rays_bounce, rays_shadow_light, rays_shadow_sky, rays_reference, paths;
   unsigned long long nodes_fetched, prims_tested, rays_counted;  // PTB_OPT_COUNT_TRAVERSAL
@@ -149,7 +139,7 @@ struct Ctx {
   PathPool pool;
   size_t pool_budget_bytes = 0;  // half of the device memory that was free at the first large render (0 = not asked yet)
   WaveCounters* h_counters = nullptr;  // pinned: [0..7] per-iteration mirrors (a ring of 4 per slot), [8..9] end-of-render copy of each slot
-  cudaEvent_t ev_a = nullptr, ev_b = nullptr, ev_iter = nullptr;
+  cudaEvent_t ev_a = nullptr, ev_b = nullptr;
   cudaEvent_t ev_prof[64] = {};  // PTB_OPT_TIME_KERNELS: 2 slots x 4 iterations (ring) x 4 kernel classes x (start, stop)
   bool opt_time_kernels = false, opt_count_traversal = false;
 

@@ -2,8 +2,8 @@
 // (implementations/src/samplers/random_sampler.rs:23-99, integrators/mod.rs:22-78, integrators/mis.rs:6-157) and
 // everything they call per bounce (materials/*.rs, sky.rs, textures/mod.rs, primitives light sampling).
 //
-// Window mode (default; see "window wavefront" below): every camera path of a chunk is resident, path g owns slot g, and
-// one iteration traces and shades bounce k of ALL of them:
+// Window wavefront (see "window wavefront" below): a call runs in chunks, every camera path of a chunk is resident, path g
+// owns slot g, and one iteration traces and shades bounce k of ALL of them:
 //   k_win_scan / k_win_prepare / k_win_fill   live counts -> ordered trace queue (slot order, direction-ordered per window)
 //   k_trace     K1 + K8      closest hit for every live path (persistent warps pulling 32-ray batches); the first
 //                            iteration of a chunk computes its camera rays in the fetch (random_sampler.rs:50-61,
@@ -11,8 +11,6 @@
 //   k_shade     K10 + K12    emission, MIS weights, NEE sample -> shadow queue, BSDF sample -> next ray (written in place),
 //                            Russian roulette, path termination -> accumulator
 //   k_shadow    K9           any-hit for the NEE queue; unoccluded contributions are added to the path's radiance
-// Queue mode (pools smaller than the call): k_prepare / k_generate refill freed slots with camera paths every iteration,
-// k_trace pushes its results to one queue per material kind, k_shade walks those queues.
 //
 // The RNG is counter-based (Philox4x32-10 keyed by seed; counter = pixel, absolute sample, depth|purpose, block):
 // the image is a pure function of (scene, seed, sample range) — independent of pool size, scheduling and GPU count.
@@ -25,20 +23,18 @@ namespace ptb {
 struct RenderParams {
   uint32_t width, height, npix;  // npix = width * (rows of this call's image tile)
   uint32_t row_begin;            // first pixel row of the tile (ptb_render_opts::row_begin)
-  uint32_t tile_w, tile_h;  // pixel issue order (k_generate); tile_h == 1 -> row-major
+  uint32_t tile_w, tile_h;  // pixel issue order (camera_pixel_sample); tile_h == 1 -> row-major
   uint32_t group;           // samples of one pixel issued back to back (a divisor of the call's spp)
-  uint32_t dir_bins;        // window mode: order a window's live rays by direction bin (PTB_DIRBINS=0 disables)
+  uint32_t dir_bins;        // order a window's live rays by direction bin (PTB_DIRBINS=0 disables)
   uint32_t sample_offset;
   uint32_t method, max_depth, rr_threshold;
   uint32_t k0, k1;  // Philox key
 };
 
 struct Queues {
-  uint32_t* active[2];
-  uint32_t* free_slots;
-  uint32_t* kind[kNumKinds];
+  uint32_t* live;  // [capacity] this iteration's trace queue: the live slots, ordered by k_win_fill
   float4* shadow;  // 3 x float4 per entry: o.xyz|tmax, d.xyz|exclude slot, contrib.rgb|path slot
-  // window mode (see "window wavefront" below)
+  // see "window wavefront" below
   uint32_t* win_count;   // [n_windows] live paths of each kWindow-slot window
   uint32_t* win_prefix;  // [n_windows] exclusive prefix of win_count inside the window's 4096-window segment
   uint32_t* seg_total;   // [n_windows / 4096 + 1] live paths per segment
@@ -219,58 +215,16 @@ PTB_DEV v3 uniform_sphere_dir(float r1, float r2) {
 }
 
 // ------------------------------------------------------------------------------------------ bookkeeping kernels
-__global__ void k_init_pool(uint32_t* free_slots, uint32_t capacity, WaveCounters* wc, unsigned long long total_samples) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < capacity) free_slots[i] = capacity - 1u - i;  // popped from the end: slot 0 first
-  if (i == 0) {
-    wc->n_free = capacity;
-    wc->push_pair = wc->shadow_pair = 0;
-    wc->n_active[0] = wc->n_active[1] = 0;
-    wc->n_new = wc->n_trace = wc->free_base = 0;
-    for (int k = 0; k < kNumKinds; ++k) wc->n_kind[k] = 0;
-    wc->n_shadow = 0;
-    wc->cur = 0;
-    wc->trace_head = wc->shade_head = wc->shadow_head = 0;
-    wc->next_sample = 0;
-    wc->total_samples = total_samples;
-    wc->rays_camera = wc->rays_bounce = wc->rays_shadow_light = wc->rays_shadow_sky = wc->rays_reference = wc->paths = 0;
-    wc->nodes_fetched = wc->prims_tested = wc->rays_counted = 0;
-    wc->tail_t0 = ~0ull;
-    wc->tail_t1 = wc->tail_ns = 0ull;
-  }
-}
-
-// Runs between iterations. Folds the finished iteration's counts into the statistics, flips the active queues and
-// decides how many camera paths the next k_generate starts.
-__global__ void k_prepare(WaveCounters* wc, uint32_t method, uint32_t first) {
-  if (!first) {
-    const uint32_t cur = wc->cur, nxt = cur ^ 1u;
-    const unsigned long long pp = wc->push_pair, sp = wc->shadow_pair;
-    const uint32_t traced = wc->n_trace, survivors = (uint32_t)pp;
-    wc->n_active[nxt] = survivors;
-    wc->n_free = (uint32_t)(pp >> 32);
-    wc->rays_shadow_sky += sp >> 32;
-    wc->rays_shadow_light += (uint32_t)sp - (uint32_t)(sp >> 32);
-    wc->rays_camera += wc->n_new;
-    wc->rays_bounce += traced - wc->n_new;
-    wc->rays_reference += method == PTB_METHOD_NAIVE ? traced : survivors;  // Q7: naive 1/check_hit, MIS 1/bounce iteration
-    wc->paths += traced - survivors;
-    wc->n_active[cur] = 0;
-    wc->cur = nxt;
-  }
-  const uint32_t cur = wc->cur;
-  const unsigned long long remaining = wc->total_samples - wc->next_sample;
-  const uint32_t n_free = wc->n_free;
-  const uint32_t n_new = remaining < (unsigned long long)n_free ? (uint32_t)remaining : n_free;
-  wc->n_new = n_new;
-  wc->free_base = n_free - n_new;
-  wc->n_free = n_free - n_new;
-  wc->n_trace = wc->n_active[cur] + n_new;
-  for (int k = 0; k < kNumKinds; ++k) wc->n_kind[k] = 0;
-  wc->n_shadow = 0;
-  wc->push_pair = (unsigned long long)(n_free - n_new) << 32;  // finished slots append after the remaining free ones
+// A slot's counters at the start of a render: work cursors and statistics zeroed, no fused-tail hand-over timed yet
+// (k_win_init folds a finished one into tail_ns only when tail_t0 != ~0). k_win_init sets the per-chunk state (mode,
+// n_tail, tail_iter, tail_head).
+__global__ void k_reset_counters(WaveCounters* wc) {
+  wc->n_trace = wc->trace_head = wc->shadow_head = 0;
   wc->shadow_pair = 0;
-  wc->trace_head = wc->shade_head = wc->shadow_head = 0;
+  wc->rays_camera = wc->rays_bounce = wc->rays_shadow_light = wc->rays_shadow_sky = wc->rays_reference = wc->paths = 0;
+  wc->nodes_fetched = wc->prims_tested = wc->rays_counted = 0;
+  wc->tail_t0 = ~0ull;
+  wc->tail_t1 = wc->tail_ns = 0ull;
 }
 
 // ------------------------------------------------------------------------------------------ K1 camera rays
@@ -305,34 +259,10 @@ PTB_DEV v3 camera_direction(const DevScene& sc, const RenderParams& rp, uint32_t
   const v3 dir = sc.cam_lower_left + sc.cam_horizontal * u + sc.cam_vertical * v - sc.cam_origin;
   return dir / mag(dir);
 }
-// One camera path (queue mode): written to `slot` as the 64-byte path block.
-PTB_DEV void emit_camera_path(const DevScene& sc, const PathPool& pool, const RenderParams& rp, unsigned long long g, uint32_t slot) {
-  uint32_t x, y, sample;
-  camera_pixel_sample(rp, g, x, y, sample);
-  const v3 d = camera_direction(sc, rp, x, y, sample);
-  // two 32-byte stores (STG.256, sm_100): half the L1 data-pipe wavefronts of four STG.128
-  stg256(pool.ray + 4u * (size_t)slot, make_float4(sc.cam_origin.x, sc.cam_origin.y, sc.cam_origin.z, 0.0f),
-         make_float4(d.x, d.y, d.z, __uint_as_float(kNone)));
-  stg256(pool.col + 4u * (size_t)slot, make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(y * rp.width + x)),
-         make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(sample << 9)));
-}
 
-__global__ void __launch_bounds__(256)
-k_generate(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp) {
-  const uint32_t n_new = wc->n_new;
-  const uint32_t cur = wc->cur;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_new; i += gridDim.x * blockDim.x) {
-    const uint32_t slot = q.free_slots[wc->free_base + (n_new - 1u - i)];
-    emit_camera_path(sc, pool, rp, wc->next_sample + i, slot);
-    q.active[cur][wc->n_active[cur] + i] = slot;
-  }
-}
-// next_sample is advanced by a separate 1-thread launch: every k_generate thread reads it
-__global__ void k_advance(WaveCounters* wc) { wc->next_sample += wc->n_new; }
-
-// ------------------------------------------------------------------------------------------ K8 closest hit + K11 queueing
-// CAMERA (window mode, first iteration of a chunk): work item i IS slot i and its ray is the camera ray of path
-// first + i, computed here — the chunk's camera rays are never written to and read back from memory.
+// ------------------------------------------------------------------------------------------ K8 closest hit
+// CAMERA (first iteration of a chunk): work item i IS slot i and its ray is the camera ray of path first + i, computed
+// here — the chunk's camera rays are never written to and read back from memory.
 template <bool CAMERA>
 struct TraceFetch {
   const PathPool& pool;
@@ -355,48 +285,30 @@ struct TraceFetch {
     ray = make_ray(from4(o), from4(d));
   }
 };
-template <bool DENSE, bool CAMERA>
+template <bool CAMERA>
 struct TraceRetire {
-  const DevScene& sc;
   const PathPool& pool;
-  const Queues& q;
-  WaveCounters* wc;
   const TraceFetch<CAMERA>& f;
-  // called by all 32 lanes: write the hit (the whole 32-byte ray record, so the store is a full sector), then a
-  // warp-aggregated push into the per-material-kind shade queue
+  // write the hit: the whole 32-byte ray record, so the store is a full sector
   PTB_DEV void operator()(bool fin, const TraceResult& tr, const Ray& ray) {
-    const uint32_t lane = threadIdx.x & 31u;
-    uint32_t kind = 0xFFu;
-    if (fin) {
+    if (fin)
       stg256(pool.ray + 4u * (size_t)f.slot, make_float4(ray.o.x, ray.o.y, ray.o.z, tr.t),
              make_float4(ray.d.x, ray.d.y, ray.d.z, __uint_as_float(tr.ref)));
-      if (!DENSE) kind = tr.ref == kNone ? 0u : 1u + (__ldg(sc.slot_mat + (tr.ref & kSlotMask)) >> 24);
-    }
-    if (DENSE) return;  // window mode: k_shade walks the windows, there is no per-kind queue
-    if (!__any_sync(0xffffffffu, fin)) return;
-    const uint32_t peers = __match_any_sync(0xffffffffu, kind);
-    if (fin) {
-      const uint32_t leader = __ffs(peers) - 1u;
-      uint32_t pos = 0;
-      if (lane == leader) pos = atomicAdd(&wc->n_kind[kind], __popc(peers));
-      pos = __shfl_sync(peers, pos, leader);
-      q.kind[kind][pos + __popc(peers & ((1u << lane) - 1u))] = f.slot;
-    }
   }
 };
 
 #ifndef PTB_SHADE_MIN_BLOCKS
-#define PTB_SHADE_MIN_BLOCKS 4  // caps k_shade at 64 registers (32 B of spills). Window mode streams its records, so occupancy
-                                // pays now: 2 -> 4 blocks: C3 3664 -> 3746 Mrays/s, rtweekend1 4K MIS 8439 -> 8967 (queue mode
-                                // preferred 2: 128 registers, profiles/r1_sweeps.md)
+#define PTB_SHADE_MIN_BLOCKS 4  // caps k_shade at 64 registers (32 B of spills). The window wavefront streams its records, so
+                                // occupancy pays: 2 -> 4 blocks: C3 3664 -> 3746 Mrays/s, rtweekend1 4K MIS 8439 -> 8967
+                                // (profiles/r1_sweeps.md)
 #endif
-template <class TR, bool COUNT, bool DENSE, bool CAMERA>
+template <class TR, bool COUNT, bool CAMERA>
 __global__ void __launch_bounds__(256, TR::kTraceMinBlocks)
 k_trace(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp, unsigned long long first) {
   const uint32_t lane = threadIdx.x & 31u;
   uint32_t cnt_nodes = 0, cnt_prims = 0, cnt_rays = 0;
-  TraceFetch<CAMERA> fetch{pool, q.active[DENSE ? 0u : wc->cur], 0u, sc, rp, first};
-  TraceRetire<DENSE, CAMERA> retire{sc, pool, q, wc, fetch};
+  TraceFetch<CAMERA> fetch{pool, q.live, 0u, sc, rp, first};
+  TraceRetire<CAMERA> retire{pool, fetch};
   persistent_trace<TR, false, COUNT>(sc, wc->n_trace, &wc->trace_head, fetch, retire, cnt_nodes, cnt_prims, cnt_rays);
   if (COUNT) {
     for (int off = 16; off > 0; off >>= 1) {
@@ -474,7 +386,7 @@ struct Surface {  // what the integrators read from `hit` + `mat`
 // ------------------------------------------------------------------------------------------ Trowbridge-Reitz (GGX)
 // statistics/bxdfs/trowbridge_reitz.rs:17-24 (d), 62-78 (g2), 80-89 (g1); trowbridge_reitz_vndf.rs:9-15 (vndf),
 // 84-113 (sample_vndf, a_x = a_y), 35-52 (sample, pdf); materials/trowbridge_reitz.rs:26-88. Kept out of line: the
-// code is only reached from the Trowbridge-Reitz shade queue and must not cost the other materials registers.
+// code is only reached for Trowbridge-Reitz surfaces and must not cost the other materials registers.
 PTB_DEV float tr_d(float alpha, float cos_theta) {
   if (cos_theta <= 0.0f) return 0.0f;
   const float a_sq = alpha * alpha;
@@ -646,11 +558,11 @@ PTB_DEV uint32_t direction_bin(v3 d) {
 
 // One path, one bounce: everything the integrators do between two check_hit calls (emission, MIS weights, NEE sample, BSDF
 // sample, Russian roulette, termination). Reads the path's records (ray + hit, colour) from the pool and writes the
-// continuing path's records back; what the caller has to route (queues, accumulator, shadow ray) comes back in `o`.
+// continuing path's records back; what the caller has to route (direction bin, accumulator, shadow ray) comes back in `o`.
 // Shared by the wavefront kernel k_shade and the fused tail kernel k_tail.
 struct ShadeOut {
-  bool alive = false;       // path continues: goes to the next active queue
-  bool finished = false;    // path ended: slot returns to the free list
+  bool alive = false;       // path continues: its next ray is in the slot's ray record
+  bool finished = false;    // path ended: the slot is marked dead
   bool shadow = false;      // an NEE ray was produced
   bool contributes = false; // finished with a radiance that passes the NaN test (integrators/mod.rs:74-76, mis.rs:88-90)
   uint32_t shadow_is_sky = 0, fin_pixel = 0;
@@ -925,51 +837,29 @@ PTB_DEV void shade_path(const DevScene& sc, const PathPool& pool, const RenderPa
   }
 }
 
-// DENSE = window mode (ordered live-slot queue in, per-slot direction bin and per-window live count out), else the
-// per-material-kind queues of the regenerating queue mode.
+// Ordered live-slot queue in, per-slot direction bin and per-window live count out.
 // MIS shades at one block more per SM than naive (48 registers): rtweekend1 4K 9133 -> 9179 Mrays/s, C3 (naive) would lose 2 %
-template <int METHOD, bool FULL, bool DENSE>
+template <int METHOD, bool FULL>
 __global__ void __launch_bounds__(256, PTB_SHADE_MIN_BLOCKS + (METHOD == PTB_METHOD_MIS ? 1 : 0))
 k_shade(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp, float* __restrict__ accum,
         unsigned long long camera_first, uint32_t sort_kinds) {
-  // window mode, first iteration of a chunk (camera_first != kNoCamera): work item i is slot i, every slot is live and its
-  // colour record is the camera path's initial state, derived from the path index instead of read from memory
-  const bool depth0 = DENSE && camera_first != kNoCamera;
+  // first iteration of a chunk (camera_first != kNoCamera): work item i is slot i, every slot is live and its colour
+  // record is the camera path's initial state, derived from the path index instead of read from memory
+  const bool depth0 = camera_first != kNoCamera;
   const uint32_t lane = threadIdx.x & 31u;
-  const uint32_t nxt = wc->cur ^ 1u;
-  uint32_t n_kind[kNumKinds], n_total = 0;
-  if (DENSE) {
-    n_total = wc->n_trace;
-  } else {
-#pragma unroll
-    for (int k = 0; k < kNumKinds; ++k) { n_kind[k] = wc->n_kind[k]; n_total += n_kind[k]; }
-  }
-  // queue mode: grid-stride over the concatenation of the kind queues; window mode: over the ordered live-slot queue.
-  // Whole blocks iterate together (ballots below).
+  const uint32_t n_total = wc->n_trace;
+  // grid-stride over the ordered live-slot queue; whole blocks iterate together (ballots below)
   for (uint32_t base = blockIdx.x * blockDim.x; base < n_total; base += gridDim.x * blockDim.x) {
   const uint32_t i = base + threadIdx.x;
-  uint32_t kq = kNumKinds, off = 0;
-  bool active;
-  if (DENSE) {
-    active = i < n_total;
-  } else {
-    uint32_t total = 0;
-#pragma unroll
-    for (int k = 0; k < kNumKinds; ++k) {
-      const uint32_t c = n_kind[k];
-      if (kq == (uint32_t)kNumKinds && i < total + c) { kq = k; off = i - total; }
-      total += c;
-    }
-    active = kq != (uint32_t)kNumKinds;
-  }
+  bool active = i < n_total;
 
   uint32_t slot = 0;
   ShadeOut so;
   so.fin_L = mk(0.0f, 0.0f, 0.0f);
 
-  if (active) slot = DENSE ? (depth0 ? i : q.active[0][i]) : q.kind[kq][off];
-  if (DENSE && sort_kinds) {
-    // Window mode orders a window's rays by direction, so the hits a block shades arrive with their materials mixed. A
+  if (active) slot = depth0 ? i : q.live[i];
+  if (sort_kinds) {
+    // The window wavefront orders a window's rays by direction, so the hits a block shades arrive with their materials mixed. A
     // scene with more than two material kinds (sort_kinds, decided at commit) has its block's work items counting-sorted
     // by the kind of the surface hit (0 = sky, 1 + PTB_MAT_*) before they are shaded: warps then run one material's code
     // instead of all of them one after the other. Costs one extra 16-byte read per path (the hit reference) and two
@@ -1005,60 +895,31 @@ k_shade(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp,
   if (active) shade_path<METHOD, FULL>(sc, pool, rp, slot, depth0, camera_first, so);
   finish_paths(accum, so.contributes, so.fin_pixel, so.fin_L);
 
-  if (DENSE) {
-    // ---- window mode: paths stay in their slot. A finished path is marked dead and leaves its window's live count
-    // (lanes of a warp nearly always share the window: one atomic per warp); NEE rays go to the shadow queue.
-    if (so.alive) q.bin[slot] = (uint8_t)so.bin;
-    if (so.finished) q.bin[slot] = (uint8_t)kBinDead;
-    const uint32_t window = slot / kWindow;
-    const uint32_t peers = __match_any_sync(0xffffffffu, so.finished ? window : 0xffffffffu);
-    if (so.finished && lane == (uint32_t)__ffs(peers) - 1u) atomicSub(&q.win_count[window], (uint32_t)__popc(peers));
-    if (METHOD == PTB_METHOD_MIS) {
-      const uint32_t m_sh = __ballot_sync(0xffffffffu, so.shadow), m_sky = __ballot_sync(0xffffffffu, so.shadow && so.shadow_is_sky);
-      unsigned long long p2 = 0ull;
-      if (lane == 0u && m_sh)
-        p2 = atomicAdd(&wc->shadow_pair, ((unsigned long long)__popc(m_sky) << 32) | (unsigned long long)__popc(m_sh));
-      p2 = __shfl_sync(0xffffffffu, p2, 0);
-      if (so.shadow) {
-        float4* e = q.shadow + 3u * (size_t)((uint32_t)p2 + __popc(m_sh & ((1u << lane) - 1u)));
-        e[0] = so.sh_o;
-        e[1] = so.sh_d;
-        e[2] = so.sh_c;
-      }
+  // Paths stay in their slot. A finished path is marked dead and leaves its window's live count (lanes of a warp nearly
+  // always share the window: one atomic per warp); NEE rays go to the shadow queue.
+  if (so.alive) q.bin[slot] = (uint8_t)so.bin;
+  if (so.finished) q.bin[slot] = (uint8_t)kBinDead;
+  const uint32_t window = slot / kWindow;
+  const uint32_t peers = __match_any_sync(0xffffffffu, so.finished ? window : 0xffffffffu);
+  if (so.finished && lane == (uint32_t)__ffs(peers) - 1u) atomicSub(&q.win_count[window], (uint32_t)__popc(peers));
+  if (METHOD == PTB_METHOD_MIS) {
+    const uint32_t m_sh = __ballot_sync(0xffffffffu, so.shadow), m_sky = __ballot_sync(0xffffffffu, so.shadow && so.shadow_is_sky);
+    unsigned long long p2 = 0ull;
+    if (lane == 0u && m_sh)
+      p2 = atomicAdd(&wc->shadow_pair, ((unsigned long long)__popc(m_sky) << 32) | (unsigned long long)__popc(m_sh));
+    p2 = __shfl_sync(0xffffffffu, p2, 0);
+    if (so.shadow) {
+      float4* e = q.shadow + 3u * (size_t)((uint32_t)p2 + __popc(m_sh & ((1u << lane) - 1u)));
+      e[0] = so.sh_o;
+      e[1] = so.sh_d;
+      e[2] = so.sh_c;
     }
-  } else {
-  // ---- warp-aggregated queue pushes: lane 0 issues both returning atomics back to back (their round trips overlap)
-  {
-    const uint32_t m_alive = __ballot_sync(0xffffffffu, so.alive), m_fin = __ballot_sync(0xffffffffu, so.finished);
-    const uint32_t m_sh = METHOD == PTB_METHOD_MIS ? __ballot_sync(0xffffffffu, so.shadow) : 0u;
-    const uint32_t m_sky = METHOD == PTB_METHOD_MIS ? __ballot_sync(0xffffffffu, so.shadow && so.shadow_is_sky) : 0u;
-    unsigned long long p1 = 0ull, p2 = 0ull;
-    if (lane == 0u) {
-      if (m_alive | m_fin)
-        p1 = atomicAdd(&wc->push_pair, ((unsigned long long)__popc(m_fin) << 32) | (unsigned long long)__popc(m_alive));
-      if (METHOD == PTB_METHOD_MIS && m_sh)
-        p2 = atomicAdd(&wc->shadow_pair, ((unsigned long long)__popc(m_sky) << 32) | (unsigned long long)__popc(m_sh));
-    }
-    p1 = __shfl_sync(0xffffffffu, p1, 0);
-    const uint32_t below = (1u << lane) - 1u;
-    if (so.alive) q.active[nxt][(uint32_t)p1 + __popc(m_alive & below)] = slot;
-    if (so.finished) q.free_slots[(uint32_t)(p1 >> 32) + __popc(m_fin & below)] = slot;
-    if (METHOD == PTB_METHOD_MIS) {
-      p2 = __shfl_sync(0xffffffffu, p2, 0);
-      if (so.shadow) {
-        float4* e = q.shadow + 3u * (size_t)((uint32_t)p2 + __popc(m_sh & below));
-        e[0] = so.sh_o;
-        e[1] = so.sh_d;
-        e[2] = so.sh_c;
-      }
-    }
-  }
   }
   }  // grid-stride
 }
 
 // ------------------------------------------------------------------------------------------ window wavefront
-// When every camera path of a chunk fits the pool, the wavefront needs no free list and no compaction of scattered slots:
+// Every camera path of a chunk is resident, so the wavefront needs no free list and no compaction of scattered slots:
 // path g of the chunk lives in slot g for its whole life (pixel-major, the samples of a pixel adjacent), and each
 // iteration's trace queue is rebuilt IN SLOT ORDER from per-slot state: k_shade leaves a direction bin (or "dead") per
 // slot and keeps a live count per 4096-slot window; a prefix sum over the window counts places every window's live slots
@@ -1147,7 +1008,7 @@ __global__ void k_win_prepare(WaveCounters* wc, Queues q, uint32_t n_segments, u
     wc->rays_shadow_light += (uint32_t)sp - (uint32_t)(sp >> 32);
     if (prev == 1u) wc->rays_camera += traced;
     else wc->rays_bounce += traced;
-    wc->rays_reference += method == PTB_METHOD_NAIVE ? traced : survivors;  // Q7, as k_prepare
+    wc->rays_reference += method == PTB_METHOD_NAIVE ? traced : survivors;  // Q7: naive 1/check_hit, MIS 1/bounce iteration
     wc->paths += traced - survivors;
   }
   if (mode == 0u) {
@@ -1158,9 +1019,8 @@ __global__ void k_win_prepare(WaveCounters* wc, Queues q, uint32_t n_segments, u
   }
   wc->mode = mode;
   wc->n_trace = mode == 0u ? total : 0u;
-  wc->cur = 0;
   wc->shadow_pair = 0;
-  wc->trace_head = wc->shade_head = wc->shadow_head = 0;
+  wc->trace_head = wc->shadow_head = 0;
 }
 
 constexpr uint32_t kFillGroup = 8u;  // windows whose live counts a k_win_fill block fetches (and skips) together
@@ -1240,7 +1100,7 @@ __global__ void __launch_bounds__(256) k_win_fill(Queues q, WaveCounters* wc) {
       __syncthreads();
 #pragma unroll
       for (uint32_t k = 0; k < kWinItems; ++k)
-        if (bins[k] != kBinDead) q.active[0][hist[bins[k]] + offs[k]] = first_slot + tid * kWinItems + k;
+        if (bins[k] != kBinDead) q.live[hist[bins[k]] + offs[k]] = first_slot + tid * kWinItems + k;
       buf ^= 1u;
     }
   }
@@ -1341,7 +1201,7 @@ template <class TR, int METHOD, bool FULL>
 __global__ void __launch_bounds__(kTailThreads)
 k_tail(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp, float* __restrict__ accum, uint32_t depth) {
   if (wc->tail_iter != depth) return;  // launched after every iteration >= 2; only the hand-over iteration's launch has work
-  const uint32_t n = wc->n_tail;   // live paths, listed in q.active[0] by k_win_fill
+  const uint32_t n = wc->n_tail;   // live paths, listed in q.live by k_win_fill
   if (threadIdx.x == 0u) atomicMin(&wc->tail_t0, global_timer_ns());
 #ifdef PTB_TAIL_STATS
   if (threadIdx.x == 0u) atomicMin(&g_tail_stats[9], global_timer_ns());
@@ -1365,7 +1225,7 @@ k_tail(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp, 
         if (t < n) {
           uint32_t i = t;
           do { i = (i * 0x9E3779B1u) & mask; } while (i >= n);
-          slot = q.active[0][i];
+          slot = q.live[i];
         } else {
           exhausted = true;
         }
@@ -1432,7 +1292,7 @@ k_tail(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp, 
     for (;;) {
       const uint32_t i = atomicAdd(&wc->tail_head, 1u);
       if (i >= n) break;
-      const uint32_t s = q.active[0][i];
+      const uint32_t s = q.live[i];
       for (;;) {
         float4 o4, d4;
         ldg256_rw(pool.ray + 4u * (size_t)s, o4, d4);
@@ -1730,13 +1590,12 @@ int32_t sampler_hook(Ctx* c, const ptb_sampler_query& q, size_t n, const float* 
 
 // ---- kernel tables: every persistent traversal kernel exists once per tree (BinTrav / CwTrav)
 template <class TR>
-static const void* trace_kernel_of(bool count, bool dense, bool camera) {
-  if (!dense) return count ? (const void*)k_trace<TR, true, false, false> : (const void*)k_trace<TR, false, false, false>;
-  if (camera) return count ? (const void*)k_trace<TR, true, true, true> : (const void*)k_trace<TR, false, true, true>;
-  return count ? (const void*)k_trace<TR, true, true, false> : (const void*)k_trace<TR, false, true, false>;
+static const void* trace_kernel_of(bool count, bool camera) {
+  if (camera) return count ? (const void*)k_trace<TR, true, true> : (const void*)k_trace<TR, false, true>;
+  return count ? (const void*)k_trace<TR, true, false> : (const void*)k_trace<TR, false, false>;
 }
-static const void* trace_kernel(const Ctx* c, bool count, bool dense, bool camera) {
-  return c->wide ? trace_kernel_of<CwTrav>(count, dense, camera) : trace_kernel_of<BinTrav>(count, dense, camera);
+static const void* trace_kernel(const Ctx* c, bool count, bool camera) {
+  return c->wide ? trace_kernel_of<CwTrav>(count, camera) : trace_kernel_of<BinTrav>(count, camera);
 }
 static const void* shadow_kernel(const Ctx* c) { return c->wide ? (const void*)k_shadow<CwTrav> : (const void*)k_shadow<BinTrav>; }
 static const void* api_kernel(const Ctx* c, bool count) {
@@ -1851,10 +1710,9 @@ int32_t launch_visibility(Ctx* c, const void* d_rays, const void* d_index, size_
 }
 
 // bytes of device state per path in flight
-static unsigned long long bytes_per_path(bool mis, bool windows) {
-  // 64-byte path block + queues (window mode: the live-slot queue + one bin byte; queue mode: 2 active, free, kNumKinds
-  // shade queues) + MIS: previous-hit record, 48-byte shadow entry
-  return 64ull + (windows ? 4ull + 1ull : 4ull * (3 + kNumKinds)) + (mis ? 16ull + 48ull : 0ull);
+static unsigned long long bytes_per_path(bool mis) {
+  // 64-byte path block + the live-slot queue + one bin byte + MIS: previous-hit record, 48-byte shadow entry
+  return 64ull + 4ull + 1ull + (mis ? 16ull + 48ull : 0ull);
 }
 
 void free_render_state(Ctx* c) {
@@ -1869,16 +1727,16 @@ void free_render_state(Ctx* c) {
 // the path state is bounded: two chunk slots of together PTB_POOL_BYTES (default 8 GiB), never more than half of the
 // device memory that was free at the context's first large render. A call is cut into equal chunks of at most one slot;
 // all tails but the last chunk's are hidden under the next chunk.
-// PTB_POOL_PATHS sets the slot size directly (tests; the queue mode's pool).
+// PTB_POOL_PATHS sets the slot size directly (tests).
 struct PoolPlan {
   uint32_t slot_paths;  // capacity of one slot (multiple of kWindow)
   uint32_t n_chunks;
   uint32_t chunk_paths; // paths per chunk (the last one may be shorter)
 };
-static PoolPlan plan_pool(Ctx* c, unsigned long long total, bool mis, bool windows) {
+static PoolPlan plan_pool(Ctx* c, unsigned long long total, bool mis) {
   unsigned long long budget = 8ull << 30;
   if (const char* e = getenv("PTB_POOL_BYTES")) { unsigned long long v = strtoull(e, nullptr, 10); if (v >= (64ull << 20)) budget = v; }
-  const unsigned long long per_path = bytes_per_path(mis, windows);
+  const unsigned long long per_path = bytes_per_path(mis);
   unsigned long long cap = 0;
   if (const char* e = getenv("PTB_POOL_PATHS")) {
     unsigned long long v = strtoull(e, nullptr, 10);
@@ -1897,7 +1755,7 @@ static PoolPlan plan_pool(Ctx* c, unsigned long long total, bool mis, bool windo
     // extra chunk adds the drain of five more persistent launches: measured, profiles/r2_sweeps.md); a larger one
     // alternates between two slots of half the budget each
     cap = budget / per_path;
-    if (windows && total > cap) cap = budget / 2ull / per_path;
+    if (total > cap) cap = budget / 2ull / per_path;
     if (cap > (1ull << 29)) cap = 1ull << 29;
     if (cap < (1ull << 20)) cap = 1ull << 20;
   }
@@ -1917,47 +1775,36 @@ static PoolPlan plan_pool(Ctx* c, unsigned long long total, bool mis, bool windo
 
 struct RenderSetup {
   RenderParams rp;
-  Queues q;            // slot 0 (queue mode: the only one)
-  Queues q2;           // slot 1 (window mode, calls of more than one chunk)
+  Queues q;            // slot 0
+  Queues q2;           // slot 1 (calls of more than one chunk)
   PathPool pool2;
   WaveCounters* wc;
   WaveCounters* wc2;
   float* accum;
-  uint32_t P;          // slot capacity in paths
   uint32_t chunk_paths, n_chunks;
   bool mis, full, count, prof;
-  bool sort_kinds = false;  // window mode: k_shade sorts each block's hits by material kind
+  bool sort_kinds = false;  // k_shade sorts each block's hits by material kind
 };
 
-static int32_t render_queue_mode(Ctx* c, const ptb_render_opts& o, const RenderSetup& rs, ptb_progress_fn progress, void* user);
 static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const RenderSetup& rs, ptb_progress_fn progress, void* user);
 
 // carve one slot's queue / window arrays out of its buffers
-static void bind_slot(Queues& q, PathPool& pool, uint32_t P, bool windows, DevBuf& pool_mem, DevBuf& prev, DevBuf& queues,
-                      DevBuf& shadow, DevBuf& win) {
+static void bind_slot(Queues& q, PathPool& pool, uint32_t P, DevBuf& pool_mem, DevBuf& prev, DevBuf& queues, DevBuf& shadow,
+                      DevBuf& win) {
   pool.capacity = P;
   pool.ray = pool_mem.as<float4>();
   pool.col = pool.ray + 2;
   pool.prev = prev.as<float4>();
-  uint32_t* b = queues.as<uint32_t>();
-  q.active[0] = b; b += P;
-  if (windows) b = queues.as<uint32_t>();  // window mode uses active[0] only
-  q.active[1] = b; b += windows ? 0 : P;
-  q.free_slots = b; b += windows ? 0 : P;
-  for (int k = 0; k < kNumKinds; ++k) { q.kind[k] = b; b += windows ? 0 : P; }
+  q.live = queues.as<uint32_t>();
   q.shadow = shadow.as<float4>();
   q.n_windows = P / kWindow;  // P is a multiple of kWindow
   const size_t n_seg = (q.n_windows + kSegWindows - 1) / kSegWindows;
-  q.win_count = q.win_prefix = q.seg_total = nullptr;
-  q.bin = nullptr;
-  if (windows) {
-    const size_t words = ((size_t)q.n_windows * 2 + n_seg + 3) & ~(size_t)3;  // keeps the byte array 16-byte aligned
-    uint32_t* w = win.as<uint32_t>();
-    q.win_count = w;
-    q.win_prefix = w + q.n_windows;
-    q.seg_total = w + 2 * (size_t)q.n_windows;
-    q.bin = reinterpret_cast<uint8_t*>(w + words);  // k_win_fill reads a window's 256 bytes as 32 x uint2
-  }
+  const size_t words = ((size_t)q.n_windows * 2 + n_seg + 3) & ~(size_t)3;  // keeps the byte array 16-byte aligned
+  uint32_t* w = win.as<uint32_t>();
+  q.win_count = w;
+  q.win_prefix = w + q.n_windows;
+  q.seg_total = w + 2 * (size_t)q.n_windows;
+  q.bin = reinterpret_cast<uint8_t*>(w + words);  // k_win_fill reads a window's 256 bytes as 32 x uint2
 }
 
 int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progress, void* user) {
@@ -1967,36 +1814,25 @@ int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progr
   if (total == 0) return PTB_OK;
   RenderSetup rs;
   rs.mis = o.method == PTB_METHOD_MIS;
-  // Window mode (default) needs chunks long enough to keep its wide iterations wide: at least 32 Mi paths per slot, or the
-  // whole call in one chunk. PTB_WAVEFRONT=queue forces the regenerating queue mode, =window the window mode.
-  bool windows = true, forced_windows = false;
-  if (const char* e = getenv("PTB_WAVEFRONT")) {
-    windows = strcmp(e, "queue") != 0;
-    forced_windows = strcmp(e, "window") == 0;
-  }
-  PoolPlan plan = plan_pool(c, total, rs.mis, windows);
-  if (windows && !forced_windows && plan.n_chunks > 1 && plan.slot_paths < (1u << 22)) {
-    windows = false;
-    plan = plan_pool(c, total, rs.mis, false);
-  }
+  PoolPlan plan = plan_pool(c, total, rs.mis);
   // ---- device state (grow-only across calls; the MIS-only arrays are allocated by the first MIS call)
   // one 64-byte block per path: ray record then colour record (a DRAM access atom; two scattered 32-byte sectors per
-  // path cost generate/shade ~1 TB/s of effective write bandwidth). If the device cannot provide the slots (another
+  // path cost ~1 TB/s of effective write bandwidth). If the device cannot provide the slots (another
   // process holds the memory), they are halved and the call runs in more chunks.
   uint32_t P = plan.slot_paths;
   for (;;) {
-    const bool two = windows && plan.n_chunks > 1;
+    const bool two = plan.n_chunks > 1;
     const size_t n_seg = ((size_t)P / kWindow + kSegWindows - 1) / kSegWindows;
-    const size_t win_bytes = windows ? ((((size_t)P / kWindow * 2 + n_seg + 3) & ~(size_t)3) * 4 + (size_t)P) : 0;
+    const size_t win_bytes = (((size_t)P / kWindow * 2 + n_seg + 3) & ~(size_t)3) * 4 + (size_t)P;
     cudaError_t e = cudaSuccess;
     DevBuf* sets[2][5] = {{&c->d_pool_mem, &c->d_queues, &c->d_prev, &c->d_shadow, &c->d_windows},
                           {&c->d_pool_mem2, &c->d_queues2, &c->d_prev2, &c->d_shadow2, &c->d_windows2}};
     for (int sl = 0; sl < (two ? 2 : 1) && e == cudaSuccess; ++sl) {
       e = sets[sl][0]->reserve((size_t)P * 64);
-      if (e == cudaSuccess) e = sets[sl][1]->reserve((size_t)P * 4 * (windows ? 1 : 3 + kNumKinds));
+      if (e == cudaSuccess) e = sets[sl][1]->reserve((size_t)P * 4);
       if (e == cudaSuccess && rs.mis) e = sets[sl][2]->reserve((size_t)P * 16);
       if (e == cudaSuccess && rs.mis) e = sets[sl][3]->reserve((size_t)P * 48);
-      if (e == cudaSuccess && windows) e = sets[sl][4]->reserve(win_bytes);
+      if (e == cudaSuccess) e = sets[sl][4]->reserve(win_bytes);
     }
     if (e == cudaSuccess) break;
     if (e != cudaErrorMemoryAllocation || P <= (1u << 20)) return check_cuda(c, e, "path pool allocation");
@@ -2005,17 +1841,15 @@ int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progr
     P = (P / 2 + kWindow - 1) / kWindow * kWindow;
     plan.slot_paths = plan.chunk_paths = P;
     plan.n_chunks = (uint32_t)((total + P - 1ull) / P);
-    if (windows && P < (1u << 22) && !forced_windows) windows = false;  // too many chunks for window mode
   }
-  rs.P = P;
   rs.chunk_paths = plan.chunk_paths;
   rs.n_chunks = plan.n_chunks;
   PTB_CUDA_TRY(c, c->d_counters.reserve(sizeof(WaveCounters) + 64));
   PTB_CUDA_TRY(c, c->d_counters2.reserve(sizeof(WaveCounters) + 64));
-  bind_slot(rs.q, c->pool, P, windows, c->d_pool_mem, c->d_prev, c->d_queues, c->d_shadow, c->d_windows);
+  bind_slot(rs.q, c->pool, P, c->d_pool_mem, c->d_prev, c->d_queues, c->d_shadow, c->d_windows);
   rs.q2 = rs.q;
   rs.pool2 = c->pool;
-  if (windows && plan.n_chunks > 1) bind_slot(rs.q2, rs.pool2, P, windows, c->d_pool_mem2, c->d_prev2, c->d_queues2, c->d_shadow2, c->d_windows2);
+  if (plan.n_chunks > 1) bind_slot(rs.q2, rs.pool2, P, c->d_pool_mem2, c->d_prev2, c->d_queues2, c->d_shadow2, c->d_windows2);
   rs.wc = c->d_counters.as<WaveCounters>();
   rs.wc2 = c->d_counters2.as<WaveCounters>();
   if (!c->h_counters) PTB_CUDA_TRY(c, cudaMallocHost(&c->h_counters, 10 * sizeof(WaveCounters)));
@@ -2025,7 +1859,7 @@ int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progr
   rp.row_begin = o.row_begin;
   // Pixel issue order: 32 consecutive pixel indices cover an 8 x 4 tile when the image allows (else 16 x 2, else a row), so
   // the 16 pixels of a 4096-slot window are an 8 x 2 block instead of a 16 x 1 strip: the origins of a window's rays lie
-  // closer together. Window mode, C3: 3793 -> 3834 Mrays/s (queue mode preferred rows). PTB_TILES=0 keeps rows.
+  // closer together. C3: 3793 -> 3834 Mrays/s. PTB_TILES=0 keeps rows.
   rp.tile_w = 32u; rp.tile_h = 1u;
   bool tiles = true;
   if (const char* e = getenv("PTB_TILES")) tiles = atoi(e) != 0;
@@ -2065,12 +1899,11 @@ int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progr
     for (cudaEvent_t& e : c->ev_prof)
       if (!e) PTB_CUDA_TRY(c, cudaEventCreate(&e));
   }
-  return windows ? render_window_mode(c, o, rs, progress, user) : render_queue_mode(c, o, rs, progress, user);
+  return render_window_mode(c, o, rs, progress, user);
 }
 
-// ev_prof[(iter & 3) * 8 + 2 * k + {0,1}] brackets kernel class k (0 generate + bookkeeping, 1 trace, 2 shade, 3 shadow)
-#define PTB_PROF(k, which) \
-  if (prof) cudaEventRecord(c->ev_prof[(int)(iter & 3u) * 8 + 2 * (k) + (which)], st)
+// ev_prof[(slot * 4 + (iter & 3)) * 8 + 2 * k + {0,1}] brackets kernel class k (0 window bookkeeping, 1 trace, 2 shade,
+// 3 shadow)
 static void prof_collect(Ctx* c, int half, bool mis) {  // half = ring position (+ 4 for the second slot's ring)
   double* prof_ms[4] = {&c->stats.ms_generate, &c->stats.ms_trace, &c->stats.ms_shade, &c->stats.ms_shadow};
   static const bool timeline = getenv("PTB_TIMELINE") != nullptr;  // tuning aid: where each iteration sits inside the render
@@ -2137,16 +1970,15 @@ struct SlotRefs {  // the device state one chunk runs in
   const Queues& q;
   WaveCounters* wc;
 };
-template <bool DENSE>
 static void launch_shade(const RenderSetup& rs, Ctx* c, const SlotRefs& sl, uint32_t grid, int threads, cudaStream_t st,
-                         unsigned long long camera_first = kNoCamera) {
-  const uint32_t sort = DENSE && rs.sort_kinds ? 1u : 0u;
+                         unsigned long long camera_first) {
+  const uint32_t sort = rs.sort_kinds ? 1u : 0u;
   if (rs.mis) {
-    if (rs.full) k_shade<PTB_METHOD_MIS, true, DENSE><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
-    else k_shade<PTB_METHOD_MIS, false, DENSE><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
+    if (rs.full) k_shade<PTB_METHOD_MIS, true><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
+    else k_shade<PTB_METHOD_MIS, false><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
   } else {
-    if (rs.full) k_shade<PTB_METHOD_NAIVE, true, DENSE><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
-    else k_shade<PTB_METHOD_NAIVE, false, DENSE><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
+    if (rs.full) k_shade<PTB_METHOD_NAIVE, true><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
+    else k_shade<PTB_METHOD_NAIVE, false><<<grid, threads, 0, st>>>(c->dev, sl.pool, sl.q, sl.wc, rs.rp, rs.accum, camera_first, sort);
   }
 }
 static const void* tail_fn(const RenderSetup& rs, Ctx* c) {
@@ -2159,10 +1991,9 @@ static void launch_tail(const RenderSetup& rs, Ctx* c, const SlotRefs& sl, uint3
   void* args[] = {(void*)&c->dev, (void*)&sl.pool, (void*)&sl.q, (void*)&wc, (void*)&rs.rp, (void*)&accum, (void*)&depth};
   cudaLaunchKernel(fn, dim3(grid), dim3(kTailThreads), args, 0, st);
 }
-template <bool DENSE>
 static const void* shade_fn(const RenderSetup& rs) {
-  return rs.mis ? (rs.full ? (const void*)k_shade<PTB_METHOD_MIS, true, DENSE> : (const void*)k_shade<PTB_METHOD_MIS, false, DENSE>)
-                : (rs.full ? (const void*)k_shade<PTB_METHOD_NAIVE, true, DENSE> : (const void*)k_shade<PTB_METHOD_NAIVE, false, DENSE>);
+  return rs.mis ? (rs.full ? (const void*)k_shade<PTB_METHOD_MIS, true> : (const void*)k_shade<PTB_METHOD_MIS, false>)
+                : (rs.full ? (const void*)k_shade<PTB_METHOD_NAIVE, true> : (const void*)k_shade<PTB_METHOD_NAIVE, false>);
 }
 
 // ---- window mode: chunk by chunk, every path of a chunk resident, one bounce of all of them per iteration.
@@ -2186,16 +2017,16 @@ static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const Render
   // (window mode, C3: 256 threads 3438 Mrays/s, 128 -> 3500, 64 -> 3499)
   int TS = 128;
   if (const char* e = getenv("PTB_SHADE_THREADS")) { int v = atoi(e); if (v == 64 || v == 128 || v == 256) TS = v; }
-  uint32_t grid_shade = (uint32_t)persistent_grid(c, shade_fn<true>(rs), TS);
+  uint32_t grid_shade = (uint32_t)persistent_grid(c, shade_fn(rs), TS);
   if (grid_shade > (P + TS - 1) / TS) grid_shade = (P + TS - 1) / TS;
-  const void* fn_trace = trace_kernel(c, count, true, false);
+  const void* fn_trace = trace_kernel(c, count, false);
   // camera rays of the binary tree walk it in packets (PTB_CAMERA_PACKET=0: the persistent kernel, as the wide tree does)
   // — when a warp's 32 work items are samples of ONE pixel (group a multiple of 32). C3 on B200: 256 spp 4256 -> 4344 Mrays/s;
   // with 4 samples per pixel a warp spans eight pixels and the packet loses (7.32 vs 6.75 ms per 4-spp step).
   bool cam_packet = !c->wide && rs.rp.group % 32u == 0u;
   if (const char* e = getenv("PTB_CAMERA_PACKET")) cam_packet = !c->wide && atoi(e) != 0;
   const void* fn_trace_cam = cam_packet ? (count ? (const void*)k_trace_camera<true> : (const void*)k_trace_camera<false>)
-                                        : trace_kernel(c, count, true, true);
+                                        : trace_kernel(c, count, true);
   const void* fn_shadow = shadow_kernel(c);
   const int grid_trace = persistent_grid(c, fn_trace, T);
   const int grid_trace_cam = persistent_grid(c, fn_trace_cam, T);
@@ -2270,8 +2101,8 @@ static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const Render
   cudaStream_t wst[2] = {st, chunk_streams == 2 ? c->s_work2 : st};
 
   PTB_CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
-  k_init_pool<<<1, 32, 0, st>>>(rs.q.active[0], 0u, rs.wc, total);   // counters only
-  k_init_pool<<<1, 32, 0, st>>>(rs.q2.active[0], 0u, rs.wc2, total);
+  k_reset_counters<<<1, 1, 0, st>>>(rs.wc);
+  k_reset_counters<<<1, 1, 0, st>>>(rs.wc2);
   c->stats.kernel_launches += 2;
   if (chunk_streams == 2) {  // the second stream starts after whatever the caller queued before this render
     PTB_CUDA_TRY(c, cudaEventRecord(c->ev_fork, st));
@@ -2347,7 +2178,7 @@ static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const Render
     }
     prof_rec(sl, depth, 1, 1);
     prof_rec(sl, depth, 2, 0);
-    launch_shade<true>(rs, c, S, grid_shade, TS, s, depth == 0 ? R.first : kNoCamera);
+    launch_shade(rs, c, S, grid_shade, TS, s, depth == 0 ? R.first : kNoCamera);
     prof_rec(sl, depth, 2, 1);
     c->stats.kernel_launches += depth ? 5 : 4;
     c->stats.trace_launches += 1;
@@ -2447,99 +2278,5 @@ static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const Render
   }
   return rc;
 }
-
-// ---- queue mode: a pool smaller than the call; freed slots are refilled with new camera paths every iteration
-static int32_t render_queue_mode(Ctx* c, const ptb_render_opts& o, const RenderSetup& rs, ptb_progress_fn progress, void* user) {
-  cudaStream_t st = c->stream;
-  const Queues& q = rs.q;
-  WaveCounters* wc = rs.wc;
-  const RenderParams& rp = rs.rp;
-  const uint32_t npix = rp.npix, P = rs.P;
-  const unsigned long long total = (unsigned long long)npix * o.samples_per_pixel;
-  const bool mis = rs.mis, prof = rs.prof, count = rs.count;
-  const int T = 256;
-  const uint32_t grid_p = (P + T - 1) / T;
-  auto capped = [&](const void* k) { const int g = persistent_grid(c, k, T); return (uint32_t)g < grid_p ? (uint32_t)g : grid_p; };
-  const uint32_t grid_gen = capped((const void*)k_generate);
-  // k_shade is register-heavy (MIS: ~130): smaller blocks let more of them share an SM's register file
-  int TS = mis ? 128 : 256;
-  if (const char* e = getenv("PTB_SHADE_THREADS")) { int v = atoi(e); if (v == 64 || v == 128 || v == 256) TS = v; }
-  uint32_t grid_shade = (uint32_t)persistent_grid(c, shade_fn<false>(rs), TS);
-  if (grid_shade > (P + TS - 1) / TS) grid_shade = (P + TS - 1) / TS;
-  const void* fn_trace = trace_kernel(c, count, false, false);
-  const void* fn_shadow = shadow_kernel(c);
-  const int grid_trace = persistent_grid(c, fn_trace, T);
-  const int grid_shadow = persistent_grid(c, fn_shadow, T);
-
-  PTB_CUDA_TRY(c, cudaEventRecord(c->ev_a, st));
-  k_init_pool<<<grid_p, T, 0, st>>>(q.free_slots, P, wc, total);
-  c->stats.kernel_launches += 1;
-
-  int32_t rc = PTB_OK;
-  uint64_t iter = 0;
-  uint64_t last_pass_reported = 0;
-  bool done = false;
-  // Two pinned mirrors + events so the host inspects iteration k-1 while iteration k runs.
-  cudaEvent_t ev[2] = {c->ev_iter, c->ev_b};
-  while (!done) {
-    k_prepare<<<1, 1, 0, st>>>(wc, o.method, iter == 0 ? 1u : 0u);
-    PTB_PROF(0, 0);
-    k_generate<<<grid_gen, T, 0, st>>>(c->dev, c->pool, q, wc, rp);
-    PTB_PROF(0, 1);
-    k_advance<<<1, 1, 0, st>>>(wc);
-    PTB_PROF(1, 0);
-    PTB_CUDA_TRY(c, launch_trace(fn_trace, grid_trace, st, c->dev, c->pool, q, wc, rp, 0ull));
-    PTB_PROF(1, 1);
-    PTB_PROF(2, 0);
-    launch_shade<false>(rs, c, SlotRefs{c->pool, q, wc}, grid_shade, TS, st);
-    PTB_PROF(2, 1);
-    c->stats.kernel_launches += 5;
-    c->stats.trace_launches += 1;
-    if (mis) {
-      PTB_PROF(3, 0);
-      PTB_CUDA_TRY(c, launch_shadow(fn_shadow, grid_shadow, st, c->dev, c->pool, q, wc));
-      PTB_PROF(3, 1);
-      c->stats.kernel_launches += 1;
-    }
-    const int slot = (int)(iter & 1u);
-    PTB_CUDA_TRY(c, cudaMemcpyAsync(c->h_counters + slot, wc, sizeof(WaveCounters), cudaMemcpyDeviceToHost, st));
-    PTB_CUDA_TRY(c, cudaEventRecord(ev[slot], st));
-    if (iter > 0) {  // inspect the previous iteration (already finished or about to)
-      const int ps = slot ^ 1;
-      PTB_CUDA_TRY(c, cudaEventSynchronize(ev[ps]));
-      if (prof) prof_collect(c, (int)((iter - 1) & 3u), mis);
-      const WaveCounters& h = c->h_counters[ps];
-      if (h.next_sample >= h.total_samples && (uint32_t)h.push_pair == 0u) done = true;
-      if (progress && !done) {
-        const uint64_t passes = h.next_sample / npix;
-        if (passes != last_pass_reported) {
-          last_pass_reported = passes;
-          if (progress(user, passes, h.rays_reference)) { rc = PTB_ERR_ABORTED; done = true; }
-        }
-      }
-    }
-    ++iter;
-    if (iter > (1ull << 40)) return set_error(c, PTB_ERR_INVALID, "wavefront did not terminate");
-  }
-  // fold the last iteration's counts into the statistics
-  k_prepare<<<1, 1, 0, st>>>(wc, o.method, 0u);
-  c->stats.kernel_launches += 1;
-  PTB_CUDA_TRY(c, cudaMemcpyAsync(c->h_counters, wc, sizeof(WaveCounters), cudaMemcpyDeviceToHost, st));
-  PTB_CUDA_TRY(c, cudaEventRecord(c->ev_b, st));
-  PTB_CUDA_TRY(c, cudaStreamSynchronize(st));
-  PTB_CUDA_TRY(c, cudaGetLastError());
-  if (prof && iter > 0) prof_collect(c, (int)((iter - 1) & 3u), mis);
-  float ms = 0.f;
-  cudaEventElapsedTime(&ms, c->ev_a, c->ev_b);
-  const WaveCounters& h = c->h_counters[0];
-  fold_counters(c, h, iter);
-  c->stats.render_ms = ms;
-  if (rc == PTB_OK) {
-    c->accum_samples += o.samples_per_pixel;
-    if (progress) progress(user, o.samples_per_pixel, h.rays_reference);
-  }
-  return rc;
-}
-#undef PTB_PROF
 
 }  // namespace ptb

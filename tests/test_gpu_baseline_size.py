@@ -103,10 +103,8 @@ def test_c3_bench_chunking_is_the_same_image(ptb, gpu_ctx, c3_full, monkeypatch)
     sc = ptb.Scene(c3_full, ctx=gpu_ctx)
     o = ptb.RenderOptions(samples_per_pixel=spp, render_method=0, width=w, height=h, seed=23)
     a = sc.render(o)
-    monkeypatch.setenv("PTB_WAVEFRONT", "window")
     monkeypatch.setenv("PTB_POOL_PATHS", str(1 << 21))
     b = sc.render(o)
-    monkeypatch.delenv("PTB_WAVEFRONT")
     monkeypatch.delenv("PTB_POOL_PATHS")
     assert np.max(np.abs(a - b)) < 1e-5
 

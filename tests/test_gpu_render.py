@@ -122,6 +122,7 @@ def test_sample_offset_sharding_is_exact(ptb, gpu_ctx, rtweekend1):
 
 
 def test_determinism_and_pool_size_independence(ptb, gpu_ctx, rtweekend1, monkeypatch):
+    """The image does not depend on the pool size: one chunk vs 4096-path slots (18 chunks of the window wavefront)."""
     sc = ptb.Scene(rtweekend1, ctx=gpu_ctx)
     o = ptb.RenderOptions(samples_per_pixel=8, render_method=1, width=128, height=72, seed=5)
     a = sc.render(o)
@@ -132,6 +133,8 @@ def test_determinism_and_pool_size_independence(ptb, gpu_ctx, rtweekend1, monkey
 
 
 def test_progress_callback_and_abort(ptb, gpu_ctx, rtweekend1):
+    """The progress callback ends at the call's spp; a non-zero return aborts a render of many small chunks
+    (PTB_POOL_PATHS=1024 rounds up to one 4096-slot window per chunk)."""
     sc = ptb.Scene(rtweekend1, ctx=gpu_ctx)
     seen = []
     sc.render(ptb.RenderOptions(samples_per_pixel=4, render_method=0, width=64, height=36), update=lambda s, r: seen.append((s, r)) or False)
@@ -215,9 +218,9 @@ def test_converged_images_agree_with_independent_samples(ptb, orc, gpu_ctx, rtwe
 
 
 @pytest.mark.parametrize("method", [0, 1])
-def test_window_and_queue_wavefronts_agree(ptb, gpu_ctx, overshadowed, method, monkeypatch):
-    """The window wavefront (default: every path resident, slot = generation index), its chunked form and the
-    regenerating queue mode trace the same paths: same image (f32 summation order aside), same ray counters."""
+def test_chunked_window_wavefront_agrees(ptb, gpu_ctx, overshadowed, method, monkeypatch):
+    """The window wavefront in one chunk (every path resident, slot = generation index) and in 8 chunks trace the same
+    paths: same image (f32 summation order aside), same ray counters."""
     sc = ptb.Scene(overshadowed, ctx=gpu_ctx)
     o = ptb.RenderOptions(samples_per_pixel=12, render_method=method, width=96, height=54, seed=9)
 
@@ -228,29 +231,23 @@ def test_window_and_queue_wavefronts_agree(ptb, gpu_ctx, overshadowed, method, m
         return img, (st.rays_camera, st.rays_bounce, st.rays_shadow_light, st.rays_shadow_sky, st.rays_reference, st.paths)
 
     a, ca = run()
-    monkeypatch.setenv("PTB_WAVEFRONT", "window")
     monkeypatch.setenv("PTB_POOL_PATHS", "8192")  # 62 208 paths -> 8 chunks
     b, cb = run()
-    monkeypatch.setenv("PTB_WAVEFRONT", "queue")
-    c, cc = run()
-    monkeypatch.delenv("PTB_WAVEFRONT")
     monkeypatch.delenv("PTB_POOL_PATHS")
     assert ca[0] == 96 * 54 * 12 and ca[5] == 96 * 54 * 12
-    assert ca == cb == cc
-    assert np.allclose(a, b, rtol=1e-5, atol=1e-5) and np.allclose(a, c, rtol=1e-5, atol=1e-5)
+    assert ca == cb
+    assert np.allclose(a, b, rtol=1e-5, atol=1e-5)
 
 
 def test_abort_between_chunks_in_window_mode(ptb, gpu_ctx, rtweekend1, monkeypatch):
     """Window mode calls the progress callback after each chunk; a non-zero return aborts the render (PTB_ERR_ABORTED),
     as `true` from the reference's per-pass closure does (random_sampler.rs:82-88)."""
     sc = ptb.Scene(rtweekend1, ctx=gpu_ctx)
-    monkeypatch.setenv("PTB_WAVEFRONT", "window")
     monkeypatch.setenv("PTB_POOL_PATHS", "8192")
     seen = []
     with pytest.raises(ptb.PtbError) as e:
         sc.render(ptb.RenderOptions(samples_per_pixel=16, render_method=0, width=64, height=36),
                   update=lambda s, r: seen.append(s) or len(seen) >= 2)
-    monkeypatch.delenv("PTB_WAVEFRONT")
     monkeypatch.delenv("PTB_POOL_PATHS")
     assert e.value.code == 7 and len(seen) == 2 and seen[0] < seen[1] < 16
     # the context stays usable
@@ -268,13 +265,11 @@ def test_abort_clears_the_accumulator(ptb, gpu_ctx, rtweekend1, monkeypatch):
     ctx.accum_clear()
     ctx.render(o)
     want = ctx.accum_read(64, 36, normalise=True).copy()
-    monkeypatch.setenv("PTB_WAVEFRONT", "window")
     monkeypatch.setenv("PTB_POOL_PATHS", "8192")
     ctx.accum_clear()
     with pytest.raises(ptb.PtbError) as e:
         ctx.render(o, progress=lambda s, r: True)
     assert e.value.code == 7
-    monkeypatch.delenv("PTB_WAVEFRONT")
     monkeypatch.delenv("PTB_POOL_PATHS")
     assert not np.any(ctx.accum_read(64, 36, normalise=False))      # nothing left behind
     ctx.render(o)                                                     # no accum_clear in between: starts from zero
@@ -372,11 +367,10 @@ def test_fused_tail_hand_over_does_not_change_the_result(ptb, gpu_ctx, overshado
         b, cb = run()                                      # 230 400 paths: handed over once <= 65 536 are alive
         monkeypatch.setenv("PTB_TAIL_PATHS", str(1 << 24))
         c, cc = run()                                      # handed over after the first bounce
-        monkeypatch.setenv("PTB_WAVEFRONT", "window")
         monkeypatch.setenv("PTB_POOL_PATHS", "32768")      # 8 chunks alternating between the two slots, tails overlapping
         monkeypatch.setenv("PTB_TAIL_PATHS", "8192")
         d, cd = run()
-        for k in ("PTB_TAIL_PATHS", "PTB_WAVEFRONT", "PTB_POOL_PATHS"):
+        for k in ("PTB_TAIL_PATHS", "PTB_POOL_PATHS"):
             monkeypatch.delenv(k)
         assert ca == cb == cc == cd, (ca, cb, cc, cd)
         assert ca[5] == 160 * 90 * 16
