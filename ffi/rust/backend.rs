@@ -134,6 +134,19 @@ impl CudaScene {
         check(self.ctx, unsafe { ptb_scene_update_mesh_vertices(self.ctx, base, out.as_ptr(), out.len()) })
     }
 
+    /// Place ranges of the indexed mesh (triangle order of `new_indexed`'s mesh) as instances, one transform each: the
+    /// scene's triangles become the instances' transformed copies, in order. Call `rebuild` afterwards.
+    pub fn set_mesh_instances(&self, instances: &[ptb_mesh_instance], xforms: &[ptb_instance_xform]) -> Result<(), String> {
+        if instances.len() != xforms.len() { return Err("set_mesh_instances: one transform per instance".into()); }
+        check(self.ctx, unsafe { ptb_scene_set_mesh_instances(self.ctx, instances.as_ptr(), xforms.as_ptr(), instances.len()) })
+    }
+
+    /// Rigid animation of an instanced scene: overwrite transforms [first, first + xforms.len()). Call `refit` afterwards;
+    /// the device expands the instances again at the commit.
+    pub fn update_instance_xforms(&self, first: usize, xforms: &[ptb_instance_xform]) -> Result<(), String> {
+        check(self.ctx, unsafe { ptb_scene_update_instance_xforms(self.ctx, first, xforms.as_ptr(), xforms.len()) })
+    }
+
     /// Commit the updates keeping the tree (PTB_BUILD_REFIT); returns the refitted tree's SAH cost, which the caller
     /// compares with the cost after the last full build to decide when to call `rebuild`.
     pub fn refit(&self) -> Result<f64, String> {

@@ -13,6 +13,10 @@ pub const PTB_METHOD_MIS: u32 = 1;
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_triangle { pub p: [ptb_vec3; 3], pub n: [ptb_vec3; 3], pub material: u32 }
 /// MeshTriangle (implementations/primitives/triangle.rs:30-36): indices into the scene's vertex / normal arrays (28 B)
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_mesh_triangle { pub p: [u32; 3], pub n: [u32; 3], pub material: u32 }
+/// One placed copy of mesh triangles [first_triangle, first_triangle + n_triangles); material PTB_MISS keeps theirs (12 B)
+#[repr(C)] #[derive(Clone, Copy)] pub struct ptb_mesh_instance { pub first_triangle: u32, pub n_triangles: u32, pub material: u32 }
+/// Object-to-world transform, row-major: m = 3x4 position map, n = 3x3 normal map (84 B)
+#[repr(C)] #[derive(Clone, Copy)] pub struct ptb_instance_xform { pub m: [f32; 12], pub n: [f32; 9] }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_material { pub kind: u32, pub texture: u32, pub param: f32, pub ior: ptb_vec3, pub metallic: f32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_texture { pub kind: u32, pub a: ptb_vec3, pub b: ptb_vec3 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_camera { pub origin: ptb_vec3, pub lower_left: ptb_vec3, pub horizontal: ptb_vec3, pub vertical: ptb_vec3 }
@@ -74,6 +78,9 @@ extern "C" {
     pub fn ptb_scene_update_mesh_vertices_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
     pub fn ptb_scene_update_mesh_normals_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
     pub fn ptb_scene_update_mesh_triangles_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
+    pub fn ptb_scene_set_mesh_instances(ctx: *mut ptb_ctx, instances: *const ptb_mesh_instance, xforms: *const ptb_instance_xform, n: usize) -> i32;
+    pub fn ptb_scene_update_instance_xforms(ctx: *mut ptb_ctx, first: usize, p: *const ptb_instance_xform, n: usize) -> i32;
+    pub fn ptb_scene_update_instance_xforms_device(ctx: *mut ptb_ctx, first: usize, d_p: *const c_void, n: usize) -> i32;
     pub fn ptb_scene_commit(ctx: *mut ptb_ctx, build_flags: u32) -> i32;
     pub fn ptb_bvh_sah_cost(ctx: *mut ptb_ctx, cost: *mut f64) -> i32;
     pub fn ptb_bvh_export_quantised(ctx: *mut ptb_ctx, frame: *mut f32, nodes32: *mut c_void) -> i32;

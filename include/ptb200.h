@@ -286,6 +286,48 @@ int32_t ptb_scene_update_mesh_triangles(ptb_ctx* ctx, size_t first, const ptb_me
 int32_t ptb_scene_update_mesh_vertices_device(ptb_ctx* ctx, size_t first, const void* d_vertices, size_t n);
 int32_t ptb_scene_update_mesh_normals_device(ptb_ctx* ctx, size_t first, const void* d_normals, size_t n);
 int32_t ptb_scene_update_mesh_triangles_device(ptb_ctx* ctx, size_t first, const void* d_triangles, size_t n);
+
+/* Mesh instances: placed copies of ranges of the indexed mesh, each under its own transform. One placed copy of mesh
+ * triangles [first_triangle, first_triangle + n_triangles). 12 bytes. */
+typedef struct ptb_mesh_instance {
+  uint32_t first_triangle;
+  uint32_t n_triangles;
+  uint32_t material;   /* PTB_MISS: every triangle keeps its own material; otherwise all of the instance's triangles get this one */
+} ptb_mesh_instance;
+/* Object-to-world transform, row-major f32. 84 bytes.
+ * position: x' = ((m[0]*x + m[1]*y) + m[2]*z) + m[3], likewise rows 1 and 2 (m[4..7], m[8..11]);
+ * normal:   n'.x = (n[0]*nx + n[1]*ny) + n[2]*nz, likewise rows 1 and 2; no translation, no normalisation.
+ * Each product and sum is one IEEE f32 operation, with no fused multiply-add (the library is built with -fmad=false). */
+typedef struct ptb_instance_xform {
+  float m[12];
+  float n[9];
+} ptb_instance_xform;
+/* ptb_scene_set_mesh_instances (host pointers, copied before returning) replaces the triangles of a mesh scene with the
+ * concatenation, in instance order, of each instance's range of mesh triangles under that instance's transform: triangle id
+ * = the sum of the earlier instances' n_triangles + the position inside the range, and primitive ids are still spheres
+ * first, then triangles. Ranges may overlap, repeat or be empty; zero instances means zero triangles. At commit (full or
+ * PTB_BUILD_REFIT) the device expands every instance into the ptb_triangle records the flat path uploads, whenever the
+ * mesh, the instance list or a transform changed since the last successful commit; the expansion counts in
+ * ptb_stats.build_ms and kernel_launches. Nothing after the expansion knows about instances: the device memory of the
+ * scene grows with the placed triangles, not with the mesh.
+ *   - ptb_scene_set_mesh drops the instance list (the scene's triangles are the mesh's own again); ptb_scene_set_triangles
+ *     drops the mesh and the instance list. On a flat scene ptb_scene_set_mesh_instances fails with PTB_ERR_INVALID.
+ *   - A range beyond the mesh's triangle count, a total of more than 2^32 - 1 triangles and a null pointer with n > 0 fail
+ *     with PTB_ERR_INVALID and a message naming the instance, before anything is allocated.
+ *   - ptb_scene_update_mesh_{vertices,normals,triangles}(_device) keep working: their ranges are over the mesh's arrays, and
+ *     every instance that places a changed triangle moves with it. Index validation names the mesh triangle, and covers only
+ *     the triangles some instance places. ptb_scene_update_triangles(_device) fails, as on every mesh scene.
+ *   - A material override goes into each placed triangle's material word and is validated and collected as a light like
+ *     any other.
+ *   - PTB_BUILD_REFIT keeps the tree while the sphere and total triangle counts are those of the last full commit. */
+int32_t ptb_scene_set_mesh_instances(ptb_ctx* ctx, const ptb_mesh_instance* instances, const ptb_instance_xform* xforms, size_t n);
+/* Overwrite transforms [first, first + n) of the instance list in place, with the range and pointer rules of
+ * ptb_scene_update_* (the host variant copies before returning; the _device variant copies device to device on the
+ * context's stream without synchronising). Without an instance list they fail with PTB_ERR_INVALID. Ranges and materials
+ * change only through ptb_scene_set_mesh_instances. The rigid animation loop: ptb_scene_update_instance_xforms ->
+ * ptb_scene_commit(PTB_BUILD_REFIT), 84 bytes per moving instance. */
+int32_t ptb_scene_update_instance_xforms(ptb_ctx* ctx, size_t first, const ptb_instance_xform* xforms, size_t n);
+int32_t ptb_scene_update_instance_xforms_device(ptb_ctx* ctx, size_t first, const void* d_xforms, size_t n);
 /* SAH cost of the committed binary tree in the reference's cost model (traversal 0.125, intersection 1, split.rs:161-176):
  * (0.125 * sum over inner nodes of SA(node) + sum over leaves of SA(leaf box)) / SA(root), SA = 2 (xy + yz + zx) of the f32
  * box evaluated in f64, root box = union of node 0's two child boxes. 1 primitive: 1.125; 0 primitives or a root of zero

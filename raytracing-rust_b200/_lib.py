@@ -34,6 +34,8 @@ BUILD_DEFAULT, BUILD_BINARY, BUILD_WIDE, BUILD_SAH, BUILD_REFIT = 0, 1, 2, 4, 8
 sphere_dtype = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4")])
 triangle_dtype = np.dtype([("p", "<f4", (3, 3)), ("n", "<f4", (3, 3)), ("material", "<u4")])
 mesh_triangle_dtype = np.dtype([("p", "<u4", 3), ("n", "<u4", 3), ("material", "<u4")])  # indices into vertices / normals
+mesh_instance_dtype = np.dtype([("first_triangle", "<u4"), ("n_triangles", "<u4"), ("material", "<u4")])
+instance_xform_dtype = np.dtype([("m", "<f4", (3, 4)), ("n", "<f4", (3, 3))])  # row-major object-to-world, normal matrix
 material_dtype = np.dtype([("kind", "<u4"), ("texture", "<u4"), ("param", "<f4"), ("ior", "<f4", 3), ("metallic", "<f4")])
 texture_dtype = np.dtype([("kind", "<u4"), ("a", "<f4", 3), ("b", "<f4", 3)])
 camera_dtype = np.dtype([("origin", "<f4", 3), ("lower_left", "<f4", 3), ("horizontal", "<f4", 3), ("vertical", "<f4", 3)])
@@ -113,6 +115,9 @@ SYMBOLS = [
     ("ptb_scene_update_mesh_vertices_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
     ("ptb_scene_update_mesh_normals_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
     ("ptb_scene_update_mesh_triangles_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_set_mesh_instances", C.c_int32, [_P, _P, _P, C.c_size_t]),
+    ("ptb_scene_update_instance_xforms", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
+    ("ptb_scene_update_instance_xforms_device", C.c_int32, [_P, C.c_size_t, _P, C.c_size_t]),
     ("ptb_scene_commit", C.c_int32, [_P, C.c_uint32]),
     ("ptb_bvh_sah_cost", C.c_int32, [_P, C.POINTER(C.c_double)]),
     ("ptb_bvh_info", C.c_int32, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),

@@ -84,9 +84,10 @@ class Context:
     def synchronize(self):
         _check(self._h, L.lib.ptb_synchronize(self._h))
 
-    def upload(self, s: HostScene, mesh: IndexedMesh | None = None):
+    def upload(self, s: HostScene, mesh: IndexedMesh | None = None, instances=None):
         """ptb_scene_set_* for every array (host -> library copy). With `mesh`, the scene's triangles are that indexed mesh
-        (set_mesh) and s.triangles is not uploaded."""
+        (set_mesh) and s.triangles is not uploaded; with `instances` = (instances, xforms) as well, they are those placed
+        copies of the mesh (set_mesh_instances)."""
         h = self._h
         _check(h, L.lib.ptb_scene_set_textures(h, L.ptr(s.textures), len(s.textures)))
         for i, (w, hh, words) in s.texture_data.items():
@@ -97,6 +98,8 @@ class Context:
             _check(h, L.lib.ptb_scene_set_triangles(h, L.ptr(s.triangles), len(s.triangles)))
         else:
             self.set_mesh(mesh)
+            if instances is not None:
+                self.set_mesh_instances(*instances)
         _check(h, L.lib.ptb_scene_set_camera(h, L.ptr(s.camera)))
         _check(h, L.lib.ptb_scene_set_sky(h, L.ptr(s.sky)))
 
@@ -158,6 +161,26 @@ class Context:
     def update_mesh_triangles_device(self, first: int, d_ptr: int, n: int):
         """n records of mesh_triangle_dtype's layout (28 bytes each)."""
         _check(self._h, L.lib.ptb_scene_update_mesh_triangles_device(self._h, first, C.c_void_p(d_ptr), n))
+
+    # ---- mesh instances: placed, transformed copies of mesh triangle ranges, expanded on the device at commit
+    def set_mesh_instances(self, instances: np.ndarray, xforms: np.ndarray):
+        """The scene's triangles become the instances (mesh_instance_dtype) in order, each under its transform
+        (instance_xform_dtype); set_mesh drops the list. Needs a mesh scene."""
+        i = np.ascontiguousarray(instances, L.mesh_instance_dtype).reshape(-1)
+        x = np.ascontiguousarray(xforms, L.instance_xform_dtype).reshape(-1)
+        if len(i) != len(x):
+            raise ValueError(f"{len(i)} instances but {len(x)} transforms")
+        _check(self._h, L.lib.ptb_scene_set_mesh_instances(self._h, L.ptr(i), L.ptr(x), len(i)))
+
+    def update_instance_xforms(self, first: int, xforms: np.ndarray):
+        """Overwrite transforms [first, first + len(xforms)) (instance_xform_dtype); then commit, e.g. with L.BUILD_REFIT."""
+        x = np.ascontiguousarray(xforms, L.instance_xform_dtype).reshape(-1)
+        _check(self._h, L.lib.ptb_scene_update_instance_xforms(self._h, first, L.ptr(x), len(x)))
+
+    def update_instance_xforms_device(self, first: int, d_ptr: int, n: int):
+        """Same from device memory (n records of 84 bytes: 21 float32 each), enqueued on the context's stream without a
+        synchronise (as update_triangles_device)."""
+        _check(self._h, L.lib.ptb_scene_update_instance_xforms_device(self._h, first, C.c_void_p(d_ptr), n))
 
     def bvh_sah_cost(self) -> float:
         """SAH cost of the committed binary tree (traversal 0.125, intersection 1; normalised by the root's area). Compare

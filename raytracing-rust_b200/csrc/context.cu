@@ -169,18 +169,27 @@ int32_t ptb_scene_set_spheres(ptb_ctx* ctx, const ptb_sphere* p, size_t n) {
   c->n_spheres = n;
   return PTB_OK;
 }
+// the instance list goes with ptb_scene_set_mesh and ptb_scene_set_triangles (the caller has drained the stream)
+static void drop_instances(Ctx* c) {
+  c->instanced = false;
+  c->n_instances = 0;
+  c->d_inst.release();
+  c->d_inst_first.release();
+  c->d_inst_xforms.release();
+}
 int32_t ptb_scene_set_triangles(ptb_ctx* ctx, const ptb_triangle* p, size_t n) {
   CTX_OR_FAIL(ctx);
   if (n && !p) return set_error(c, PTB_ERR_INVALID, "null triangles");
   c->committed = false;
   c->n_tris = 0;
-  if (c->mesh) {  // flat mode: the mesh is dropped
+  if (c->mesh) {  // flat mode: the mesh and its instances are dropped
     PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));  // a device update may still read into its buffers
     c->mesh = c->mesh_dirty = false;
-    c->n_mesh_vertices = c->n_mesh_normals = 0;
+    c->n_mesh_vertices = c->n_mesh_normals = c->n_mesh_tris = 0;
     c->d_mesh_vertices.release();
     c->d_mesh_normals.release();
     c->d_mesh_tris.release();
+    drop_instances(c);
   }
   PTB_CUDA_TRY(c, c->d_raw_tris.reserve(n * sizeof(ptb_triangle)));
   if (n) PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_raw_tris.p, p, n * sizeof(ptb_triangle), cudaMemcpyHostToDevice, c->stream));
@@ -197,7 +206,11 @@ int32_t ptb_scene_set_mesh(ptb_ctx* ctx, const ptb_vec3* v, size_t nv, const ptb
   c->committed = false;
   c->n_tris = 0;
   c->mesh = false;
-  c->n_mesh_vertices = c->n_mesh_normals = 0;
+  c->n_mesh_vertices = c->n_mesh_normals = c->n_mesh_tris = 0;
+  if (c->instanced) {
+    PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));  // a device transform update may still write into its buffer
+    drop_instances(c);
+  }
   PTB_CUDA_TRY(c, c->d_mesh_vertices.reserve(nv * sizeof(ptb_vec3)));
   PTB_CUDA_TRY(c, c->d_mesh_normals.reserve(nn * sizeof(ptb_vec3)));
   PTB_CUDA_TRY(c, c->d_mesh_tris.reserve(nt * sizeof(ptb_mesh_triangle)));
@@ -208,8 +221,46 @@ int32_t ptb_scene_set_mesh(ptb_ctx* ctx, const ptb_vec3* v, size_t nv, const ptb
   PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   c->n_mesh_vertices = nv;
   c->n_mesh_normals = nn;
-  c->n_tris = nt;
+  c->n_mesh_tris = c->n_tris = nt;
   c->mesh = c->mesh_dirty = true;
+  return PTB_OK;
+}
+int32_t ptb_scene_set_mesh_instances(ptb_ctx* ctx, const ptb_mesh_instance* inst, const ptb_instance_xform* xf, size_t n) {
+  CTX_OR_FAIL(ctx);
+  if (!c->mesh)
+    return set_error(c, PTB_ERR_INVALID, "mesh instances: the scene's triangles are flat, not an indexed mesh (ptb_scene_set_mesh)");
+  if (n && (!inst || !xf)) return set_error(c, PTB_ERR_INVALID, "null mesh instances or transforms (%zu instances)", n);
+  if (n > 0xFFFFFFFFull) return set_error(c, PTB_ERR_INVALID, "at most 2^32 - 1 mesh instances (%zu)", n);
+  // every instance is checked before anything is allocated; the prefix sums are what k_expand_instances searches
+  std::vector<uint32_t> first(n);
+  uint64_t total = 0;
+  for (size_t i = 0; i < n; ++i) {
+    if ((uint64_t)inst[i].first_triangle + inst[i].n_triangles > c->n_mesh_tris)
+      return set_error(c, PTB_ERR_INVALID, "mesh instance %zu: triangles [%u, %u + %u) outside the %zu the mesh holds", i,
+                       inst[i].first_triangle, inst[i].first_triangle, inst[i].n_triangles, c->n_mesh_tris);
+    first[i] = (uint32_t)total;
+    total += inst[i].n_triangles;
+    if (total > 0xFFFFFFFFull)
+      return set_error(c, PTB_ERR_INVALID, "mesh instance %zu: the instances place more than 2^32 - 1 triangles", i);
+  }
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));  // a device transform update may still write into the old list
+  c->committed = false;
+  c->n_tris = 0;
+  c->instanced = false;
+  c->n_instances = 0;
+  PTB_CUDA_TRY(c, c->d_inst.reserve(n * sizeof(ptb_mesh_instance)));
+  PTB_CUDA_TRY(c, c->d_inst_first.reserve(n * sizeof(uint32_t)));
+  PTB_CUDA_TRY(c, c->d_inst_xforms.reserve(n * sizeof(ptb_instance_xform)));
+  PTB_CUDA_TRY(c, c->d_raw_tris.reserve(total * sizeof(ptb_triangle)));  // the expansion's output
+  if (n) {
+    PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_inst.p, inst, n * sizeof(ptb_mesh_instance), cudaMemcpyHostToDevice, c->stream));
+    PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_inst_first.p, first.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+    PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_inst_xforms.p, xf, n * sizeof(ptb_instance_xform), cudaMemcpyHostToDevice, c->stream));
+  }
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  c->n_instances = n;
+  c->n_tris = total;
+  c->instanced = c->mesh_dirty = true;
   return PTB_OK;
 }
 // ptb_scene_update_*: primitives [first, first + n) of `raw` (count `have`, records of `rec` bytes) in place
@@ -267,7 +318,7 @@ int32_t ptb_scene_update_mesh_normals(ptb_ctx* ctx, size_t first, const ptb_vec3
 }
 int32_t ptb_scene_update_mesh_triangles(ptb_ctx* ctx, size_t first, const ptb_mesh_triangle* p, size_t n) {
   CTX_OR_FAIL(ctx);
-  return update_mesh(c, c->d_mesh_tris, c->n_tris, sizeof(ptb_mesh_triangle), first, p, n, cudaMemcpyHostToDevice, "mesh triangles");
+  return update_mesh(c, c->d_mesh_tris, c->n_mesh_tris, sizeof(ptb_mesh_triangle), first, p, n, cudaMemcpyHostToDevice, "mesh triangles");
 }
 int32_t ptb_scene_update_mesh_vertices_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
   CTX_OR_FAIL(ctx);
@@ -279,7 +330,23 @@ int32_t ptb_scene_update_mesh_normals_device(ptb_ctx* ctx, size_t first, const v
 }
 int32_t ptb_scene_update_mesh_triangles_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
   CTX_OR_FAIL(ctx);
-  return update_mesh(c, c->d_mesh_tris, c->n_tris, sizeof(ptb_mesh_triangle), first, d_p, n, cudaMemcpyDeviceToDevice, "mesh triangles");
+  return update_mesh(c, c->d_mesh_tris, c->n_mesh_tris, sizeof(ptb_mesh_triangle), first, d_p, n, cudaMemcpyDeviceToDevice, "mesh triangles");
+}
+// ptb_scene_update_instance_xforms*: update_prims on the transform list, which the next commit expands again
+static int32_t update_xforms(Ctx* c, size_t first, const void* p, size_t n, cudaMemcpyKind kind) {
+  if (!c->instanced)
+    return set_error(c, PTB_ERR_INVALID, "instance transform update: the scene has no instance list (ptb_scene_set_mesh_instances)");
+  const int32_t rc = update_prims(c, c->d_inst_xforms, c->n_instances, sizeof(ptb_instance_xform), first, p, n, kind, "instance transforms");
+  if (rc == PTB_OK && n) c->mesh_dirty = true;
+  return rc;
+}
+int32_t ptb_scene_update_instance_xforms(ptb_ctx* ctx, size_t first, const ptb_instance_xform* p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_xforms(c, first, p, n, cudaMemcpyHostToDevice);
+}
+int32_t ptb_scene_update_instance_xforms_device(ptb_ctx* ctx, size_t first, const void* d_p, size_t n) {
+  CTX_OR_FAIL(ctx);
+  return update_xforms(c, first, d_p, n, cudaMemcpyDeviceToDevice);
 }
 int32_t ptb_scene_set_materials(ptb_ctx* ctx, const ptb_material* p, size_t n) {
   CTX_OR_FAIL(ctx);

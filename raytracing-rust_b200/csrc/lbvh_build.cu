@@ -722,10 +722,78 @@ k_expand_mesh(const uint32_t* __restrict__ vtx, uint32_t nv, const uint32_t* __r
     reinterpret_cast<uint4*>(dst)[q] = reinterpret_cast<const uint4*>(s_rec)[q];
   for (uint32_t w = (out_words & ~3u) + threadIdx.x; w < out_words; w += kExpandThreads) dst[w] = s_rec[w];
 }
+// ptb_scene_set_mesh_instances: output triangle t belongs to the last instance whose first triangle id (the exclusive prefix
+// sum `inst_first`) is <= t; empty instances share their successor's prefix and are never chosen. The record is gathered
+// as k_expand_mesh gathers it, with the same index checks naming the mesh triangle, then transformed in shared memory in
+// the header's statement order (__fmul_rn / __fadd_rn: never contracted into an FMA).
+constexpr uint32_t kInstWords = sizeof(ptb_mesh_instance) / 4, kXformWords = sizeof(ptb_instance_xform) / 4;  // 3, 21
+static_assert(sizeof(ptb_mesh_instance) == 12 && sizeof(ptb_instance_xform) == 84, "record layouts");
+
+__device__ __forceinline__ float xf_point(const float* r, float x, float y, float z) {
+  return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(r[0], x), __fmul_rn(r[1], y)), __fmul_rn(r[2], z)), r[3]);
+}
+__device__ __forceinline__ float xf_normal(const float* r, float x, float y, float z) {
+  return __fadd_rn(__fadd_rn(__fmul_rn(r[0], x), __fmul_rn(r[1], y)), __fmul_rn(r[2], z));
+}
+__global__ void __launch_bounds__(kExpandThreads)
+k_expand_instances(const uint32_t* __restrict__ vtx, uint32_t nv, const uint32_t* __restrict__ nrm, uint32_t nn,
+                   const uint32_t* __restrict__ mesh_tris, const uint32_t* __restrict__ inst, const uint32_t* __restrict__ inst_first,
+                   const float* __restrict__ xforms, uint32_t n_inst, uint32_t n_tris, uint32_t* __restrict__ tris, uint32_t* out) {
+  // the output side is k_expand_mesh's: records staged in shared memory, stored with 16-byte accesses
+  __shared__ __align__(16) uint32_t s_rec[kExpandThreads * kTriWords];
+  const uint32_t first = blockIdx.x * kExpandThreads, count = min(kExpandThreads, n_tris - first);
+  if (threadIdx.x < count) {
+    const uint32_t t = first + threadIdx.x;
+    uint32_t lo = 0, hi = n_inst;  // the first instance whose prefix is > t, minus one
+    while (hi - lo > 1) {
+      const uint32_t mid = (lo + hi) >> 1;
+      if (__ldg(inst_first + mid) <= t) lo = mid;
+      else hi = mid;
+    }
+    const uint32_t mt = __ldg(inst + kInstWords * lo) + (t - __ldg(inst_first + lo)), material = __ldg(inst + kInstWords * lo + 2);
+    uint32_t idx[kMeshWords];
+#pragma unroll
+    for (uint32_t w = 0; w < kMeshWords; ++w) idx[w] = __ldg(mesh_tris + (size_t)mt * kMeshWords + w);
+    uint32_t* rec = s_rec + threadIdx.x * kTriWords;
+    expand_record(idx, rec, mt, vtx, nv, nrm, nn, out);
+    const float* m = xforms + (size_t)lo * kXformWords;
+    float mr[12], nr[9];
+#pragma unroll
+    for (int w = 0; w < 12; ++w) mr[w] = __ldg(m + w);
+#pragma unroll
+    for (int w = 0; w < 9; ++w) nr[w] = __ldg(m + 12 + w);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      float* p = reinterpret_cast<float*>(rec + 3 * k);
+      float* q = reinterpret_cast<float*>(rec + 9 + 3 * k);
+      const float x = p[0], y = p[1], z = p[2], a = q[0], b = q[1], d = q[2];
+#pragma unroll
+      for (int r = 0; r < 3; ++r) {
+        p[r] = xf_point(mr + 4 * r, x, y, z);
+        q[r] = xf_normal(nr + 3 * r, a, b, d);
+      }
+    }
+    if (material != PTB_MISS) rec[18] = material;
+  }
+  __syncthreads();
+  const uint32_t out_words = count * kTriWords;
+  uint32_t* dst = tris + (size_t)first * kTriWords;
+  for (uint32_t q = threadIdx.x; q < out_words / 4; q += kExpandThreads)
+    reinterpret_cast<uint4*>(dst)[q] = reinterpret_cast<const uint4*>(s_rec)[q];
+  for (uint32_t w = (out_words & ~3u) + threadIdx.x; w < out_words; w += kExpandThreads) dst[w] = s_rec[w];
+}
 // Enqueued after the memset of the light-list words and before k_collect_lights, in both commit paths.
 static void expand_mesh(Ctx* c, uint32_t* out) {
   if (!c->mesh || !c->mesh_dirty || c->n_tris == 0) return;
   const uint32_t nt = (uint32_t)c->n_tris;
+  if (c->instanced) {
+    k_expand_instances<<<(nt + kExpandThreads - 1) / kExpandThreads, kExpandThreads, 0, c->stream>>>(
+        c->d_mesh_vertices.as<uint32_t>(), (uint32_t)c->n_mesh_vertices, c->d_mesh_normals.as<uint32_t>(), (uint32_t)c->n_mesh_normals,
+        c->d_mesh_tris.as<uint32_t>(), c->d_inst.as<uint32_t>(), c->d_inst_first.as<uint32_t>(), c->d_inst_xforms.as<float>(),
+        (uint32_t)c->n_instances, nt, c->d_raw_tris.as<uint32_t>(), out);
+    c->stats.kernel_launches += 1;
+    return;
+  }
   k_expand_mesh<<<(nt + kExpandThreads - 1) / kExpandThreads, kExpandThreads, 0, c->stream>>>(
       c->d_mesh_vertices.as<uint32_t>(), (uint32_t)c->n_mesh_vertices, c->d_mesh_normals.as<uint32_t>(), (uint32_t)c->n_mesh_normals,
       c->d_mesh_tris.as<uint32_t>(), nt, c->d_raw_tris.as<uint32_t>(), out);

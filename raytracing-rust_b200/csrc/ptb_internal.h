@@ -84,10 +84,16 @@ struct Ctx {
   DevBuf d_raw_spheres, d_raw_tris;
   size_t n_spheres = 0, n_tris = 0;
   // indexed mesh (ptb_scene_set_mesh): when `mesh` is set, d_raw_tris is the mesh's expansion (k_expand_mesh), redone at
-  // the next commit whenever `mesh_dirty`; n_tris is the number of mesh triangles
+  // the next commit whenever `mesh_dirty`; n_tris is the number of mesh triangles, n_mesh_tris too unless `instanced`
   DevBuf d_mesh_vertices, d_mesh_normals, d_mesh_tris;
-  size_t n_mesh_vertices = 0, n_mesh_normals = 0;
+  size_t n_mesh_vertices = 0, n_mesh_normals = 0, n_mesh_tris = 0;
   bool mesh = false, mesh_dirty = false;
+  // mesh instances (ptb_scene_set_mesh_instances): when `instanced` is set (on a mesh scene), d_raw_tris is the expansion
+  // of every instance (k_expand_instances) and n_tris the sum of their n_triangles; d_inst_first is the exclusive prefix
+  // sum of n_triangles (the first triangle id of each instance)
+  DevBuf d_inst, d_inst_first, d_inst_xforms;
+  size_t n_instances = 0;
+  bool instanced = false;
   DevBuf scratch[16];  // LBVH build temporaries, grow-only (lbvh_build.cu)
   std::vector<ptb_material> materials;
   std::vector<ptb_texture> textures;

@@ -5,6 +5,11 @@
   c3_deform()         one frame of an animated C3: terrain wave + glass sphere pushed into the terrain (same counts)
   c3_indexed(), heightfield_indexed(), c3_deform_vertices()
                       the same scenes as indexed meshes over their grid points (expand() == the flat triangles)
+  c3_instanced(), c3_instanced_frame()
+                      c3_indexed's mesh placed as two instances (terrain, glass sphere), and the sphere's transform for
+                      c3_deform's motion
+  rock(), scatter_instances()
+                      a small closed mesh, and many rotated, scaled, translated copies of a mesh over a terrain
   heightfield_scene() R x C quads in [-1,1]^2 x [-0.2,0.2]; 2500 x 2000 -> 10 000 000 triangles      ("C5")
   philox_rays()       incoherent rays from Philox4x32-10 (seed 0x5EED, counter = ray index): origin uniform in the
                       ball of radius 2 about the mesh centre, direction uniform on the sphere
@@ -18,7 +23,7 @@ import copy
 import numpy as np
 
 from . import _lib as L
-from .scene import HostScene, IndexedMesh
+from .scene import HostScene, IndexedMesh, instance_xform
 
 F = np.float32
 
@@ -207,6 +212,69 @@ def c3_deform_vertices(mesh: IndexedMesh, wave: float, shift: float) -> IndexedM
     v[~glass] = t
     v[glass] = v[glass] + (F(shift) * F(C3_GLASS_RADIUS) * np.array([0.6, 0.0, -0.8], F)).astype(F)
     return IndexedMesh(v, mesh.normals, mesh.triangles)
+
+
+def _instances(ranges) -> np.ndarray:
+    """mesh_instance_dtype records from (first_triangle, n_triangles, material) tuples."""
+    inst = np.zeros(len(ranges), L.mesh_instance_dtype)
+    for i, (first, n, material) in enumerate(ranges):
+        inst[i] = (first, n, material)
+    return inst
+
+
+def c3_instanced(scale: float = 1.0):
+    """c3_indexed's mesh placed as two instances, the terrain's triangle range and the glass sphere's, each under an
+    identity transform: (scene without triangles, mesh, instances, xforms). Upload with
+    Context.upload(scene, mesh=mesh, instances=(instances, xforms)); mesh.expand_instances(instances, xforms) is the flat
+    scene (c3_scene's triangles up to the sign of zero coordinates)."""
+    s, mesh = c3_indexed(scale)
+    n_terrain = int(np.count_nonzero(mesh.triangles["material"] == 0))
+    inst = _instances([(0, n_terrain, L.PTB_MISS), (n_terrain, len(mesh.triangles) - n_terrain, L.PTB_MISS)])
+    return s, mesh, inst, np.concatenate([instance_xform(), instance_xform()])
+
+
+def c3_instanced_frame(shift: float) -> np.ndarray:
+    """The glass sphere instance's transform (instance 1 of c3_instanced) for c3_deform's motion: a translation by `shift`
+    radii along (0.6, 0, -0.8)."""
+    return instance_xform(translation=(F(shift) * F(C3_GLASS_RADIUS) * np.array([0.6, 0.0, -0.8], F)).astype(F))
+
+
+def rock(slices: int = 25, stacks: int = 21) -> IndexedMesh:
+    """A small closed mesh about the origin: a unit UV sphere with closed-form bumps on its radius and radial normals,
+    2 * slices * (stacks - 1) triangles (1000 by default), material 0."""
+    P, D = _uv_sphere_vertices((0.0, 0.0, 0.0), 1.0, slices, stacks)
+    bump = F(1) + F(0.15) * np.sin(F(3) * D[..., 0] + F(2) * D[..., 2]) * np.cos(F(4) * D[..., 1])
+    return _mesh([((P * bump[..., None]).astype(F), D, _uv_sphere_indices(slices, stacks), 0)])
+
+
+def scatter_instances(mesh: IndexedMesh, count: int, seed: int = 0, terrain=(200, 80)):
+    """`count` copies of `mesh` over a C3-like terrain of 2 * terrain[0] * terrain[1] triangles: (scene without triangles,
+    combined mesh, instances, xforms). The combined mesh is the terrain's grid followed by `mesh`; instance 0 places the
+    terrain under the identity, instances 1..count place `mesh` with a uniformly random rotation, a scale in [0.05, 0.2]
+    and a translation onto the terrain, all drawn from numpy's default_rng(seed)."""
+    nx, ny = terrain
+    s = _base_scene()
+    xs, ys = _c3_axes(nx, ny)
+    P, N = _grid_vertices(xs, ys, _terrain_height, _terrain_normal)
+    ground = _mesh([(P, N, _grid_indices(nx + 1, ny + 1), 0)])
+    t = mesh.triangles.copy()
+    t["p"] += np.uint32(len(ground.vertices))
+    t["n"] += np.uint32(len(ground.normals))
+    combined = IndexedMesh(np.concatenate([ground.vertices, mesh.vertices]), np.concatenate([ground.normals, mesh.normals]),
+                           np.concatenate([ground.triangles, t]))
+    nt = len(ground.triangles)
+    inst = np.zeros(count + 1, L.mesh_instance_dtype)
+    inst["first_triangle"][0], inst["n_triangles"][0] = 0, nt
+    inst["first_triangle"][1:], inst["n_triangles"][1:] = nt, len(mesh.triangles)
+    inst["material"] = L.PTB_MISS
+    rng = np.random.default_rng(seed)
+    q = rng.normal(size=(count, 4))
+    scale = rng.uniform(0.05, 0.2, count)
+    x, y = rng.uniform(-12.0, 12.0, count), rng.uniform(0.5, 10.0, count)
+    z = _terrain_height(x.astype(F), y.astype(F)).astype(np.float64)
+    xf = np.concatenate([instance_xform()] + [instance_xform(q[i], scale[i], (x[i], y[i], z[i])) for i in range(count)])
+    s.set_camera(*C3_CAMERA)
+    return s, combined, inst, xf
 
 
 def _hf_height(X, Y):

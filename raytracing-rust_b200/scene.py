@@ -117,8 +117,55 @@ class IndexedMesh:
         tri["material"] = self.triangles["material"]
         return tri
 
+    def expand_instances(self, instances: np.ndarray, xforms: np.ndarray) -> np.ndarray:
+        """The flat triangles (triangle_dtype) an instance list over this mesh stands for (Context.set_mesh_instances): for
+        each instance in order, mesh triangles [first_triangle, first_triangle + n_triangles) expanded, positions and normals
+        transformed in float32 in the header's statement order, and the material replaced unless it is PTB_MISS. Byte for
+        byte what the device expansion writes."""
+        inst = np.ascontiguousarray(instances, L.mesh_instance_dtype).reshape(-1)
+        xf = np.ascontiguousarray(xforms, L.instance_xform_dtype).reshape(-1)
+        if len(inst) != len(xf):
+            raise ValueError(f"{len(inst)} instances but {len(xf)} transforms")
+        count = inst["n_triangles"].astype(np.int64)
+        owner = np.repeat(np.arange(len(inst)), count)
+        start = np.cumsum(count) - count
+        mt = inst["first_triangle"].astype(np.int64)[owner] + (np.arange(len(owner)) - start[owner])
+        tri = IndexedMesh(self.vertices, self.normals, self.triangles[mt]).expand()
+        m, n = xf["m"][owner], xf["n"][owner]  # (T, 3, 4), (T, 3, 3)
+        p, q = tri["p"].copy(), tri["n"].copy()  # (T, 3 corners, 3)
+        for r in range(3):
+            tri["p"][:, :, r] = ((m[:, r, 0, None] * p[:, :, 0] + m[:, r, 1, None] * p[:, :, 1]) + m[:, r, 2, None] * p[:, :, 2]) \
+                + m[:, r, 3, None]
+            tri["n"][:, :, r] = (n[:, r, 0, None] * q[:, :, 0] + n[:, r, 1, None] * q[:, :, 1]) + n[:, r, 2, None] * q[:, :, 2]
+        over = inst["material"][owner]
+        tri["material"] = np.where(over != L.PTB_MISS, over, tri["material"])
+        return tri
+
     def nbytes(self) -> int:
         return int(self.vertices.nbytes + self.normals.nbytes + self.triangles.nbytes)
+
+
+def instance_xform(rotation=None, scale: float = 1.0, translation=(0.0, 0.0, 0.0)) -> np.ndarray:
+    """One instance_xform_dtype record: m = [s R | t], n = R. `rotation` is a 3x3 rotation matrix or a quaternion
+    (w, x, y, z), normalised here; None is the identity. With R orthonormal, unit normals stay unit up to rounding. For a
+    general affine map build the record yourself with n = the inverse transpose of its linear part: the library does not
+    renormalise normals (neither does the reference's interpolated normal)."""
+    if rotation is None:
+        R = np.eye(3)
+    else:
+        r = np.asarray(rotation, np.float64)
+        if r.shape == (4,):
+            w, x, y, z = r / np.linalg.norm(r)
+            R = np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y)],
+                          [2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x)],
+                          [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
+        else:
+            R = r.reshape(3, 3)
+    out = np.zeros(1, L.instance_xform_dtype)
+    out["m"][0, :, :3] = (float(scale) * R).astype(np.float32)
+    out["m"][0, :, 3] = np.asarray(translation, np.float32)
+    out["n"][0] = R.astype(np.float32)
+    return out
 
 
 def _dedup_rows(a: np.ndarray):
