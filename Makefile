@@ -25,7 +25,7 @@ cli: $(PKG)/ptb200-cli
 $(PKG)/ptb200-cli: $(PKG)/host/cli_main.cpp $(PKG)/libptb200.so include/ptb200.h
 	$(CXX) -O2 -std=c++17 -Wall -Wextra -o $@ $(PKG)/host/cli_main.cpp -L$(PKG) -lptb200 -Wl,-rpath,'$$ORIGIN' -ldl -lpthread
 
-oracle: oracle/libvisibility_oracle.so oracle/librefit_oracle.so
+oracle: oracle/libvisibility_oracle.so oracle/librefit_oracle.so oracle/libaov_oracle.so
 	$(MAKE) -C oracle
 # test infrastructure beside liboracle.so: the reference's visibility queries for a batch (oracle/visibility_api.cpp)
 oracle/libvisibility_oracle.so: oracle/visibility_api.cpp $(wildcard oracle/*.hpp) include/ptb200.h
@@ -33,8 +33,11 @@ oracle/libvisibility_oracle.so: oracle/visibility_api.cpp $(wildcard oracle/*.hp
 # ... and the refit of a kept binary tree (oracle/refit_api.cpp, PTB_BUILD_REFIT)
 oracle/librefit_oracle.so: oracle/refit_api.cpp $(wildcard oracle/*.hpp) include/ptb200.h
 	$(CXX) -O2 -std=c++17 -fno-fast-math -ffp-contract=off -fPIC -Wall -Wextra -pthread -shared -o $@ $<
+# ... and the denoiser feature buffers of the render's camera rays (oracle/aov_api.cpp, ptb_render_aov)
+oracle/libaov_oracle.so: oracle/aov_api.cpp $(wildcard oracle/*.hpp) include/ptb200.h
+	$(CXX) -O2 -std=c++17 -fno-fast-math -ffp-contract=off -fPIC -Wall -Wextra -pthread -shared -o $@ $<
 
 clean:
-	rm -f $(OBJS) $(PKG)/csrc/*.ptxas.log $(PKG)/libptb200.so $(PKG)/ptb200-cli oracle/libvisibility_oracle.so oracle/librefit_oracle.so
+	rm -f $(OBJS) $(PKG)/csrc/*.ptxas.log $(PKG)/libptb200.so $(PKG)/ptb200-cli oracle/libvisibility_oracle.so oracle/librefit_oracle.so oracle/libaov_oracle.so
 	$(MAKE) -C oracle clean
 .PHONY: all oracle clean cli

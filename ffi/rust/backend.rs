@@ -106,6 +106,24 @@ impl CudaScene {
         }
         Ok((image, st.rays_reference))
     }
+
+    /// Denoiser feature buffers of the camera rays `render(opts, seed)` traces: (albedo, normal, depth, coverage), each
+    /// normalised, row-major with the top row first; albedo and normal hold 3 floats per pixel, depth and coverage one
+    /// (depth is the mean t over the samples that hit, 0 where none did). Feed them to the denoiser with the beauty image.
+    pub fn render_aov(&self, opts: RenderOptions, seed: u64) -> Result<(Vec<f32>, Vec<f32>, Vec<f32>, Vec<f32>), String> {
+        let o = self.opts(opts, seed);
+        let n = (opts.width * opts.height) as usize;
+        let (mut albedo, mut normal, mut depth, mut coverage) = (vec![0.0f32; 3 * n], vec![0.0f32; 3 * n], vec![0.0f32; n], vec![0.0f32; n]);
+        unsafe {
+            check(self.ctx, ptb_aov_clear(self.ctx))?;
+            check(self.ctx, ptb_render_aov(self.ctx, &o))?;
+            for (aov, buf) in [(PTB_AOV_ALBEDO, &mut albedo), (PTB_AOV_NORMAL, &mut normal), (PTB_AOV_DEPTH, &mut depth),
+                               (PTB_AOV_COVERAGE, &mut coverage)] {
+                check(self.ctx, ptb_aov_read(self.ctx, aov, buf.as_mut_ptr(), buf.len(), 1))?;
+            }
+        }
+        Ok((albedo, normal, depth, coverage))
+    }
 }
 
 impl CudaScene {

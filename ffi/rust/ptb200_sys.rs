@@ -7,6 +7,11 @@ pub const PTB_MISS: u32 = 0xFFFF_FFFF;
 pub const PTB_RR_DEFAULT: u32 = 0xFFFF_FFFF;
 pub const PTB_METHOD_NAIVE: u32 = 0;
 pub const PTB_METHOD_MIS: u32 = 1;
+/// Denoiser feature buffers (ptb_aov_read)
+pub const PTB_AOV_ALBEDO: u32 = 0;
+pub const PTB_AOV_NORMAL: u32 = 1;
+pub const PTB_AOV_DEPTH: u32 = 2;
+pub const PTB_AOV_COVERAGE: u32 = 3;
 
 #[repr(C)] #[derive(Clone, Copy, Default)] pub struct ptb_vec3 { pub x: f32, pub y: f32, pub z: f32 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct ptb_sphere { pub center: ptb_vec3, pub radius: f32, pub material: u32 }
@@ -101,6 +106,9 @@ extern "C" {
     pub fn ptb_accum_clear(ctx: *mut ptb_ctx) -> i32;
     pub fn ptb_accum_read(ctx: *mut ptb_ctx, rgb: *mut f32, n_floats: usize, normalise: i32) -> i32;
     pub fn ptb_accum_device_ptr(ctx: *mut ptb_ctx, d_ptr: *mut *mut c_void, n_floats: *mut usize) -> i32;
+    pub fn ptb_render_aov(ctx: *mut ptb_ctx, opts: *const ptb_render_opts) -> i32;
+    pub fn ptb_aov_clear(ctx: *mut ptb_ctx) -> i32;
+    pub fn ptb_aov_read(ctx: *mut ptb_ctx, aov: u32, out: *mut f32, n_floats: usize, normalise: i32) -> i32;
     pub fn ptb_sample_only(ctx: *mut ptb_ctx, query: *const ptb_sampler_query, n: usize, dirs: *mut f32, pdf: *mut f32) -> i32;
     pub fn ptb_sampler_pdf(ctx: *mut ptb_ctx, query: *const ptb_sampler_query, dirs: *const f32, n: usize, pdf: *mut f32) -> i32;
     pub fn ptb_stats_get(ctx: *mut ptb_ctx, out: *mut ptb_stats) -> i32;

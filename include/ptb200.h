@@ -432,6 +432,34 @@ int32_t ptb_accum_device_ptr(ptb_ctx* ctx, void** d_ptr, size_t* n_floats);
 /* After an external reduce wrote sums of `total_samples` samples into the accumulator. */
 int32_t ptb_accum_set_samples(ptb_ctx* ctx, uint64_t total_samples);
 
+/* ------------------------------------------------ denoiser feature buffers -- */
+/* The inputs a denoiser (Open Image Denoise, the OptiX denoiser, an SVGF-style filter) reads beside the beauty image,
+ * aligned with it sample for sample: ptb_render_aov traces the camera ray of every (pixel, sample) that ptb_render with
+ * the same opts traces (width, height, seed, sample_offset, samples_per_pixel, row_begin, row_count: the same jitter, the
+ * same ray, bit for bit) and adds per sample, at the ray's closest hit h (wo = the unit camera direction):
+ *   albedo   3 floats  LAMBERTIAN: param * texture(wo, h.point); REFLECT, REFRACT, TROWBRIDGE_REITZ: texture(wo, h.point);
+ *                      EMIT: the emission the first bounce adds; a miss: the sky's emission. Each channel clamped to [0, 1]
+ *                      (a NaN becomes 0).
+ *   normal   3 floats  the hit record's normal, as every scatter uses it (not turned towards the camera); 0 on a miss
+ *   depth    1 float   t along the unit direction (what ptb_closest_hit reports for that ray); 0 on a miss
+ *   coverage 1 float   1 on a hit, 0 on a miss
+ * into a separate AOV accumulator. method, max_depth, rr_threshold and flags are not read, so a host passes the opts of
+ * its render unchanged; the other checks and messages are ptb_render's. The sums of a pixel are formed in sample order
+ * without atomics: the buffers are deterministic, and sample ranges or row tiles of a call add up bit for bit to the one
+ * call. The beauty accumulator and its sample count are not touched. Each sample is one traversal launch (counted in
+ * ptb_stats.kernel_launches and trace_launches, no ray counters). Enqueues on the context's stream and may return before
+ * the work is done; ptb_aov_read synchronises.
+ * The first call allocates 8 floats per pixel; a call with another width or height reallocates and resets them. */
+enum { PTB_AOV_ALBEDO = 0, PTB_AOV_NORMAL = 1, PTB_AOV_DEPTH = 2, PTB_AOV_COVERAGE = 3 };
+int32_t ptb_render_aov(ptb_ctx* ctx, const ptb_render_opts* opts);
+/* Zeroes the AOV sums and their sample count. */
+int32_t ptb_aov_clear(ptb_ctx* ctx);
+/* Reads one buffer (PTB_AOV_*): n_floats = width*height*3 for albedo and normal, width*height for depth and coverage;
+ * row-major, top row first, as ptb_accum_read. normalise != 0 divides albedo, normal and coverage by the AOV sample count
+ * and depth by the pixel's coverage sum (0 where nothing was hit); the mean normal is not renormalised. Synchronises the
+ * stream. A read before any ptb_render_aov, an unknown aov or a wrong n_floats fails with PTB_ERR_INVALID. */
+int32_t ptb_aov_read(ptb_ctx* ctx, uint32_t aov, float* out, size_t n_floats, int32_t normalise);
+
 /* ------------------------------------------------------------ multi-GPU -- */
 /* The path shards by samples (independent), scene and BVH replicated per GPU: rank r of `world` renders the absolute
  * samples [first, first + count) of every pixel. */

@@ -29,6 +29,7 @@ METHOD_NAIVE, METHOD_MIS = 0, 1
 PERLIN_TABLE_WORDS = 1024
 OPT_TIME_KERNELS, OPT_COUNT_TRAVERSAL = 1, 2
 BUILD_DEFAULT, BUILD_BINARY, BUILD_WIDE, BUILD_SAH, BUILD_REFIT = 0, 1, 2, 4, 8
+PTB_AOV_ALBEDO, PTB_AOV_NORMAL, PTB_AOV_DEPTH, PTB_AOV_COVERAGE = range(4)
 
 # numpy mirrors of the POD structs (sizes asserted against the header's layout in tests/test_abi.py)
 sphere_dtype = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4")])
@@ -138,6 +139,9 @@ SYMBOLS = [
     ("ptb_accum_read", C.c_int32, [_P, _P, C.c_size_t, C.c_int32]),
     ("ptb_accum_device_ptr", C.c_int32, [_P, C.POINTER(_P), C.POINTER(C.c_size_t)]),
     ("ptb_accum_set_samples", C.c_int32, [_P, C.c_uint64]),
+    ("ptb_render_aov", C.c_int32, [_P, C.POINTER(RenderOpts)]),
+    ("ptb_aov_clear", C.c_int32, [_P]),
+    ("ptb_aov_read", C.c_int32, [_P, C.c_uint32, _P, C.c_size_t, C.c_int32]),
     ("ptb_shard_samples", None, [C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     ("ptb_shard_rows", None, [C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     ("ptb_render_multi", C.c_int32, [_P, C.c_int32, C.POINTER(RenderOpts)]),

@@ -317,6 +317,23 @@ class Context:
     def accum_set_samples(self, n: int):
         _check(self._h, L.lib.ptb_accum_set_samples(self._h, n))
 
+    # ---- denoiser feature buffers
+    def render_aov(self, opts: RenderOptions):
+        """Adds the first-hit albedo, normal, depth and coverage of the camera rays `render(opts)` traces into the AOV
+        sums (render_method, max_depth and rr_threshold are not read)."""
+        o = opts.to_c()
+        _check(self._h, L.lib.ptb_render_aov(self._h, C.byref(o)))
+
+    def aov_clear(self):
+        _check(self._h, L.lib.ptb_aov_clear(self._h))
+
+    def aov_read(self, width: int, height: int, aov: int, normalise: bool = True) -> np.ndarray:
+        """One AOV buffer (L.PTB_AOV_*): (H, W, 3) float32 for albedo and normal, (H, W) for depth and coverage."""
+        c = 3 if aov in (L.PTB_AOV_ALBEDO, L.PTB_AOV_NORMAL) else 1
+        out = np.empty(width * height * c, np.float32)
+        _check(self._h, L.lib.ptb_aov_read(self._h, aov, L.ptr(out), out.size, 1 if normalise else 0))
+        return out.reshape((height, width, 3) if c == 3 else (height, width))
+
     # ---- sampler test hook (the reference's chi-squared harness pointed at the device samplers)
     @staticmethod
     def _query(kind, alpha, normal, aux, light_index, seed) -> L.SamplerQuery:
@@ -392,6 +409,14 @@ class Scene:
         self.ctx.accum_clear()
         RandomSampler().sample_image(opts, self.acceleration, update, presentation_update)
         return self.ctx.accum_read(opts.width, opts.height, normalise=True)
+
+    def render_aov(self, opts: RenderOptions) -> dict:
+        """The denoiser feature buffers of the samples `render(opts)` takes: {"albedo", "normal"} (H, W, 3) and {"depth",
+        "coverage"} (H, W), normalised (depth is the mean over the samples that hit)."""
+        self.ctx.aov_clear()
+        self.ctx.render_aov(opts)
+        names = {"albedo": L.PTB_AOV_ALBEDO, "normal": L.PTB_AOV_NORMAL, "depth": L.PTB_AOV_DEPTH, "coverage": L.PTB_AOV_COVERAGE}
+        return {k: self.ctx.aov_read(opts.width, opts.height, a) for k, a in names.items()}
 
 
 def render_multi(contexts, opts: RenderOptions) -> np.ndarray:

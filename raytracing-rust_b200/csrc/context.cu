@@ -647,17 +647,24 @@ static int32_t ensure_accum(Ctx* c, uint32_t w, uint32_t h) {
   return PTB_OK;
 }
 
-int32_t ptb_render(ptb_ctx* ctx, const ptb_render_opts* opts, ptb_progress_fn progress, void* user) {
-  CTX_OR_FAIL(ctx);
+// the option checks of every render entry point; `method` is not read by ptb_render_aov
+static int32_t check_render_opts(Ctx* c, const ptb_render_opts* opts, bool method) {
   if (!opts) return set_error(c, PTB_ERR_INVALID, "null render opts");
   if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
   if (opts->width < 2 || opts->height < 2) return set_error(c, PTB_ERR_INVALID, "width and height must be >= 2");
   if ((uint64_t)opts->width * opts->height > 0x7FFFFFFFull) return set_error(c, PTB_ERR_INVALID, "image too large");
-  if (opts->method != PTB_METHOD_NAIVE && opts->method != PTB_METHOD_MIS) return set_error(c, PTB_ERR_INVALID, "unknown method");
+  if (method && opts->method != PTB_METHOD_NAIVE && opts->method != PTB_METHOD_MIS) return set_error(c, PTB_ERR_INVALID, "unknown method");
   if (opts->row_begin >= opts->height || (uint64_t)opts->row_begin + opts->row_count > opts->height)
     return set_error(c, PTB_ERR_INVALID, "image tile rows [%u, %u) outside the %u rows of the image", opts->row_begin,
                      opts->row_begin + opts->row_count, opts->height);
-  int32_t rc = ensure_accum(c, opts->width, opts->height);
+  return PTB_OK;
+}
+
+int32_t ptb_render(ptb_ctx* ctx, const ptb_render_opts* opts, ptb_progress_fn progress, void* user) {
+  CTX_OR_FAIL(ctx);
+  int32_t rc = check_render_opts(c, opts, true);
+  if (rc != PTB_OK) return rc;
+  rc = ensure_accum(c, opts->width, opts->height);
   if (rc != PTB_OK) return rc;
   rc = render_wavefront(c, *opts, progress, user);
   if (rc == PTB_ERR_ABORTED) {
@@ -678,15 +685,9 @@ __global__ void k_add_into(const float* __restrict__ src, float* __restrict__ ds
 
 int32_t ptb_render_passes(ptb_ctx* ctx, const ptb_render_opts* opts, ptb_pass_fn update, void* user) {
   CTX_OR_FAIL(ctx);
-  if (!opts) return set_error(c, PTB_ERR_INVALID, "null render opts");
-  if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
-  if (opts->width < 2 || opts->height < 2) return set_error(c, PTB_ERR_INVALID, "width and height must be >= 2");
-  if ((uint64_t)opts->width * opts->height > 0x7FFFFFFFull) return set_error(c, PTB_ERR_INVALID, "image too large");
-  if (opts->method != PTB_METHOD_NAIVE && opts->method != PTB_METHOD_MIS) return set_error(c, PTB_ERR_INVALID, "unknown method");
-  if (opts->row_begin >= opts->height || (uint64_t)opts->row_begin + opts->row_count > opts->height)
-    return set_error(c, PTB_ERR_INVALID, "image tile rows [%u, %u) outside the %u rows of the image", opts->row_begin,
-                     opts->row_begin + opts->row_count, opts->height);
-  int32_t rc = ensure_accum(c, opts->width, opts->height);
+  int32_t rc = check_render_opts(c, opts, true);
+  if (rc != PTB_OK) return rc;
+  rc = ensure_accum(c, opts->width, opts->height);
   if (rc != PTB_OK) return rc;
   const size_t n = (size_t)opts->width * opts->height * 3;
   PTB_CUDA_TRY(c, c->d_pass.reserve(n * sizeof(float)));
@@ -765,6 +766,77 @@ int32_t ptb_accum_device_ptr(ptb_ctx* ctx, void** d_ptr, size_t* n_floats) {
 int32_t ptb_accum_set_samples(ptb_ctx* ctx, uint64_t total_samples) {
   CTX_OR_FAIL(ctx);
   c->accum_samples = total_samples;
+  return PTB_OK;
+}
+
+// ---------------------------------------------------------------- denoiser feature buffers
+static int32_t ensure_aov(Ctx* c, uint32_t w, uint32_t h) {
+  if (c->aov_w == w && c->aov_h == h && c->d_aov.p) return PTB_OK;
+  const size_t bytes = (size_t)w * h * 8 * sizeof(float);
+  PTB_CUDA_TRY(c, c->d_aov.alloc(bytes));
+  PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_aov.p, 0, bytes, c->stream));
+  c->aov_w = w;
+  c->aov_h = h;
+  c->aov_samples = 0;
+  return PTB_OK;
+}
+
+int32_t ptb_render_aov(ptb_ctx* ctx, const ptb_render_opts* opts) {
+  CTX_OR_FAIL(ctx);
+  int32_t rc = check_render_opts(c, opts, false);
+  if (rc != PTB_OK) return rc;
+  if ((uint64_t)opts->sample_offset + opts->samples_per_pixel > kMaxSampleIndex)
+    return set_error(c, PTB_ERR_INVALID, "sample_offset + samples_per_pixel must be <= %u", kMaxSampleIndex);
+  rc = ensure_aov(c, opts->width, opts->height);
+  if (rc != PTB_OK) return rc;
+  rc = launch_aov(c, *opts);
+  if (rc != PTB_OK) return rc;
+  c->aov_samples += opts->samples_per_pixel;
+  return PTB_OK;
+}
+
+int32_t ptb_aov_clear(ptb_ctx* ctx) {
+  CTX_OR_FAIL(ctx);
+  if (c->d_aov.p) PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_aov.p, 0, (size_t)c->aov_w * c->aov_h * 8 * sizeof(float), c->stream));
+  c->aov_samples = 0;
+  return PTB_OK;
+}
+
+// one buffer out of the per-pixel records [albedo.rgb | coverage] [normal.xyz | depth]; normalise: albedo, normal and
+// coverage over the sample count, depth over the pixel's coverage (0 where nothing was hit)
+__global__ void k_aov_read(const float4* __restrict__ sums, float* __restrict__ out, size_t npix, uint32_t aov,
+                           int normalise, float samples) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= npix) return;
+  const float4 s0 = sums[2 * i], s1 = sums[2 * i + 1];
+  if (aov == PTB_AOV_ALBEDO || aov == PTB_AOV_NORMAL) {
+    const float4 s = aov == PTB_AOV_ALBEDO ? s0 : s1;
+    out[3 * i + 0] = normalise ? s.x / samples : s.x;
+    out[3 * i + 1] = normalise ? s.y / samples : s.y;
+    out[3 * i + 2] = normalise ? s.z / samples : s.z;
+  } else if (aov == PTB_AOV_DEPTH) {
+    out[i] = normalise ? (s0.w > 0.0f ? s1.w / s0.w : 0.0f) : s1.w;
+  } else {
+    out[i] = normalise ? s0.w / samples : s0.w;
+  }
+}
+
+int32_t ptb_aov_read(ptb_ctx* ctx, uint32_t aov, float* out, size_t n_floats, int32_t normalise) {
+  CTX_OR_FAIL(ctx);
+  if (!c->d_aov.p) return set_error(c, PTB_ERR_INVALID, "no AOV rendered yet");
+  if (aov > PTB_AOV_COVERAGE) return set_error(c, PTB_ERR_INVALID, "unknown AOV %u", aov);
+  const size_t npix = (size_t)c->aov_w * c->aov_h;
+  const size_t n = npix * (aov == PTB_AOV_ALBEDO || aov == PTB_AOV_NORMAL ? 3 : 1);
+  if (!out || n_floats != n) return set_error(c, PTB_ERR_INVALID, "aov_read expects %zu floats", n);
+  PTB_CUDA_TRY(c, c->d_hits.reserve(n * sizeof(float)));
+  // with no samples yet there is nothing to divide by: the (zero) sums are returned, as ptb_accum_read does
+  const int norm = normalise && c->aov_samples > 0;
+  k_aov_read<<<(unsigned)((npix + 255) / 256), 256, 0, c->stream>>>(c->d_aov.as<float4>(), c->d_hits.as<float>(), npix, aov,
+                                                                    norm, (float)c->aov_samples);
+  c->stats.kernel_launches += 1;
+  PTB_CUDA_TRY(c, cudaGetLastError());
+  PTB_CUDA_TRY(c, cudaMemcpyAsync(out, c->d_hits.p, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
   return PTB_OK;
 }
 

@@ -133,6 +133,11 @@ struct Ctx {
   size_t h_pass_floats = 0;
   uint32_t accum_w = 0, accum_h = 0;
   uint64_t accum_samples = 0;
+  // denoiser feature buffers (ptb_render_aov): 8 float sums per pixel, [albedo.rgb | coverage] [normal.xyz | depth],
+  // and the work cursors of one call's k_aov launches (one per sample)
+  DevBuf d_aov, d_aov_heads;
+  uint32_t aov_w = 0, aov_h = 0;
+  uint64_t aov_samples = 0;
   DevBuf d_pool_mem, d_prev, d_queues, d_shadow, d_counters, d_windows;
   // second chunk slot of the window wavefront: chunk k+1's wide iterations run on the main stream while chunk k's fused
   // tail (k_tail) finishes on `s_tail` in the other slot
@@ -197,6 +202,8 @@ size_t radix_sort_hist_words(uint32_t n);
 // wavefront.cu
 int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progress, void* user);
 int32_t launch_closest_hit(Ctx* c, const void* d_rays, size_t n, void* d_hits);
+// ptb_render_aov's launches, opts validated; adds into d_aov
+int32_t launch_aov(Ctx* c, const ptb_render_opts& o);
 // check_hit_index (d_index != nullptr: ptb_ray in, ptb_hit out) or occlusion (ptb_occlusion_ray in, one byte out)
 int32_t launch_visibility(Ctx* c, const void* d_rays, const void* d_index, size_t n, void* d_out);
 void free_render_state(Ctx* c);

@@ -1432,6 +1432,70 @@ k_closest_hit_api(DevScene sc, const float4* __restrict__ rays, const uint32_t* 
   }
 }
 
+// ------------------------------------------------------------------------------------------ denoiser feature buffers
+// ptb_render_aov: the first hit of the camera ray of every (pixel, sample) that ptb_render traces, reduced to what a
+// denoiser reads. One launch per sample; work item i is the i-th pixel of the tile in the render's issue order
+// (camera_pixel_sample with group 1, so rp.sample_offset is the launch's sample), and its ray is the render's camera
+// ray: camera_direction + make_ray. Each pixel occurs once per launch, so its sums are updated with a plain
+// read-add-write and are formed in sample order: deterministic, and independent of how a call is split.
+// Sums per pixel, two 16-byte records: [albedo.rgb | coverage], [normal.xyz | depth].
+struct AovFetch {
+  const DevScene& sc;
+  const RenderParams& rp;
+  uint32_t pixel;
+  PTB_DEV void operator()(uint32_t i, Ray& r, float& /*tmax*/, uint32_t& /*exclude*/) {
+    uint32_t x, y, sample;
+    camera_pixel_sample(rp, i, x, y, sample);
+    pixel = y * rp.width + x;
+    r = make_ray(sc.cam_origin, camera_direction(sc, rp, x, y, sample));
+  }
+};
+struct AovRetire {
+  const DevScene& sc;
+  float4* __restrict__ sums;
+  const AovFetch& f;
+  PTB_DEV void operator()(bool fin, const TraceResult& tr, const Ray& ray) {
+    if (!fin) return;
+    const bool hit = tr.ref != kNone;
+    HitRec h;
+    uint32_t kind = PTB_MAT_EMIT, tex = sc.sky_tex;
+    float param = 1.0f;
+    if (hit) {
+      prim_hit(sc, ray, tr.ref, h);
+      const DevMaterial* m = sc.materials + (__ldg(sc.slot_mat + (tr.ref & kSlotMask)) & 0x00FFFFFFu);
+      kind = __ldg(&m->kind);
+      tex = __ldg(&m->tex);
+      param = __ldg(&m->param);
+    } else {  // sky.rs:79-91: zero Hit + Emit(sky texture, 1.0), as k_shade treats a miss
+      h.t = 0.0f;
+      h.point = h.error = h.normal = mk(0.0f, 0.0f, 0.0f);
+    }
+    v3 a;
+    if (kind == PTB_MAT_EMIT) {  // the emission the depth-0 integrator adds (emissive.rs:23-26)
+      a = param * texture_colour<true>(sc, tex, ray.d, offset_ray(h.point, h.normal, h.error, true));
+    } else {
+      a = texture_colour<true>(sc, tex, ray.d, h.point);
+      if (kind == PTB_MAT_LAMBERTIAN) a = a * param;  // the colour factor of mat_eval
+    }
+    // denoisers expect albedo in [0, 1]; fminf / fmaxf also turn a NaN into 0
+    a = mk(fminf(fmaxf(a.x, 0.0f), 1.0f), fminf(fmaxf(a.y, 0.0f), 1.0f), fminf(fmaxf(a.z, 0.0f), 1.0f));
+    float4* p = sums + 2u * (size_t)f.pixel;
+    float4 s0 = p[0], s1 = p[1];
+    s0.x += a.x; s0.y += a.y; s0.z += a.z; s0.w += hit ? 1.0f : 0.0f;
+    s1.x += h.normal.x; s1.y += h.normal.y; s1.z += h.normal.z; s1.w += h.t;
+    p[0] = s0;
+    p[1] = s1;
+  }
+};
+template <class TR>
+__global__ void __launch_bounds__(256, TR::kApiMinBlocks)
+k_aov(DevScene sc, RenderParams rp, float4* __restrict__ sums, uint32_t* head) {
+  uint32_t a = 0, b = 0, r = 0;
+  AovFetch fetch{sc, rp, 0u};
+  AovRetire retire{sc, sums, fetch};
+  persistent_trace<TR, false, false>(sc, rp.npix, head, fetch, retire, a, b, r);
+}
+
 // ------------------------------------------------------------------------------------------ visibility API kernel
 // Batch any-hit through the walk k_shadow runs (persistent_trace<TR, ANYHIT = true>), fed from caller records.
 //   CHI  : check_hit_index (acceleration/mod.rs:226-263): ptb_ray + target id in, ptb_hit out. The target's own hit is
@@ -1602,6 +1666,7 @@ static const void* api_kernel(const Ctx* c, bool count) {
   if (c->wide) return count ? (const void*)k_closest_hit_api<CwTrav, true> : (const void*)k_closest_hit_api<CwTrav, false>;
   return count ? (const void*)k_closest_hit_api<BinTrav, true> : (const void*)k_closest_hit_api<BinTrav, false>;
 }
+static const void* aov_kernel(const Ctx* c) { return c->wide ? (const void*)k_aov<CwTrav> : (const void*)k_aov<BinTrav>; }
 static const void* visibility_kernel(const Ctx* c, bool chi) {
   if (c->wide) return chi ? (const void*)k_visibility_api<CwTrav, true> : (const void*)k_visibility_api<CwTrav, false>;
   return chi ? (const void*)k_visibility_api<BinTrav, true> : (const void*)k_visibility_api<BinTrav, false>;
@@ -1705,6 +1770,47 @@ int32_t launch_visibility(Ctx* c, const void* d_rays, const void* d_index, size_
   PTB_CUDA_TRY(c, cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(256), args, 0, c->stream));
   c->stats.kernel_launches += 1;
   c->stats.trace_launches += 1;
+  PTB_CUDA_TRY(c, cudaGetLastError());
+  return PTB_OK;
+}
+
+// Pixel issue order: 32 consecutive pixel indices cover an 8 x 4 tile when the image allows (else 16 x 2, else a row), so
+// the 16 pixels of a 4096-slot window are an 8 x 2 block instead of a 16 x 1 strip: the origins of a window's rays lie
+// closer together. C3: 3793 -> 3834 Mrays/s. PTB_TILES=0 keeps rows.
+static void pick_tiles(RenderParams& rp, uint32_t width, uint32_t rows) {
+  rp.tile_w = 32u; rp.tile_h = 1u;
+  bool tiles = true;
+  if (const char* e = getenv("PTB_TILES")) tiles = atoi(e) != 0;
+  if (tiles)
+    for (uint32_t th = 4u; th > 1u; th >>= 1)
+      if (rows % th == 0u && width % (32u / th) == 0u) { rp.tile_h = th; rp.tile_w = 32u / th; break; }
+}
+
+// ptb_render_aov after validation: one k_aov launch per sample of the call, each over the tile's pixels in the render's
+// tile order. Every launch has its own work cursor, all zeroed by one memset.
+int32_t launch_aov(Ctx* c, const ptb_render_opts& o) {
+  const uint32_t rows = o.row_count ? o.row_count : o.height - o.row_begin;
+  const uint32_t spp = o.samples_per_pixel;
+  if (spp == 0) return PTB_OK;
+  RenderParams rp{};
+  rp.width = o.width; rp.height = o.height; rp.npix = o.width * rows;
+  rp.row_begin = o.row_begin;
+  pick_tiles(rp, o.width, rows);
+  rp.group = 1u;
+  rp.k0 = (uint32_t)o.seed; rp.k1 = (uint32_t)(o.seed >> 32);
+  PTB_CUDA_TRY(c, c->d_aov_heads.reserve((size_t)spp * 4));
+  PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_aov_heads.p, 0, (size_t)spp * 4, c->stream));
+  const void* fn = aov_kernel(c);
+  const int grid = persistent_grid(c, fn, 256);
+  float4* sums = c->d_aov.as<float4>();
+  for (uint32_t s = 0; s < spp; ++s) {
+    rp.sample_offset = o.sample_offset + s;
+    uint32_t* head = c->d_aov_heads.as<uint32_t>() + s;
+    void* args[] = {(void*)&c->dev, (void*)&rp, (void*)&sums, (void*)&head};
+    PTB_CUDA_TRY(c, cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(256), args, 0, c->stream));
+    c->stats.kernel_launches += 1;
+    c->stats.trace_launches += 1;
+  }
   PTB_CUDA_TRY(c, cudaGetLastError());
   return PTB_OK;
 }
@@ -1857,15 +1963,7 @@ int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progr
   RenderParams& rp = rs.rp;
   rp.width = o.width; rp.height = o.height; rp.npix = npix;
   rp.row_begin = o.row_begin;
-  // Pixel issue order: 32 consecutive pixel indices cover an 8 x 4 tile when the image allows (else 16 x 2, else a row), so
-  // the 16 pixels of a 4096-slot window are an 8 x 2 block instead of a 16 x 1 strip: the origins of a window's rays lie
-  // closer together. C3: 3793 -> 3834 Mrays/s. PTB_TILES=0 keeps rows.
-  rp.tile_w = 32u; rp.tile_h = 1u;
-  bool tiles = true;
-  if (const char* e = getenv("PTB_TILES")) tiles = atoi(e) != 0;
-  if (tiles)
-    for (uint32_t th = 4u; th > 1u; th >>= 1)
-      if (rows % th == 0u && o.width % (32u / th) == 0u) { rp.tile_h = th; rp.tile_w = 32u / th; break; }
+  pick_tiles(rp, o.width, rows);
   // samples of one pixel issued back to back: the largest divisor of spp <= 1024 (PTB_SAMPLE_GROUP). Measured on C3 at
   // 256 spp: group 1 -> 2760 Mrays/s, 32 -> 3066, 256 -> 3197 (camera rays of a warp walk the same nodes).
   rp.group = 1u;
