@@ -124,6 +124,21 @@ impl CudaScene {
         }
         Ok((albedo, normal, depth, coverage))
     }
+
+    /// `render(opts, seed)` denoised on the device: the samples, the feature buffers of the same camera rays, then the
+    /// spatial SVGF filter (`denoise`: ptb_denoise_opts, all zeros for the defaults). Same layout as `render`'s image.
+    pub fn render_denoised(&self, opts: RenderOptions, seed: u64, denoise: ptb_denoise_opts) -> Result<Vec<Float>, String> {
+        let o = self.opts(opts, seed);
+        let mut image = vec![0.0 as Float; (opts.width * opts.height * 3) as usize];
+        unsafe {
+            check(self.ctx, ptb_accum_clear(self.ctx))?;
+            check(self.ctx, ptb_render(self.ctx, &o, None, ptr::null_mut()))?;
+            check(self.ctx, ptb_aov_clear(self.ctx))?;
+            check(self.ctx, ptb_render_aov(self.ctx, &o))?;
+            check(self.ctx, ptb_denoise(self.ctx, &denoise, image.as_mut_ptr(), image.len()))?;
+        }
+        Ok(image)
+    }
 }
 
 impl CudaScene {

@@ -37,6 +37,9 @@ pub struct ptb_render_opts {
     /// image tile (ABI 2): rows [row_begin, row_begin + row_count) only; row_count 0 = to the last row
     pub row_begin: u32, pub row_count: u32,
 }
+/// denoiser options (ptb_denoise); 0 selects a default: 5 levels, sigma_luminance 4, sigma_normal 128, sigma_depth 1
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct ptb_denoise_opts { pub iterations: u32, pub sigma_luminance: f32, pub sigma_normal: f32, pub sigma_depth: f32, pub flags: u32 }
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct ptb_stats {
     pub rays_camera: u64, pub rays_bounce: u64, pub rays_shadow_light: u64, pub rays_shadow_sky: u64,
@@ -109,6 +112,8 @@ extern "C" {
     pub fn ptb_render_aov(ctx: *mut ptb_ctx, opts: *const ptb_render_opts) -> i32;
     pub fn ptb_aov_clear(ctx: *mut ptb_ctx) -> i32;
     pub fn ptb_aov_read(ctx: *mut ptb_ctx, aov: u32, out: *mut f32, n_floats: usize, normalise: i32) -> i32;
+    pub fn ptb_denoise(ctx: *mut ptb_ctx, opts: *const ptb_denoise_opts, rgb: *mut f32, n_floats: usize) -> i32;
+    pub fn ptb_denoise_device(ctx: *mut ptb_ctx, opts: *const ptb_denoise_opts, d_rgb: *mut c_void) -> i32;
     pub fn ptb_sample_only(ctx: *mut ptb_ctx, query: *const ptb_sampler_query, n: usize, dirs: *mut f32, pdf: *mut f32) -> i32;
     pub fn ptb_sampler_pdf(ctx: *mut ptb_ctx, query: *const ptb_sampler_query, dirs: *const f32, n: usize, pdf: *mut f32) -> i32;
     pub fn ptb_stats_get(ctx: *mut ptb_ctx, out: *mut ptb_stats) -> i32;

@@ -460,6 +460,55 @@ int32_t ptb_aov_clear(ptb_ctx* ctx);
  * stream. A read before any ptb_render_aov, an unknown aov or a wrong n_floats fails with PTB_ERR_INVALID. */
 int32_t ptb_aov_read(ptb_ctx* ctx, uint32_t aov, float* out, size_t n_floats, int32_t normalise);
 
+/* ------------------------------------------------------------- denoiser -- */
+/* The spatial part of SVGF (Schied et al., "Spatiotemporal Variance-Guided Filtering", HPG 2017, §4.3-4.5): Dammertz et
+ * al. 2010's edge-avoiding à-trous wavelet filter with albedo demodulation and variance-guided luminance weights, over the
+ * beauty accumulator (sums of S_b = the accumulated sample count) and the AOV sums (S_a samples). All arithmetic is f32,
+ * without contraction, in the order written; only exp2f, log2f (and sqrtf, IEEE) are the platform's.
+ * Inputs per pixel p:
+ *   c = beauty sum * (1/S_b)   (as ptb_accum_read normalises)      a = albedo sum / S_a      α = coverage sum / S_a
+ *   n = normal sum / |normal sum|, |v| = sqrtf((v.x*v.x + v.y*v.y) + v.z*v.z); (0,0,0) where that length is 0
+ *   z = depth sum / coverage sum, 0 where the coverage sum is 0 (as ptb_aov_read normalises)
+ * Prepare:  d = max(a, 1e-3) per channel; irradiance e = c / d per channel; luminance ℓ(e) = (0.2126 e.r + 0.7152 e.g)
+ *   + 0.0722 e.b. Depth gradient ∂x z: of the one-sided differences f = z[x+1] - z[x] and b = z[x] - z[x-1], counting only
+ *   neighbours inside the image whose coverage sum is > 0: both -> |f| <= |b| ? f : b; one -> that one; none -> 0. ∂y z alike
+ *   (y + 1 is the next row down). The sums are finite (the render zeroes non-finite samples); there is no guard.
+ * Edge stopping, centre p, tap q at pixel offset Δ = (Δx, Δy):
+ *   w_α = 1 - |α_p - α_q|
+ *   w_n: both normals zero -> 1; exactly one zero -> 0 (the tap is dropped); otherwise max(0, n_p·n_q)^σ_n,
+ *        n_p·n_q = (n_p.x*n_q.x + n_p.y*n_q.y) + n_p.z*n_q.z
+ *   D_z = (σ_z * |∂x z_p * Δx + ∂y z_p * Δy| + 1e-3 * z_p) + 1e-6,  t_z = |z_p - z_q| / D_z,  w_z = exp(-t_z)
+ *   D_l = σ_l * sqrtf(g_p) + 1e-10,  t_l = |ℓ_p - ℓ_q| / D_l,  w_l = exp(-t_l); g_p = Σ k var / Σ k over the 3x3
+ *        neighbours inside the image (row by row), k = 1/4 at the centre, 1/8 beside it, 1/16 at the corners
+ *   w_n * w_z (* w_l) is ONE exp2: exp2f(σ_n * log2f(max(0, n_p·n_q)) - (t_z (+ t_l)) * log2(e)) (σ_n * log2f(...) is 0 when
+ *   both normals are zero), so the product is w_α * that.
+ * Variance (SVGF's spatial estimate): over the 7x7 window inside the image, row by row, w = w_α * exp2f(σ_n log2f(n·n) -
+ *   t_z log2(e)) (no w_l; the centre's w is exactly 1): μ1 = Σ w ℓ / Σ w, μ2 = Σ w ℓ² / Σ w, var = max(0, μ2 - μ1*μ1).
+ * Level i = 0 .. L-1, step s = 2^i: taps q = p + s*(dx, dy), dx, dy in [-2, 2], inside the image, row by row;
+ *   W_q = (h(dx)*h(dy)) * w_α * exp2f(σ_n log2f(n·n) - (t_z + t_l) log2(e)), Δ = s*(dx, dy), h = (3/8, 1/4, 1/16) by |d|;
+ *   the centre's W is exactly h(0)² (the sum is never 0). e'_p = Σ W e / Σ W per channel; var'_p = Σ (W*W) var / (ΣW*ΣW).
+ * Output: e^(L) * d, RGB, W*H*3 floats in ptb_accum_read's layout.
+ * Defaults (0 selects them): L = 5, σ_l = 4, σ_n = 128, σ_z = 1 (SVGF's). Temporal accumulation is not part of this filter.
+ *
+ * Both accumulators are read and left bit-identical, sums and sample counts. The output is a pure function of them and
+ * the options (no atomics: two calls give the same bits). Each launch (one prepare, one variance, one per level) counts in
+ * ptb_stats.kernel_launches; none in trace_launches or the ray counters. The scratch (ping-pong irradiance + variance and
+ * the guide records, 60 bytes per pixel) belongs to the context: allocated at first use, reallocated on a size change.
+ * Errors, PTB_ERR_INVALID before anything is enqueued: null opts; nothing rendered or no AOV rendered yet; beauty and AOV
+ * sizes differ; a sample count of 0 (e.g. after a clear); iterations > 10; a negative, NaN or infinite sigma; flags != 0;
+ * a null output or n_floats != W*H*3. */
+typedef struct ptb_denoise_opts {
+  uint32_t iterations;      /* à-trous levels, step 2^i; 0 -> 5; at most 10 */
+  float sigma_luminance;    /* 0 -> 4   */
+  float sigma_normal;       /* 0 -> 128 */
+  float sigma_depth;        /* 0 -> 1   */
+  uint32_t flags;           /* reserved, 0 */
+} ptb_denoise_opts;
+/* Denoises into host memory (W*H*3 floats); synchronises the stream. */
+int32_t ptb_denoise(ptb_ctx* ctx, const ptb_denoise_opts* opts, float* rgb, size_t n_floats);
+/* Enqueues the same work on the context's stream into a device buffer of W*H*3 floats and returns without waiting. */
+int32_t ptb_denoise_device(ptb_ctx* ctx, const ptb_denoise_opts* opts, void* d_rgb);
+
 /* ------------------------------------------------------------ multi-GPU -- */
 /* The path shards by samples (independent), scene and BVH replicated per GPU: rank r of `world` renders the absolute
  * samples [first, first + count) of every pixel. */

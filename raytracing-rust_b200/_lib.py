@@ -55,6 +55,11 @@ class RenderOpts(C.Structure):
                 ("row_begin", C.c_uint32), ("row_count", C.c_uint32)]
 
 
+class DenoiseOpts(C.Structure):
+    _fields_ = [("iterations", C.c_uint32), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float),
+                ("sigma_depth", C.c_float), ("flags", C.c_uint32)]
+
+
 class Stats(C.Structure):
     _fields_ = [("rays_camera", C.c_uint64), ("rays_bounce", C.c_uint64), ("rays_shadow_light", C.c_uint64),
                 ("rays_shadow_sky", C.c_uint64), ("rays_reference", C.c_uint64), ("paths", C.c_uint64),
@@ -142,6 +147,8 @@ SYMBOLS = [
     ("ptb_render_aov", C.c_int32, [_P, C.POINTER(RenderOpts)]),
     ("ptb_aov_clear", C.c_int32, [_P]),
     ("ptb_aov_read", C.c_int32, [_P, C.c_uint32, _P, C.c_size_t, C.c_int32]),
+    ("ptb_denoise", C.c_int32, [_P, C.POINTER(DenoiseOpts), _P, C.c_size_t]),
+    ("ptb_denoise_device", C.c_int32, [_P, C.POINTER(DenoiseOpts), _P]),
     ("ptb_shard_samples", None, [C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     ("ptb_shard_rows", None, [C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     ("ptb_render_multi", C.c_int32, [_P, C.c_int32, C.POINTER(RenderOpts)]),

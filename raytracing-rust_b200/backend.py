@@ -45,6 +45,12 @@ class RenderOptions:
                             self.max_depth, self.rr_threshold, 0, self.seed, self.row_begin, self.row_count)
 
 
+def denoise_opts(iterations: int = 0, sigma_luminance: float = 0.0, sigma_normal: float = 0.0, sigma_depth: float = 0.0,
+                 flags: int = 0) -> L.DenoiseOpts:
+    """ptb_denoise_opts; 0 selects a default (5 levels, sigma_luminance 4, sigma_normal 128, sigma_depth 1)."""
+    return L.DenoiseOpts(iterations, sigma_luminance, sigma_normal, sigma_depth, flags)
+
+
 class Context:
     """One ptb_ctx == one GPU."""
 
@@ -334,6 +340,20 @@ class Context:
         _check(self._h, L.lib.ptb_aov_read(self._h, aov, L.ptr(out), out.size, 1 if normalise else 0))
         return out.reshape((height, width, 3) if c == 3 else (height, width))
 
+    # ---- denoiser
+    def denoise(self, width: int, height: int, **opts) -> np.ndarray:
+        """The beauty accumulator filtered by the spatial SVGF filter, guided by the AOV sums: (H, W, 3) float32. Keyword
+        options (0 selects the default): iterations (5), sigma_luminance (4), sigma_normal (128), sigma_depth (1)."""
+        o = denoise_opts(**opts)
+        out = np.empty(width * height * 3, np.float32)
+        _check(self._h, L.lib.ptb_denoise(self._h, C.byref(o), L.ptr(out), out.size))
+        return out.reshape(height, width, 3)
+
+    def denoise_device(self, d_rgb_ptr: int, **opts):
+        """As denoise, into a device buffer of W*H*3 floats; enqueued on the context's stream, not waited for."""
+        o = denoise_opts(**opts)
+        _check(self._h, L.lib.ptb_denoise_device(self._h, C.byref(o), C.c_void_p(d_rgb_ptr)))
+
     # ---- sampler test hook (the reference's chi-squared harness pointed at the device samplers)
     @staticmethod
     def _query(kind, alpha, normal, aux, light_index, seed) -> L.SamplerQuery:
@@ -417,6 +437,15 @@ class Scene:
         self.ctx.render_aov(opts)
         names = {"albedo": L.PTB_AOV_ALBEDO, "normal": L.PTB_AOV_NORMAL, "depth": L.PTB_AOV_DEPTH, "coverage": L.PTB_AOV_COVERAGE}
         return {k: self.ctx.aov_read(opts.width, opts.height, a) for k, a in names.items()}
+
+    def render_denoised(self, opts: RenderOptions, **denoise) -> np.ndarray:
+        """render(opts) and the feature buffers of the same samples, then the denoised image (H, W, 3); `denoise` takes
+        Context.denoise's keyword options."""
+        self.ctx.accum_clear()
+        self.ctx.render(opts)
+        self.ctx.aov_clear()
+        self.ctx.render_aov(opts)
+        return self.ctx.denoise(opts.width, opts.height, **denoise)
 
 
 def render_multi(contexts, opts: RenderOptions) -> np.ndarray:

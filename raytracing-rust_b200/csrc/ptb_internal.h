@@ -138,6 +138,10 @@ struct Ctx {
   DevBuf d_aov, d_aov_heads;
   uint32_t aov_w = 0, aov_h = 0;
   uint64_t aov_samples = 0;
+  // denoiser scratch (denoise.cu), dn_w x dn_h pixels: ping-pong [e.rgb | var] and the guide records [n.xyz | z],
+  // coverage α and the depth gradient [∂x z, ∂y z]
+  DevBuf d_dn_e[2], d_dn_nz, d_dn_alpha, d_dn_grad;
+  uint32_t dn_w = 0, dn_h = 0;
   DevBuf d_pool_mem, d_prev, d_queues, d_shadow, d_counters, d_windows;
   // second chunk slot of the window wavefront: chunk k+1's wide iterations run on the main stream while chunk k's fused
   // tail (k_tail) finishes on `s_tail` in the other slot

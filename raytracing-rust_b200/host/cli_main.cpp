@@ -5,6 +5,8 @@
 //              [--gpus 1] [--seed 0] [--max-depth 50] [-b sah|middle|equal-counts (accepted, ignored: the device builds its own tree)]
 // --gpus N renders on GPUs device .. device+N-1 through ptb_render_multi (samples split N ways, or bands of image rows
 // when there are fewer samples than GPUs; one ncclReduce of the accumulators) — the rayon fan-out of random_sampler.rs:40-80.
+// --denoise renders the first-hit feature buffers of the same camera samples (ptb_render_aov, on GPU `device` after the
+// reduce) and writes the image ptb_denoise makes of them instead of the noisy one; use .pfm or .exr to keep it linear f32.
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -33,6 +35,7 @@ struct Cli {
   int gpus = 1;
   unsigned long long seed = 0;
   unsigned max_depth = 50;
+  bool denoise = false;
 };
 
 void log_line(const char* level, const char* target, const std::string& msg) {
@@ -80,7 +83,9 @@ int usage(const char* argv0, const char* err) {
                "      --device <INDEX>                 [default: 0]\n"
                "      --gpus <N>                       [default: 1] GPUs device .. device+N-1 of this box\n"
                "      --seed <SEED>                    [default: 0]\n"
-               "      --max-depth <DEPTH>              [default: 50]\n",
+               "      --max-depth <DEPTH>              [default: 50]\n"
+               "      --denoise                        write the denoised image (spatial SVGF guided by first-hit albedo,\n"
+               "                                       normal and depth of the same samples)\n",
                argv0);
   return 2;
 }
@@ -123,6 +128,7 @@ int main(int argc, char** argv) {
     else if (a == "--gpus") cli.gpus = std::atoi(value("--gpus"));
     else if (a == "--seed") cli.seed = std::strtoull(value("--seed"), nullptr, 10);
     else if (a == "--max-depth") cli.max_depth = (unsigned)std::atoi(value("--max-depth"));
+    else if (a == "--denoise") cli.denoise = true;
     else if (a == "-h" || a == "--help") return usage(argv[0], nullptr), 0;
     else return usage(argv[0], ("unexpected argument '" + a + "'").c_str());
   }
@@ -207,7 +213,13 @@ int main(int argc, char** argv) {
     if (ptb_render_multi(ctxs.data(), cli.gpus, &o) != PTB_OK) return fail("multi-GPU render");
   }
   std::vector<float> image((size_t)cli.width * cli.height * 3);
-  if (ptb_accum_read(ctx, image.data(), image.size(), 1) != PTB_OK) return fail("accumulator read-back");
+  if (cli.denoise) {  // the feature buffers of the same samples, then the filter with its defaults
+    ptb_denoise_opts d{};
+    if (ptb_render_aov(ctx, &o) != PTB_OK) return fail("feature buffers");
+    if (ptb_denoise(ctx, &d, image.data(), image.size()) != PTB_OK) return fail("denoise");
+  } else if (ptb_accum_read(ctx, image.data(), image.size(), 1) != PTB_OK) {
+    return fail("accumulator read-back");
+  }
   const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - start).count();
   ptb_stats st{};
   ptb_stats_get(ctx, &st);
