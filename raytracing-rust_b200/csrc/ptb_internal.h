@@ -142,6 +142,8 @@ struct Ctx {
   // coverage α and the depth gradient [∂x z, ∂y z]
   DevBuf d_dn_e[2], d_dn_nz, d_dn_alpha, d_dn_grad;
   uint32_t dn_w = 0, dn_h = 0;
+  // camera candidate lists of the window wavefront (ptb_camcand.cuh), grow-only: entries [npix * k] and counts [npix]
+  DevBuf d_camcand, d_camcand_count;
   DevBuf d_pool_mem, d_prev, d_queues, d_shadow, d_counters, d_windows;
   // second chunk slot of the window wavefront: chunk k+1's wide iterations run on the main stream while chunk k's fused
   // tail (k_tail) finishes on `s_tail` in the other slot

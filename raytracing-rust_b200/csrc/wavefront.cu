@@ -17,6 +17,7 @@
 #include "ptb_internal.h"
 #include "ptb_traverse.cuh"
 #include "ptb_packet.cuh"
+#include "ptb_camcand.cuh"
 
 namespace ptb {
 
@@ -327,14 +328,18 @@ k_trace(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp,
 // K1 + K8 for the first iteration of a window-mode chunk on the binary tree: packets (ptb_packet.cuh). Work item i is slot i
 // and its ray is the camera ray of path first + i, computed here; a warp takes 32 consecutive slots — samples of one pixel
 // (or of one 8 x 4 pixel tile when the call has fewer samples) — and walks the tree once for all of them.
+// With candidate lists (cl.count set; ptb_camcand.cuh) a warp's 32 samples belong to one pixel, and the warp answers them
+// from that pixel's list unless it overflowed — same hits as the packet walk, bit for bit. Counted renders
+// (PTB_OPT_COUNT_TRAVERSAL) count a listed ray's primitive tests as prims and no nodes; k_cam_candidates counts the beam
+// walk's nodes, once per pixel.
 #ifndef PTB_CAMERA_MIN_BLOCKS
-// 4 blocks per SM = 62 registers, no spills. (Before the octant-specialised slab test the kernel needed 71 registers and
+// 4 blocks per SM = 64 registers (62 before the candidate-list path), no spills. (Before the octant-specialised slab test the kernel needed 71 registers and
 // lost at 4 blocks: 4252 vs 4344 Mrays/s on C3; with it, 3 -> 4 blocks: 4849 -> 4925 at 256 spp, 4475 -> 4570 at 32 spp.)
 #define PTB_CAMERA_MIN_BLOCKS 4
 #endif
 template <bool COUNT>
 __global__ void __launch_bounds__(256, PTB_CAMERA_MIN_BLOCKS)
-k_trace_camera(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp, unsigned long long first) {
+k_trace_camera(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderParams rp, unsigned long long first, CamCandList cl) {
   const uint32_t lane = threadIdx.x & 31u;
   const uint32_t n = wc->n_trace;
   uint32_t cnt_nodes = 0, cnt_prims = 0, cnt_rays = 0;
@@ -346,9 +351,11 @@ k_trace_camera(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderPar
     const uint32_t i = base + lane;
     const bool valid = i < n;
     Ray ray;
+    uint32_t lin = 0;
     if (valid) {
       uint32_t x, y, sample;
       camera_pixel_sample(rp, first + i, x, y, sample);
+      lin = (y - rp.row_begin) * rp.width + x;
       ray = make_ray(sc.cam_origin, camera_direction(sc, rp, x, y, sample));
       if (COUNT) ++cnt_rays;
     } else {
@@ -356,7 +363,16 @@ k_trace_camera(DevScene sc, PathPool pool, Queues q, WaveCounters* wc, RenderPar
     }
     float best_t;
     uint32_t best_ref;
-    packet_trace<COUNT>(sc, ray, valid, best_t, best_ref, cnt_nodes, cnt_prims);
+    uint32_t cnt = kNone;
+    if (cl.count) {  // lane 0 is always valid; a warp whose valid lanes span two pixels keeps the packet walk
+      const uint32_t lin0 = __shfl_sync(0xffffffffu, lin, 0);
+      if (__all_sync(0xffffffffu, !valid || lin == lin0)) {
+        lin = lin0;
+        cnt = __ldg(cl.count + lin);
+      }
+    }
+    if (cnt != kNone) cand_trace<COUNT>(sc, cl, lin, cnt, ray, valid, best_t, best_ref, cnt_prims);
+    else packet_trace<COUNT>(sc, ray, valid, best_t, best_ref, cnt_nodes, cnt_prims);
     if (valid)
       stg256(pool.ray + 4u * (size_t)i, make_float4(ray.o.x, ray.o.y, ray.o.z, best_ref == kNone ? 0.0f : best_t),
              make_float4(ray.d.x, ray.d.y, ray.d.z, __uint_as_float(best_ref == kNone ? kNone : (best_ref & ~PTB_LEAF_BIT))));
@@ -1681,6 +1697,12 @@ static cudaError_t launch_trace(const void* fn, int grid, cudaStream_t st, const
   void* args[] = {(void*)&sc, (void*)&pool, (void*)&q, (void*)&wc, (void*)&rp, (void*)&first};
   return cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(256), args, 0, st);
 }
+static cudaError_t launch_trace_camera(const void* fn, int grid, cudaStream_t st, const DevScene& sc, const PathPool& pool,
+                                       const Queues& q, WaveCounters* wc, const RenderParams& rp, unsigned long long first,
+                                       const CamCandList& cl) {
+  void* args[] = {(void*)&sc, (void*)&pool, (void*)&q, (void*)&wc, (void*)&rp, (void*)&first, (void*)&cl};
+  return cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(256), args, 0, st);
+}
 static cudaError_t launch_shadow(const void* fn, int grid, cudaStream_t st, const DevScene& sc, const PathPool& pool, const Queues& q,
                                  WaveCounters* wc) {
   void* args[] = {(void*)&sc, (void*)&pool, (void*)&q, (void*)&wc};
@@ -2125,6 +2147,21 @@ static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const Render
   if (const char* e = getenv("PTB_CAMERA_PACKET")) cam_packet = !c->wide && atoi(e) != 0;
   const void* fn_trace_cam = cam_packet ? (count ? (const void*)k_trace_camera<true> : (const void*)k_trace_camera<false>)
                                         : trace_kernel(c, count, true);
+  // Camera samples answered from per-pixel candidate lists (ptb_camcand.cuh): one beam walk per pixel and call, then each
+  // sample tests only what its pixel can see. Taken where the packets run, on scenes whose geometry is not L1 resident
+  // anyway (>= 4096 primitives, as for the chunk streams below); PTB_CAMERA_CAND=0|1 overrides, PTB_CAMERA_CAND_K=1..16
+  // shortens the lists (tests: forces the overflow fallback).
+  const bool cand_ok = cam_packet && rs.rp.group % 32u == 0u;
+  bool cam_cand = cand_ok && c->n_prims >= 4096;
+  if (const char* e = getenv("PTB_CAMERA_CAND")) cam_cand = cand_ok && atoi(e) != 0;
+  CamCandList cand{nullptr, nullptr, kCamCandMaxK};
+  if (const char* e = getenv("PTB_CAMERA_CAND_K")) { int v = atoi(e); if (v >= 1 && v <= (int)kCamCandMaxK) cand.k = (uint32_t)v; }
+  if (cam_cand) {
+    PTB_CUDA_TRY(c, c->d_camcand.reserve((size_t)npix * cand.k * sizeof(uint4)));
+    PTB_CUDA_TRY(c, c->d_camcand_count.reserve((size_t)npix * sizeof(uint32_t)));
+    cand.entries = c->d_camcand.as<uint4>();
+    cand.count = c->d_camcand_count.as<uint32_t>();
+  }
   const void* fn_shadow = shadow_kernel(c);
   const int grid_trace = persistent_grid(c, fn_trace, T);
   const int grid_trace_cam = persistent_grid(c, fn_trace_cam, T);
@@ -2202,6 +2239,14 @@ static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const Render
   k_reset_counters<<<1, 1, 0, st>>>(rs.wc);
   k_reset_counters<<<1, 1, 0, st>>>(rs.wc2);
   c->stats.kernel_launches += 2;
+  if (cam_cand) {
+    const DevScene& d = c->dev;
+    k_cam_candidates<<<(npix + 127) / 128, 128, 0, st>>>(d, rs.rp.width, rs.rp.height, rs.rp.row_begin, npix,
+                                                        cam_cand_camera(d.cam_origin, d.cam_lower_left, d.cam_horizontal, d.cam_vertical),
+                                                        cand.k, c->d_camcand.as<uint4>(), c->d_camcand_count.as<uint32_t>(),
+                                                        count ? &rs.wc->nodes_fetched : nullptr);
+    c->stats.kernel_launches += 1;
+  }
   if (chunk_streams == 2) {  // the second stream starts after whatever the caller queued before this render
     PTB_CUDA_TRY(c, cudaEventRecord(c->ev_fork, st));
     PTB_CUDA_TRY(c, cudaStreamWaitEvent(wst[1], c->ev_fork, 0));
@@ -2270,7 +2315,8 @@ static int32_t render_window_mode(Ctx* c, const ptb_render_opts& o, const Render
       // (C3, camera rays only: threshold 8 -> 8105 Mrays/s, 4 -> 8311; bounce rays prefer 8, profiles/r1_sweeps.md)
       DevScene cam = c->dev;
       cam.trace_fetch_threshold = cam_fetch;
-      PTB_CUDA_TRY(c, launch_trace(fn_trace_cam, grid_trace_cam, s, cam, S.pool, q, wc, rs.rp, R.first));
+      if (cam_packet) PTB_CUDA_TRY(c, launch_trace_camera(fn_trace_cam, grid_trace_cam, s, cam, S.pool, q, wc, rs.rp, R.first, cand));
+      else PTB_CUDA_TRY(c, launch_trace(fn_trace_cam, grid_trace_cam, s, cam, S.pool, q, wc, rs.rp, R.first));
     } else {
       PTB_CUDA_TRY(c, launch_trace(fn_trace, grid_trace, s, c->dev, S.pool, q, wc, rs.rp, 0ull));
     }
