@@ -19,12 +19,19 @@
 // distance from the apex) outside a side plane. (c) box_entry accepts a box up to its widened slabs: near planes moved by
 // 2 eps |o_i| along axis i, far side stretched by 1 + 4 gamma(3), one rounding of the fma: a few eps of the box's distance.
 // Every box is grown by 2^-16 * max(|o|, |box|) per side, which covers (c) many times over. The CPU statement of all
-// this (scripts/camcand_ref.cpp) checks the lists against the ordered walk over millions of jittered camera rays.
+// this (scripts/camcand_ref.cpp) checks the lists against the ordered walk over millions of jittered camera rays, and
+// checks (b) alone on the corner rays of every pixel's jitter square with the growth switched off. The f64 camera and
+// the margins live in ptb_camcand_frustum.h, which that statement includes. sin_a alone also covers (a): it is twice
+// (b)'s bound, and the spare half, 4 eps |S| / dmin >= 4 eps (|h| + |vv|) / dmin, exceeds the angle of at most
+// 2 eps (|h| + |vv|) / dmin by which (a) turns a direction. So the uv margin is redundant (the corner check passes
+// without it).
 //
 // List. Up to K entries per pixel, sorted by key: (key, leaf reference, parent node | side << 31). The key is the
 // distance from the apex to the grown box, times (1 - eps), less 2^-16 of its farthest distance, rounded down to f32: a
 // lower bound, for every ray of the pixel, on box_entry's cull key tmin - kCullSlack * max(|tmin|, |hmin|) of the leaf box
-// (tmin * |d| >= that distance, |d| = 1 within 2 eps, and kCullSlack = 32 eps < 2^-16). More than K candidates: the pixel
+// (tmin * |d| >= that distance, |d| = 1 within 2 eps, and kCullSlack = 32 eps < 2^-16) wherever that key is positive. A
+// box around the apex has a key below 0 and a cull key that may be lower still; neither stops anything, since every best
+// t is positive. More than K candidates: the pixel
 // is marked overflowed (count = kNone) and its samples take the packet walk.
 //
 // Why the answer is the walk's, bit for bit (the argument k_trace_camera's list path rests on):
@@ -41,6 +48,7 @@
 //    it too. So the lane computes the same minimum over the same set, with the same tie rule.
 #pragma once
 #include <cmath>
+#include "ptb_camcand_frustum.h"
 #include "ptb_intersect.cuh"
 
 namespace ptb {
@@ -52,47 +60,16 @@ constexpr uint32_t kCamCandMaxK = PTB_CAMCAND_K;
 // The frustum starts every ray at the pinhole: a camera with an aperture (a lens radius in ptb_camera) would break the lists.
 static_assert(sizeof(ptb_camera) == 4 * sizeof(ptb_vec3), "camera candidate lists assume a pinhole camera (no aperture)");
 
-struct CamCandCamera {  // f64 camera of the frustum test (cam_cand_camera)
-  double o[3], ll[3], h[3], vv[3];
-  double f[3];   // unit normal of the image plane, away from the apex
-  double sin_a;  // bound on the angle between a computed camera direction and the exact cone (see above)
-};
 struct CamCandList {  // what k_trace_camera reads; count == nullptr: the list path is off
   const uint4* entries;   // [npix * k] (key bits, leaf reference, parent node | side << 31, 0), nearest key first
   const uint32_t* count;  // [npix] entries of the pixel, kNone: overflowed
   uint32_t k;
 };
-constexpr double kCcEps = 1.0 / 8388608.0;
-constexpr double kCcUvMargin = 1.0 / 1048576.0;
-constexpr double kCcBoxGrow = 1.0 / 65536.0;
-constexpr double kCcKeySlack = 1.0 / 65536.0;
 
-PTB_HD void cc_cross(const double a[3], const double b[3], double r[3]) {
-  r[0] = a[1] * b[2] - a[2] * b[1];
-  r[1] = a[2] * b[0] - a[0] * b[2];
-  r[2] = a[0] * b[1] - a[1] * b[0];
-}
-PTB_HD double cc_dot(const double a[3], const double b[3]) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; }
-
-// host: the f64 camera of the frustum test
+// host: cam_cand_camera (ptb_camcand_frustum.h) of the device scene's camera
 inline CamCandCamera cam_cand_camera(v3 o, v3 ll, v3 h, v3 vv) {
-  CamCandCamera c;
-  const v3 src[4] = {o, ll, h, vv};
-  double* dst[4] = {c.o, c.ll, c.h, c.vv};
-  for (int i = 0; i < 4; ++i) { dst[i][0] = src[i].x; dst[i][1] = src[i].y; dst[i][2] = src[i].z; }
-  double s2 = 0.0;
-  for (int k = 0; k < 3; ++k) {
-    const double s = std::fabs(c.ll[k]) + 2.0 * std::fabs(c.h[k]) + 2.0 * std::fabs(c.vv[k]) + std::fabs(c.o[k]);
-    s2 += s * s;
-  }
-  cc_cross(c.h, c.vv, c.f);
-  const double fm = std::sqrt(cc_dot(c.f, c.f));
-  for (int k = 0; k < 3; ++k) c.f[k] /= fm;
-  const double llo[3] = {c.ll[0] - c.o[0], c.ll[1] - c.o[1], c.ll[2] - c.o[2]};
-  double dmin = cc_dot(llo, c.f);
-  if (dmin < 0.0) { for (int k = 0; k < 3; ++k) c.f[k] = -c.f[k]; dmin = -dmin; }
-  c.sin_a = 8.0 * kCcEps * std::sqrt(s2) / dmin + 2.0 * kCcEps;
-  return c;
+  const float fo[3] = {o.x, o.y, o.z}, fll[3] = {ll.x, ll.y, ll.z}, fh[3] = {h.x, h.y, h.z}, fvv[3] = {vv.x, vv.y, vv.z};
+  return cam_cand_camera(fo, fll, fh, fvv);
 }
 
 #ifdef __CUDACC__

@@ -10,6 +10,7 @@
 
 #include "../oracle/sah_ref.hpp"
 #include "../oracle/ref_integrators.hpp"
+#include "../raytracing-rust_b200/csrc/ptb_camcand_frustum.h"
 
 namespace ref {
 thread_local RngCursor g_rng;
@@ -18,52 +19,33 @@ using namespace ref;
 
 namespace {
 
-// ---- the frustum of one pixel (restates ptb_camcand.cuh: cc_camera / cc_pixel / cc_box) ------------------------------
-struct CcCamera {
-  double o[3], ll[3], h[3], vv[3];
-  double f[3];   // unit normal of the image plane, pointing away from the apex
-  double sin_a;  // bound on the angle between a computed camera direction and the exact cone
-};
+// ---- the frustum of one pixel (restates ptb_camcand.cuh: cam_candidates_pixel / cc_box; the f64 camera and the margins
+// are the device's own, ptb_camcand_frustum.h) ------------------------------------------------------------------------
+using ptb::CamCandCamera;
+using ptb::kCcEps;
+using ptb::kCcUvMargin;
+using ptb::kCcBoxGrow;
+using ptb::kCcKeySlack;
 struct CcPixel {
   double n[4][3];  // outward unit normals of the four side planes (through the apex)
 };
-const double kEps = 1.0 / 8388608.0;    // 2^-23
-const double kUvMargin = 1.0 / 1048576.0;  // 2^-20
-const double kBoxGrow = 1.0 / 65536.0;     // 2^-16
-const double kKeySlack = 1.0 / 65536.0;    // 2^-16
 
-void cross3(const double a[3], const double b[3], double r[3]) {
-  r[0] = a[1] * b[2] - a[2] * b[1];
-  r[1] = a[2] * b[0] - a[0] * b[2];
-  r[2] = a[0] * b[1] - a[1] * b[0];
-}
-double dot3(const double a[3], const double b[3]) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; }
+void cross3(const double a[3], const double b[3], double r[3]) { ptb::cc_cross(a, b, r); }
+double dot3(const double a[3], const double b[3]) { return ptb::cc_dot(a, b); }
 void unit3(double a[3]) {
   const double m = std::sqrt(dot3(a, a));
   for (int k = 0; k < 3; ++k) a[k] /= m;
 }
 
-CcCamera cc_camera(const Camera& cam) {
-  CcCamera c;
+CamCandCamera cc_camera(const Camera& cam) {
   const Vec3* src[4] = {&cam.origin, &cam.lower_left, &cam.horizontal, &cam.vertical};
-  double* dst[4] = {c.o, c.ll, c.h, c.vv};
-  for (int i = 0; i < 4; ++i) { dst[i][0] = src[i]->x; dst[i][1] = src[i]->y; dst[i][2] = src[i]->z; }
-  double s2 = 0.0;
-  for (int k = 0; k < 3; ++k) {
-    const double s = std::fabs(c.ll[k]) + 2.0 * std::fabs(c.h[k]) + 2.0 * std::fabs(c.vv[k]) + std::fabs(c.o[k]);
-    s2 += s * s;
-  }
-  cross3(c.h, c.vv, c.f);
-  unit3(c.f);
-  double llo[3] = {c.ll[0] - c.o[0], c.ll[1] - c.o[1], c.ll[2] - c.o[2]};
-  double dmin = dot3(llo, c.f);
-  if (dmin < 0.0) { for (int k = 0; k < 3; ++k) c.f[k] = -c.f[k]; dmin = -dmin; }
-  c.sin_a = 8.0 * kEps * std::sqrt(s2) / dmin + 2.0 * kEps;
-  return c;
+  float v[4][3];
+  for (int i = 0; i < 4; ++i) { v[i][0] = src[i]->x; v[i][1] = src[i]->y; v[i][2] = src[i]->z; }
+  return ptb::cam_cand_camera(v[0], v[1], v[2], v[3]);
 }
-CcPixel cc_pixel(const CcCamera& c, uint32_t x, uint32_t y, uint32_t W, uint32_t H) {
-  const double u0 = (double)x / (double)(W - 1) - kUvMargin, u1 = (double)(x + 1) / (double)(W - 1) + kUvMargin;
-  const double v0 = 1.0 - (double)(y + 1) / (double)(H - 1) - kUvMargin, v1 = 1.0 - (double)y / (double)(H - 1) + kUvMargin;
+CcPixel cc_pixel(const CamCandCamera& c, uint32_t x, uint32_t y, uint32_t W, uint32_t H) {
+  const double u0 = (double)x / (double)(W - 1) - kCcUvMargin, u1 = (double)(x + 1) / (double)(W - 1) + kCcUvMargin;
+  const double v0 = 1.0 - (double)(y + 1) / (double)(H - 1) - kCcUvMargin, v1 = 1.0 - (double)y / (double)(H - 1) + kCcUvMargin;
   const double us[4] = {u0, u1, u1, u0}, vs[4] = {v0, v0, v1, v1};
   double d[4][3], dc[3] = {0, 0, 0};
   for (int i = 0; i < 4; ++i)
@@ -80,15 +62,17 @@ CcPixel cc_pixel(const CcCamera& c, uint32_t x, uint32_t y, uint32_t W, uint32_t
   return p;
 }
 // may a camera ray of the pixel reach the box? On acceptance `key` is a lower bound on the box_entry cull key of every
-// such ray (float, rounded down)
-bool cc_box(const CcCamera& c, const CcPixel& p, const float* bmn, const float* bmx, float& key) {
+// such ray (float, rounded down). grow = false: the box as given, without the 2^-16 growth (the directed frustum check).
+// rejected (may be null): 1 = outside a side plane, 2 = behind the apex.
+bool cc_box(const CamCandCamera& c, const CcPixel& p, const double* bmn, const double* bmx, float& key, bool grow = true,
+            int* rejected = nullptr) {
   double mx_abs = 0.0;
-  for (int k = 0; k < 3; ++k) mx_abs = std::fmax(mx_abs, std::fmax(std::fabs(c.o[k]), std::fmax(std::fabs((double)bmn[k]), std::fabs((double)bmx[k]))));
-  const double g = kBoxGrow * mx_abs;
+  for (int k = 0; k < 3; ++k) mx_abs = std::fmax(mx_abs, std::fmax(std::fabs(c.o[k]), std::fmax(std::fabs(bmn[k]), std::fabs(bmx[k]))));
+  const double g = grow ? kCcBoxGrow * mx_abs : 0.0;
   double lo[3], hi[3], far2 = 0.0, near2 = 0.0;
   for (int k = 0; k < 3; ++k) {
-    lo[k] = (double)bmn[k] - g - c.o[k];
-    hi[k] = (double)bmx[k] + g - c.o[k];
+    lo[k] = bmn[k] - g - c.o[k];
+    hi[k] = bmx[k] + g - c.o[k];
     far2 += std::fmax(lo[k] * lo[k], hi[k] * hi[k]);
     const double nd = std::fmax(std::fmax(lo[k], 0.0), -hi[k]);
     near2 += nd * nd;
@@ -97,15 +81,25 @@ bool cc_box(const CcCamera& c, const CcPixel& p, const float* bmn, const float* 
   for (int i = 0; i < 4; ++i) {
     const double* n = p.n[i];
     const double pmin = n[0] * (n[0] > 0.0 ? lo[0] : hi[0]) + n[1] * (n[1] > 0.0 ? lo[1] : hi[1]) + n[2] * (n[2] > 0.0 ? lo[2] : hi[2]);
-    if (pmin > c.sin_a * rmax) return false;
+    if (pmin > c.sin_a * rmax) {
+      if (rejected) *rejected = 1;
+      return false;
+    }
   }
   const double fmax_ = c.f[0] * (c.f[0] > 0.0 ? hi[0] : lo[0]) + c.f[1] * (c.f[1] > 0.0 ? hi[1] : lo[1]) + c.f[2] * (c.f[2] > 0.0 ? hi[2] : lo[2]);
-  if (fmax_ < 0.0) return false;
-  const double kd = std::sqrt(near2) * (1.0 - kEps) - kKeySlack * rmax;
+  if (fmax_ < 0.0) {
+    if (rejected) *rejected = 2;
+    return false;
+  }
+  const double kd = std::sqrt(near2) * (1.0 - kCcEps) - kCcKeySlack * rmax;
   float kf = (float)kd;
   if ((double)kf > kd) kf = std::nextafter(kf, -INF_F);
   key = kf;
   return true;
+}
+bool cc_box(const CamCandCamera& c, const CcPixel& p, const float* bmn, const float* bmx, float& key) {
+  const double dmn[3] = {bmn[0], bmn[1], bmn[2]}, dmx[3] = {bmx[0], bmx[1], bmx[2]};
+  return cc_box(c, p, dmn, dmx, key);
 }
 
 struct Entry {
@@ -176,7 +170,7 @@ void ccr_destroy(ccr_scene* s) { delete s; }
 // min(count, K) of them, sorted; count > K: overflowed); visits[i] = nodes expanded by the beam walk.
 void ccr_lists(const ccr_scene* s, uint32_t W, uint32_t H, uint32_t row_begin, uint32_t rows, uint32_t K, uint32_t* count,
                float* keys, uint32_t* refs, uint32_t* nodes, uint32_t* visits, int threads) {
-  const CcCamera c = cc_camera(s->cam);
+  const CamCandCamera c = cc_camera(s->cam);
   const std::vector<ptb_bvh_node>& nd = s->l.nodes;
   parallel_for((size_t)W * rows, threads, [&](size_t b, size_t e) {
     std::vector<Entry> list;
@@ -221,7 +215,8 @@ void ccr_lists(const ccr_scene* s, uint32_t W, uint32_t H, uint32_t row_begin, u
 // tested (box + primitive), [4] primitive tests of the list path, [5] walk nodes, [6] walk primitive tests over the list
 // rays, [7] list entries whose primitive is hit (t > 0) although the walk's box test rejects its leaf box, [8] list
 // entries (all of the list, not only those a ray reached) whose key exceeds the cull key box_entry computes for the ray on
-// their leaf box while its geometric test passes (the key must be a lower bound). hist (3 x kHistBins, may be null): per
+// their leaf box while its geometric test passes, and is positive (the key must bound the cull key from below wherever
+// that decides anything: a best t is positive, so a key at or below 0, a box around the apex, never stops a list). hist (3 x kHistBins, may be null): per
 // list ray, the entries tested, the primitive tests of the list path and the ordered walk's nodes (last bin: that many or
 // more).
 static const int kHistBins = 256;
@@ -263,7 +258,7 @@ void ccr_check(const ccr_scene* s, uint32_t W, uint32_t H, uint32_t row_begin, u
           const ptb_bvh_node& q = l.nodes[nodes[j] & 0x7FFFFFFFu];
           const bool side = (nodes[j] >> 31) != 0;
           Float tk;
-          if (Lbvh::box_hit(side ? q.rmin : q.lmin, side ? q.rmax : q.lmax, slab, INF_F, tk) && keys[j] > tk) ++loc[8];
+          if (Lbvh::box_hit(side ? q.rmin : q.lmin, side ? q.rmax : q.lmax, slab, INF_F, tk) && keys[j] > tk && keys[j] > 0.0f) ++loc[8];
         }
         const uint64_t e0 = loc[3], p0 = loc[4];
         Float best_t = INF_F;
@@ -300,6 +295,59 @@ void ccr_check(const ccr_scene* s, uint32_t W, uint32_t H, uint32_t row_begin, u
   });
   for (int k = 0; k < 9; ++k) out[k] = acc[k];
   if (hist) for (size_t k = 0; k < hacc.size(); ++k) hist[k] = hacc[k];
+}
+
+// Directed check of the frustum predicate alone (argument (b) of ptb_camcand.cuh: sin_a and the uv margin cover the
+// rounding of the computed camera directions; the box growth is switched off). For every pixel of rows [row_begin,
+// row_begin + rows): the four corner rays of its jitter square (jitter 0 and 1 - 2^-24 on each axis, the extremes of
+// u32_to_unit), built with the device's camera arithmetic (camera_direction + make_ray), and on each of them the
+// zero-extent boxes at dist[j] times the ray's distance from the apex to the image plane, placed in f64 on the computed
+// ray. Every such box must pass the pixel's side planes and lie ahead of the apex. out[0] boxes tested, [1] rejected by a
+// side plane, [2] rejected as behind the apex. worst[0]: the largest (signed distance outside a side plane) / (sin_a *
+// distance from the apex) over the boxes, which stays below 1 while the check passes.
+void ccr_frustum_corners(const ccr_scene* s, uint32_t W, uint32_t H, uint32_t row_begin, uint32_t rows, const double* dist,
+                         uint32_t ndist, int threads, uint64_t out[3], double* worst) {
+  const CamCandCamera c = cc_camera(s->cam);
+  std::atomic<uint64_t> acc[3];
+  for (auto& a : acc) a = 0;
+  std::vector<double> worst_part((size_t)W * rows, -INFINITY);
+  const Float j1 = u32_to_unit(0xFFFFFFFFu);  // 1 - 2^-24
+  parallel_for((size_t)W * rows, threads, [&](size_t b, size_t e) {
+    uint64_t loc[3] = {0, 0, 0};
+    for (size_t i = b; i < e; ++i) {
+      const uint32_t x = (uint32_t)(i % W), y = row_begin + (uint32_t)(i / W);
+      const CcPixel p = cc_pixel(c, x, y, W, H);
+      double wmax = -INFINITY;
+      for (int corner = 0; corner < 4; ++corner) {
+        const Float ju = (corner & 1) ? j1 : 0.0f, jv = (corner & 2) ? j1 : 0.0f;
+        const Float u = (ju + (Float)x) / (Float)(W - 1u);
+        const Float v = 1.0f - (jv + (Float)y) / (Float)(H - 1u);
+        const Ray ray = s->cam.get_ray(u, v);
+        const double d[3] = {ray.direction.x, ray.direction.y, ray.direction.z};
+        const double llo[3] = {c.ll[0] - c.o[0], c.ll[1] - c.o[1], c.ll[2] - c.o[2]};
+        const double to_plane = dot3(llo, c.f) / dot3(d, c.f);  // along the ray, to the image plane
+        for (uint32_t j = 0; j < ndist; ++j) {
+          double pt[3], rel[3];
+          for (int k = 0; k < 3; ++k) {
+            pt[k] = c.o[k] + dist[j] * to_plane * d[k];
+            rel[k] = pt[k] - c.o[k];
+          }
+          float key;
+          int why = 0;
+          ++loc[0];
+          if (!cc_box(c, p, pt, pt, key, false, &why)) ++loc[why];
+          const double r = std::sqrt(dot3(rel, rel));
+          for (int q = 0; q < 4; ++q) wmax = std::fmax(wmax, dot3(p.n[q], rel) / (c.sin_a * r));
+        }
+      }
+      worst_part[i] = wmax;
+    }
+    for (int k = 0; k < 3; ++k) acc[k] += loc[k];
+  });
+  for (int k = 0; k < 3; ++k) out[k] = acc[k];
+  double w = -INFINITY;
+  for (double v : worst_part) w = std::fmax(w, v);
+  *worst = w;
 }
 
 }  // extern "C"

@@ -21,7 +21,8 @@ def _load():
     if _lib is not None:
         return _lib
     deps = [_SRC] + [os.path.join(_HERE, "..", "oracle", f) for f in sorted(os.listdir(os.path.join(_HERE, "..", "oracle")))
-                     if f.endswith(".hpp")] + [os.path.join(_HERE, "..", "include", "ptb200.h")]
+                     if f.endswith(".hpp")] + [os.path.join(_HERE, "..", "include", "ptb200.h"),
+                                os.path.join(_HERE, "..", "raytracing-rust_b200", "csrc", "ptb_camcand_frustum.h")]
     h = hashlib.sha1()
     for f in deps:
         with open(f, "rb") as fh:
@@ -42,6 +43,7 @@ def _load():
     u32 = C.c_uint32
     lib.ccr_lists.argtypes = [P, u32, u32, u32, u32, u32, P, P, P, P, P, C.c_int]
     lib.ccr_check.argtypes = [P, u32, u32, u32, u32, u32, P, P, P, P, u32, u32, C.c_uint64, C.c_int, P, P]
+    lib.ccr_frustum_corners.argtypes = [P, u32, u32, u32, u32, P, u32, C.c_int, P, P]
     _lib = lib
     return lib
 
@@ -98,3 +100,13 @@ class CamCandScene:
         r = {k: int(v) for k, v in zip(names, out)}
         r["hist"] = dict(zip(("list_entries", "list_prim_tests", "walk_nodes"), hist))
         return r
+
+    def frustum_corners(self, W, H, dist, row_begin=0, rows=None, threads=0) -> dict:
+        """The directed check of the frustum predicate (ccr_frustum_corners): the corner rays of every pixel's jitter
+        square, zero-extent boxes on them at `dist` times their distance to the image plane, the box growth off."""
+        rows = H - row_begin if rows is None else rows
+        d = np.ascontiguousarray(dist, np.float64)
+        out = np.zeros(3, np.uint64)
+        worst = np.zeros(1, np.float64)
+        _lib.ccr_frustum_corners(self._h, W, H, row_begin, rows, _p(d), len(d), threads, _p(out), _p(worst))
+        return {"boxes": int(out[0]), "side_rejected": int(out[1]), "behind_rejected": int(out[2]), "worst": float(worst[0])}
