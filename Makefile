@@ -25,7 +25,8 @@ cli: $(PKG)/ptb200-cli
 $(PKG)/ptb200-cli: $(PKG)/host/cli_main.cpp $(PKG)/libptb200.so include/ptb200.h
 	$(CXX) -O2 -std=c++17 -Wall -Wextra -o $@ $(PKG)/host/cli_main.cpp -L$(PKG) -lptb200 -Wl,-rpath,'$$ORIGIN' -ldl -lpthread
 
-oracle: oracle/libvisibility_oracle.so oracle/librefit_oracle.so oracle/libaov_oracle.so oracle/libdenoise_oracle.so
+oracle: oracle/libvisibility_oracle.so oracle/librefit_oracle.so oracle/libaov_oracle.so oracle/libdenoise_oracle.so \
+        oracle/libmotion_oracle.so oracle/libtemporal_oracle.so
 	$(MAKE) -C oracle
 # test infrastructure beside liboracle.so: the reference's visibility queries for a batch (oracle/visibility_api.cpp)
 oracle/libvisibility_oracle.so: oracle/visibility_api.cpp $(wildcard oracle/*.hpp) include/ptb200.h
@@ -39,8 +40,15 @@ oracle/libaov_oracle.so: oracle/aov_api.cpp $(wildcard oracle/*.hpp) include/ptb
 # ... and the denoiser over the beauty and AOV sums (oracle/denoise_api.cpp, ptb_denoise)
 oracle/libdenoise_oracle.so: oracle/denoise_api.cpp include/ptb200.h
 	$(CXX) -O2 -std=c++17 -fno-fast-math -ffp-contract=off -fPIC -Wall -Wextra -pthread -shared -o $@ $<
+# ... and the motion vectors of ptb_render_aov after a mark (oracle/motion_api.cpp, over the AOV oracle's scene)
+oracle/libmotion_oracle.so: oracle/motion_api.cpp oracle/aov_api.cpp $(wildcard oracle/*.hpp) include/ptb200.h
+	$(CXX) -O2 -std=c++17 -fno-fast-math -ffp-contract=off -fPIC -Wall -Wextra -pthread -shared -o $@ $<
+# ... and one step of the temporal denoiser (oracle/temporal_api.cpp, over the spatial oracle's helpers)
+oracle/libtemporal_oracle.so: oracle/temporal_api.cpp oracle/denoise_api.cpp include/ptb200.h
+	$(CXX) -O2 -std=c++17 -fno-fast-math -ffp-contract=off -fPIC -Wall -Wextra -pthread -shared -o $@ $<
 
 clean:
-	rm -f $(OBJS) $(PKG)/csrc/*.ptxas.log $(PKG)/libptb200.so $(PKG)/ptb200-cli oracle/libvisibility_oracle.so oracle/librefit_oracle.so oracle/libaov_oracle.so oracle/libdenoise_oracle.so
+	rm -f $(OBJS) $(PKG)/csrc/*.ptxas.log $(PKG)/libptb200.so $(PKG)/ptb200-cli oracle/libvisibility_oracle.so oracle/librefit_oracle.so oracle/libaov_oracle.so oracle/libdenoise_oracle.so \
+	      oracle/libmotion_oracle.so oracle/libtemporal_oracle.so
 	$(MAKE) -C oracle clean
 .PHONY: all oracle clean cli

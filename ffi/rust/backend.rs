@@ -139,6 +139,29 @@ impl CudaScene {
         }
         Ok(image)
     }
+
+    /// Keeps the committed scene's primitives and camera as the previous frame of the motion vectors (ptb_motion_mark).
+    pub fn motion_mark(&self) -> Result<(), String> {
+        unsafe { check(self.ctx, ptb_motion_mark(self.ctx)) }
+    }
+
+    /// One frame of an animation denoised with the history of the earlier ones: the samples, the feature buffers and
+    /// motion vectors of the same camera rays, SVGF's temporal accumulation and spatial filter (`denoise`:
+    /// ptb_temporal_opts, all zeros for the defaults), then this frame becomes the previous one. Give every frame its own
+    /// seed: the same samples every frame average nothing. Same layout as `render`'s image.
+    pub fn denoise_temporal(&self, opts: RenderOptions, seed: u64, denoise: ptb_temporal_opts) -> Result<Vec<Float>, String> {
+        let o = self.opts(opts, seed);
+        let mut image = vec![0.0 as Float; (opts.width * opts.height * 3) as usize];
+        unsafe {
+            check(self.ctx, ptb_accum_clear(self.ctx))?;
+            check(self.ctx, ptb_render(self.ctx, &o, None, ptr::null_mut()))?;
+            check(self.ctx, ptb_aov_clear(self.ctx))?;
+            check(self.ctx, ptb_render_aov(self.ctx, &o))?;
+            check(self.ctx, ptb_denoise_temporal(self.ctx, &denoise, image.as_mut_ptr(), image.len()))?;
+            check(self.ctx, ptb_motion_mark(self.ctx))?;
+        }
+        Ok(image)
+    }
 }
 
 impl CudaScene {

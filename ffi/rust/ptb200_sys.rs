@@ -40,6 +40,9 @@ pub struct ptb_render_opts {
 /// denoiser options (ptb_denoise); 0 selects a default: 5 levels, sigma_luminance 4, sigma_normal 128, sigma_depth 1
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct ptb_denoise_opts { pub iterations: u32, pub sigma_luminance: f32, pub sigma_normal: f32, pub sigma_depth: f32, pub flags: u32 }
+/// temporal denoiser options (ptb_denoise_temporal); 0 selects a default: alpha_color 0.2, alpha_moments 0.2, max_history 32
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct ptb_temporal_opts { pub spatial: ptb_denoise_opts, pub alpha_color: f32, pub alpha_moments: f32, pub max_history: u32, pub flags: u32 }
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct ptb_stats {
     pub rays_camera: u64, pub rays_bounce: u64, pub rays_shadow_light: u64, pub rays_shadow_sky: u64,
@@ -114,6 +117,11 @@ extern "C" {
     pub fn ptb_aov_read(ctx: *mut ptb_ctx, aov: u32, out: *mut f32, n_floats: usize, normalise: i32) -> i32;
     pub fn ptb_denoise(ctx: *mut ptb_ctx, opts: *const ptb_denoise_opts, rgb: *mut f32, n_floats: usize) -> i32;
     pub fn ptb_denoise_device(ctx: *mut ptb_ctx, opts: *const ptb_denoise_opts, d_rgb: *mut c_void) -> i32;
+    pub fn ptb_motion_mark(ctx: *mut ptb_ctx) -> i32;
+    pub fn ptb_motion_read(ctx: *mut ptb_ctx, out: *mut f32, n_floats: usize) -> i32;
+    pub fn ptb_denoise_temporal(ctx: *mut ptb_ctx, opts: *const ptb_temporal_opts, rgb: *mut f32, n_floats: usize) -> i32;
+    pub fn ptb_denoise_temporal_device(ctx: *mut ptb_ctx, opts: *const ptb_temporal_opts, d_rgb: *mut c_void) -> i32;
+    pub fn ptb_denoise_temporal_reset(ctx: *mut ptb_ctx) -> i32;
     pub fn ptb_sample_only(ctx: *mut ptb_ctx, query: *const ptb_sampler_query, n: usize, dirs: *mut f32, pdf: *mut f32) -> i32;
     pub fn ptb_sampler_pdf(ctx: *mut ptb_ctx, query: *const ptb_sampler_query, dirs: *const f32, n: usize, pdf: *mut f32) -> i32;
     pub fn ptb_stats_get(ctx: *mut ptb_ctx, out: *mut ptb_stats) -> i32;

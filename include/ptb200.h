@@ -460,6 +460,33 @@ int32_t ptb_aov_clear(ptb_ctx* ctx);
  * stream. A read before any ptb_render_aov, an unknown aov or a wrong n_floats fails with PTB_ERR_INVALID. */
 int32_t ptb_aov_read(ptb_ctx* ctx, uint32_t aov, float* out, size_t n_floats, int32_t normalise);
 
+/* ------------------------------------------------------- motion vectors -- */
+/* Per-sample screen motion of the first hit between a marked previous frame and the committed scene, the input temporal
+ * denoisers (ptb_denoise_temporal, the OptiX denoiser's flow image) need. A typical animated frame is
+ *   update -> commit(REFIT) -> accum_clear / aov_clear -> render -> render_aov -> denoise_temporal -> motion_mark.
+ * ptb_motion_mark keeps the committed scene's primitives (d_raw_spheres, d_raw_tris in original order: in mesh and
+ * instance mode the expansion, so every scene kind works alike) and its camera as "the previous frame", by device-to-device
+ * copies on the context's stream. The copy costs 20 B per sphere and 76 B per triangle (76 MB for 1 M triangles), held
+ * until ptb_destroy; a later mark replaces it. Before a commit it fails with PTB_ERR_INVALID.
+ * While a mark exists whose sphere and triangle counts equal the committed scene's (primitive ids are stable then, across
+ * refits and full rebuilds alike), ptb_render_aov also adds, per sample whose camera ray hits primitive p at P:
+ *   P'   P if the mark's record of p is bit-identical to the committed one (sphere: centre and radius; triangle: the three
+ *        positions); else triangle: b0*p0' + b1*p1' + b2*p2' with the hit's own barycentrics (the expression of the hit
+ *        point); sphere: c' + (P - c) * (r'/r)
+ *   proj(cam, X) = (u, v, λ) with X - o = λ (ll - o + u*h + v*vv), the inverse of the camera ray, computed as
+ *        d = X - o, a = ll - o, n = cross(h, vv), s = dot(d, n); λ = s / dot(a, n), u = dot(d, cross(vv, a)) / s,
+ *        v = dot(d, cross(a, h)) / s   (dot(a, b) = a.x*b.x + a.y*b.y + a.z*b.z, cross component-wise a.y*b.z - a.z*b.y ..)
+ *   (u, v, λ) = proj(committed camera, P), (u', v', λ') = proj(marked camera, P')
+ *   Δx = (u' - u) * (W - 1), Δy = -(v' - v) * (H - 1) (image rows, top row first), t' = |P' - o'|
+ * when λ' > 0 (P' in front of the marked camera). Both points are projected, not the sample's jitter: a static frame gives
+ * exactly 0. Per pixel the sums [Σ Δx, Σ Δy, Σ t', valid samples] (one float4, 16 B per pixel beside the AOV sums) are
+ * formed in sample order without atomics, like the AOV sums; ptb_aov_clear and the reallocation on a size change zero
+ * them. Without a mark, or with one of other counts, nothing is added and no error is raised. */
+int32_t ptb_motion_mark(ptb_ctx* ctx);
+/* W*H*3 floats, row-major, top row first: the mean Δx, Δy, t' over each pixel's valid samples, 0 where there are none.
+ * Synchronises. Before any ptb_render_aov, or with n_floats != W*H*3 or a null buffer: PTB_ERR_INVALID. */
+int32_t ptb_motion_read(ptb_ctx* ctx, float* out, size_t n_floats);
+
 /* ------------------------------------------------------------- denoiser -- */
 /* The spatial part of SVGF (Schied et al., "Spatiotemporal Variance-Guided Filtering", HPG 2017, §4.3-4.5): Dammertz et
  * al. 2010's edge-avoiding à-trous wavelet filter with albedo demodulation and variance-guided luminance weights, over the
@@ -508,6 +535,46 @@ typedef struct ptb_denoise_opts {
 int32_t ptb_denoise(ptb_ctx* ctx, const ptb_denoise_opts* opts, float* rgb, size_t n_floats);
 /* Enqueues the same work on the context's stream into a device buffer of W*H*3 floats and returns without waiting. */
 int32_t ptb_denoise_device(ptb_ctx* ctx, const ptb_denoise_opts* opts, void* d_rgb);
+
+/* ---------------------------------------------------- temporal denoiser -- */
+/* SVGF's temporal part (Schied et al. 2017, §4.1-4.2) in front of ptb_denoise's spatial stages, for animated scenes
+ * rendered at a few samples per frame. Reads the beauty, AOV and motion sums (ptb_motion_mark, ptb_render_aov) and the
+ * context's history; changes none of the sums. All work is in irradiance e, prepared as ptb_denoise does, with the same
+ * arithmetic rules. Per pixel p = (x, y):
+ * 1. Reproject. With a history and a valid motion sample count > 0: Δ̄ = mean Δx, Δy, t̄' = mean t'; q = (x + Δ̄x, y + Δ̄y),
+ *    x0 = floor(q.x), y0 = floor(q.y), f = q - (x0, y0); taps (x0, y0), (x0+1, y0), (x0, y0+1), (x0+1, y0+1) with weights
+ *    (1-fx)(1-fy), fx(1-fy), (1-fx)fy, fx fy. A tap is accepted when it is inside the image with weight > 0, its history
+ *    coverage α > 0, its history normal is non-zero with n_p·n_q >= 0.9 (n_p·n_q as the spatial filter forms it), and
+ *    |t̄' - z_q| <= 4 * (|∂x z_q| + |∂y z_q|) + 0.02 * z_q (z, ∂z: the history's depth and gradient). With W = Σ accepted
+ *    weights > 0.01 the history colour, moments and length are the accepted Σ w * value / W; otherwise (and for pixels
+ *    without valid motion, and everywhere without a history) the history is 0 and its length 0.
+ * 2. Integrate. len = min(len_h + 1, max_history); a_c = max(alpha_color, 1/len), a_m = max(alpha_moments, 1/len);
+ *    e_int = (1 - a_c) * e_h + a_c * e per channel; with ℓ = ℓ(e): m1 = (1 - a_m) * m1_h + a_m * ℓ,
+ *    m2 = (1 - a_m) * m2_h + a_m * (ℓ * ℓ). With no history len = 1 and e_int == e exactly.
+ * 3. Variance. len >= 4: max(0, m2 - m1 * m1); otherwise ptb_denoise's 7x7 spatial estimate over e_int.
+ * 4. Filter. ptb_denoise's à-trous levels over [e_int | var]; level 0's output (irradiance) becomes the next history's
+ *    colour, also when it is the last level.
+ * 5. History: level 0's irradiance, [m1, m2, len], and this frame's guides ([n | z], α, depth gradient; swapped in by
+ *    pointer). It belongs to the context (92 bytes per pixel beside the denoiser scratch); a size change or
+ *    ptb_denoise_temporal_reset drops it.
+ * A call without history (the first, after a reset or a size change, or a frame where every tap is rejected) gives exactly
+ * ptb_denoise's image for the same spatial options. No atomics: the same sums and history give the same bits. Launches
+ * (prepare, integrate, variance, one per level, plus one when there is a single level) count in ptb_stats.kernel_launches.
+ * Errors (PTB_ERR_INVALID, nothing enqueued): ptb_denoise's, plus a null opts, alpha_* outside (0, 1] and not 0,
+ * max_history > 255, flags != 0. */
+typedef struct ptb_temporal_opts {
+  ptb_denoise_opts spatial; /* as ptb_denoise, same defaults and checks */
+  float alpha_color;        /* 0 -> 0.2 */
+  float alpha_moments;      /* 0 -> 0.2 */
+  uint32_t max_history;     /* 0 -> 32; at most 255 */
+  uint32_t flags;           /* reserved, 0 */
+} ptb_temporal_opts;
+/* Denoises into host memory (W*H*3 floats); synchronises the stream. */
+int32_t ptb_denoise_temporal(ptb_ctx* ctx, const ptb_temporal_opts* opts, float* rgb, size_t n_floats);
+/* Enqueues the same work into a device buffer of W*H*3 floats and returns without waiting. */
+int32_t ptb_denoise_temporal_device(ptb_ctx* ctx, const ptb_temporal_opts* opts, void* d_rgb);
+/* Drops the history: the next call filters as ptb_denoise does. */
+int32_t ptb_denoise_temporal_reset(ptb_ctx* ctx);
 
 /* ------------------------------------------------------------ multi-GPU -- */
 /* The path shards by samples (independent), scene and BVH replicated per GPU: rank r of `world` renders the absolute

@@ -8,7 +8,7 @@ from ._lib import (METHOD_MIS, METHOD_NAIVE, MAT_EMIT, MAT_LAMBERTIAN, MAT_REFLE
                    PTB_AOV_ALBEDO, PTB_AOV_COVERAGE, PTB_AOV_DEPTH, PTB_AOV_NORMAL, PTB_MISS, TEX_CHECKERED, TEX_IMAGE, TEX_LERP, TEX_PERLIN, TEX_SOLID, PtbError, Stats, hit_dtype,
                    instance_xform_dtype, mesh_instance_dtype, mesh_triangle_dtype, occlusion_ray_dtype, ray_dtype)
 from .backend import (Bvh, Context, RandomSampler, RenderOptions, Scene, denoise_opts, make_occlusion_rays, make_rays,
-                      render_multi)
+                      render_multi, temporal_opts)
 from .multi import accumulator_tensor, reduce_accumulators, shard_samples
 from .scene import HostScene, IndexedMesh, index_triangles, instance_xform, load_file, load_image, load_str, save_image
 from . import meshgen
@@ -19,5 +19,5 @@ __all__ = [
     "save_image", "load_image", "meshgen", "shard_samples", "accumulator_tensor", "reduce_accumulators", "PtbError", "Stats",
     "METHOD_MIS", "METHOD_NAIVE", "PTB_MISS", "hit_dtype", "ray_dtype", "occlusion_ray_dtype", "mesh_triangle_dtype",
     "mesh_instance_dtype", "instance_xform_dtype", "PTB_AOV_ALBEDO", "PTB_AOV_NORMAL", "PTB_AOV_DEPTH", "PTB_AOV_COVERAGE",
-    "denoise_opts",
+    "denoise_opts", "temporal_opts",
 ]

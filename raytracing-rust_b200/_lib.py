@@ -60,6 +60,11 @@ class DenoiseOpts(C.Structure):
                 ("sigma_depth", C.c_float), ("flags", C.c_uint32)]
 
 
+class TemporalOpts(C.Structure):
+    _fields_ = [("spatial", DenoiseOpts), ("alpha_color", C.c_float), ("alpha_moments", C.c_float),
+                ("max_history", C.c_uint32), ("flags", C.c_uint32)]
+
+
 class Stats(C.Structure):
     _fields_ = [("rays_camera", C.c_uint64), ("rays_bounce", C.c_uint64), ("rays_shadow_light", C.c_uint64),
                 ("rays_shadow_sky", C.c_uint64), ("rays_reference", C.c_uint64), ("paths", C.c_uint64),
@@ -149,6 +154,11 @@ SYMBOLS = [
     ("ptb_aov_read", C.c_int32, [_P, C.c_uint32, _P, C.c_size_t, C.c_int32]),
     ("ptb_denoise", C.c_int32, [_P, C.POINTER(DenoiseOpts), _P, C.c_size_t]),
     ("ptb_denoise_device", C.c_int32, [_P, C.POINTER(DenoiseOpts), _P]),
+    ("ptb_motion_mark", C.c_int32, [_P]),
+    ("ptb_motion_read", C.c_int32, [_P, _P, C.c_size_t]),
+    ("ptb_denoise_temporal", C.c_int32, [_P, C.POINTER(TemporalOpts), _P, C.c_size_t]),
+    ("ptb_denoise_temporal_device", C.c_int32, [_P, C.POINTER(TemporalOpts), _P]),
+    ("ptb_denoise_temporal_reset", C.c_int32, [_P]),
     ("ptb_shard_samples", None, [C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     ("ptb_shard_rows", None, [C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     ("ptb_render_multi", C.c_int32, [_P, C.c_int32, C.POINTER(RenderOpts)]),

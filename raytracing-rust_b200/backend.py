@@ -51,6 +51,13 @@ def denoise_opts(iterations: int = 0, sigma_luminance: float = 0.0, sigma_normal
     return L.DenoiseOpts(iterations, sigma_luminance, sigma_normal, sigma_depth, flags)
 
 
+def temporal_opts(alpha_color: float = 0.0, alpha_moments: float = 0.0, max_history: int = 0, flags: int = 0,
+                  **spatial) -> L.TemporalOpts:
+    """ptb_temporal_opts; 0 selects a default (alpha_color 0.2, alpha_moments 0.2, max_history 32); `spatial` takes
+    denoise_opts' keywords."""
+    return L.TemporalOpts(denoise_opts(**spatial), alpha_color, alpha_moments, max_history, flags)
+
+
 class Context:
     """One ptb_ctx == one GPU."""
 
@@ -354,6 +361,33 @@ class Context:
         o = denoise_opts(**opts)
         _check(self._h, L.lib.ptb_denoise_device(self._h, C.byref(o), C.c_void_p(d_rgb_ptr)))
 
+    # ---- motion vectors and the temporal denoiser
+    def motion_mark(self):
+        """Keeps the committed scene's primitives and camera as the previous frame of the motion vectors."""
+        _check(self._h, L.lib.ptb_motion_mark(self._h))
+
+    def motion_read(self, width: int, height: int) -> np.ndarray:
+        """(H, W, 3) float32: mean Δx, Δy (pixels, rows downwards) and t' over each pixel's valid samples, 0 where none."""
+        out = np.empty(width * height * 3, np.float32)
+        _check(self._h, L.lib.ptb_motion_read(self._h, L.ptr(out), out.size))
+        return out.reshape(height, width, 3)
+
+    def denoise_temporal(self, width: int, height: int, **opts) -> np.ndarray:
+        """The beauty accumulator through SVGF's temporal accumulation and the spatial filter, with the context's history:
+        (H, W, 3) float32. Keyword options: temporal_opts' (alpha_color, alpha_moments, max_history) and denoise's."""
+        o = temporal_opts(**opts)
+        out = np.empty(width * height * 3, np.float32)
+        _check(self._h, L.lib.ptb_denoise_temporal(self._h, C.byref(o), L.ptr(out), out.size))
+        return out.reshape(height, width, 3)
+
+    def denoise_temporal_device(self, d_rgb_ptr: int, **opts):
+        """As denoise_temporal, into a device buffer of W*H*3 floats; enqueued on the context's stream, not waited for."""
+        o = temporal_opts(**opts)
+        _check(self._h, L.lib.ptb_denoise_temporal_device(self._h, C.byref(o), C.c_void_p(d_rgb_ptr)))
+
+    def denoise_temporal_reset(self):
+        _check(self._h, L.lib.ptb_denoise_temporal_reset(self._h))
+
     # ---- sampler test hook (the reference's chi-squared harness pointed at the device samplers)
     @staticmethod
     def _query(kind, alpha, normal, aux, light_index, seed) -> L.SamplerQuery:
@@ -446,6 +480,18 @@ class Scene:
         self.ctx.aov_clear()
         self.ctx.render_aov(opts)
         return self.ctx.denoise(opts.width, opts.height, **denoise)
+
+    def render_denoised_temporal(self, opts: RenderOptions, **denoise) -> np.ndarray:
+        """One frame of an animation: render(opts) and its feature buffers and motion vectors, the temporally denoised image
+        (H, W, 3), then this frame is marked as the next one's previous frame. Give each frame its own sample_offset or
+        seed: the same samples every frame average nothing. `denoise` takes Context.denoise_temporal's keyword options."""
+        self.ctx.accum_clear()
+        self.ctx.render(opts)
+        self.ctx.aov_clear()
+        self.ctx.render_aov(opts)
+        out = self.ctx.denoise_temporal(opts.width, opts.height, **denoise)
+        self.ctx.motion_mark()
+        return out
 
 
 def render_multi(contexts, opts: RenderOptions) -> np.ndarray:

@@ -775,6 +775,8 @@ static int32_t ensure_aov(Ctx* c, uint32_t w, uint32_t h) {
   const size_t bytes = (size_t)w * h * 8 * sizeof(float);
   PTB_CUDA_TRY(c, c->d_aov.alloc(bytes));
   PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_aov.p, 0, bytes, c->stream));
+  PTB_CUDA_TRY(c, c->d_motion.alloc(bytes / 2));
+  PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_motion.p, 0, bytes / 2, c->stream));
   c->aov_w = w;
   c->aov_h = h;
   c->aov_samples = 0;
@@ -798,6 +800,7 @@ int32_t ptb_render_aov(ptb_ctx* ctx, const ptb_render_opts* opts) {
 int32_t ptb_aov_clear(ptb_ctx* ctx) {
   CTX_OR_FAIL(ctx);
   if (c->d_aov.p) PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_aov.p, 0, (size_t)c->aov_w * c->aov_h * 8 * sizeof(float), c->stream));
+  if (c->d_motion.p) PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_motion.p, 0, (size_t)c->aov_w * c->aov_h * 4 * sizeof(float), c->stream));
   c->aov_samples = 0;
   return PTB_OK;
 }
@@ -833,6 +836,53 @@ int32_t ptb_aov_read(ptb_ctx* ctx, uint32_t aov, float* out, size_t n_floats, in
   const int norm = normalise && c->aov_samples > 0;
   k_aov_read<<<(unsigned)((npix + 255) / 256), 256, 0, c->stream>>>(c->d_aov.as<float4>(), c->d_hits.as<float>(), npix, aov,
                                                                     norm, (float)c->aov_samples);
+  c->stats.kernel_launches += 1;
+  PTB_CUDA_TRY(c, cudaGetLastError());
+  PTB_CUDA_TRY(c, cudaMemcpyAsync(out, c->d_hits.p, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  return PTB_OK;
+}
+
+// ---------------------------------------------------------------- motion vectors
+int32_t ptb_motion_mark(ptb_ctx* ctx) {
+  CTX_OR_FAIL(ctx);
+  if (!c->committed) return set_error(c, PTB_ERR_INVALID, "scene not committed");
+  PTB_CUDA_TRY(c, c->d_mark_spheres.reserve(c->n_spheres * sizeof(ptb_sphere)));
+  PTB_CUDA_TRY(c, c->d_mark_tris.reserve(c->n_tris * sizeof(ptb_triangle)));
+  if (c->n_spheres)
+    PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_mark_spheres.p, c->d_raw_spheres.p, c->n_spheres * sizeof(ptb_sphere),
+                                    cudaMemcpyDeviceToDevice, c->stream));
+  if (c->n_tris)
+    PTB_CUDA_TRY(c, cudaMemcpyAsync(c->d_mark_tris.p, c->d_raw_tris.p, c->n_tris * sizeof(ptb_triangle), cudaMemcpyDeviceToDevice,
+                                    c->stream));
+  c->mark_spheres = c->n_spheres;
+  c->mark_tris = c->n_tris;
+  c->mark_cam[0] = c->dev.cam_origin;
+  c->mark_cam[1] = c->dev.cam_lower_left;
+  c->mark_cam[2] = c->dev.cam_horizontal;
+  c->mark_cam[3] = c->dev.cam_vertical;
+  c->have_mark = true;
+  return PTB_OK;
+}
+
+// mean Δx, Δy, t' over the valid samples of each pixel, 0 where there are none
+__global__ void k_motion_read(const float4* __restrict__ sums, float* __restrict__ out, size_t npix) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= npix) return;
+  const float4 s = sums[i];
+  const bool any = s.w > 0.0f;
+  out[3 * i + 0] = any ? s.x / s.w : 0.0f;
+  out[3 * i + 1] = any ? s.y / s.w : 0.0f;
+  out[3 * i + 2] = any ? s.z / s.w : 0.0f;
+}
+
+int32_t ptb_motion_read(ptb_ctx* ctx, float* out, size_t n_floats) {
+  CTX_OR_FAIL(ctx);
+  if (!c->d_aov.p) return set_error(c, PTB_ERR_INVALID, "no AOV rendered yet");
+  const size_t npix = (size_t)c->aov_w * c->aov_h, n = npix * 3;
+  if (!out || n_floats != n) return set_error(c, PTB_ERR_INVALID, "motion_read expects %zu floats", n);
+  PTB_CUDA_TRY(c, c->d_hits.reserve(n * sizeof(float)));
+  k_motion_read<<<(unsigned)((npix + 255) / 256), 256, 0, c->stream>>>(c->d_motion.as<float4>(), c->d_hits.as<float>(), npix);
   c->stats.kernel_launches += 1;
   PTB_CUDA_TRY(c, cudaGetLastError());
   PTB_CUDA_TRY(c, cudaMemcpyAsync(out, c->d_hits.p, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));

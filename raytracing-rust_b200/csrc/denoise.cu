@@ -8,9 +8,14 @@
 //   k_denoise_variance  7x7 feature-weighted moments of ℓ(e) -> [e.rgb | var]
 //   k_denoise_atrous    one launch per level (step 2^i), ping-pong [e.rgb | var]; the last level multiplies the albedo
 //                       back in and stores RGB
+// ptb_denoise_temporal (SVGF §4.1-4.2, CPU restatement oracle/temporal_api.cpp) runs k_denoise_prepare, then
+//   k_temporal_integrate  reprojects the context's history through the motion sums and integrates colour and moments
+//   k_temporal_variance   [e_int | var]: the moments' variance from 4 frames of history on, the 7x7 estimate before
+// and the same levels, level 0 writing the next history (k_temporal_modulate stores RGB when it is also the last).
 // A tap reads 36 bytes: [e.rgb | var] and [n.xyz | z] (16 B each) and the coverage α (4 B). The taps go through L1; a
 // shared-memory tile for the small steps was not built.
 #include <cmath>
+#include <utility>
 
 #include "ptb_internal.h"
 
@@ -81,13 +86,11 @@ __global__ void k_denoise_prepare(const float* __restrict__ beauty, const float4
   grad_out[i] = make_float2(gx, depth_gradient(nz.w, zf, cf, zb, cb));
 }
 
-__global__ void __launch_bounds__(kBlockX * kBlockY)
-k_denoise_variance(const float4* __restrict__ e_in, const float4* __restrict__ nz, const float* __restrict__ alpha,
-                   const float2* __restrict__ grad, int w, int h, DenoiseSigmas sg, float4* __restrict__ out) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-  if (x >= w || y >= h) return;
-  const size_t i = (size_t)y * w + x;
-  const float4 ep = e_in[i], np = nz[i];
+// SVGF's spatial variance estimate of pixel (x, y) over `e_in`: 7x7 feature-weighted moments of ℓ(e)
+__device__ __forceinline__ float spatial_variance(const float4* __restrict__ e_in, const float4* __restrict__ nz,
+                                                  const float* __restrict__ alpha, const float2* __restrict__ grad, int w,
+                                                  int h, DenoiseSigmas sg, int x, int y, size_t i, const float4& ep) {
+  const float4 np = nz[i];
   const float ap = alpha[i], lp = luminance(ep.x, ep.y, ep.z);
   const float2 gp = grad[i];
   const bool zp = zero3(np);
@@ -119,7 +122,17 @@ k_denoise_variance(const float4* __restrict__ e_in, const float4* __restrict__ n
     }
   }
   const float mu1 = m1 / sw, mu2 = m2 / sw;
-  out[i] = make_float4(ep.x, ep.y, ep.z, fmaxf(0.0f, mu2 - mu1 * mu1));
+  return fmaxf(0.0f, mu2 - mu1 * mu1);
+}
+
+__global__ void __launch_bounds__(kBlockX * kBlockY)
+k_denoise_variance(const float4* __restrict__ e_in, const float4* __restrict__ nz, const float* __restrict__ alpha,
+                   const float2* __restrict__ grad, int w, int h, DenoiseSigmas sg, float4* __restrict__ out) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+  if (x >= w || y >= h) return;
+  const size_t i = (size_t)y * w + x;
+  const float4 ep = e_in[i];
+  out[i] = make_float4(ep.x, ep.y, ep.z, spatial_variance(e_in, nz, alpha, grad, w, h, sg, x, y, i, ep));
 }
 
 // one à-trous level; `rgb` != nullptr marks the last one: e * max(albedo, 1e-3) goes there instead of `out`
@@ -189,6 +202,86 @@ k_denoise_atrous(const float4* __restrict__ in, const float4* __restrict__ nz, c
   }
 }
 
+// ---- temporal accumulation (SVGF §4.1-4.2, include/ptb200.h "temporal denoiser")
+struct TemporalParams {
+  float alpha_c, alpha_m, max_len;
+  int have_history;
+};
+constexpr float kTapNormal = 0.9f, kTapDepthGrad = 4.0f, kTapDepthRel = 0.02f, kMinHistoryWeight = 0.01f;
+
+// Reprojects the history through the pixel's mean motion (bilinear taps, each kept only when its guides match) and
+// integrates: e_int = (1 - a_c) e_hist + a_c e, moments alike. e_int -> e_out (w = 0), [m1, m2, len, 0] -> m_out.
+__global__ void __launch_bounds__(kBlockX * kBlockY)
+k_temporal_integrate(const float4* __restrict__ e_in, const float4* __restrict__ motion, const float4* __restrict__ nz,
+                     const float4* __restrict__ h_e, const float4* __restrict__ h_m, const float4* __restrict__ h_nz,
+                     const float* __restrict__ h_alpha, const float2* __restrict__ h_grad, int w, int h, TemporalParams tp,
+                     float4* __restrict__ e_out, float4* __restrict__ m_out) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+  if (x >= w || y >= h) return;
+  const size_t i = (size_t)y * w + x;
+  const float4 e = e_in[i], mot = motion[i], np = nz[i];
+  float er = 0.0f, eg = 0.0f, eb = 0.0f, m1 = 0.0f, m2 = 0.0f, len_h = 0.0f;
+  if (tp.have_history && mot.w > 0.0f) {
+    const float qx = (float)x + mot.x / mot.w, qy = (float)y + mot.y / mot.w, tq = mot.z / mot.w;
+    const float x0 = floorf(qx), y0 = floorf(qy), fx = qx - x0, fy = qy - y0;
+    float sw = 0.0f, sr = 0.0f, sg = 0.0f, sb = 0.0f, s1 = 0.0f, s2 = 0.0f, sl = 0.0f;
+    for (int dy = 0; dy <= 1; ++dy) {
+      for (int dx = 0; dx <= 1; ++dx) {
+        const float wq = (dx ? fx : 1.0f - fx) * (dy ? fy : 1.0f - fy);
+        const float xq = x0 + (float)dx, yq = y0 + (float)dy;
+        if (!(wq > 0.0f) || !(xq >= 0.0f && xq < (float)w && yq >= 0.0f && yq < (float)h)) continue;
+        const size_t j = (size_t)yq * w + (size_t)xq;
+        if (!(h_alpha[j] > 0.0f)) continue;
+        const float4 nq = h_nz[j];
+        if (zero3(nq) || (np.x * nq.x + np.y * nq.y) + np.z * nq.z < kTapNormal) continue;
+        const float2 gq = h_grad[j];
+        if (fabsf(tq - nq.w) > kTapDepthGrad * (fabsf(gq.x) + fabsf(gq.y)) + kTapDepthRel * nq.w) continue;
+        const float4 ce = h_e[j], cm = h_m[j];
+        sw += wq;
+        sr += wq * ce.x;
+        sg += wq * ce.y;
+        sb += wq * ce.z;
+        s1 += wq * cm.x;
+        s2 += wq * cm.y;
+        sl += wq * cm.z;
+      }
+    }
+    if (sw > kMinHistoryWeight) {
+      er = sr / sw; eg = sg / sw; eb = sb / sw;
+      m1 = s1 / sw; m2 = s2 / sw; len_h = sl / sw;
+    }
+  }
+  const float len = fminf(len_h + 1.0f, tp.max_len);
+  const float ac = fmaxf(tp.alpha_c, 1.0f / len), am = fmaxf(tp.alpha_m, 1.0f / len);
+  e_out[i] = make_float4((1.0f - ac) * er + ac * e.x, (1.0f - ac) * eg + ac * e.y, (1.0f - ac) * eb + ac * e.z, 0.0f);
+  const float l = luminance(e.x, e.y, e.z);
+  m_out[i] = make_float4((1.0f - am) * m1 + am * l, (1.0f - am) * m2 + am * (l * l), len, 0.0f);
+}
+
+// [e_int | var]: the integrated moments' variance once 4 frames are in the history, the spatial estimate before
+__global__ void __launch_bounds__(kBlockX * kBlockY)
+k_temporal_variance(const float4* __restrict__ e_in, const float4* __restrict__ m, const float4* __restrict__ nz,
+                    const float* __restrict__ alpha, const float2* __restrict__ grad, int w, int h, DenoiseSigmas sg,
+                    float4* __restrict__ out) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+  if (x >= w || y >= h) return;
+  const size_t i = (size_t)y * w + x;
+  const float4 ep = e_in[i], mi = m[i];
+  const float var = mi.z >= 4.0f ? fmaxf(0.0f, mi.y - mi.x * mi.x) : spatial_variance(e_in, nz, alpha, grad, w, h, sg, x, y, i, ep);
+  out[i] = make_float4(ep.x, ep.y, ep.z, var);
+}
+
+// rgb = e * max(albedo, 1e-3): the last level's output when level 0 (kept as history) is also the last
+__global__ void k_temporal_modulate(const float4* __restrict__ e, const float4* __restrict__ aov, size_t npix, float s_a,
+                                    float* __restrict__ rgb) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= npix) return;
+  const float4 ei = e[i], s0 = aov[2 * i];
+  rgb[3 * i + 0] = ei.x * fmaxf(s0.x / s_a, 1e-3f);
+  rgb[3 * i + 1] = ei.y * fmaxf(s0.y / s_a, 1e-3f);
+  rgb[3 * i + 2] = ei.z * fmaxf(s0.z / s_a, 1e-3f);
+}
+
 int32_t check_denoise(Ctx* c, const ptb_denoise_opts* opts) {
   if (!opts) return set_error(c, PTB_ERR_INVALID, "null denoise opts");
   if (!c->d_accum.p) return set_error(c, PTB_ERR_INVALID, "nothing rendered yet");
@@ -209,7 +302,8 @@ int32_t check_denoise(Ctx* c, const ptb_denoise_opts* opts) {
 }
 
 // opts checked; writes W*H*3 floats to the device buffer `rgb`
-int32_t launch_denoise(Ctx* c, const ptb_denoise_opts& o, float* rgb) {
+// the scratch at the beauty image's size
+int32_t ensure_denoise_scratch(Ctx* c) {
   const uint32_t w = c->accum_w, h = c->accum_h;
   const size_t npix = (size_t)w * h;
   if (c->dn_w != w || c->dn_h != h || !c->d_dn_nz.p) {
@@ -221,9 +315,20 @@ int32_t launch_denoise(Ctx* c, const ptb_denoise_opts& o, float* rgb) {
     c->dn_w = w;
     c->dn_h = h;
   }
+  return PTB_OK;
+}
+
+DenoiseSigmas sigmas_of(const ptb_denoise_opts& o) {
+  return DenoiseSigmas{o.sigma_luminance != 0.0f ? o.sigma_luminance : 4.0f, o.sigma_normal != 0.0f ? o.sigma_normal : 128.0f,
+                       o.sigma_depth != 0.0f ? o.sigma_depth : 1.0f};
+}
+
+int32_t launch_denoise(Ctx* c, const ptb_denoise_opts& o, float* rgb) {
+  const uint32_t w = c->accum_w, h = c->accum_h;
+  const int32_t rc = ensure_denoise_scratch(c);
+  if (rc != PTB_OK) return rc;
   const uint32_t levels = o.iterations ? o.iterations : 5u;
-  const DenoiseSigmas sg{o.sigma_luminance != 0.0f ? o.sigma_luminance : 4.0f, o.sigma_normal != 0.0f ? o.sigma_normal : 128.0f,
-                         o.sigma_depth != 0.0f ? o.sigma_depth : 1.0f};
+  const DenoiseSigmas sg = sigmas_of(o);
   const float s_a = (float)c->aov_samples;
   float4* e[2] = {c->d_dn_e[0].as<float4>(), c->d_dn_e[1].as<float4>()};
   const float4* aov = c->d_aov.as<float4>();
@@ -242,6 +347,80 @@ int32_t launch_denoise(Ctx* c, const ptb_denoise_opts& o, float* rgb) {
   }
   c->stats.kernel_launches += 2 + levels;
   PTB_CUDA_TRY(c, cudaGetLastError());
+  return PTB_OK;
+}
+
+int32_t check_temporal(Ctx* c, const ptb_temporal_opts* opts) {
+  if (!opts) return set_error(c, PTB_ERR_INVALID, "null temporal opts");
+  const int32_t rc = check_denoise(c, &opts->spatial);
+  if (rc != PTB_OK) return rc;
+  const struct { const char* name; float v; } al[2] = {{"alpha_color", opts->alpha_color}, {"alpha_moments", opts->alpha_moments}};
+  for (const auto& a : al)
+    if (!(a.v == 0.0f || (a.v > 0.0f && a.v <= 1.0f)))
+      return set_error(c, PTB_ERR_INVALID, "%s must be in (0, 1] or 0 (got %g)", a.name, (double)a.v);
+  if (opts->max_history > 255) return set_error(c, PTB_ERR_INVALID, "max_history must be <= 255 (got %u)", opts->max_history);
+  if (opts->flags != 0) return set_error(c, PTB_ERR_INVALID, "temporal flags must be 0 (got 0x%x)", opts->flags);
+  return PTB_OK;
+}
+
+void swap_buf(DevBuf& a, DevBuf& b) {
+  std::swap(a.p, b.p);
+  std::swap(a.bytes, b.bytes);
+}
+
+// opts checked; writes W*H*3 floats to the device buffer `rgb` and makes this frame the history
+int32_t launch_temporal(Ctx* c, const ptb_temporal_opts& o, float* rgb) {
+  const uint32_t w = c->accum_w, h = c->accum_h;
+  const size_t npix = (size_t)w * h;
+  int32_t rc = ensure_denoise_scratch(c);
+  if (rc != PTB_OK) return rc;
+  if (c->th_w != w || c->th_h != h || !c->d_th_nz.p) {
+    c->have_history = false;
+    for (DevBuf* b : {&c->d_th_e[0], &c->d_th_e[1], &c->d_th_m[0], &c->d_th_m[1], &c->d_th_nz})
+      PTB_CUDA_TRY(c, b->alloc(npix * sizeof(float4)));
+    PTB_CUDA_TRY(c, c->d_th_alpha.alloc(npix * sizeof(float)));
+    PTB_CUDA_TRY(c, c->d_th_grad.alloc(npix * sizeof(float2)));
+    c->th_w = w;
+    c->th_h = h;
+  }
+  const uint32_t levels = o.spatial.iterations ? o.spatial.iterations : 5u;
+  const DenoiseSigmas sg = sigmas_of(o.spatial);
+  const TemporalParams tp{o.alpha_color != 0.0f ? o.alpha_color : 0.2f, o.alpha_moments != 0.0f ? o.alpha_moments : 0.2f,
+                          (float)(o.max_history ? o.max_history : 32u), c->have_history ? 1 : 0};
+  const float s_a = (float)c->aov_samples;
+  const uint32_t cur = c->th_cur, nxt = cur ^ 1u;
+  float4* e[2] = {c->d_dn_e[0].as<float4>(), c->d_dn_e[1].as<float4>()};
+  float4* hist_out = c->d_th_e[nxt].as<float4>();
+  const float4* aov = c->d_aov.as<float4>();
+  float4* nz = c->d_dn_nz.as<float4>();
+  float* alpha = c->d_dn_alpha.as<float>();
+  float2* grad = c->d_dn_grad.as<float2>();
+  const dim3 block(kBlockX, kBlockY), grid((w + kBlockX - 1) / kBlockX, (h + kBlockY - 1) / kBlockY);
+  k_denoise_prepare<<<grid, block, 0, c->stream>>>(c->d_accum.as<float>(), aov, (int)w, (int)h, 1.0f / (float)c->accum_samples,
+                                                   s_a, e[0], nz, alpha, grad);
+  k_temporal_integrate<<<grid, block, 0, c->stream>>>(e[0], c->d_motion.as<float4>(), nz, c->d_th_e[cur].as<float4>(),
+                                                      c->d_th_m[cur].as<float4>(), c->d_th_nz.as<float4>(),
+                                                      c->d_th_alpha.as<float>(), c->d_th_grad.as<float2>(), (int)w, (int)h, tp,
+                                                      e[1], c->d_th_m[nxt].as<float4>());
+  k_temporal_variance<<<grid, block, 0, c->stream>>>(e[1], c->d_th_m[nxt].as<float4>(), nz, alpha, grad, (int)w, (int)h, sg, e[0]);
+  // level 0 writes the next history; later levels ping-pong through the scratch from there
+  k_denoise_atrous<<<grid, block, 0, c->stream>>>(e[0], nz, alpha, grad, (int)w, (int)h, 1, sg, hist_out, nullptr, aov, s_a);
+  for (uint32_t l = 1; l < levels; ++l) {
+    const bool last = l + 1 == levels;
+    const float4* src = l == 1 ? hist_out : e[(l + 1) & 1u];
+    k_denoise_atrous<<<grid, block, 0, c->stream>>>(src, nz, alpha, grad, (int)w, (int)h, 1 << l, sg, e[l & 1u],
+                                                    last ? rgb : nullptr, aov, s_a);
+  }
+  if (levels == 1)
+    k_temporal_modulate<<<(unsigned)((npix + 255) / 256), 256, 0, c->stream>>>(hist_out, aov, npix, s_a, rgb);
+  c->stats.kernel_launches += 3 + levels + (levels == 1 ? 1 : 0);
+  PTB_CUDA_TRY(c, cudaGetLastError());
+  // this frame's guides become the history's; the old history's buffers are the next call's scratch
+  swap_buf(c->d_dn_nz, c->d_th_nz);
+  swap_buf(c->d_dn_alpha, c->d_th_alpha);
+  swap_buf(c->d_dn_grad, c->d_th_grad);
+  c->th_cur = nxt;
+  c->have_history = true;
   return PTB_OK;
 }
 
@@ -276,6 +455,38 @@ int32_t ptb_denoise_device(ptb_ctx* ctx, const ptb_denoise_opts* opts, void* d_r
   if (rc != PTB_OK) return rc;
   if (!d_rgb) return set_error(c, PTB_ERR_INVALID, "null device output");
   return launch_denoise(c, *opts, static_cast<float*>(d_rgb));
+}
+
+int32_t ptb_denoise_temporal(ptb_ctx* ctx, const ptb_temporal_opts* opts, float* rgb, size_t n_floats) {
+  if (!ctx) return PTB_ERR_INVALID;
+  Ctx* c = &ctx->c;
+  if (cudaSetDevice(c->device) != cudaSuccess) return set_error(c, PTB_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
+  int32_t rc = check_temporal(c, opts);
+  if (rc != PTB_OK) return rc;
+  const size_t n = (size_t)c->accum_w * c->accum_h * 3;
+  if (!rgb || n_floats != n) return set_error(c, PTB_ERR_INVALID, "denoise expects %zu floats", n);
+  PTB_CUDA_TRY(c, c->d_hits.reserve(n * sizeof(float)));
+  rc = launch_temporal(c, *opts, c->d_hits.as<float>());
+  if (rc != PTB_OK) return rc;
+  PTB_CUDA_TRY(c, cudaMemcpyAsync(rgb, c->d_hits.p, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  PTB_CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+  return PTB_OK;
+}
+
+int32_t ptb_denoise_temporal_device(ptb_ctx* ctx, const ptb_temporal_opts* opts, void* d_rgb) {
+  if (!ctx) return PTB_ERR_INVALID;
+  Ctx* c = &ctx->c;
+  if (cudaSetDevice(c->device) != cudaSuccess) return set_error(c, PTB_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
+  const int32_t rc = check_temporal(c, opts);
+  if (rc != PTB_OK) return rc;
+  if (!d_rgb) return set_error(c, PTB_ERR_INVALID, "null device output");
+  return launch_temporal(c, *opts, static_cast<float*>(d_rgb));
+}
+
+int32_t ptb_denoise_temporal_reset(ptb_ctx* ctx) {
+  if (!ctx) return PTB_ERR_INVALID;
+  ctx->c.have_history = false;
+  return PTB_OK;
 }
 
 }  // extern "C"

@@ -138,10 +138,23 @@ struct Ctx {
   DevBuf d_aov, d_aov_heads;
   uint32_t aov_w = 0, aov_h = 0;
   uint64_t aov_samples = 0;
+  // motion sums beside the AOV sums (aov_w x aov_h): one float4 per pixel [Σ Δx, Σ Δy, Σ t', valid samples]
+  DevBuf d_motion;
+  // the previous frame (ptb_motion_mark): the primitives in original order and the camera of the committed scene
+  DevBuf d_mark_spheres, d_mark_tris;
+  size_t mark_spheres = 0, mark_tris = 0;
+  bool have_mark = false;
+  v3 mark_cam[4] = {};  // origin, lower_left, horizontal, vertical
   // denoiser scratch (denoise.cu), dn_w x dn_h pixels: ping-pong [e.rgb | var] and the guide records [n.xyz | z],
   // coverage α and the depth gradient [∂x z, ∂y z]
   DevBuf d_dn_e[2], d_dn_nz, d_dn_alpha, d_dn_grad;
   uint32_t dn_w = 0, dn_h = 0;
+  // temporal history (ptb_denoise_temporal), th_w x th_h pixels when have_history: level 0's irradiance and the
+  // integrated moments [m1, m2, len] (double-buffered, [th_cur] is the history), the guides of the frame they belong to
+  // (swapped with d_dn_nz / d_dn_alpha / d_dn_grad by pointer)
+  DevBuf d_th_e[2], d_th_m[2], d_th_nz, d_th_alpha, d_th_grad;
+  uint32_t th_w = 0, th_h = 0, th_cur = 0;
+  bool have_history = false;
   // camera candidate lists of the window wavefront (ptb_camcand.cuh), grow-only: entries [npix * k] and counts [npix]
   DevBuf d_camcand, d_camcand_count;
   DevBuf d_pool_mem, d_prev, d_queues, d_shadow, d_counters, d_windows;
@@ -208,7 +221,7 @@ size_t radix_sort_hist_words(uint32_t n);
 // wavefront.cu
 int32_t render_wavefront(Ctx* c, const ptb_render_opts& o, ptb_progress_fn progress, void* user);
 int32_t launch_closest_hit(Ctx* c, const void* d_rays, size_t n, void* d_hits);
-// ptb_render_aov's launches, opts validated; adds into d_aov
+// ptb_render_aov's launches, opts validated; adds into d_aov (and d_motion when the mark's counts match the scene's)
 int32_t launch_aov(Ctx* c, const ptb_render_opts& o);
 // check_hit_index (d_index != nullptr: ptb_ray in, ptb_hit out) or occlusion (ptb_occlusion_ray in, one byte out)
 int32_t launch_visibility(Ctx* c, const void* d_rays, const void* d_index, size_t n, void* d_out);

@@ -1512,6 +1512,86 @@ k_aov(DevScene sc, RenderParams rp, float4* __restrict__ sums, uint32_t* head) {
   persistent_trace<TR, false, false>(sc, rp.npix, head, fetch, retire, a, b, r);
 }
 
+// Motion vectors (ptb_render_aov after ptb_motion_mark, include/ptb200.h "motion vectors"): k_aov's sums plus, per hit
+// sample, the hit point's position in the marked frame P' and both projections. One float4 per pixel [Σ Δx, Σ Δy, Σ t',
+// valid count], updated like the AOV sums (each pixel once per launch, in sample order).
+struct MotionParams {
+  const ptb_sphere* cur_s;  // the committed primitives and the mark's, original order
+  const ptb_sphere* prev_s;
+  const ptb_triangle* cur_t;
+  const ptb_triangle* prev_t;
+  uint32_t n_spheres;
+  float wm1, hm1;  // W - 1, H - 1
+  v3 o, ll, hz, vt;  // the marked camera
+  float4* out;
+};
+// proj(cam, X): X - o = λ (ll - o + u h + v vv), the inverse of camera_direction, by Cramer's rule in this order:
+// d = X - o, a = ll - o, n = cross(h, vv), s = dot(d, n); λ = s / dot(a, n), u = dot(d, cross(vv, a)) / s,
+// v = dot(d, cross(a, h)) / s
+PTB_DEV void cam_project(v3 o, v3 ll, v3 hz, v3 vt, v3 x, float& u, float& v, float& lambda) {
+  const v3 d = x - o, a = ll - o, n = cross(hz, vt);
+  const float s = dot(d, n);
+  lambda = s / dot(a, n);
+  u = dot(d, cross(vt, a)) / s;
+  v = dot(d, cross(a, hz)) / s;
+}
+PTB_DEV bool same_bits(const float* a, const float* b, int n) {
+  bool same = true;
+  for (int k = 0; k < n; ++k) same = same && __float_as_uint(__ldg(a + k)) == __float_as_uint(__ldg(b + k));
+  return same;
+}
+struct AovMotionRetire {
+  AovRetire aov;
+  const MotionParams& mp;
+  PTB_DEV void operator()(bool fin, const TraceResult& tr, const Ray& ray) {
+    aov(fin, tr, ray);
+    if (!fin || tr.ref == kNone) return;
+    const DevScene& sc = aov.sc;
+    HitRec h;
+    prim_hit(sc, ray, tr.ref, h);  // the record the AOV sums were formed from
+    const uint32_t slot = tr.ref & kSlotMask, p = __ldg(sc.slot_prim + slot);
+    v3 q = h.point;  // P' = P while the marked record is bit-identical to the committed one
+    if (tr.ref & kSphereBit) {
+      const float* cur = &mp.cur_s[p].center.x;
+      const float* prv = &mp.prev_s[p].center.x;
+      if (!same_bits(cur, prv, 4))
+        q = mk(__ldg(prv), __ldg(prv + 1), __ldg(prv + 2)) +
+            (h.point - mk(__ldg(cur), __ldg(cur + 1), __ldg(cur + 2))) * (__ldg(prv + 3) / __ldg(cur + 3));
+    } else {
+      const float* cur = &mp.cur_t[p - mp.n_spheres].p[0].x;
+      const float* prv = &mp.prev_t[p - mp.n_spheres].p[0].x;
+      if (!same_bits(cur, prv, 9)) {
+        // the hit's barycentrics, all three: triangle_core on the same ray and vertices gives prim_hit's b0, b1, b2
+        const float4* g = sc.geom + 3u * (size_t)slot;
+        TriCore tc;
+        triangle_core(ray, from4(__ldg(g)), from4(__ldg(g + 1)), from4(__ldg(g + 2)), tc);
+        const v3 p0 = mk(__ldg(prv), __ldg(prv + 1), __ldg(prv + 2)), p1 = mk(__ldg(prv + 3), __ldg(prv + 4), __ldg(prv + 5)),
+                 p2 = mk(__ldg(prv + 6), __ldg(prv + 7), __ldg(prv + 8));
+        q = tc.b0 * p0 + tc.b1 * p1 + tc.b2 * p2;
+      }
+    }
+    float u, v, l, u1, v1, l1;
+    cam_project(sc.cam_origin, sc.cam_lower_left, sc.cam_horizontal, sc.cam_vertical, h.point, u, v, l);
+    cam_project(mp.o, mp.ll, mp.hz, mp.vt, q, u1, v1, l1);
+    if (!(l1 > 0.0f)) return;  // behind the marked camera (or degenerate): not a valid sample
+    float4* m = mp.out + aov.f.pixel;
+    float4 s = *m;
+    s.x += (u1 - u) * mp.wm1;
+    s.y += -(v1 - v) * mp.hm1;
+    s.z += mag(q - mp.o);
+    s.w += 1.0f;
+    *m = s;
+  }
+};
+template <class TR>
+__global__ void __launch_bounds__(256, TR::kApiMinBlocks)
+k_aov_motion(DevScene sc, RenderParams rp, float4* __restrict__ sums, uint32_t* head, MotionParams mp) {
+  uint32_t a = 0, b = 0, r = 0;
+  AovFetch fetch{sc, rp, 0u};
+  AovMotionRetire retire{AovRetire{sc, sums, fetch}, mp};
+  persistent_trace<TR, false, false>(sc, rp.npix, head, fetch, retire, a, b, r);
+}
+
 // ------------------------------------------------------------------------------------------ visibility API kernel
 // Batch any-hit through the walk k_shadow runs (persistent_trace<TR, ANYHIT = true>), fed from caller records.
 //   CHI  : check_hit_index (acceleration/mod.rs:226-263): ptb_ray + target id in, ptb_hit out. The target's own hit is
@@ -1822,13 +1902,27 @@ int32_t launch_aov(Ctx* c, const ptb_render_opts& o) {
   rp.k0 = (uint32_t)o.seed; rp.k1 = (uint32_t)(o.seed >> 32);
   PTB_CUDA_TRY(c, c->d_aov_heads.reserve((size_t)spp * 4));
   PTB_CUDA_TRY(c, cudaMemsetAsync(c->d_aov_heads.p, 0, (size_t)spp * 4, c->stream));
-  const void* fn = aov_kernel(c);
+  // motion vectors while a mark of the same primitive counts exists (ids are stable only then)
+  const bool motion = c->have_mark && c->mark_spheres == c->n_spheres && c->mark_tris == c->n_tris;
+  MotionParams mp{};
+  if (motion) {
+    mp.cur_s = c->d_raw_spheres.as<ptb_sphere>();
+    mp.prev_s = c->d_mark_spheres.as<ptb_sphere>();
+    mp.cur_t = c->d_raw_tris.as<ptb_triangle>();
+    mp.prev_t = c->d_mark_tris.as<ptb_triangle>();
+    mp.n_spheres = (uint32_t)c->n_spheres;
+    mp.wm1 = (float)(o.width - 1u);
+    mp.hm1 = (float)(o.height - 1u);
+    mp.o = c->mark_cam[0]; mp.ll = c->mark_cam[1]; mp.hz = c->mark_cam[2]; mp.vt = c->mark_cam[3];
+    mp.out = c->d_motion.as<float4>();
+  }
+  const void* fn = motion ? (c->wide ? (const void*)k_aov_motion<CwTrav> : (const void*)k_aov_motion<BinTrav>) : aov_kernel(c);
   const int grid = persistent_grid(c, fn, 256);
   float4* sums = c->d_aov.as<float4>();
   for (uint32_t s = 0; s < spp; ++s) {
     rp.sample_offset = o.sample_offset + s;
     uint32_t* head = c->d_aov_heads.as<uint32_t>() + s;
-    void* args[] = {(void*)&c->dev, (void*)&rp, (void*)&sums, (void*)&head};
+    void* args[] = {(void*)&c->dev, (void*)&rp, (void*)&sums, (void*)&head, (void*)&mp};
     PTB_CUDA_TRY(c, cudaLaunchKernel(fn, dim3((unsigned)grid), dim3(256), args, 0, c->stream));
     c->stats.kernel_launches += 1;
     c->stats.trace_launches += 1;
